@@ -1,8 +1,11 @@
 #!/usr/bin/env python
 """bench.py — AVFormer hot-path throughput on B200 (clips/s), with roofline and CPU baseline.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--mode fwd|train] [--check]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--mode fwd|train] [--check] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
+
+`--dump-outputs DIR` writes what the last timed step computed on rank 0 as DIR/<name>.npy (fp32; sample indices in fp64), so
+that two builds can be compared output for output: the inputs and weights are seeded, identical from run to run.
 
 `--mode train` makes the hot-path TRAINING step (BASELINE config 4 restricted to the transformer stack: forward with tape,
 AULoss, backward, gradient all-reduce overlapped with the backward at N > 1, fused Adam) the measured thing, with the same JSON
@@ -34,6 +37,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True           # a benchmark run leaves the tree as it found it (no __pycache__ of the modules it imports)
 
 CLIPS_PER_GPU = 512
 N_FRAMES = 16
@@ -48,6 +52,33 @@ FLOP_FUSION_PER_CLIP = 28_760_064
 
 def hot_path_flops_per_clip(T):
     return T * FLOP_SFORMER_PER_FRAME + FLOP_TFORMER_PER_CLIP[T] + 2 * FLOP_AU_FORMER_PER_CLIP + FLOP_FUSION_PER_CLIP
+
+
+# --dump-outputs: the full SFormer output (8192 maps, 411 MB in fp32) and the flat parameter / gradient buckets of the training step
+# (41.7 MB each) are larger than the dump may be, so a fixed, seeded sample of them is written
+DUMP_MAX_BYTES = 64 << 20
+DUMP_SFORMER_FRAMES = 512                # 25.7 MB in fp32
+DUMP_BUCKET_ELEMENTS = 1 << 20           # 4 MB per bucket in fp32
+
+
+def dump_sample(n, k):
+    """k indices of range(n), sorted, the same in every run."""
+    import torch
+    return torch.randperm(n, generator=torch.Generator().manual_seed(SEED))[:k].sort().values
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each tensor as out_dir/<name>.npy: fp64 stays fp64, everything else becomes fp32."""
+    import numpy as np
+    import torch
+    host = {k: v.detach().cpu() for k, v in arrays.items()}
+    host = {k: (v.double() if v.dtype == torch.float64 else v.float()).numpy() for k, v in host.items()}
+    total = sum(a.nbytes for a in host.values())
+    if total > DUMP_MAX_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_MAX_BYTES} byte budget")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in host.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def measured_peaks():
@@ -405,6 +436,14 @@ def run_ours(args):
             chk = torch.stack([tbl.double().sum(), -tbl.double().sum(), torch.tensor(0.0 if mine_ok else 1.0, dtype=torch.float64, device=dev)])
             dist.all_reduce(chk, op=dist.ReduceOp.MAX)
             gather_ok = bool(chk[0].item() == -chk[1].item() and chk[2].item() == 0.0)
+        if args.dump_outputs and rank == 0:
+            s_out, out21, dec = graphed.out
+            frames = dump_sample(s_out.shape[0], DUMP_SFORMER_FRAMES)
+            dumped = {"out21": out21, "decisions": dec, "sformer_out_sample": s_out[frames.to(dev)],
+                      "sformer_out_sample_frames": frames.double()}
+            if gather_ok is not None:
+                dumped["gathered_out21"] = tbl
+            dump_outputs(args.dump_outputs, dumped)
         parity = timed_outputs_vs_oracle(model, graphed.out, host, T) if rank == 0 else None
 
         # ---- end to end from pinned host buffers ---------------------------------------------
@@ -600,6 +639,12 @@ def run_train(model, A, dev, rank, world, args):
         e1.record()
         barrier()
     ms_total = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:
+        # the last timed step: its loss, the gradients it computed and the parameters its Adam update wrote (flat buckets, sampled)
+        bucket = opt._buckets[0]
+        idx = dump_sample(bucket["p"].numel(), DUMP_BUCKET_ELEMENTS)
+        dump_outputs(args.dump_outputs, {"loss": graphed.loss.reshape(1), "params_sample": bucket["p"][idx.to(dev)],
+                                         "grads_sample": bucket["g"][idx.to(dev)], "bucket_sample_index": idx.double()})
 
     # end to end: inputs and labels from pinned host memory every step, the loss read back
     loss_host = torch.zeros(1, dtype=torch.float32).pin_memory()
@@ -775,7 +820,13 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--mode", default="fwd", choices=["fwd", "train"], help="what a step is: the evaluation hot path (default) or its training step")
     ap.add_argument("--check", action="store_true", help="data-parallel parity checks instead of timing (run under torchrun with N > 1)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write what the last timed step computed (rank 0) as DIR/<name>.npy, at most 64 MB in all")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.check):
+        ap.error("--dump-outputs goes with the timed GPU path (--impl ours, without --check)")
     if args.impl == "reference":
         run_reference_arm(args)
     else:
