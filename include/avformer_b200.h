@@ -80,10 +80,14 @@ uint64_t    avf_launch_count(void);
 /* SM count, compute capability major*10+minor, and whether the tcgen05 path is usable. */
 int         avf_device_info(int32_t* sm_count, int32_t* cc, int32_t* has_tcgen05);
 
-/* The encoder stacks with dim 256 / 8 heads x 32 (SFormer, fusion head) run as ONE persistent tcgen05 kernel per
- * stack in mode AVF_BF16 (residual stream in TMEM, see csrc/avf_layer_fused.cu).  avf_set_fused_enabled(0) forces the
- * kernel-per-operation path instead (used by the A/B parity tests); returns the previous setting. */
+/* The encoder stacks with dim 256 or 128 / 8 heads x 32 (SFormer, fusion head, AU_formers, VA_former) run as ONE persistent
+ * tcgen05 kernel per stack in mode AVF_BF16 (residual stream in TMEM, see csrc/avf_layer_fused.cu).  avf_set_fused_enabled(0) forces
+ * the kernel-per-operation path instead (used by the A/B parity tests); returns the previous setting. */
 int         avf_set_fused_enabled(int enabled);
+/* 0: dim-128 stacks run kernel per operation, and avf_token_stack_fwd runs its separate positional-add and AU-logit kernels
+ * (the launch sequence before they were folded into the fused kernel; developer A/B, also AVF_FUSED_SMALL=0 in the Python
+ * package).  Returns the previous setting. */
+int         avf_set_fused_small_enabled(int enabled);
 int         avf_encoder_fused_supported(const avf_stack_shape* s, int mode);
 /* Upper bound on the grid of the persistent kernels (fused encoder, tcgen05 GEMM) launched AFTER the call; 0 = all SMs.
  * Returns the previous value.  Lets a caller run two kernel chains side by side on disjoint SM sets (each persistent CTA
@@ -119,6 +123,15 @@ size_t avf_encoder_workspace_bytes(const avf_stack_shape* s, int mode);
 int avf_encoder_stack_fwd(int mode, const avf_stack_shape* s, const avf_layer_weights* layers,
                           float* x, int32_t ld_x, float* out, int32_t ld_out,
                           void* workspace, size_t workspace_bytes, void* stream);
+/* The encoder stack of a token head (AU_former, VA_former, fusion head): x [n_seq*n_tok, ld_x] fp32 (+ pos[n_tok, dim] when
+ * pos != NULL) -> `depth` layers -> out (or x in place when out == NULL), like avf_encoder_stack_fwd.  With w_last [12, dim]
+ * (n_tok = 12) the AU logits of the result follow as in avf_au_logits_fwd: out21 [n_seq, 21] (required) and decisions [n_seq, 12]
+ * (may be NULL); the token rows are then only stored when out != NULL.  x is scratch whenever out != NULL or w_last != NULL.
+ * Same workspace as avf_encoder_stack_fwd.  In mode AVF_BF16 a stack the fused kernel supports (dim 256 or 128) is ONE launch,
+ * positional add and logits included; otherwise the sequence avf_add_row_periodic -> avf_encoder_stack_fwd -> avf_au_logits_fwd. */
+int avf_token_stack_fwd(int mode, const avf_stack_shape* s, const avf_layer_weights* layers, float* x, int32_t ld_x, const float* pos,
+                        float* out, int32_t ld_out, const float* w_last, float* out21, int32_t* decisions,
+                        void* workspace, size_t workspace_bytes, void* stream);
 
 /* Building blocks (exposed for tests and for callers that fuse differently). */
 /* y[r,:] = LayerNorm(x[r,:]) * gamma + beta, eps 1e-5; y is bf16 (mode BF16) or fp32. */
@@ -164,14 +177,15 @@ int avf_tformer_cls_extract(const float* x, float* cls, int32_t n_clips, int32_t
 /* ---- a8: AU_former front end, models/heads.py:293-323 --------------------------------------- */
 /* emb [n_clips, 512] fp32 (row stride ld_emb, so the cls rows of a TFormer output can be read in
  * place) -> BatchNorm1d with running statistics (eval) -> 12 Linear(512,128)+b stacked as
- * w_cat [12*128, 512], b_cat [12*128] -> + pos[12,128] -> x [n_clips*12, 128] fp32. */
+ * w_cat [12*128, 512], b_cat [12*128] -> + pos[12,128] -> x [n_clips*12, 128] fp32.  pos == NULL: no positional add
+ * (avf_token_stack_fwd adds it inside the stack launch). */
 int avf_au_former_front_fwd(int mode, const float* emb, int32_t ld_emb,
                             const float* bn_gamma, const float* bn_beta, const float* bn_mean, const float* bn_var,
                             const void* w_cat, const float* b_cat, const float* pos, float* x,
                             int32_t n_clips, int32_t in_dim, int32_t emb_dim,
                             void* workspace, size_t workspace_bytes, void* stream);
 /* The same front for any number of tokens per clip: BatchNorm1d (running statistics) -> n_tok stacked Linear(in_dim, emb_dim) ->
- * view [n_clips*n_tok, emb_dim] -> + pos[n_tok, emb_dim].  n_tok = 12 is the AU_former above; n_tok = 2 is VA_former
+ * view [n_clips*n_tok, emb_dim] -> + pos[n_tok, emb_dim] (if pos != NULL).  n_tok = 12 is the AU_former above; n_tok = 2 is VA_former
  * (models/heads.py:341-372: VA_BN1, VA_linear_p1..2). */
 int avf_token_front_fwd(int mode, const float* emb, int32_t ld_emb,
                         const float* bn_gamma, const float* bn_beta, const float* bn_mean, const float* bn_var,

@@ -55,11 +55,14 @@ SIGNATURES = {
     "avf_launch_count": (ctypes.c_uint64, []),
     "avf_device_info": (ctypes.c_int, [ctypes.POINTER(_i32)] * 3),
     "avf_set_fused_enabled": (ctypes.c_int, [ctypes.c_int]),
+    "avf_set_fused_small_enabled": (ctypes.c_int, [ctypes.c_int]),
     "avf_encoder_fused_supported": (ctypes.c_int, [ctypes.POINTER(StackShape), ctypes.c_int]),
     "avf_debug_fused_prof": (ctypes.c_int, [ctypes.POINTER(ctypes.c_uint64), ctypes.c_int]),
     "avf_encoder_workspace_bytes": (_sz, [ctypes.POINTER(StackShape), ctypes.c_int]),
     "avf_encoder_stack_fwd": (ctypes.c_int, [ctypes.c_int, ctypes.POINTER(StackShape), ctypes.POINTER(LayerWeights), _c_p, _i32,
                                              _c_p, _i32, _c_p, _sz, _c_p]),
+    "avf_token_stack_fwd": (ctypes.c_int, [ctypes.c_int, ctypes.POINTER(StackShape), ctypes.POINTER(LayerWeights), _c_p, _i32, _c_p,
+                                           _c_p, _i32, _c_p, _c_p, _c_p, _c_p, _sz, _c_p]),
     "avf_layernorm_fwd": (ctypes.c_int, [ctypes.c_int, _c_p, _i32, _c_p, _c_p, _c_p, _i32, _i32, _c_p]),
     "avf_linear_fwd": (ctypes.c_int, [ctypes.c_int, _c_p, _i32, _c_p, _c_p, _c_p, _i32, _c_p, _i32, ctypes.c_int, _i32, _i32, _i32,
                                       ctypes.c_int, _c_p]),
@@ -180,6 +183,8 @@ def lib() -> ctypes.CDLL:
                 fn.restype, fn.argtypes = res, args
             if os.environ.get("AVF_PDL", "") in ("0", "off"):
                 handle.avf_set_pdl_enabled(0)
+            if os.environ.get("AVF_FUSED_SMALL", "") in ("0", "off"):
+                handle.avf_set_fused_small_enabled(0)
             if handle.avf_abi_version() != 1:
                 raise RuntimeError("avformer_b200: ABI version mismatch")
             _lib = handle

@@ -17,6 +17,7 @@ bool pdl_enabled() { return g_pdl.load() != 0; }
 static std::atomic<int> g_sm_cap{0};     // avf_set_sm_cap
 int sm_cap() { return g_sm_cap.load(); }
 static std::atomic<int> g_fused{1};      // avf_set_fused_enabled: 0 forces the kernel-per-op path (A/B tests)
+static std::atomic<int> g_fused_small{1};  // avf_set_fused_small_enabled: 0 keeps dim-128 stacks, positional adds and AU logits out of the fused kernel
 
 void count_launch() { g_launches.fetch_add(1, std::memory_order_relaxed); }
 
@@ -107,14 +108,20 @@ int linear(int mode, const void* a, int lda, const void* w, const float* bias, c
   return linear_f32(static_cast<const float*>(a), lda, static_cast<const float*>(w), bias, res, ld_res, c, ldc, c_mode, m, n, k, flags, st);
 }
 
+// Does a stack of fp32 token rows run as one fused kernel?
+static bool fused_rows(int mode, const avf_stack_shape* s, int ld_x, const float* out, int ld_out) {
+  return mode == AVF_BF16 && g_fused.load() && tcgen05_ok() && encoder_fused_supported(s) && (s->dim == 256 || g_fused_small.load()) &&
+         ld_x % 4 == 0 && (out == nullptr || ld_out % 4 == 0);
+}
+
 static int encoder_stack(int mode, const avf_stack_shape* s, const avf_layer_weights* L, float* x, int ld_x, float* out, int ld_out,
                          void* ws, size_t ws_bytes, cudaStream_t st) {
   int e = check_shape(s);
   if (e) return e;
   AVF_REQUIRE(mode == AVF_BF16 || mode == AVF_FP32, AVF_EINVAL, "mode=%d", mode);
   AVF_REQUIRE(L != nullptr && x != nullptr && ws != nullptr, AVF_EINVAL, "null pointer argument");
-  if (mode == AVF_BF16 && g_fused.load() && tcgen05_ok() && encoder_fused_supported(s) && ld_x % 4 == 0 && (out == nullptr || ld_out % 4 == 0))
-    return encoder_fused(1, s, L, x, ld_x, out ? out : x, out ? ld_out : ld_x, nullptr, nullptr, st);     // whole stack, one persistent kernel
+  if (fused_rows(mode, s, ld_x, out, ld_out))     // whole stack, one persistent kernel
+    return encoder_fused(1, s, L, x, ld_x, out ? out : x, out ? ld_out : ld_x, nullptr, nullptr, nullptr, nullptr, nullptr, st);
   const EncoderWs w = carve_encoder_ws(s, mode, ws);
   AVF_REQUIRE(ws_bytes >= w.total, AVF_EWORKSPACE, "workspace too small: %zu < %zu bytes", ws_bytes, w.total);
   const int R = s->n_seq * s->n_tok, D = s->dim, I = s->heads * s->dim_head, M = s->mlp_dim;
@@ -153,12 +160,14 @@ int avf_set_fused_enabled(int enabled) {
   return old;
 }
 
+int avf_set_fused_small_enabled(int enabled) { return g_fused_small.exchange(enabled ? 1 : 0); }
+
 int avf_set_pdl_enabled(int enabled) { return g_pdl.exchange(enabled ? 1 : 0); }
 
 int avf_set_sm_cap(int cap) { return g_sm_cap.exchange(cap > 0 ? cap : 0); }
 
 int avf_encoder_fused_supported(const avf_stack_shape* s, int mode) {
-  return (s != nullptr && mode == AVF_BF16 && s->n_seq > 0 && encoder_fused_supported(s)) ? 1 : 0;
+  return (s != nullptr && mode == AVF_BF16 && s->n_seq > 0 && encoder_fused_supported(s) && (s->dim == 256 || g_fused_small.load())) ? 1 : 0;
 }
 
 /* Debug: per-phase cycle counters of the fused encoder kernel (library built with -DAVF_FUSED_PROF); else AVF_EUNSUPPORTED. */
@@ -198,6 +207,22 @@ int avf_encoder_stack_fwd(int mode, const avf_stack_shape* s, const avf_layer_we
   int e = require_device();
   if (e) return e;
   return encoder_stack(mode, s, layers, x, ld_x, out, ld_out, workspace, workspace_bytes, static_cast<cudaStream_t>(stream));
+}
+
+int avf_token_stack_fwd(int mode, const avf_stack_shape* s, const avf_layer_weights* layers, float* x, int32_t ld_x, const float* pos, float* out,
+                        int32_t ld_out, const float* w_last, float* out21, int32_t* decisions, void* workspace, size_t workspace_bytes, void* stream) {
+  int e = require_device();
+  if (e) return e;
+  if ((e = check_shape(s))) return e;
+  AVF_REQUIRE(layers && x && workspace, AVF_EINVAL, "token_stack: null pointer");
+  AVF_REQUIRE(w_last == nullptr || (s->n_tok == 12 && out21 != nullptr), AVF_EINVAL, "token_stack: AU logits need 12 tokens per clip and out21 (n_tok=%d)",
+              s->n_tok);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (g_fused_small.load() && fused_rows(mode, s, ld_x, out, ld_out))      // positional add, stack and AU logits in one launch
+    return encoder_fused(1, s, layers, x, ld_x, (out || w_last) ? out : x, out ? ld_out : ld_x, pos, nullptr, w_last, out21, decisions, st);
+  if (pos != nullptr && (e = add_row_periodic(x, ld_x, pos, s->n_seq * s->n_tok, s->dim, s->n_tok, st))) return e;
+  if ((e = encoder_stack(mode, s, layers, x, ld_x, out, ld_out, workspace, workspace_bytes, st))) return e;
+  return w_last == nullptr ? 0 : au_logits(out ? out : x, out ? ld_out : ld_x, w_last, out21, decisions, s->n_seq, s->dim, st);
 }
 
 int avf_layernorm_fwd(int out_mode, const float* x, int32_t ld_x, const float* gamma, const float* beta, void* y, int32_t rows,
@@ -253,8 +278,8 @@ int avf_sformer_fwd(int mode, int io_mode, const avf_stack_shape* s, const avf_l
   const size_t need = avf_sformer_workspace_bytes(s, mode);
   AVF_REQUIRE(workspace_bytes >= need, AVF_EWORKSPACE, "workspace too small: %zu < %zu bytes", workspace_bytes, need);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (mode == AVF_BF16 && io_mode == AVF_BF16 && g_fused.load() && tcgen05_ok() && encoder_fused_supported(s))
-    return encoder_fused(0, s, layers, fmap_in, 0, fmap_out, 0, pos, workspace, st);   // frames in, frames out: nothing else touches HBM
+  if (mode == AVF_BF16 && io_mode == AVF_BF16 && g_fused.load() && tcgen05_ok() && encoder_fused_supported(s) && s->dim == 256)
+    return encoder_fused(0, s, layers, fmap_in, 0, fmap_out, 0, pos, workspace, nullptr, nullptr, nullptr, st);   // frames in, frames out: nothing else touches HBM
   float* x = static_cast<float*>(workspace);
   const size_t xbytes = align_up(size_t(s->n_seq) * s->n_tok * s->dim * 4);
   if ((e = sformer_pack(io_mode, fmap_in, pos, x, s->n_seq, s->dim, s->n_tok, st))) return e;
@@ -333,7 +358,7 @@ int avf_token_front_fwd(int mode, const float* emb, int32_t ld_emb, const float*
                         int32_t in_dim, int32_t emb_dim, int32_t n_tok, void* workspace, size_t workspace_bytes, void* stream) {
   int e = require_device();
   if (e) return e;
-  AVF_REQUIRE(emb && bn_gamma && bn_beta && bn_mean && bn_var && w_cat && b_cat && pos && x && workspace, AVF_EINVAL, "token_front: null pointer");
+  AVF_REQUIRE(emb && bn_gamma && bn_beta && bn_mean && bn_var && w_cat && b_cat && x && workspace, AVF_EINVAL, "token_front: null pointer");
   AVF_REQUIRE(n_clips > 0 && in_dim > 0 && emb_dim > 0 && n_tok > 0, AVF_EINVAL, "token_front: n_clips=%d n_tok=%d", n_clips, n_tok);
   const size_t need = align_up(size_t(n_clips) * in_dim * elt(mode));
   AVF_REQUIRE(workspace_bytes >= need, AVF_EWORKSPACE, "workspace too small: %zu < %zu bytes", workspace_bytes, need);
@@ -341,7 +366,7 @@ int avf_token_front_fwd(int mode, const float* emb, int32_t ld_emb, const float*
   if ((e = bn_rows(mode, emb, ld_emb, bn_gamma, bn_beta, bn_mean, bn_var, workspace, n_clips, in_dim, st))) return e;
   // [n_clips, n_tok*emb_dim] row-major IS [n_clips*n_tok, emb_dim]: token i = the i-th stacked projection  (models/heads.py:294-319, 356-364)
   if ((e = linear(mode, workspace, in_dim, w_cat, b_cat, nullptr, 0, x, n_tok * emb_dim, AVF_FP32, n_clips, n_tok * emb_dim, in_dim, AVF_EPI_BIAS, st))) return e;
-  return add_row_periodic(x, emb_dim, pos, n_clips * n_tok, emb_dim, n_tok, st);
+  return pos == nullptr ? 0 : add_row_periodic(x, emb_dim, pos, n_clips * n_tok, emb_dim, n_tok, st);     // NULL: added by avf_token_stack_fwd
 }
 
 int avf_au_former_front_fwd(int mode, const float* emb, int32_t ld_emb, const float* bn_gamma, const float* bn_beta, const float* bn_mean,

@@ -67,13 +67,13 @@ int adam_step(float* p, const float* g, float* m, float* v, void* shadow, size_t
 int attention_mma_bf16(const void* qkv, void* out, int n_seq, int n_tok, int heads, int dim_head, cudaStream_t st, int q_rows = 0);
 int attention_bwd_mma_bf16(const void* qkv, const void* dout, void* dqkv, int n_seq, int n_tok, int heads, int dim_head, cudaStream_t st);
 
-// avf_layer_fused.cu: whole encoder stack in one persistent tcgen05 kernel (dim 256, 8 heads x 32)
+// avf_layer_fused.cu: whole encoder stack in one persistent tcgen05 kernel (dim 256 or 128, 8 heads x 32)
 bool encoder_fused_supported(const avf_stack_shape* s);
 int fused_prof_read(unsigned long long* out64, int reset);   // phase counters, only with -DAVF_FUSED_PROF
 int fused_set_trap_buffer(void* host_mapped_words);          // 4 host-mapped words a timed-out wait fills in before trapping
 size_t encoder_fused_scratch_bytes();                        // scratch of the NCHW form (channel-major positional table)
 int encoder_fused(int io_kind, const avf_stack_shape* s, const avf_layer_weights* L, const void* in, int ld_in, void* out, int ld_out,
-                  const float* pos, void* scratch, cudaStream_t st);
+                  const float* pos, void* scratch, const float* w_last, float* out21, int* decisions, cudaStream_t st);
 
 // avf_gemm_umma.cu
 int gemm_umma(int trans_a, int trans_b, const void* a, int lda, const void* w, int ldw, const float* bias, const float* res, int ld_res,

@@ -1,8 +1,8 @@
-// Fused pre-LN encoder stack for dim 256 / 8 heads x 32 (SFormer, fusion head): ONE persistent kernel runs
+// Fused pre-LN encoder stack for dim 256 or 128 / 8 heads x 32 (SFormer, fusion head; AU_formers, VA_former): ONE persistent kernel runs
 //   x + to_out(softmax(q k^T / sqrt(dh)) v)   and   x + W2 gelu(W1 LN(x) + b1) + b2        (models/heads.py:164-256)
 // for `depth` layers on 128-row tiles (floor(128 / n_tok) whole sequences per tile) without touching HBM in between.
 //
-//   * the fp32 residual stream of the tile lives in TMEM columns [0,256): the out-projection and the second MLP GEMM
+//   * the fp32 residual stream of the tile lives in TMEM columns [0,D): the out-projection and the second MLP GEMM
 //     ACCUMULATE onto it (tcgen05.mma with accumulate=1 on a tile pre-loaded with x + bias), so both residual adds
 //     and both bias adds cost nothing;
 //   * LayerNorm runs on the row workers (one TMEM lane = one token row, two threads per row) and writes the bf16
@@ -16,7 +16,11 @@
 //     "head full" barrier per head), so QKV(h+1) never waits for L2;
 //   * the other weights are streamed from L2 by TMA through 16 KB slots (two during attention, nine in the MLP phase, when the
 //     Q/K/V staging and the QKV ring are idle; one barrier per group of four), activations enter / leave as whole NCHW frames
-//     by bulk copies (SFormer, models/vformer.py:245-259) or as fp32 rows;
+//     by bulk copies (SFormer, models/vformer.py:245-259) or as fp32 rows (+ an optional positional table; the fusion head's
+//     12 AU logits and decisions can be taken from the last layer's output sweep instead of storing the token rows);
+//   * the model width D (256 or 128) is a template parameter.  The shared-memory map, the TMEM map and the per-layer vector
+//     block are laid out for D = 256; at D = 128 the A0 operand, the residual columns and the vectors use their first halves,
+//     and every GEMM whose K or N is the model width has half the panels (QKV / FF1 K, out-projection / FF2 N);
 //   * tiles are handed out by an atomic counter (NCHW form): the weight producer fetches the next index one tile ahead and
 //     publishes it to the other roles through a four-entry queue in shared memory (see next_tile).
 //
@@ -52,12 +56,14 @@ using namespace fused;
 #define AVF_O_TMEM 1
 #endif
 
+// DIM: the widest model (256) — the layouts below are sized for it — and the only width of the NCHW form.  Kernels take the
+// model width as the template parameter D (256 or 128).
 constexpr int DIM = 256, HEADS = 8, DH = 32;
 constexpr int MAX_DEPTH = 3, MAX_MLP = 1024;
 #ifndef AVF_FUSED_NSPLIT
 #define AVF_FUSED_NSPLIT 2
 #endif
-constexpr int NSPLIT = AVF_FUSED_NSPLIT;   // threads per token row (each owns DIM / NSPLIT columns of the residual stream)
+constexpr int NSPLIT = AVF_FUSED_NSPLIT;   // threads per token row (each owns D / NSPLIT columns of the residual stream)
 static_assert(NSPLIT == 2, "two threads per token row (the packed softmax exchanges a pair)");
 constexpr int WORKER_T0 = 96;              // first worker thread
 constexpr int NUM_WORKERS = 128 * NSPLIT;
@@ -73,15 +79,29 @@ constexpr int RING = 9, RING_LO = 2, RING_HI = 4, SLOT_BYTES = 16384;
 #define AVF_QRING 6
 #endif
 constexpr int QRING = AVF_QRING, QSLOT_BYTES = 12288;
+// K panels per head in the QKV ring (= K panels of A0) at model width D
+template <int D> constexpr int KPH = D / 64;
+// "Head full" barriers of the QKV ring: head hq signals barrier hq % NQG, whose phase (hq / NQG) & 1 the MMA thread waits for.
+// Head hq + NQG re-arms that barrier (expect_tx) when its first panel is issued, i.e. after the producer's wait for the slot of
+// panel KPH * (hq + NQG) - QRING to be consumed.  With NQG = ceil(QRING / KPH) that panel number lies in
+// [KPH * hq, KPH * hq + KPH - 1]: it is one of head hq's OWN panels, consumed only after the MMA thread's wait for head hq.  So a
+// barrier never completes a second phase before its first one has been waited for.  (D = 256, QRING = 6: KPH = 4, NQG = 2, head
+// hq + 2 reuses the slot of head hq's third panel; D = 128: KPH = 2, NQG = 3, head hq + 3 reuses the slot of head hq's first panel.)
+template <int D> constexpr int NQG = (QRING + KPH<D> - 1) / KPH<D>;
+constexpr int MAX_QG = NQG<128>;
+static_assert(KPH<256> * (NQG<256> - 1) < QRING && QRING <= KPH<256> * NQG<256>, "head-full barrier parity (D = 256)");
+static_assert(KPH<128> * (NQG<128> - 1) < QRING && QRING <= KPH<128> * NQG<128>, "head-full barrier parity (D = 128)");
 // MLP weight slots per "group full" barrier: 4 = one barrier per GEMM, 2 = one per half GEMM (the first MMAs start one slot pair earlier)
 #ifndef AVF_MLP_GROUP
 #define AVF_MLP_GROUP 4
 #endif
 constexpr int MLPG = AVF_MLP_GROUP;
 static_assert(MLPG == 2 || MLPG == 4, "MLP group size");
+// At D = 128 an MLP GEMM (FF1: K = D, FF2: N = D) is two 16 KB slots: one group per GEMM
+template <int D> constexpr int GSLOTS = MLPG < D / 64 ? MLPG : D / 64;
 
 // shared memory map (offsets from a 1024-byte aligned base)
-constexpr int OFF_A0 = 0;                          // 64 KB  LN output [128 x 256] bf16, 4 K-panels; also the NCHW input staging
+constexpr int OFF_A0 = 0;                          // 64 KB  LN output [128 x D] bf16, D / 64 K-panels of 16 KB; also the NCHW input staging
 constexpr int OFF_Q = 65536;                       // 8 KB   Q_h [128 x 32] K-major SW64
 constexpr int OFF_K = OFF_Q + 8192;                // 8 KB   K_h
 constexpr int OFF_V = OFF_K + 8192;                // 2x8 KB V_h [128 tok x 32] MN-major SW64, double buffered
@@ -90,15 +110,15 @@ constexpr int OFF_OST = OFF_RING + (RING_HI - RING_LO) * SLOT_BYTES;   // 8 KB  
 constexpr int OFF_QRING = OFF_OST + (AVF_O_TMEM ? 0 : 8192);   // QRING x 12 KB QKV weight ring (right behind slot 3 when O_h stays in TMEM); also the NCHW output staging (2 x 64 x 256 bf16 at most)
 constexpr int OFF_OUTST = OFF_QRING;
 static_assert(QRING * QSLOT_BYTES >= 2 * 64 * 256 * 2, "the NCHW output staging lives in the QKV ring");
-static_assert(QRING >= 6 && QRING < 8, "one head-full barrier per head parity needs 6 or 7 sub-slots (see qkv_producer_main)");
+static_assert(QRING >= 6 && QRING < 8, "six or seven QKV sub-slots (one and a half heads in flight at D = 256; see NQG)");
 constexpr int QRING_END = OFF_QRING + QRING * QSLOT_BYTES;
 constexpr int OFF_XCH = QRING_END > OFF_Q + RING * SLOT_BYTES ? QRING_END : OFF_Q + RING * SLOT_BYTES;      // row exchange [2][128][4] floats
 static_assert(OFF_XCH - OFF_Q >= RING * SLOT_BYTES, "the nine MLP ring slots fit in [OFF_Q, OFF_XCH)");
 static_assert(OFF_RING == OFF_Q + RING_LO * SLOT_BYTES, "ring slots are contiguous from OFF_Q");
 __host__ __device__ constexpr int slot_offset(uint32_t s) { return OFF_Q + int(s) * SLOT_BYTES; }
-constexpr int OFF_VEC = OFF_XCH + 2 * 128 * 4 * 4;      // per-layer vectors
-constexpr int V_BOUT = 0, V_BFF2 = 256, V_BFF1 = 512;   // fp32 biases
-constexpr int V_B16 = V_BFF1 + MAX_MLP;             // then bf16 copies of the LayerNorm affine vectors: [ln1_g | ln1_b | ln2_g | ln2_b] x 256
+constexpr int OFF_VEC = OFF_XCH + 2 * 128 * 4 * 4;      // per-layer vectors (first D entries of each used)
+constexpr int V_BOUT = 0, V_BFF2 = DIM, V_BFF1 = 2 * DIM;   // fp32 biases
+constexpr int V_B16 = V_BFF1 + MAX_MLP;             // then bf16 copies of the LayerNorm affine vectors: [ln1_g | ln1_b | ln2_g | ln2_b] x DIM
 constexpr int OFF_BAR = OFF_VEC + (V_B16 + 512) * 4;
 constexpr int SMEM_USED = OFF_BAR + 512;
 constexpr int SMEM_ALLOC = SMEM_USED + 1024;       // slack for the 1024-byte alignment of the base
@@ -106,23 +126,22 @@ static_assert(SMEM_ALLOC <= 232448, "shared memory budget");
 
 // K-panel order of the two GEMMs that read a fresh LayerNorm output (QKV, FF1).  The two threads of a row write panels {0,1} and {2,3}
 // of A0, so panels 0 and 2 are complete when every thread is half-way through its normalisation sweep (B_A0_HALF): the first GEMM behind
-// a LayerNorm starts on them and only then waits for the whole operand (B_A0_READY).  AVF_A0_HALF=0: plain order, one barrier.
+// a LayerNorm starts on them and only then waits for the whole operand (B_A0_READY).  AVF_A0_HALF=0: plain order, one barrier.  At
+// D = 128 each thread writes ONE panel, both at the same time: plain order, one barrier.
 #ifndef AVF_A0_HALF
 #define AVF_A0_HALF 1
 #endif
-#if AVF_A0_HALF
-__device__ __forceinline__ constexpr int kpanel(int i) { return ((i & 1) << 1) | (i >> 1); }      // 0, 2, 1, 3
-#else
-__device__ __forceinline__ constexpr int kpanel(int i) { return i; }
-#endif
+template <int D> constexpr bool A0_HALF = AVF_A0_HALF && D == 256;
+template <int D>
+__device__ __forceinline__ constexpr int kpanel(int i) { return A0_HALF<D> ? (((i & 1) << 1) | (i >> 1)) : i; }      // 0, 2, 1, 3
 
-// TMEM columns
+// TMEM columns (residual stream: [0, D))
 constexpr uint32_t TM_X = 0, TM_D1 = 256, TM_O = 352, TM_S = 384, TM_H0 = 256, TM_H1 = 384;
 
 enum {
   B_RING_FULL = 0, B_RING_EMPTY = RING, B_X0_FULL = 2 * RING, B_A0_FREE, B_A0_READY, B_D1_FULL, B_STAGED, B_S_FULL, B_P_READY, B_O_FULL,
   B_O_DRAINED, B_X1_FULL, B_HACC_FULL, B_HACC_FULL1, B_H_READY, B_H_READY1, B_X2_FULL,
-  B_QG_FULL, B_QR_EMPTY = B_QG_FULL + 2, B_A1_FREE = B_QR_EMPTY + QRING, B_OUT_READ, B_QKV_FREE, B_G_FULL, B_TQ_FULL = B_G_FULL + 8, B_A0_HALF = B_TQ_FULL + 4, NUM_BARS
+  B_QG_FULL, B_QR_EMPTY = B_QG_FULL + MAX_QG, B_A1_FREE = B_QR_EMPTY + QRING, B_OUT_READ, B_QKV_FREE, B_G_FULL, B_TQ_FULL = B_G_FULL + 8, B_A0_HALF = B_TQ_FULL + 4, NUM_BARS
 };
 static_assert(NUM_BARS * 8 + 8 + 16 <= 512, "barrier block (+ TMEM slot + tile queue)");
 
@@ -159,8 +178,11 @@ struct LayerArgs {
 struct FusedArgs {
   LayerArgs layer[MAX_DEPTH];
   const void* in;
-  void* out;
-  const float* pos;          // [n_tok, 256] or nullptr (IO_ROWS_F32)
+  void* out;                 // IO_ROWS_F32: nullptr = the token rows are not stored (w_last given)
+  const float* pos;          // [n_tok, D] or nullptr (IO_ROWS_F32)
+  const float* w_last;       // IO_ROWS_F32, n_tok = 12: [12, D] AU weights or nullptr; out21 [n_seq, 21] and decisions [n_seq, 12]
+  float* out21;              // (nullable) are then written by the last layer's output sweep
+  int* decisions;
   const float* pos_t;        // IO_NCHW_BF16: the same table as [256 / 4][POS_LD tokens][4 channels]: one 16-byte load per 4 channels,
                              // and the lanes of a warp (consecutive tokens) read consecutive 16-byte words
   int ld_in, ld_out;         // IO_ROWS_F32 row strides (elements)
@@ -174,11 +196,12 @@ struct FusedArgs {
 __device__ unsigned* g_trap_buffer = nullptr;
 
 // ---------------------------------------------------------------------------------------------
-// row workers: thread (row, g) owns columns [g*CW, g*CW+CW) of token row `row` (= TMEM lane), CW = 256 / NSPLIT
+// row workers: thread (row, g) owns columns [g*CW, g*CW+CW) of token row `row` (= TMEM lane), CW = D / NSPLIT
 // ---------------------------------------------------------------------------------------------
-constexpr int CW = DIM / NSPLIT;
-
+template <int D>
 struct Worker {
+  static constexpr int CW = D / NSPLIT;
+
   uint8_t* smem;
   uint64_t* bars;
   const float* vec;     // per-layer vectors in shared memory
@@ -255,7 +278,7 @@ struct Worker {
     mean = exchange_sum(mean_g) * (1.f / NSPLIT);
     const float dm = mean_g - mean;
     const float m2 = exchange_sum(fmaf(dm * dm, n, m2_g));
-    rstd = rsqrtf(m2 * (1.f / DIM) + 1e-5f);
+    rstd = rsqrtf(m2 * (1.f / D) + 1e-5f);
   }
   // Sweep 1 of a LayerNorm whose input already sits in TMEM (x1 after the out-projection, x2 after the MLP).
   __device__ __forceinline__ void stats_from_tmem(float& mean, float& rstd) {
@@ -285,8 +308,8 @@ struct Worker {
       const int chunk0 = (col0 & 63) >> 3;
 #pragma unroll
       for (int ch = 0; ch < 4; ++ch) {
-        const __nv_bfloat16* v16 = reinterpret_cast<const __nv_bfloat16*>(vec + V_B16) + ln_sel * 512 + col0 + ch * 8;
-        const uint4 gm = *reinterpret_cast<const uint4*>(v16), bt = *reinterpret_cast<const uint4*>(v16 + 256);
+        const __nv_bfloat16* v16 = reinterpret_cast<const __nv_bfloat16*>(vec + V_B16) + ln_sel * (2 * DIM) + col0 + ch * 8;
+        const uint4 gm = *reinterpret_cast<const uint4*>(v16), bt = *reinterpret_cast<const uint4*>(v16 + DIM);
         uint4 pk;
         pk.x = fma_bf16x2(cvt_bf16x2_pair(f2_fma(f2_pack(x[ch * 8], x[ch * 8 + 1]), rstd2, nmr2)), gm.x, bt.x);
         pk.y = fma_bf16x2(cvt_bf16x2_pair(f2_fma(f2_pack(x[ch * 8 + 2], x[ch * 8 + 3]), rstd2, nmr2)), gm.y, bt.y);
@@ -301,9 +324,7 @@ struct Worker {
         f2_unpack(f2_add(f2_pack(x[j + 2], x[j + 3]), b.y), x[j + 2], x[j + 3]);
       }
       tmem_st32(tl + TM_X + col0, reinterpret_cast<const uint32_t(&)[32]>(x));
-#if AVF_A0_HALF
-      if (c0 == 32) arrive(B_A0_HALF);          // this thread's first panel (0 or 2) is written
-#endif
+      if (A0_HALF<D> && c0 == 32) arrive(B_A0_HALF);          // this thread's first panel (0 or 2) is written
     }
     tmem_st_wait();
     arrive(B_A0_READY);
@@ -313,8 +334,8 @@ struct Worker {
 // Softmax of one head for a thread that owns NC whole 8-column chunks of its row's window, geometry known at compile time
 // (TAILV > 0: only the first TAILV columns of the last chunk exist).  S is read at `ts`, P (bf16 pairs) written at `tp`;
 // returns the thread's partial row sum.  Same arithmetic as the general path in worker_main.
-template <int NC, int TAILV>
-__device__ __forceinline__ float softmax_fixed(Worker& w, uint32_t ts, uint32_t tp, float sm_scale, Prof& pf) {
+template <int NC, int TAILV, class W>
+__device__ __forceinline__ float softmax_fixed(W& w, uint32_t ts, uint32_t tp, float sm_scale, Prof& pf) {
   float s[NC][8];
 #pragma unroll
   for (int c = 0; c < NC; ++c) tmem_ld8(ts + c * 8, reinterpret_cast<uint32_t(&)[8]>(s[c]));
@@ -370,9 +391,11 @@ __host__ __device__ constexpr int log2_of(int v) { return v == 16 ? 4 : (v == 32
 
 // NTOK > 0: the sequence length is a compile-time constant (the SFormer's 49): the transposing tile sweeps address the staged
 // NCHW frames with immediate offsets and the softmax geometry folds away.  NTOK = 0: everything from FusedArgs.
-template <int IO, int NTOK>
+template <int IO, int NTOK, int D>
 __device__ void worker_main(const FusedArgs& a, uint8_t* smem, uint64_t* bars, uint32_t tmem) {
-  Worker w;
+  using W = Worker<D>;
+  constexpr int CW = W::CW;
+  W w;
   w.smem = smem;
   w.bars = bars;
   w.vec = reinterpret_cast<const float*>(smem + OFF_VEC);
@@ -416,14 +439,14 @@ __device__ void worker_main(const FusedArgs& a, uint8_t* smem, uint64_t* bars, u
     // ---- tile input: x (+ pos) -> TMEM, statistics of LN1 on the way --------------------------------------
     float mean, rstd;
     {
-      Worker::Stats st{0.f, 0.f, 0.f};
+      typename W::Stats st{0.f, 0.f, 0.f};
       // Branch-free: padding rows (and sequences beyond the end of the batch) read a valid location, i.e. they carry a copy of a
       // real token.  Nothing ever looks at them: as keys they are outside every row's softmax window, as rows they are not stored.
       const int t_safe = valid ? t_in_seq : 0, seq_safe = valid ? seq_in_tile : 0;
-      const float* pp = (IO == IO_ROWS_F32 && a.pos != nullptr) ? a.pos + t_safe * DIM + g * CW : nullptr;
+      const float* pp = (IO == IO_ROWS_F32 && a.pos != nullptr) ? a.pos + t_safe * D + g * CW : nullptr;
       const float4* ppt = reinterpret_cast<const float4*>(a.pos_t) + size_t(g * CW / 4) * POS_LD + t_safe;
       if constexpr (IO == IO_NCHW_BF16) mbar_wait(&bars[B_X0_FULL], (n_x0++) & 1);
-      const __nv_bfloat16* src16 = reinterpret_cast<const __nv_bfloat16*>(smem + OFF_A0) + size_t(seq_safe * DIM + g * CW) * n_tok + t_safe;
+      const __nv_bfloat16* src16 = reinterpret_cast<const __nv_bfloat16*>(smem + OFF_A0) + size_t(seq_safe * D + g * CW) * n_tok + t_safe;
       const float* src32 = static_cast<const float*>(a.in) + ((size_t(tile) * spt + seq_safe) * n_tok + t_safe) * a.ld_in + g * CW;
 #pragma unroll 1
       for (int c0 = 0; c0 < CW; c0 += 32) {
@@ -485,11 +508,11 @@ __device__ void worker_main(const FusedArgs& a, uint8_t* smem, uint64_t* bars, u
       if (a.depth > 1 || !vec_loaded) {          // per-layer vectors -> shared memory (once per CTA when there is one layer)
         if (vec_loaded) bar_sync(5, NUM_WORKERS);  // previous layer's readers are done
         float* vs = reinterpret_cast<float*>(smem + OFF_VEC);
-        for (int i = wt; i < DIM; i += NUM_WORKERS) {
+        for (int i = wt; i < D; i += NUM_WORKERS) {
           vs[V_BOUT + i] = L.b_out[i]; vs[V_BFF2 + i] = L.b_ff2[i];
           __nv_bfloat16* v16 = reinterpret_cast<__nv_bfloat16*>(vs + V_B16);
-          v16[i] = __float2bfloat16_rn(L.ln1_g[i]); v16[256 + i] = __float2bfloat16_rn(L.ln1_b[i]);
-          v16[512 + i] = __float2bfloat16_rn(L.ln2_g[i]); v16[768 + i] = __float2bfloat16_rn(L.ln2_b[i]);
+          v16[i] = __float2bfloat16_rn(L.ln1_g[i]); v16[DIM + i] = __float2bfloat16_rn(L.ln1_b[i]);
+          v16[2 * DIM + i] = __float2bfloat16_rn(L.ln2_g[i]); v16[3 * DIM + i] = __float2bfloat16_rn(L.ln2_b[i]);
         }
         for (int i = wt; i < a.n_chunks * 128; i += NUM_WORKERS) vs[V_BFF1 + i] = L.b_ff1[i];
         bar_sync(5, NUM_WORKERS);
@@ -727,16 +750,20 @@ __device__ void worker_main(const FusedArgs& a, uint8_t* smem, uint64_t* bars, u
       if (l + 1 < a.depth) w.stats_from_tmem(mean, rstd);
     }
 
-    // ---- tile output ----------------------------------------------------------------------------
+    // ---- tile output (+ the AU logits: token t of a clip dotted with w_last[t]) -------------------------------
     {
-      __nv_bfloat16* dst16 = reinterpret_cast<__nv_bfloat16*>(smem + OFF_OUTST) + size_t(seq_in_tile * DIM + g * CW) * n_tok + t_in_seq;
+      __nv_bfloat16* dst16 = reinterpret_cast<__nv_bfloat16*>(smem + OFF_OUTST) + size_t(seq_in_tile * D + g * CW) * n_tok + t_in_seq;
+      const bool store = valid && (IO == IO_NCHW_BF16 || a.out != nullptr);
       float* dst32 = static_cast<float*>(a.out) + grow * a.ld_out + g * CW;
+      const bool logits = IO == IO_ROWS_F32 && a.w_last != nullptr;
+      const float* wl = logits ? a.w_last + (valid ? t_in_seq : 0) * D + g * CW : nullptr;
+      float dot = 0.f;
 #pragma unroll 1
       for (int c0 = 0; c0 < CW; c0 += 32) {
         float x[32];
         tmem_ld32(tl + TM_X + g * CW + c0, reinterpret_cast<uint32_t(&)[32]>(x));
         tmem_ld_wait();
-        if (valid) {
+        if (store) {
           if constexpr (IO == IO_NCHW_BF16) {
 #pragma unroll
             for (int j = 0; j < 32; ++j) dst16[(c0 + j) * n_tok] = __float2bfloat16_rn(x[j]);
@@ -745,13 +772,33 @@ __device__ void worker_main(const FusedArgs& a, uint8_t* smem, uint64_t* bars, u
             for (int j = 0; j < 32; j += 4) *reinterpret_cast<float4*>(dst32 + c0 + j) = make_float4(x[j], x[j + 1], x[j + 2], x[j + 3]);
           }
         }
+        if constexpr (IO == IO_ROWS_F32) {
+          if (logits) {
+#pragma unroll
+            for (int j = 0; j < 32; j += 4) {
+              const float4 w4 = __ldg(reinterpret_cast<const float4*>(wl + c0 + j));
+              dot = fmaf(x[j], w4.x, fmaf(x[j + 1], w4.y, fmaf(x[j + 2], w4.z, fmaf(x[j + 3], w4.w, dot))));
+            }
+          }
+        }
+      }
+      if constexpr (IO == IO_ROWS_F32) {
+        if (logits) {      // n_tok = 12 (checked on the host): token t_in_seq of clip `grow / 12` is AU t_in_seq
+          const float lg = w.exchange_sum(dot);
+          const size_t clip = grow / 12;
+          if (valid && g == 0) {
+            if (a.out21 != nullptr) a.out21[clip * 21 + t_in_seq] = lg;
+            if (a.decisions != nullptr) a.decisions[clip * 12 + t_in_seq] = lg > 0.f ? 1 : 0;     // round(sigmoid(x)) == x > 0
+          }
+          if (valid && g == 1 && t_in_seq < 9 && a.out21 != nullptr) a.out21[clip * 21 + 12 + t_in_seq] = 0.f;      // zero padding to 21
+        }
       }
       if constexpr (IO == IO_NCHW_BF16) {
         fence_proxy_async_smem();
         bar_sync(5, NUM_WORKERS);
         if (threadIdx.x == WORKER_T0) {
-          __nv_bfloat16* gdst = static_cast<__nv_bfloat16*>(a.out) + size_t(tile) * spt * n_tok * DIM;
-          bulk_store_1d(gdst, smem + OFF_OUTST, uint32_t(seqs_here) * n_tok * DIM * 2);   // read completion: see the next tile's input sweep
+          __nv_bfloat16* gdst = static_cast<__nv_bfloat16*>(a.out) + size_t(tile) * spt * n_tok * D;
+          bulk_store_1d(gdst, smem + OFF_OUTST, uint32_t(seqs_here) * n_tok * D * 2);   // read completion: see the next tile's input sweep
         }
       }
     }
@@ -767,7 +814,7 @@ __device__ void worker_main(const FusedArgs& a, uint8_t* smem, uint64_t* bars, u
 // ---------------------------------------------------------------------------------------------
 // weight producer (one thread): must issue slots in exactly the order the MMA thread consumes them
 // ---------------------------------------------------------------------------------------------
-template <int IO>
+template <int IO, int D>
 __device__ void producer_main(const FusedArgs& a, uint8_t* smem, uint64_t* bars) {
   // (one lane only: this loop polls with try_wait between slots, and a whole-warp version — every lane polling and adopting the
   //  issuing lane's observation — measured 7x slower; the MMA warp, which blocks instead of polling, does run warp-wide)
@@ -788,9 +835,9 @@ __device__ void producer_main(const FusedArgs& a, uint8_t* smem, uint64_t* bars)
       ++n_free;
     }
     const int seqs_here = min(a.spt, a.n_seq - load_tile * a.spt);
-    const uint32_t bytes = uint32_t(seqs_here) * a.n_tok * DIM * 2;
+    const uint32_t bytes = uint32_t(seqs_here) * a.n_tok * D * 2;
     mbar_expect_tx(&bars[B_X0_FULL], bytes);
-    bulk_load_1d(smem + OFF_A0, static_cast<const __nv_bfloat16*>(a.in) + size_t(load_tile) * a.spt * a.n_tok * DIM, bytes, &bars[B_X0_FULL]);
+    bulk_load_1d(smem + OFF_A0, static_cast<const __nv_bfloat16*>(a.in) + size_t(load_tile) * a.spt * a.n_tok * D, bytes, &bars[B_X0_FULL]);
     load_tile = -1;
     need_free = true;
   };
@@ -857,23 +904,24 @@ __device__ void producer_main(const FusedArgs& a, uint8_t* smem, uint64_t* bars)
     }
     for (int l = 0; l < a.depth; ++l) {
       const LayerArgs& L = a.layer[l];
-      for (int h = 0; h < HEADS; ++h) {                        // Wout[:, 32h .. 32h+32): [256 x 32], 64B swizzle
+      for (int h = 0; h < HEADS; ++h) {                        // Wout[:, 32h .. 32h+32): [D x 32], 64B swizzle
         const uint32_t s = RING_LO + h % (RING_HI - RING_LO);
-        load(s, &L.tm_out, h * DH, 0, &bars[B_RING_FULL + s], SLOT_BYTES);
+        load(s, &L.tm_out, h * DH, 0, &bars[B_RING_FULL + s], D * DH * 2);
       }
       poll_wait(&bars[B_QKV_FREE], (n_gate++) & 1);          // the attention MMAs are done with the Q/K/V staging and A1 = slots 0-1, 5-8
       uint32_t m = 0;
-      auto ff1 = [&](int c) {
-        for (int kp = 0; kp < 4; ++kp) {
-          if (kp % MLPG == 0) ++gidx;
-          load((m++) % RING, &L.tm_w1, kpanel(kp) * 64, c * 128, &bars[B_G_FULL + ((gidx - 1) & 7u)], kp % MLPG == 0 ? MLPG * SLOT_BYTES : 0);
+      constexpr int G = GSLOTS<D>, NH = D / 128;
+      auto ff1 = [&](int c) {                                  // K = D: D / 64 panels of W1[c*128 .. +128, :]
+        for (int kp = 0; kp < D / 64; ++kp) {
+          if (kp % G == 0) ++gidx;
+          load((m++) % RING, &L.tm_w1, kpanel<D>(kp) * 64, c * 128, &bars[B_G_FULL + ((gidx - 1) & 7u)], kp % G == 0 ? G * SLOT_BYTES : 0);
         }
       };
-      auto ff2 = [&](int c) {
-        for (int i = 0; i < 4; ++i) {
-          const int kp = i >> 1, nh = i & 1;
-          if (i % MLPG == 0) ++gidx;
-          load((m++) % RING, &L.tm_w2, c * 128 + kp * 64, nh * 128, &bars[B_G_FULL + ((gidx - 1) & 7u)], i % MLPG == 0 ? MLPG * SLOT_BYTES : 0);
+      auto ff2 = [&](int c) {                                  // K = 128 (two panels) x N = D (D / 128 halves)
+        for (int i = 0; i < 2 * NH; ++i) {
+          const int kp = i / NH, nh = i % NH;
+          if (i % G == 0) ++gidx;
+          load((m++) % RING, &L.tm_w2, c * 128 + kp * 64, nh * 128, &bars[B_G_FULL + ((gidx - 1) & 7u)], i % G == 0 ? G * SLOT_BYTES : 0);
         }
       };
       ff1(0);
@@ -891,7 +939,7 @@ __device__ void producer_main(const FusedArgs& a, uint8_t* smem, uint64_t* bars)
 // ---------------------------------------------------------------------------------------------
 // QKV weight producer (one thread of its own warp): the 4 x 12 KB ring inside A1
 // ---------------------------------------------------------------------------------------------
-template <int IO>
+template <int IO, int D>
 __device__ void qkv_producer_main(const FusedArgs& a, uint8_t* smem, uint64_t* bars) {
   uint32_t qit = 0, hq = 0, n_free = 0, n_read = 0;
   bool first = true;
@@ -903,16 +951,15 @@ __device__ void qkv_producer_main(const FusedArgs& a, uint8_t* smem, uint64_t* b
       if (!first) mbar_wait(&bars[B_A1_FREE], (n_free++) & 1);   // the previous layer's MLP weights (ring slots 5-8 live in A1) are consumed
       first = false;
       for (int h = 0; h < HEADS; ++h, ++hq) {
-        // the four panels of a head signal ONE barrier (armed with the head's 48 KB at its first panel): the MMA thread waits once
-        // per head.  Barrier hq % 2: head hq + 2 reuses sub-slots that head hq's third and fourth panel occupied, so it is armed
-        // only after the MMA thread's wait for head hq.
-        uint64_t* fb = &bars[B_QG_FULL + (hq & 1u)];
-        for (int kp = 0; kp < 4; ++kp) {
+        // the KPH panels of a head signal ONE barrier (armed with the head's KPH x 12 KB at its first panel): the MMA thread waits
+        // once per head.  Barrier hq % NQG is re-armed only after the MMA thread's wait for head hq (see NQG).
+        uint64_t* fb = &bars[B_QG_FULL + (hq % uint32_t(NQG<D>))];
+        for (int kp = 0; kp < KPH<D>; ++kp) {
           const uint32_t s = qit % QRING, ph = (qit / QRING) & 1;
           mbar_wait(&bars[B_QR_EMPTY + s], ph ^ 1);
           uint8_t* d = smem + OFF_QRING + s * QSLOT_BYTES;
-          if (kp == 0) mbar_expect_tx(fb, 4 * QSLOT_BYTES);
-          for (int s3 = 0; s3 < 3; ++s3) tma_load_2d(d + s3 * 4096, &L.tm_qkv, fb, kpanel(kp) * 64, s3 * (HEADS * DH) + h * DH);
+          if (kp == 0) mbar_expect_tx(fb, KPH<D> * QSLOT_BYTES);
+          for (int s3 = 0; s3 < 3; ++s3) tma_load_2d(d + s3 * 4096, &L.tm_qkv, fb, kpanel<D>(kp) * 64, s3 * (HEADS * DH) + h * DH);
           ++qit;
         }
       }
@@ -925,6 +972,7 @@ __device__ void qkv_producer_main(const FusedArgs& a, uint8_t* smem, uint64_t* b
 // ---------------------------------------------------------------------------------------------
 // Executed by ALL 32 lanes of warp 1 with warp-uniform values (so that descriptors and addresses live in uniform registers and
 // the issue loop is a handful of instructions per MMA); only the elected lane issues tcgen05.mma / tcgen05.commit.
+template <int D>
 __device__ void mma_main(const FusedArgs& a, uint8_t* smem, uint64_t* bars, uint32_t tmem) {
   const bool leader = elect_one();
   const uint32_t a0 = smem_u32(smem + OFF_A0);
@@ -932,7 +980,7 @@ __device__ void mma_main(const FusedArgs& a, uint8_t* smem, uint64_t* bars, uint
   const uint32_t smem0 = smem_u32(smem), qring = smem_u32(smem + OFF_QRING), ost = smem_u32(smem + OFF_OST);
   const int kmax = 128;                        // S / P span the whole tile: sequences sit in power-of-two row slots
   const uint32_t id_qkv = make_idesc_bf16(128, 96), id_s = make_idesc_bf16(128, kmax), id_pv = make_idesc_bf16(128, DH, 0, 1),
-                 id_128 = make_idesc_bf16(128, 128), id_256 = make_idesc_bf16(128, 256);
+                 id_128 = make_idesc_bf16(128, 128), id_out = make_idesc_bf16(128, D);
   uint32_t obits = 0, m = 0, qit = 0, hq = 0, gidx = 0, n_a0 = 0, n_hready[2] = {0, 0};
   Prof pf;
   pf.start(blockIdx.x == 0 && leader);
@@ -957,27 +1005,27 @@ __device__ void mma_main(const FusedArgs& a, uint8_t* smem, uint64_t* bars, uint
   };
   // fresh = the first GEMM behind a LayerNorm: its first two panels (0, 2) only need B_A0_HALF, the other two B_A0_READY
   auto a0_wait = [&](int i, bool fresh) {
-#if AVF_A0_HALF
-    if (!fresh || (i != 0 && i != 2)) return;
-    pf.mark(ring_phase);
-    if (i == 0) mbar_wait(&bars[B_A0_HALF], n_a0 & 1);
-    else mbar_wait(&bars[B_A0_READY], (n_a0++) & 1);
-#else
-    if (!fresh || i != 0) return;
-    pf.mark(ring_phase);
-    mbar_wait(&bars[B_A0_READY], (n_a0++) & 1);
-#endif
+    if constexpr (A0_HALF<D>) {
+      if (!fresh || (i != 0 && i != 2)) return;
+      pf.mark(ring_phase);
+      if (i == 0) mbar_wait(&bars[B_A0_HALF], n_a0 & 1);
+      else mbar_wait(&bars[B_A0_READY], (n_a0++) & 1);
+    } else {
+      if (!fresh || i != 0) return;
+      pf.mark(ring_phase);
+      mbar_wait(&bars[B_A0_READY], (n_a0++) & 1);
+    }
     tc_fence_after();
     pf.mark(ring_phase == PM_QKV ? PM_WAIT_A0 : PM_WAIT_A0B);
   };
   auto qkv = [&](bool fresh) {                // D1[128 x 96] = LN(x) [Wq_h; Wk_h; Wv_h]^T, weights from the QKV ring
     pf.mark(ring_phase);
-    mbar_wait(&bars[B_QG_FULL + (hq & 1u)], (hq >> 1) & 1u);      // all four panels of the head
+    mbar_wait(&bars[B_QG_FULL + (hq % uint32_t(NQG<D>))], (hq / uint32_t(NQG<D>)) & 1u);      // all KPH panels of the head
     ++hq;
     tc_fence_after();
     pf.mark(PM_RW_QKV);
-    for (int i = 0; i < 4; ++i) {
-      const int kp = kpanel(i);
+    for (int i = 0; i < KPH<D>; ++i) {
+      const int kp = kpanel<D>(i);
       a0_wait(i, fresh);
       const uint32_t s = qit % QRING;
       const uint64_t da = make_desc_sw128_kmajor(a0 + kp * 16384), db = make_desc_sw128_kmajor(qring + s * QSLOT_BYTES);
@@ -992,21 +1040,21 @@ __device__ void mma_main(const FusedArgs& a, uint8_t* smem, uint64_t* bars, uint
     const uint32_t s = RING_LO + h % (RING_HI - RING_LO), sb = slot_wait(s);
     const uint64_t db = desc_sw64(sb);
 #if AVF_O_TMEM
-    if (leader) umma_bf16_ts(tmem + TM_X, tmem + TM_O, db, id_256, 1u);               // k-step 0: thread 0's packed columns
-    if (leader) umma_bf16_ts(tmem + TM_X, tmem + TM_O + 16, db + 2, id_256, 1u);      // k-step 1: thread 1's
+    if (leader) umma_bf16_ts(tmem + TM_X, tmem + TM_O, db, id_out, 1u);               // k-step 0: thread 0's packed columns
+    if (leader) umma_bf16_ts(tmem + TM_X, tmem + TM_O + 16, db + 2, id_out, 1u);      // k-step 1: thread 1's
 #else
     const uint64_t da = desc_sw64(ost);
-    if (leader) umma_bf16(tmem + TM_X, da, db, id_256, 1u);
-    if (leader) umma_bf16(tmem + TM_X, da + 2, db + 2, id_256, 1u);
+    if (leader) umma_bf16(tmem + TM_X, da, db, id_out, 1u);
+    if (leader) umma_bf16(tmem + TM_X, da + 2, db + 2, id_out, 1u);
 #endif
     slot_release(s);
   };
   bool last_layer = false;
   auto ff1 = [&](int c, bool fresh) {         // H[c&1][128 x 128] = LN2(x) W1[c*128.., :]^T
     const uint32_t d = tmem + ((c & 1) ? TM_H1 : TM_H0);
-    for (int i = 0; i < 4; ++i) {
-      const int kp = kpanel(i);
-      if (i % MLPG == 0) group_wait();
+    for (int i = 0; i < D / 64; ++i) {
+      const int kp = kpanel<D>(i);
+      if (i % GSLOTS<D> == 0) group_wait();
       a0_wait(i, fresh);
       const uint32_t s = (m++) % RING, sb = smem0 + uint32_t(slot_offset(s));
       const uint64_t da = make_desc_sw128_kmajor(a0 + kp * 16384), db = make_desc_sw128_kmajor(sb);
@@ -1075,8 +1123,8 @@ __device__ void mma_main(const FusedArgs& a, uint8_t* smem, uint64_t* bars, uint
         pf.mark(PM_WAIT_H);
         ring_phase = PM_FF2;
         for (int kp = 0; kp < 2; ++kp)        // x += gelu(H_c) W2[:, c*128..]^T
-          for (int nh = 0; nh < 2; ++nh) {
-            if ((kp * 2 + nh) % MLPG == 0) group_wait();
+          for (int nh = 0; nh < D / 128; ++nh) {
+            if ((kp * (D / 128) + nh) % GSLOTS<D> == 0) group_wait();
             const uint32_t s = (m++) % RING, sb = smem0 + uint32_t(slot_offset(s));
             const uint32_t ta = tmem + (b ? TM_H1 : TM_H0) + uint32_t(kp * 64);       // gelu(H_c) as bf16, 8 columns per 16-wide k-step
             const uint64_t db = make_desc_sw128_kmajor(sb);
@@ -1095,7 +1143,7 @@ __device__ void mma_main(const FusedArgs& a, uint8_t* smem, uint64_t* bars, uint
   pf.flush(32, 64);
 }
 
-template <int IO, int NTOK>
+template <int IO, int NTOK, int D>
 __global__ void __launch_bounds__(NUM_THREADS, 1) encoder_fused_kernel(const __grid_constant__ FusedArgs a) {
   // The kernel has no static shared memory, so the dynamic window starts at the CTA's shared-memory base, which is 1024-byte
   // aligned (checked below).  Using the array itself — not an address rounded up through integer arithmetic — lets the compiler
@@ -1136,13 +1184,13 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) encoder_fused_kernel(const __g
   pdl_trigger();
 
   if (warp == 0) {
-    if (lane == 0) producer_main<IO>(a, smem, bars);
+    if (lane == 0) producer_main<IO, D>(a, smem, bars);
   } else if (warp == 1) {
-    mma_main(a, smem, bars, tmem);
+    mma_main<D>(a, smem, bars, tmem);
   } else if (warp == 2) {
-    if (lane == 0) qkv_producer_main<IO>(a, smem, bars);
+    if (lane == 0) qkv_producer_main<IO, D>(a, smem, bars);
   } else {
-    worker_main<IO, NTOK>(a, smem, bars, tmem);
+    worker_main<IO, NTOK, D>(a, smem, bars, tmem);
   }
 
   tc_fence_before();
@@ -1203,23 +1251,28 @@ int fused_prof_read(unsigned long long* out64, int reset) {
 }
 
 bool encoder_fused_supported(const avf_stack_shape* s) {
-  return s->dim == DIM && s->heads == HEADS && s->dim_head == DH && s->mlp_dim % 128 == 0 && s->mlp_dim >= 128 && s->mlp_dim <= MAX_MLP && s->n_tok >= 1 &&
+  return (s->dim == 256 || s->dim == 128) && s->heads == HEADS && s->dim_head == DH && s->mlp_dim % 128 == 0 && s->mlp_dim >= 128 && s->mlp_dim <= MAX_MLP && s->n_tok >= 1 &&
          s->n_tok <= 64 && s->depth >= 1 && s->depth <= MAX_DEPTH;
 }
 
-// io_kind 0: in/out are NCHW bf16 maps [n_seq, 256, n_tok] (pos required); 1: fp32 token rows with strides ld_in / ld_out.
+// io_kind 0: in/out are NCHW bf16 maps [n_seq, 256, n_tok] (pos required, dim 256); 1: fp32 token rows with strides ld_in / ld_out,
+// pos [n_tok, dim] optional, out == nullptr only with w_last (n_tok 12: AU logits [n_seq, 21] and decisions [n_seq, 12] instead of rows).
 size_t encoder_fused_scratch_bytes() { return size_t(DIM) * POS_LD * sizeof(float) + 64; }      // positional table + the tile scheduler's counter
 
 int encoder_fused(int io_kind, const avf_stack_shape* s, const avf_layer_weights* L, const void* in, int ld_in, void* out, int ld_out,
-                  const float* pos, void* scratch, cudaStream_t st) {
+                  const float* pos, void* scratch, const float* w_last, float* out21, int* decisions, cudaStream_t st) {
   AVF_REQUIRE(encoder_fused_supported(s), AVF_EUNSUPPORTED, "fused encoder: unsupported shape dim=%d heads=%d dh=%d mlp=%d n_tok=%d depth=%d",
               s->dim, s->heads, s->dim_head, s->mlp_dim, s->n_tok, s->depth);
   AVF_REQUIRE(io_kind == IO_ROWS_F32 || (pos != nullptr && scratch != nullptr), AVF_EINVAL,
               "fused encoder: NCHW input needs the positional embedding and the scratch buffer");
-  AVF_REQUIRE(io_kind == IO_NCHW_BF16 || (ld_in % 4 == 0 && ld_out % 4 == 0), AVF_EINVAL, "fused encoder: row strides must be multiples of 4");
+  AVF_REQUIRE(io_kind == IO_ROWS_F32 || s->dim == DIM, AVF_EUNSUPPORTED, "fused encoder: the NCHW form is dim %d only", DIM);
+  AVF_REQUIRE(io_kind == IO_NCHW_BF16 || (ld_in % 4 == 0 && (out == nullptr || ld_out % 4 == 0)), AVF_EINVAL, "fused encoder: row strides must be multiples of 4");
+  AVF_REQUIRE(w_last == nullptr || (io_kind == IO_ROWS_F32 && s->n_tok == 12), AVF_EINVAL, "fused encoder: AU logits need 12-token rows");
+  AVF_REQUIRE(out != nullptr || w_last != nullptr, AVF_EINVAL, "fused encoder: no output");
   static thread_local FusedArgs a;      // ~2 KB of tensor maps + pointers, passed by value (__grid_constant__) per launch
   static_assert(sizeof(FusedArgs) <= 4000, "kernel parameter space");
   a.in = in; a.out = out; a.pos = pos; a.pos_t = static_cast<const float*>(scratch); a.ld_in = ld_in; a.ld_out = ld_out;
+  a.w_last = w_last; a.out21 = out21; a.decisions = decisions;
   a.tile_counter = nullptr;
   if (io_kind == IO_NCHW_BF16) {
     if (dynamic_tiles_enabled()) a.tile_counter = reinterpret_cast<int*>(static_cast<uint8_t*>(scratch) + size_t(DIM) * POS_LD * sizeof(float));
@@ -1232,31 +1285,34 @@ int encoder_fused(int io_kind, const avf_stack_shape* s, const avf_layer_weights
   a.spt = 128 / a.slot;
   a.n_tiles = ceil_div(s->n_seq, a.spt);
   a.n_chunks = s->mlp_dim / 128; a.depth = s->depth;
-  const int inner = HEADS * DH;
+  const int inner = HEADS * DH, D = s->dim;
   for (int l = 0; l < s->depth; ++l) {
     LayerArgs& A = a.layer[l];
     int e;
-    if ((e = make_tmap_bf16_2d(&A.tm_qkv, L[l].w_qkv, 3 * inner, DIM, DIM, 32))) return e;
-    if ((e = make_tmap_bf16_2d(&A.tm_out, L[l].w_out, DIM, inner, inner, 256, DH))) return e;
-    if ((e = make_tmap_bf16_2d(&A.tm_w1, L[l].w_ff1, s->mlp_dim, DIM, DIM, 128))) return e;
-    if ((e = make_tmap_bf16_2d(&A.tm_w2, L[l].w_ff2, DIM, s->mlp_dim, s->mlp_dim, 128))) return e;
+    if ((e = make_tmap_bf16_2d(&A.tm_qkv, L[l].w_qkv, 3 * inner, D, D, 32))) return e;
+    if ((e = make_tmap_bf16_2d(&A.tm_out, L[l].w_out, D, inner, inner, D, DH))) return e;      // box [D rows x 32 cols]
+    if ((e = make_tmap_bf16_2d(&A.tm_w1, L[l].w_ff1, s->mlp_dim, D, D, 128))) return e;
+    if ((e = make_tmap_bf16_2d(&A.tm_w2, L[l].w_ff2, D, s->mlp_dim, s->mlp_dim, 128))) return e;
     A.ln1_g = L[l].ln1_gamma; A.ln1_b = L[l].ln1_beta; A.b_out = L[l].b_out;
     A.ln2_g = L[l].ln2_gamma; A.ln2_b = L[l].ln2_beta; A.b_ff1 = L[l].b_ff1; A.b_ff2 = L[l].b_ff2;
   }
   static PerDeviceOnce once;
   if (once.first()) {
-    AVF_CUDA(cudaFuncSetAttribute(encoder_fused_kernel<IO_NCHW_BF16, 49>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_ALLOC));
-    AVF_CUDA(cudaFuncSetAttribute(encoder_fused_kernel<IO_NCHW_BF16, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_ALLOC));
-    AVF_CUDA(cudaFuncSetAttribute(encoder_fused_kernel<IO_ROWS_F32, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_ALLOC));
+    AVF_CUDA(cudaFuncSetAttribute(encoder_fused_kernel<IO_NCHW_BF16, 49, 256>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_ALLOC));
+    AVF_CUDA(cudaFuncSetAttribute(encoder_fused_kernel<IO_NCHW_BF16, 0, 256>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_ALLOC));
+    AVF_CUDA(cudaFuncSetAttribute(encoder_fused_kernel<IO_ROWS_F32, 0, 256>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_ALLOC));
+    AVF_CUDA(cudaFuncSetAttribute(encoder_fused_kernel<IO_ROWS_F32, 0, 128>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_ALLOC));
   }
   const int cap = sm_cap();
   const int grid = min(a.n_tiles, cap > 0 ? min(cap, sm_count_cached()) : sm_count_cached());
   if (io_kind == IO_NCHW_BF16 && a.n_tok == 49 && NSPLIT == 2 && fixed_ntok_enabled())     // the SFormer's 7 x 7 maps: compile-time geometry
-    launch_pdl(encoder_fused_kernel<IO_NCHW_BF16, 49>, grid, NUM_THREADS, SMEM_ALLOC, st, a);
+    launch_pdl(encoder_fused_kernel<IO_NCHW_BF16, 49, 256>, grid, NUM_THREADS, SMEM_ALLOC, st, a);
   else if (io_kind == IO_NCHW_BF16)
-    launch_pdl(encoder_fused_kernel<IO_NCHW_BF16, 0>, grid, NUM_THREADS, SMEM_ALLOC, st, a);
+    launch_pdl(encoder_fused_kernel<IO_NCHW_BF16, 0, 256>, grid, NUM_THREADS, SMEM_ALLOC, st, a);
+  else if (D == 256)
+    launch_pdl(encoder_fused_kernel<IO_ROWS_F32, 0, 256>, grid, NUM_THREADS, SMEM_ALLOC, st, a);
   else
-    launch_pdl(encoder_fused_kernel<IO_ROWS_F32, 0>, grid, NUM_THREADS, SMEM_ALLOC, st, a);
+    launch_pdl(encoder_fused_kernel<IO_ROWS_F32, 0, 128>, grid, NUM_THREADS, SMEM_ALLOC, st, a);
   AVF_LAUNCH_CHECK("encoder_fused_kernel");
   return 0;
 }

@@ -179,19 +179,22 @@ class Transformer(nn.Module):
         return float(self.dropout), seed, self.dropout_salt
 
     # -- forward -------------------------------------------------------------------------------
-    def forward_(self, x2d: torch.Tensor, n_seq: int, n_tok: int, out: Optional[torch.Tensor] = None, ld_out: int = 0) -> torch.Tensor:
-        """Inference kernels, in place on an fp32 residual stream [n_seq*n_tok, dim].  In train() mode with dropout > 0 (a
-        frozen sub-model inside a training loop, models/avformer.py:78-85 + train.py:327) the tape-keeping kernels run instead,
-        because they are the ones that apply dropout."""
+    def forward_(self, x2d: torch.Tensor, n_seq: int, n_tok: int, out: Optional[torch.Tensor] = None, ld_out: int = 0,
+                 pos: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """Inference kernels, in place on an fp32 residual stream [n_seq*n_tok, dim] (+ pos [n_tok, dim] first, if given).  In
+        train() mode with dropout > 0 (a frozen sub-model inside a training loop, models/avformer.py:78-85 + train.py:327) the
+        tape-keeping kernels run instead, because they are the ones that apply dropout."""
         p, seed, salt = self.dropout_state()
         if p > 0.0:
+            if pos is not None:
+                AF.add_row_periodic_(x2d, pos, n_tok)
             y, _ = AF.encoder_stack_fwd_train(x2d, self.packed(), self.shape(n_seq, n_tok), p, seed, salt)
             if out is None:
                 x2d.copy_(y)
                 return x2d
             torch.as_strided(out, (y.shape[0], y.shape[1]), (ld_out, 1)).copy_(y)
             return out
-        return AF.encoder_stack_fwd_(x2d, self.packed(), self.shape(n_seq, n_tok), out, ld_out)
+        return AF.token_stack_fwd_(x2d, self.packed(), self.shape(n_seq, n_tok), pos, out, ld_out)
 
     def forward_train(self, x2d: torch.Tensor, n_seq: int, n_tok: int) -> torch.Tensor:
         """Autograd-visible forward on an fp32 token matrix [n_seq*n_tok, dim] (activation tape kept for backward)."""

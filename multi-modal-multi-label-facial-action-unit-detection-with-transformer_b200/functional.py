@@ -158,6 +158,28 @@ def encoder_stack_fwd_(x: torch.Tensor, packed: PackedStack, shape: StackShape, 
     return x if out is None else out
 
 
+def token_stack_fwd_(x: torch.Tensor, packed: PackedStack, shape: StackShape, pos: Optional[torch.Tensor] = None,
+                     out: Optional[torch.Tensor] = None, ld_out: int = 0, w_last: Optional[torch.Tensor] = None, want_decisions: bool = False):
+    """encoder_stack_fwd_ of a token head: + pos [n_tok, dim] first (if given); with w_last [12, dim] (12 tokens per sequence) the
+    AU logits of the result follow and [n_seq, 21] logits (+ [n_seq, 12] int32 decisions) are returned, else the tokens.  In bf16
+    mode a fused-kernel stack is one launch.  x is scratch whenever out or w_last is given."""
+    _cuda(x, "x")
+    if x.dtype != torch.float32 or x.stride(-1) != 1:
+        raise TypeError("token_stack_fwd_: x must be a float32 residual stream with unit column stride")
+    L = _lib.lib()
+    ws = workspace(L.avf_encoder_workspace_bytes(ctypes.byref(shape), packed.mode), x.device)
+    out21 = dec = None
+    if w_last is not None:
+        out21 = torch.empty((shape.n_seq, 21), dtype=torch.float32, device=x.device)
+        dec = torch.empty((shape.n_seq, 12), dtype=torch.int32, device=x.device) if want_decisions else None
+    check(L.avf_token_stack_fwd(packed.mode, ctypes.byref(shape), packed.array, _ptr(x), x.stride(0), _ptr(None if pos is None else _f32c(pos)),
+                                _ptr(out), ld_out, _ptr(None if w_last is None else _f32c(w_last)), _ptr(out21), _ptr(dec), _ptr(ws), ws.numel(),
+                                _stream()), "token_stack_fwd")
+    if w_last is not None:
+        return (out21, dec) if want_decisions else out21
+    return x if out is None else out
+
+
 def layernorm_fwd(x: torch.Tensor, gamma: torch.Tensor, beta: torch.Tensor, precision="bf16") -> torch.Tensor:
     x = _f32c(_cuda(x, "x"))
     rows, dim = x.numel() // x.shape[-1], x.shape[-1]
@@ -246,22 +268,22 @@ def tformer_cls_extract(x: torch.Tensor, n_clips: int, n_tok: int) -> torch.Tens
 
 
 def au_former_front(emb: torch.Tensor, ld_emb: int, n_clips: int, bn: Sequence[torch.Tensor], w_cat: torch.Tensor, b_cat: torch.Tensor,
-                    pos: torch.Tensor, mode: int) -> torch.Tensor:
-    """BN(eval) + 12 stacked Linear(512,128) + pos -> fp32 tokens [n_clips*12, 128] (models/heads.py:293-323)."""
+                    pos: Optional[torch.Tensor], mode: int) -> torch.Tensor:
+    """BN(eval) + 12 stacked Linear(512,128) + pos -> fp32 tokens [n_clips*12, 128] (models/heads.py:293-323); pos None: no add."""
     _cuda(emb, "emb")
     in_dim, emb_dim = w_cat.shape[1], w_cat.shape[0] // 12
     x = torch.empty((n_clips * 12, emb_dim), dtype=torch.float32, device=emb.device)
     ws = workspace(n_clips * in_dim * 4 + 256, emb.device)
     g, b, mu, var = (_f32c(t) for t in bn)
     check(_lib.lib().avf_au_former_front_fwd(mode, _ptr(emb), ld_emb, _ptr(g), _ptr(b), _ptr(mu), _ptr(var), _ptr(w_cat), _ptr(b_cat),
-                                             _ptr(_f32c(pos)), _ptr(x), n_clips, in_dim, emb_dim, _ptr(ws), ws.numel(), _stream()),
+                                             _ptr(None if pos is None else _f32c(pos)), _ptr(x), n_clips, in_dim, emb_dim, _ptr(ws), ws.numel(), _stream()),
           "au_former_front_fwd")
     return x
 
 
 def token_front(emb: torch.Tensor, ld_emb: int, n_clips: int, n_tok: int, bn: Sequence[torch.Tensor], w_cat: torch.Tensor, b_cat: torch.Tensor,
-                pos: torch.Tensor, mode: int) -> torch.Tensor:
-    """au_former_front for any token count: BN(eval) + n_tok stacked Linear + pos -> fp32 tokens [n_clips*n_tok, emb_dim]
+                pos: Optional[torch.Tensor], mode: int) -> torch.Tensor:
+    """au_former_front for any token count: BN(eval) + n_tok stacked Linear + pos (if given) -> fp32 tokens [n_clips*n_tok, emb_dim]
     (n_tok = 2: VA_former, models/heads.py:354-364)."""
     _cuda(emb, "emb")
     in_dim, emb_dim = w_cat.shape[1], w_cat.shape[0] // n_tok
@@ -269,7 +291,7 @@ def token_front(emb: torch.Tensor, ld_emb: int, n_clips: int, n_tok: int, bn: Se
     ws = workspace(n_clips * in_dim * 4 + 256, emb.device)
     g, b, mu, var = (_f32c(t) for t in bn)
     check(_lib.lib().avf_token_front_fwd(mode, _ptr(emb), ld_emb, _ptr(g), _ptr(b), _ptr(mu), _ptr(var), _ptr(w_cat), _ptr(b_cat),
-                                         _ptr(_f32c(pos)), _ptr(x), n_clips, in_dim, emb_dim, n_tok, _ptr(ws), ws.numel(), _stream()),
+                                         _ptr(None if pos is None else _f32c(pos)), _ptr(x), n_clips, in_dim, emb_dim, n_tok, _ptr(ws), ws.numel(), _stream()),
           "token_front_fwd")
     return x
 
@@ -309,8 +331,14 @@ def device_info() -> Dict[str, int]:
 
 
 def set_fused_enabled(enabled: bool) -> bool:
-    """Toggle the one-kernel-per-stack tcgen05 path (dim 256 / 8x32 stacks); returns the previous setting."""
+    """Toggle the one-kernel-per-stack tcgen05 path (dim 256 / 128, 8x32 stacks); returns the previous setting."""
     return bool(_lib.lib().avf_set_fused_enabled(1 if enabled else 0))
+
+
+def set_fused_small_enabled(enabled: bool) -> bool:
+    """Developer A/B (also AVF_FUSED_SMALL=0): False runs dim-128 stacks kernel per operation and keeps the positional adds and AU
+    logits of token_stack_fwd_ in their own kernels; returns the previous setting."""
+    return bool(_lib.lib().avf_set_fused_small_enabled(1 if enabled else 0))
 
 
 def encoder_fused_supported(shape: StackShape, precision="bf16") -> bool:

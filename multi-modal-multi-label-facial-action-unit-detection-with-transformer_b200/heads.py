@@ -72,7 +72,8 @@ class AU_former(nn.Module):
         """BN -> 12 projections -> + pos -> 2 encoder layers.  ``emb`` may be a strided view (row stride
         ld_emb): the cls rows of a TFormer token matrix are consumed in place.  The last layer's result goes
         to ``out`` (row stride ld_out) when given — that is how the audio and video halves of the
-        [B,12,256] fusion input get written side by side without a cat (models/avformer.py:100)."""
+        [B,12,256] fusion input get written side by side without a cat (models/avformer.py:100).  With
+        BatchNorm in eval() the positional add is part of the encoder-stack launch."""
         f = self._packed_front()
         bn = self.AU_BN1
         if bn.training:
@@ -81,10 +82,9 @@ class AU_former(nn.Module):
             x, _ = AF.au_former_front_train(view, n_clips, bn.weight, bn.bias, bn.running_mean, bn.running_var, True,
                                             0.1 if bn.momentum is None else bn.momentum, f.w, f.b, self.pos_embedding[0], f.mode)
             bn.num_batches_tracked += 1
-        else:
-            x = AF.au_former_front(emb, ld_emb, n_clips, (bn.weight, bn.bias, bn.running_mean, bn.running_var), f.w, f.b,
-                                   self.pos_embedding[0], f.mode)
-        return self.corr_transformer.forward_(x, n_clips, 12, out, ld_out)
+            return self.corr_transformer.forward_(x, n_clips, 12, out, ld_out)
+        x = AF.au_former_front(emb, ld_emb, n_clips, (bn.weight, bn.bias, bn.running_mean, bn.running_var), f.w, f.b, None, f.mode)
+        return self.corr_transformer.forward_(x, n_clips, 12, out, ld_out, pos=self.pos_embedding[0])
 
     def front_params(self):
         return [p for i in range(1, 13) for p in (getattr(self, f"AU_linear_p{i}").weight, getattr(self, f"AU_linear_p{i}").bias)]
@@ -126,10 +126,13 @@ class former_AU_head(nn.Module):
         return self._last
 
     def logits21_(self, tokens2d: torch.Tensor, n_clips: int, want_decisions: bool = False):
-        """In place on fp32 tokens [n_clips*12, emb_dim]: + pos, 3 layers, 12 dots -> [B,21] zero-padded."""
-        AF.add_row_periodic_(tokens2d, self.pos_embedding[0], 12)
-        self.corr_transformer.forward_(tokens2d, n_clips, 12)
-        return AF.au_logits(tokens2d, self._packed_last().w, n_clips, want_decisions)
+        """On fp32 tokens [n_clips*12, emb_dim] (used as scratch): + pos, 3 layers, 12 dots -> [B,21] zero-padded."""
+        t = self.corr_transformer
+        if t.training and t.dropout > 0.0:          # dropout: the tape-keeping kernels of forward_
+            t.forward_(tokens2d, n_clips, 12, pos=self.pos_embedding[0])
+            return AF.au_logits(tokens2d, self._packed_last().w, n_clips, want_decisions)
+        return AF.token_stack_fwd_(tokens2d, t.packed(), t.shape(n_clips, 12), self.pos_embedding[0], w_last=self._packed_last().w,
+                                   want_decisions=want_decisions)
 
     def last_params(self):
         return [getattr(self, f"AU_linear_last{i}").weight for i in range(1, 13)]
@@ -185,8 +188,8 @@ class VA_former(nn.Module):
         emb = emb.detach().float().contiguous()
         f = self._packed_front()
         bn = self.VA_BN1
-        x = AF.token_front(emb, emb.shape[1], bs, 2, (bn.weight, bn.bias, bn.running_mean, bn.running_var), f.w, f.b, self.pos_embedding[0], f.mode)
-        tok = self.corr_transformer.forward_(x, bs, 2).view(bs, 2, -1)
+        x = AF.token_front(emb, emb.shape[1], bs, 2, (bn.weight, bn.bias, bn.running_mean, bn.running_var), f.w, f.b, None, f.mode)
+        tok = self.corr_transformer.forward_(x, bs, 2, pos=self.pos_embedding[0]).view(bs, 2, -1)
         w = torch.stack([self.VA_linear_last1.weight[0], self.VA_linear_last2.weight[0]]).float()       # [2, emb]
         va_out = (tok * w.unsqueeze(0)).sum(-1)      # two 128-wide dots per clip: output glue, not a kernel of the path
         return va_out, tok
