@@ -84,10 +84,6 @@ int         avf_device_info(int32_t* sm_count, int32_t* cc, int32_t* has_tcgen05
  * tcgen05 kernel per stack in mode AVF_BF16 (residual stream in TMEM, see csrc/avf_layer_fused.cu).  avf_set_fused_enabled(0) forces
  * the kernel-per-operation path instead (used by the A/B parity tests); returns the previous setting. */
 int         avf_set_fused_enabled(int enabled);
-/* 0: dim-128 stacks run kernel per operation, and avf_token_stack_fwd runs its separate positional-add and AU-logit kernels
- * (the launch sequence before they were folded into the fused kernel; developer A/B, also AVF_FUSED_SMALL=0 in the Python
- * package).  Returns the previous setting. */
-int         avf_set_fused_small_enabled(int enabled);
 int         avf_encoder_fused_supported(const avf_stack_shape* s, int mode);
 /* Upper bound on the grid of the persistent kernels (fused encoder, tcgen05 GEMM) launched AFTER the call; 0 = all SMs.
  * Returns the previous value.  Lets a caller run two kernel chains side by side on disjoint SM sets (each persistent CTA

@@ -55,7 +55,6 @@ SIGNATURES = {
     "avf_launch_count": (ctypes.c_uint64, []),
     "avf_device_info": (ctypes.c_int, [ctypes.POINTER(_i32)] * 3),
     "avf_set_fused_enabled": (ctypes.c_int, [ctypes.c_int]),
-    "avf_set_fused_small_enabled": (ctypes.c_int, [ctypes.c_int]),
     "avf_encoder_fused_supported": (ctypes.c_int, [ctypes.POINTER(StackShape), ctypes.c_int]),
     "avf_debug_fused_prof": (ctypes.c_int, [ctypes.POINTER(ctypes.c_uint64), ctypes.c_int]),
     "avf_encoder_workspace_bytes": (_sz, [ctypes.POINTER(StackShape), ctypes.c_int]),
@@ -152,7 +151,7 @@ def build(force: bool = False, verbose: bool = False, out: str = "") -> str:
     nvcc = shutil.which("nvcc") or "/usr/local/cuda/bin/nvcc"
     if not os.path.exists(nvcc):
         raise RuntimeError("avformer_b200: nvcc not found and libavformer_b200.so is missing/stale; cannot build the CUDA path")
-    extra = os.environ.get("AVF_NVCC_EXTRA", "").split()          # e.g. -DAVF_FUSED_PROF -DAVF_FUSED_NSPLIT=4 (developer builds)
+    extra = os.environ.get("AVF_NVCC_EXTRA", "").split()          # e.g. -DAVF_FUSED_PROF (developer builds)
     cmd = [nvcc] + NVCC_FLAGS + extra + (["-Xptxas", "-v"] if verbose else []) + ["-o", out or LIB_PATH] + sources()
     res = subprocess.run(cmd, capture_output=True, text=True)
     if res.returncode != 0:
@@ -183,8 +182,6 @@ def lib() -> ctypes.CDLL:
                 fn.restype, fn.argtypes = res, args
             if os.environ.get("AVF_PDL", "") in ("0", "off"):
                 handle.avf_set_pdl_enabled(0)
-            if os.environ.get("AVF_FUSED_SMALL", "") in ("0", "off"):
-                handle.avf_set_fused_small_enabled(0)
             if handle.avf_abi_version() != 1:
                 raise RuntimeError("avformer_b200: ABI version mismatch")
             _lib = handle

@@ -17,7 +17,6 @@ bool pdl_enabled() { return g_pdl.load() != 0; }
 static std::atomic<int> g_sm_cap{0};     // avf_set_sm_cap
 int sm_cap() { return g_sm_cap.load(); }
 static std::atomic<int> g_fused{1};      // avf_set_fused_enabled: 0 forces the kernel-per-op path (A/B tests)
-static std::atomic<int> g_fused_small{1};  // avf_set_fused_small_enabled: 0 keeps dim-128 stacks, positional adds and AU logits out of the fused kernel
 
 void count_launch() { g_launches.fetch_add(1, std::memory_order_relaxed); }
 
@@ -110,7 +109,7 @@ int linear(int mode, const void* a, int lda, const void* w, const float* bias, c
 
 // Does a stack of fp32 token rows run as one fused kernel?
 static bool fused_rows(int mode, const avf_stack_shape* s, int ld_x, const float* out, int ld_out) {
-  return mode == AVF_BF16 && g_fused.load() && tcgen05_ok() && encoder_fused_supported(s) && (s->dim == 256 || g_fused_small.load()) &&
+  return mode == AVF_BF16 && g_fused.load() && tcgen05_ok() && encoder_fused_supported(s) &&
          ld_x % 4 == 0 && (out == nullptr || ld_out % 4 == 0);
 }
 
@@ -160,14 +159,12 @@ int avf_set_fused_enabled(int enabled) {
   return old;
 }
 
-int avf_set_fused_small_enabled(int enabled) { return g_fused_small.exchange(enabled ? 1 : 0); }
-
 int avf_set_pdl_enabled(int enabled) { return g_pdl.exchange(enabled ? 1 : 0); }
 
 int avf_set_sm_cap(int cap) { return g_sm_cap.exchange(cap > 0 ? cap : 0); }
 
 int avf_encoder_fused_supported(const avf_stack_shape* s, int mode) {
-  return (s != nullptr && mode == AVF_BF16 && s->n_seq > 0 && encoder_fused_supported(s) && (s->dim == 256 || g_fused_small.load())) ? 1 : 0;
+  return (s != nullptr && mode == AVF_BF16 && s->n_seq > 0 && encoder_fused_supported(s)) ? 1 : 0;
 }
 
 /* Debug: per-phase cycle counters of the fused encoder kernel (library built with -DAVF_FUSED_PROF); else AVF_EUNSUPPORTED. */
@@ -218,7 +215,7 @@ int avf_token_stack_fwd(int mode, const avf_stack_shape* s, const avf_layer_weig
   AVF_REQUIRE(w_last == nullptr || (s->n_tok == 12 && out21 != nullptr), AVF_EINVAL, "token_stack: AU logits need 12 tokens per clip and out21 (n_tok=%d)",
               s->n_tok);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (g_fused_small.load() && fused_rows(mode, s, ld_x, out, ld_out))      // positional add, stack and AU logits in one launch
+  if (fused_rows(mode, s, ld_x, out, ld_out))      // positional add, stack and AU logits in one launch
     return encoder_fused(1, s, layers, x, ld_x, (out || w_last) ? out : x, out ? ld_out : ld_x, pos, nullptr, w_last, out21, decisions, st);
   if (pos != nullptr && (e = add_row_periodic(x, ld_x, pos, s->n_seq * s->n_tok, s->dim, s->n_tok, st))) return e;
   if ((e = encoder_stack(mode, s, layers, x, ld_x, out, ld_out, workspace, workspace_bytes, st))) return e;

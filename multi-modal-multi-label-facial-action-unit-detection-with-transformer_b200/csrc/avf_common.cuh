@@ -212,23 +212,17 @@ __device__ __forceinline__ bool mbar_test_wait(uint64_t* bar, uint32_t parity) {
 }
 // The same with a suspend-time hint (ns): the thread sleeps in hardware until the phase completes or the hint expires, so a
 // waiting warp issues (almost) no instructions and leaves its scheduler's issue slots to the warps that have work.
-#ifndef AVF_SPIN_HINT_NS
-#define AVF_SPIN_HINT_NS 20000
-#endif
+constexpr uint32_t SPIN_HINT_NS = 20000;
 __device__ __forceinline__ bool mbar_try_wait_sleep(uint64_t* bar, uint32_t parity) {
-#if AVF_SPIN_HINT_NS > 0
   uint32_t ok;
   asm volatile(
       "{\n\t.reg .pred P;\n\t"
       "mbarrier.try_wait.parity.shared::cta.b64 P, [%1], %2, %3;\n\t"
       "selp.u32 %0, 1, 0, P;\n\t}\n"
       : "=r"(ok)
-      : "r"(smem_u32(bar)), "r"(parity), "r"(uint32_t(AVF_SPIN_HINT_NS))
+      : "r"(smem_u32(bar)), "r"(parity), "r"(SPIN_HINT_NS)
       : "memory");
   return ok != 0;
-#else
-  return mbar_try_wait(bar, parity);
-#endif
 }
 // Bounded wait: a protocol bug traps (-> a CUDA error the host reports) instead of hanging the GPU.  The spin loop
 // lives out of line so that the many wait sites of the fused kernels stay small.

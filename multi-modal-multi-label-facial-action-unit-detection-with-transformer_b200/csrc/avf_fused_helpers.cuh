@@ -1,4 +1,4 @@
-// Device helpers shared by the fused encoder kernels (avf_layer_fused.cu, avf_sformer_fused.cu): packed bf16x2 arithmetic,
+// Device helpers of the fused encoder kernel (avf_layer_fused.cu): packed bf16x2 arithmetic,
 // narrow TMEM load / store shapes, bulk stores, operand packing and the optional per-phase cycle counters.
 #pragma once
 #include "avf_common.cuh"
@@ -40,28 +40,9 @@ struct Prof {
 #endif
 
 __device__ __forceinline__ void bar_sync(int id, int count) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(count) : "memory"); }
-__device__ __forceinline__ float fast_exp2(float x) {
-  float y;
-  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
-  return y;
-}
-__device__ __forceinline__ float fast_tanh(float x) {
-  float y;
-  asm("tanh.approx.f32 %0, %1;" : "=f"(y) : "f"(x));
-  return y;
-}
-// tanh-GELU (models/heads.py:164-166) as 0.5x(1+tanh(x(c0 + c1 x^2))): 6 instructions per element
-__device__ __forceinline__ float gelu_fast(float x) {
-  const float u = x * fmaf(x * x, 0.7978845608028654f * 0.044715f, 0.7978845608028654f);
-  const float hx = 0.5f * x;
-  return fmaf(hx, fast_tanh(u), hx);
-}
-// Packed bf16x2 arithmetic for the two MUFU-heavy epilogues (softmax exponentials, tanh-GELU).  Their results are rounded to
-// bf16 anyway (P and gelu(h) are tensor-core operands), so evaluating the transcendental on a bf16 pair halves the MUFU work
-// (16 results / clk / SM -> 32) and the surrounding multiply-adds.  -DAVF_FUSED_PACKED=0 restores the fp32 evaluation.
-#ifndef AVF_FUSED_PACKED
-#define AVF_FUSED_PACKED 1
-#endif
+// Packed bf16x2 arithmetic for the two MUFU-heavy epilogues (softmax exponentials, tanh-GELU, models/heads.py:164-166).  Their
+// results are rounded to bf16 anyway (P and gelu(h) are tensor-core operands), so evaluating the transcendental on a bf16 pair
+// halves the MUFU work (16 results / clk / SM -> 32) and the surrounding multiply-adds.
 __device__ __forceinline__ uint32_t cvt_bf16x2(float lo, float hi) {
   uint32_t r;
   asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(hi), "f"(lo));
@@ -101,10 +82,6 @@ __device__ __forceinline__ uint32_t gelu_bf16x2(uint32_t x) {
 // row workers are bound by the issue rate of their fp32 sweeps (LayerNorm statistics / normalisation, bias and positional adds,
 // softmax scaling), so halving the instruction count of those loops is worth more than any reordering.  A pair lives in a 64-bit
 // register; consecutive TMEM columns land in consecutive registers, so building a pair from two of them costs nothing.
-// -DAVF_F32X2=0 restores the scalar forms.
-#ifndef AVF_F32X2
-#define AVF_F32X2 1
-#endif
 __device__ __forceinline__ uint64_t f2_pack(float lo, float hi) {
   uint64_t r;
   asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(lo), "f"(hi));
@@ -112,37 +89,19 @@ __device__ __forceinline__ uint64_t f2_pack(float lo, float hi) {
 }
 __device__ __forceinline__ void f2_unpack(uint64_t v, float& lo, float& hi) { asm("mov.b64 {%0, %1}, %2;" : "=f"(lo), "=f"(hi) : "l"(v)); }
 __device__ __forceinline__ uint64_t f2_add(uint64_t a, uint64_t b) {
-#if AVF_F32X2
   uint64_t r;
   asm("add.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b));
   return r;
-#else
-  float al, ah, bl, bh;
-  f2_unpack(a, al, ah); f2_unpack(b, bl, bh);
-  return f2_pack(al + bl, ah + bh);
-#endif
 }
 __device__ __forceinline__ uint64_t f2_mul(uint64_t a, uint64_t b) {
-#if AVF_F32X2
   uint64_t r;
   asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b));
   return r;
-#else
-  float al, ah, bl, bh;
-  f2_unpack(a, al, ah); f2_unpack(b, bl, bh);
-  return f2_pack(al * bl, ah * bh);
-#endif
 }
 __device__ __forceinline__ uint64_t f2_fma(uint64_t a, uint64_t b, uint64_t c) {
-#if AVF_F32X2
   uint64_t r;
   asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(r) : "l"(a), "l"(b), "l"(c));
   return r;
-#else
-  float al, ah, bl, bh, cl, ch;
-  f2_unpack(a, al, ah); f2_unpack(b, bl, bh); f2_unpack(c, cl, ch);
-  return f2_pack(fmaf(al, bl, cl), fmaf(ah, bh, ch));
-#endif
 }
 __device__ __forceinline__ uint32_t cvt_bf16x2_pair(uint64_t v) {      // (lo, hi) fp32 pair -> packed bf16 pair, round to nearest even
   float lo, hi;
@@ -198,14 +157,6 @@ __device__ __forceinline__ void bulk_wait_all0() { asm volatile("cp.async.bulk.w
 
 __device__ __forceinline__ uint64_t desc_sw64(uint32_t addr) { return make_desc(addr, 16, 512, 4); }
 
-__device__ __forceinline__ uint4 pack8(const float* x) {
-  uint4 pk;
-  pk.x = pack_bf16x2(x[0], x[1]);
-  pk.y = pack_bf16x2(x[2], x[3]);
-  pk.z = pack_bf16x2(x[4], x[5]);
-  pk.w = pack_bf16x2(x[6], x[7]);
-  return pk;
-}
 __device__ __forceinline__ uint4 pack8u(const uint32_t* r) {
   uint4 pk;
   pk.x = pack_bf16x2(__uint_as_float(r[0]), __uint_as_float(r[1]));

@@ -22,7 +22,6 @@
 #include <unordered_map>
 
 #include <algorithm>
-#include <cstdlib>
 #include <mutex>
 
 #include "avf_common.cuh"
@@ -573,10 +572,6 @@ int gemm_umma(int trans_a, int trans_b, const void* a, int lda, const void* w, i
   if (n % 256 == 0 && m_tiles * (n / 256) * 5 >= (c_mode == AVF_BF16 ? 4 : 10) * sms) bn = 256;
   else if (n % 128 == 0 && m_tiles * (n / 128) >= sms) bn = 128;
   else if (n % 128 == 0 && n / 128 * m_tiles >= sms / 2 && n >= 512) bn = 128;
-  {   // developer override for tile-shape experiments: AVF_GEMM_BN=64|128|256 (ignored when N is not a multiple of it)
-    static const int forced = [] { const char* e = getenv("AVF_GEMM_BN"); return e ? atoi(e) : 0; }();
-    if (forced > 0 && n % forced == 0) bn = forced;
-  }
 #define AVF_GEMM(BN_, ST_, BMN_)                                                                                                   \
   if (bn == BN_ && bool(trans_b) == BMN_) {                                                                                        \
     if (c_mode == AVF_BF16)                                                                                                        \

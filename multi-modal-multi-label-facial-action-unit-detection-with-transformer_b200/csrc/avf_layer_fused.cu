@@ -28,7 +28,6 @@
 // (one thread), 2 = TMA producer of the QKV ring, 3.. = row workers (warp w owns TMEM lanes 32*(w%4)..+31; the NSPLIT warps
 // of a lane quarter split the columns).
 #include <cuda.h>
-#include <stdlib.h>
 
 #include "avf_common.cuh"
 #include "avf_fused_helpers.cuh"
@@ -41,44 +40,22 @@ int make_tmap_bf16_2d(CUtensorMap* tm, const void* ptr, uint64_t rows, uint64_t 
 namespace {
 using namespace fused;
 
-// How the weight producer waits (it serves two things at once: ring slots and the next tile's input frames):
-// 0 = mbarrier.try_wait on both (each probe may suspend the thread for the hardware's time limit), 1 = non-blocking test_wait on
-// both (pure spin), 2 = try_wait on the ring slot, test_wait on the input-buffer probe.
-#ifndef AVF_PROD_POLL
-#define AVF_PROD_POLL 2
-#endif
-#ifndef AVF_PROD_FASTPATH
-#define AVF_PROD_FASTPATH 1
-#endif
-// 1: the normalised attention output O_h / l stays in TMEM (packed bf16 over its own accumulator columns) as the A operand of the
-// out-projection; 0: staged through shared memory (8 KB, needs a proxy fence per head)
-#ifndef AVF_O_TMEM
-#define AVF_O_TMEM 1
-#endif
-
 // DIM: the widest model (256) — the layouts below are sized for it — and the only width of the NCHW form.  Kernels take the
 // model width as the template parameter D (256 or 128).
 constexpr int DIM = 256, HEADS = 8, DH = 32;
 constexpr int MAX_DEPTH = 3, MAX_MLP = 1024;
-#ifndef AVF_FUSED_NSPLIT
-#define AVF_FUSED_NSPLIT 2
-#endif
-constexpr int NSPLIT = AVF_FUSED_NSPLIT;   // threads per token row (each owns D / NSPLIT columns of the residual stream)
-static_assert(NSPLIT == 2, "two threads per token row (the packed softmax exchanges a pair)");
+constexpr int NSPLIT = 2;                  // threads per token row (each owns D / NSPLIT columns of the residual stream)
 constexpr int WORKER_T0 = 96;              // first worker thread
 constexpr int NUM_WORKERS = 128 * NSPLIT;
 constexpr int NUM_THREADS = WORKER_T0 + NUM_WORKERS;
 // Main weight ring, 16 KB slots laid out contiguously from OFF_Q.  Slots 2-3 are free in every phase (out-projection slices
-// rotate over them); the MLP weights rotate over all nine: slots 0-1 alias the Q/K/V staging and slots 4-8 the O staging + QKV
-// ring, all idle in the MLP phase — 144 KB in flight cover the L2 latency at the MLP's consumption rate (16 KB per 256 tensor cycles).
+// rotate over them); the MLP weights rotate over all nine: slots 0-1 alias the Q/K/V staging and slots 4-8 the QKV ring (plus the
+// 8 KB behind it), all idle in the MLP phase — 144 KB in flight cover the L2 latency at the MLP's consumption rate (16 KB per 256 tensor cycles).
 constexpr int RING = 9, RING_LO = 2, RING_HI = 4, SLOT_BYTES = 16384;
 // QKV ring: one slot = one 64-wide K panel of [Wq_h; Wk_h; Wv_h] (3 x 32 rows x 128 B); six slots = one and a half heads in
 // flight.  With four (one head) every QKV_{h+1} waited ~400 cycles for its first panels, and the chain E1_h -> QKV_{h+1} -> E1_{h+1}
 // (D1 is single-buffered in TMEM) is what paces the attention phase.
-#ifndef AVF_QRING
-#define AVF_QRING 6
-#endif
-constexpr int QRING = AVF_QRING, QSLOT_BYTES = 12288;
+constexpr int QRING = 6, QSLOT_BYTES = 12288;
 // K panels per head in the QKV ring (= K panels of A0) at model width D
 template <int D> constexpr int KPH = D / 64;
 // "Head full" barriers of the QKV ring: head hq signals barrier hq % NQG, whose phase (hq / NQG) & 1 the MMA thread waits for.
@@ -91,12 +68,8 @@ template <int D> constexpr int NQG = (QRING + KPH<D> - 1) / KPH<D>;
 constexpr int MAX_QG = NQG<128>;
 static_assert(KPH<256> * (NQG<256> - 1) < QRING && QRING <= KPH<256> * NQG<256>, "head-full barrier parity (D = 256)");
 static_assert(KPH<128> * (NQG<128> - 1) < QRING && QRING <= KPH<128> * NQG<128>, "head-full barrier parity (D = 128)");
-// MLP weight slots per "group full" barrier: 4 = one barrier per GEMM, 2 = one per half GEMM (the first MMAs start one slot pair earlier)
-#ifndef AVF_MLP_GROUP
-#define AVF_MLP_GROUP 4
-#endif
-constexpr int MLPG = AVF_MLP_GROUP;
-static_assert(MLPG == 2 || MLPG == 4, "MLP group size");
+// MLP weight slots per "group full" barrier: one barrier per GEMM (four slots at D = 256)
+constexpr int MLPG = 4;
 // At D = 128 an MLP GEMM (FF1: K = D, FF2: N = D) is two 16 KB slots: one group per GEMM
 template <int D> constexpr int GSLOTS = MLPG < D / 64 ? MLPG : D / 64;
 
@@ -106,11 +79,9 @@ constexpr int OFF_Q = 65536;                       // 8 KB   Q_h [128 x 32] K-ma
 constexpr int OFF_K = OFF_Q + 8192;                // 8 KB   K_h
 constexpr int OFF_V = OFF_K + 8192;                // 2x8 KB V_h [128 tok x 32] MN-major SW64, double buffered
 constexpr int OFF_RING = OFF_V + 16384;            // 2 x 16 KB weight ring (slots 2-3; slots 0-1 = the 32 KB of Q/K/V staging above)
-constexpr int OFF_OST = OFF_RING + (RING_HI - RING_LO) * SLOT_BYTES;   // 8 KB  O_h / l  [128 x 32] K-major SW64 (single: out-proj(h-1) is issued before PV(h))
-constexpr int OFF_QRING = OFF_OST + (AVF_O_TMEM ? 0 : 8192);   // QRING x 12 KB QKV weight ring (right behind slot 3 when O_h stays in TMEM); also the NCHW output staging (2 x 64 x 256 bf16 at most)
+constexpr int OFF_QRING = OFF_RING + 2 * SLOT_BYTES;   // QRING x 12 KB QKV weight ring, right behind slot 3; also the NCHW output staging (2 x 64 x 256 bf16 at most)
 constexpr int OFF_OUTST = OFF_QRING;
 static_assert(QRING * QSLOT_BYTES >= 2 * 64 * 256 * 2, "the NCHW output staging lives in the QKV ring");
-static_assert(QRING >= 6 && QRING < 8, "six or seven QKV sub-slots (one and a half heads in flight at D = 256; see NQG)");
 constexpr int QRING_END = OFF_QRING + QRING * QSLOT_BYTES;
 constexpr int OFF_XCH = QRING_END > OFF_Q + RING * SLOT_BYTES ? QRING_END : OFF_Q + RING * SLOT_BYTES;      // row exchange [2][128][4] floats
 static_assert(OFF_XCH - OFF_Q >= RING * SLOT_BYTES, "the nine MLP ring slots fit in [OFF_Q, OFF_XCH)");
@@ -126,12 +97,9 @@ static_assert(SMEM_ALLOC <= 232448, "shared memory budget");
 
 // K-panel order of the two GEMMs that read a fresh LayerNorm output (QKV, FF1).  The two threads of a row write panels {0,1} and {2,3}
 // of A0, so panels 0 and 2 are complete when every thread is half-way through its normalisation sweep (B_A0_HALF): the first GEMM behind
-// a LayerNorm starts on them and only then waits for the whole operand (B_A0_READY).  AVF_A0_HALF=0: plain order, one barrier.  At
-// D = 128 each thread writes ONE panel, both at the same time: plain order, one barrier.
-#ifndef AVF_A0_HALF
-#define AVF_A0_HALF 1
-#endif
-template <int D> constexpr bool A0_HALF = AVF_A0_HALF && D == 256;
+// a LayerNorm starts on them and only then waits for the whole operand (B_A0_READY).  At D = 128 each thread writes ONE panel,
+// both at the same time: plain order, one barrier.
+template <int D> constexpr bool A0_HALF = D == 256;
 template <int D>
 __device__ __forceinline__ constexpr int kpanel(int i) { return A0_HALF<D> ? (((i & 1) << 1) | (i >> 1)) : i; }      // 0, 2, 1, 3
 
@@ -217,26 +185,13 @@ struct Worker {
     bar_sync(1 + q, 32 * NSPLIT);
     return s + row * 4;
   }
-  // exchange of a PAIR of floats between the two threads of a row (one barrier): returns the partner's pair
-  __device__ __forceinline__ float2 exchange_pair(float a, float b) {
-    static_assert(NSPLIT == 2, "pair exchange is written for two threads per row");
-    float* s = reinterpret_cast<float*>(smem + OFF_XCH) + xslot * (128 * 4);
-    xslot ^= 1;
-    *reinterpret_cast<float2*>(s + row * 4 + g * 2) = make_float2(a, b);
-    bar_sync(1 + q, 32 * NSPLIT);
-    return *reinterpret_cast<const float2*>(s + row * 4 + (g ^ 1) * 2);
-  }
   __device__ __forceinline__ float exchange_sum(float mine) {
     const float* v = exchange(mine);
-    if constexpr (NSPLIT == 2) return v[0] + v[1];
-    const float4 f = *reinterpret_cast<const float4*>(v);
-    return (f.x + f.y) + (f.z + f.w);
+    return v[0] + v[1];
   }
   __device__ __forceinline__ float exchange_max(float mine) {
     const float* v = exchange(mine);
-    if constexpr (NSPLIT == 2) return fmaxf(v[0], v[1]);
-    const float4 f = *reinterpret_cast<const float4*>(v);
-    return fmaxf(fmaxf(f.x, f.y), fmaxf(f.z, f.w));
+    return fmaxf(v[0], v[1]);
   }
   __device__ __forceinline__ void arrive(int bar) {             // one arrive per warp, after every lane's fences
     fence_proxy_async_smem();
@@ -456,11 +411,7 @@ __device__ void worker_main(const FusedArgs& a, uint8_t* smem, uint64_t* bars, u
           // shared-memory reads of the staged frame overlap their L1/L2 round trip
           float4 p[8];
 #pragma unroll
-#ifdef AVF_EXP_POS_HOT      // timing experiment only (wrong results): every block reads the first block's positional values -> L1 hits
-          for (int j = 0; j < 8; ++j) p[j] = __ldg(ppt + j * POS_LD);
-#else
           for (int j = 0; j < 8; ++j) p[j] = __ldg(ppt + (c0 / 4 + j) * POS_LD);
-#endif
 #pragma unroll
           for (int j = 0; j < 8; ++j) {
             f2_unpack(f2_add(f2_pack(__bfloat162float(src16[(c0 + 4 * j) * n_tok]), __bfloat162float(src16[(c0 + 4 * j + 1) * n_tok])),
@@ -522,7 +473,7 @@ __device__ void worker_main(const FusedArgs& a, uint8_t* smem, uint64_t* bars, u
       w.normalize_from_tmem(mean, rstd, 0, V_BOUT);
       pf.mark(PW_LN1);
 
-      // ---- attention: per head  E1 (QKV -> smem), E3 of the previous head (O -> A1), E2 (softmax) -------------
+      // ---- attention: per head  E1 (QKV -> smem), E3 of the previous head (O / l -> TMEM), E2 (softmax) -------------
       float inv_l = 0.f;
 #pragma unroll 1
       for (int h = 0; h <= HEADS; ++h) {
@@ -533,13 +484,8 @@ __device__ void worker_main(const FusedArgs& a, uint8_t* smem, uint64_t* bars, u
           constexpr int NCH = 12 / NSPLIT;
           const uint32_t sw = uint32_t((row >> 1) & 3);
           uint32_t r[NCH * 8];
-          if constexpr (NSPLIT == 2) {
-            tmem_ld32(tl + TM_D1 + g * 48, reinterpret_cast<uint32_t(&)[32]>(r[0]));
-            tmem_ld16(tl + TM_D1 + g * 48 + 32, reinterpret_cast<uint32_t(&)[16]>(r[32]));
-          } else {
-            tmem_ld16(tl + TM_D1 + g * 24, reinterpret_cast<uint32_t(&)[16]>(r[0]));
-            tmem_ld8(tl + TM_D1 + g * 24 + 16, reinterpret_cast<uint32_t(&)[8]>(r[16]));
-          }
+          tmem_ld32(tl + TM_D1 + g * 48, reinterpret_cast<uint32_t(&)[32]>(r[0]));
+          tmem_ld16(tl + TM_D1 + g * 48 + 32, reinterpret_cast<uint32_t(&)[16]>(r[32]));
           tmem_ld_wait();
 #pragma unroll
           for (int c = 0; c < NCH; ++c) {
@@ -550,54 +496,35 @@ __device__ void worker_main(const FusedArgs& a, uint8_t* smem, uint64_t* bars, u
           w.arrive(B_STAGED);
           pf.mark(PW_E1);
         }
-        if (h > 0) {             // E3 of head h-1: O / l -> bf16 -> staging buffer (h-1)&1, columns [g*OW, +OW) (A operand of the per-head out-projection)
+        if (h > 0) {             // E3 of head h-1: O / l -> bf16 over its own TMEM columns (A operand of the per-head out-projection)
           mbar_wait(&bars[B_O_FULL], (h - 1) & 1);
           tc_fence_after();
           pf.mark(PW_WAIT_O);
-          constexpr int OW = DH / NSPLIT;                  // 16 or 8 columns
+          constexpr int OW = DH / NSPLIT;                  // 16 columns
           uint32_t r[OW];
-          if constexpr (OW == 16) tmem_ld16(tl + TM_O + g * OW, reinterpret_cast<uint32_t(&)[16]>(r[0]));
-          else tmem_ld8(tl + TM_O + g * OW, reinterpret_cast<uint32_t(&)[8]>(r[0]));
+          tmem_ld16(tl + TM_O + g * OW, reinterpret_cast<uint32_t(&)[16]>(r[0]));
           tmem_ld_wait();
-#if AVF_FUSED_PACKED
           {   // l = own + partner's partial row sum of head h-1 (written before their P_READY arrive, which PV -> O_FULL follows)
             const float* sums = reinterpret_cast<const float*>(smem + OFF_XCH) + ((h - 1) & 1) * (128 * 4) + row * 4 + 2;
             asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(inv_l) : "f"(sums[0] + sums[1]));
           }
-#endif
           const uint64_t inv2 = f2_pack(inv_l, inv_l);
-#if AVF_O_TMEM
           // O_h / l goes back INTO the accumulator's TMEM columns as packed bf16 (like P over S and gelu(H) over H): thread g turns its 16
           // fp32 columns [16g, 16g + 16) into 8 packed columns at [16g, 16g + 8) — columns only it reads — and the out-projection takes
           // its A operand from TMEM, one 16-wide k-step per thread.  No shared-memory staging, no generic->async proxy fence.
-          static_assert(OW == 16, "TMEM-resident O operand is written for two threads per row");
           uint32_t pk[8];
 #pragma unroll
           for (int j = 0; j < 8; ++j) pk[j] = cvt_bf16x2_pair(f2_mul(f2_pack(__uint_as_float(r[2 * j]), __uint_as_float(r[2 * j + 1])), inv2));
           tmem_st8(tl + TM_O + g * OW, pk);
           tmem_st_wait();
           w.arrive_tmem_only(B_O_DRAINED);
-#else
-          uint8_t* ob = smem + OFF_OST + row * 64;
-          const uint32_t sw = uint32_t((row >> 1) & 3);
-#pragma unroll
-          for (int c = 0; c < OW / 8; ++c) {
-            uint4 pk;
-            pk.x = cvt_bf16x2_pair(f2_mul(f2_pack(__uint_as_float(r[c * 8]), __uint_as_float(r[c * 8 + 1])), inv2));
-            pk.y = cvt_bf16x2_pair(f2_mul(f2_pack(__uint_as_float(r[c * 8 + 2]), __uint_as_float(r[c * 8 + 3])), inv2));
-            pk.z = cvt_bf16x2_pair(f2_mul(f2_pack(__uint_as_float(r[c * 8 + 4]), __uint_as_float(r[c * 8 + 5])), inv2));
-            pk.w = cvt_bf16x2_pair(f2_mul(f2_pack(__uint_as_float(r[c * 8 + 6]), __uint_as_float(r[c * 8 + 7])), inv2));
-            *reinterpret_cast<uint4*>(ob + ((uint32_t(g * (OW / 8) + c) ^ sw) << 4)) = pk;
-          }
-          w.arrive(B_O_DRAINED);
-#endif
           pf.mark(PW_E3);
         }
         if (h < HEADS) {         // E2: softmax of this row over its own sequence's columns, P (bf16) over the S columns
           mbar_wait(&bars[B_S_FULL], h & 1);
           tc_fence_after();
           pf.mark(PW_WAIT_S);
-          if constexpr (NTOK > 32 && NSPLIT == 2 && AVF_FUSED_PACKED) {
+          if constexpr (NTOK > 32) {
             // 64-row slots, compile-time window: the row's chunks are [8 seq, 8 seq + NCH_ALL), thread 0 takes the first four, thread 1 the rest
             constexpr int NCH_ALL = (NTOK + 7) / 8, NC1 = NCH_ALL - 4, TAILV = NTOK & 7;
             static_assert(NC1 >= 1 && NC1 <= 4, "softmax split");
@@ -622,9 +549,6 @@ __device__ void worker_main(const FusedArgs& a, uint8_t* smem, uint64_t* bars, u
             if (c < my_nc) tmem_ld8(tl + TM_S + (my_c0 + c) * 8, reinterpret_cast<uint32_t(&)[8]>(s[c]));
           tmem_ld_wait();
           pf.mark(PW_E2_LD);
-          // one exchange per head: every thread exponentiates against the maximum of ITS columns first, the two threads of the
-          // row then swap (max, sum) and rescale by 2^(own max - row max) — the swap also orders every S load of the row
-          // before any P store (P is written over the S columns)
           float mloc = -INFINITY;
 #pragma unroll
           for (int c = 0; c < MAXC; ++c) {
@@ -637,7 +561,6 @@ __device__ void worker_main(const FusedArgs& a, uint8_t* smem, uint64_t* bars, u
               mloc = fmaxf(mloc, fmaxf(fmaxf(fmaxf(s[c][0], s[c][1]), fmaxf(s[c][2], s[c][3])), fmaxf(fmaxf(s[c][4], s[c][5]), fmaxf(s[c][6], s[c][7]))));
             }
           }
-#if AVF_FUSED_PACKED
           // the row maximum first (one exchange; it also orders every S load of the row before any P store — P is written over
           // the S columns), then 2^(s - max) straight to its final bf16 value, two per MUFU instruction; the partial row sums
           // (fp32, of the rounded values the MMA will see) meet again in E3 through shared memory, no second barrier
@@ -659,30 +582,6 @@ __device__ void worker_main(const FusedArgs& a, uint8_t* smem, uint64_t* bars, u
             }
           }
           reinterpret_cast<float*>(smem + OFF_XCH)[(h & 1) * (128 * 4) + row * 4 + 2 + g] = sum_g;
-#else
-          const float nml = mloc == -INFINITY ? 0.f : -mloc * sm_scale;      // a thread without valid columns contributes zeros
-          float sum_g = 0.f;
-#pragma unroll
-          for (int c = 0; c < MAXC; ++c) {
-            if (c < my_nc) {
-#pragma unroll
-              for (int j = 0; j < 8; ++j) s[c][j] = fast_exp2(fmaf(s[c][j], sm_scale, nml));
-              sum_g += ((s[c][0] + s[c][1]) + (s[c][2] + s[c][3])) + ((s[c][4] + s[c][5]) + (s[c][6] + s[c][7]));
-            }
-          }
-          pf.mark(PW_E2_EXP);
-          const float2 other = w.exchange_pair(mloc, sum_g);
-          pf.mark(PW_E2_XCH);
-          const float mrow = fmaxf(mloc, other.x);
-          const float f = fast_exp2((mloc - mrow) * sm_scale), fo = fast_exp2((other.x - mrow) * sm_scale);    // 2^(-inf) = 0
-          inv_l = 1.f / fmaf(sum_g, f, other.y * fo);
-#pragma unroll
-          for (int c = 0; c < MAXC; ++c) {
-            if (c < my_nc)
-              tmem_st4(tl + TM_S + (my_c0 + c) * 4, pack_bf16x2(s[c][0] * f, s[c][1] * f), pack_bf16x2(s[c][2] * f, s[c][3] * f),
-                       pack_bf16x2(s[c][4] * f, s[c][5] * f), pack_bf16x2(s[c][6] * f, s[c][7] * f));
-          }
-#endif
           // P columns the MMA reads (all 128) but this warp's rows never use: zeros; thread g takes TMEM columns [32g, 32g + 32)
           {
             const int z_lo = g * 32, z_hi = z_lo + 32, w_lo = c_lo * 4, w_hi = c_hi * 4;
@@ -728,13 +627,8 @@ __device__ void worker_main(const FusedArgs& a, uint8_t* smem, uint64_t* bars, u
 #pragma unroll
           for (int j = 0; j < 32; j += 4) {
             const float4 b4 = *reinterpret_cast<const float4*>(bias + j);
-#if AVF_FUSED_PACKED
             yk[j / 2] = gelu_bf16x2(cvt_bf16x2_pair(f2_add(f2_pack(__uint_as_float(r[j]), __uint_as_float(r[j + 1])), f2_pack(b4.x, b4.y))));
             yk[j / 2 + 1] = gelu_bf16x2(cvt_bf16x2_pair(f2_add(f2_pack(__uint_as_float(r[j + 2]), __uint_as_float(r[j + 3])), f2_pack(b4.z, b4.w))));
-#else
-            yk[j / 2] = pack_bf16x2(gelu_fast(__uint_as_float(r[j]) + b4.x), gelu_fast(__uint_as_float(r[j + 1]) + b4.y));
-            yk[j / 2 + 1] = pack_bf16x2(gelu_fast(__uint_as_float(r[j + 2]) + b4.z), gelu_fast(__uint_as_float(r[j + 3]) + b4.w));
-#endif
           }
           tmem_st16(hbase + c0 / 2, yk);
         }
@@ -827,11 +721,7 @@ __device__ void producer_main(const FusedArgs& a, uint8_t* smem, uint64_t* bars)
   auto poll_loader = [&]() {
     if (IO != IO_NCHW_BF16 || load_tile < 0) return;
     if (need_free) {
-#if AVF_PROD_POLL >= 1
       if (!mbar_test_wait(&bars[B_A0_FREE], n_free & 1)) return;     // a probe that never suspends: this thread has weight slots to serve
-#else
-      if (!mbar_try_wait(&bars[B_A0_FREE], n_free & 1)) return;
-#endif
       ++n_free;
     }
     const int seqs_here = min(a.spt, a.n_seq - load_tile * a.spt);
@@ -845,18 +735,12 @@ __device__ void producer_main(const FusedArgs& a, uint8_t* smem, uint64_t* bars)
   // slots 2-4, the MLP weights over all five — slots 0-1 alias the Q/K/V staging and are only loaded after the attention MMAs).
   uint32_t pbits = 0, n_gate = 0;
   auto poll_wait = [&](uint64_t* bar, uint32_t parity) {
-#if AVF_PROD_FASTPATH
     // Fast path first: in the MLP phase this thread issues a 16 KB slot per ~250 tensor cycles, and every probe (of the slot's
     // barrier or of the input buffer's) costs it ~100 cycles.  The input loader is polled only while the slot is not free yet.
     if (mbar_try_wait(bar, parity)) return;
-#endif
     poll_loader();
     const long long t0 = clock64();
-#if AVF_PROD_POLL == 1
-    while (!mbar_test_wait(bar, parity)) {
-#else
     while (!mbar_try_wait(bar, parity)) {
-#endif
       poll_loader();
       if (clock64() - t0 > 4000000000LL) {
         unsigned* tb = g_trap_buffer;
@@ -937,7 +821,7 @@ __device__ void producer_main(const FusedArgs& a, uint8_t* smem, uint64_t* bars)
 }
 
 // ---------------------------------------------------------------------------------------------
-// QKV weight producer (one thread of its own warp): the 4 x 12 KB ring inside A1
+// QKV weight producer (one thread of its own warp): the QRING x 12 KB ring inside A1
 // ---------------------------------------------------------------------------------------------
 template <int IO, int D>
 __device__ void qkv_producer_main(const FusedArgs& a, uint8_t* smem, uint64_t* bars) {
@@ -977,7 +861,7 @@ __device__ void mma_main(const FusedArgs& a, uint8_t* smem, uint64_t* bars, uint
   const bool leader = elect_one();
   const uint32_t a0 = smem_u32(smem + OFF_A0);
   const uint32_t qs = smem_u32(smem + OFF_Q), ks = smem_u32(smem + OFF_K), vs = smem_u32(smem + OFF_V);
-  const uint32_t smem0 = smem_u32(smem), qring = smem_u32(smem + OFF_QRING), ost = smem_u32(smem + OFF_OST);
+  const uint32_t smem0 = smem_u32(smem), qring = smem_u32(smem + OFF_QRING);
   const int kmax = 128;                        // S / P span the whole tile: sequences sit in power-of-two row slots
   const uint32_t id_qkv = make_idesc_bf16(128, 96), id_s = make_idesc_bf16(128, kmax), id_pv = make_idesc_bf16(128, DH, 0, 1),
                  id_128 = make_idesc_bf16(128, 128), id_out = make_idesc_bf16(128, D);
@@ -1039,14 +923,8 @@ __device__ void mma_main(const FusedArgs& a, uint8_t* smem, uint64_t* bars, uint
   auto outproj = [&](int h) {                 // x += (O_h / l) Wout[:, 32h .. 32h+32)^T   (x + b_out was stored by the workers)
     const uint32_t s = RING_LO + h % (RING_HI - RING_LO), sb = slot_wait(s);
     const uint64_t db = desc_sw64(sb);
-#if AVF_O_TMEM
     if (leader) umma_bf16_ts(tmem + TM_X, tmem + TM_O, db, id_out, 1u);               // k-step 0: thread 0's packed columns
     if (leader) umma_bf16_ts(tmem + TM_X, tmem + TM_O + 16, db + 2, id_out, 1u);      // k-step 1: thread 1's
-#else
-    const uint64_t da = desc_sw64(ost);
-    if (leader) umma_bf16(tmem + TM_X, da, db, id_out, 1u);
-    if (leader) umma_bf16(tmem + TM_X, da + 2, db + 2, id_out, 1u);
-#endif
     slot_release(s);
   };
   bool last_layer = false;
@@ -1085,7 +963,7 @@ __device__ void mma_main(const FusedArgs& a, uint8_t* smem, uint64_t* bars, uint
         pf.mark(PM_S);
         if (h + 1 < HEADS) qkv(false);
         pf.mark(PM_QKV);
-        if (h > 0) {                          // O(h-1) is out of TMEM and staged: its slice of the out-projection
+        if (h > 0) {                          // O(h-1) / l is packed in TMEM: its slice of the out-projection
           mbar_wait(&bars[B_O_DRAINED], (h - 1) & 1);
           tc_fence_after();
           pf.mark(PM_WAIT_OD7);
@@ -1207,24 +1085,6 @@ __global__ void __launch_bounds__(256) pos_transpose_kernel(const float* __restr
   pos_t[(blockIdx.x * POS_LD + t) * 4 + (threadIdx.x & 3)] = t < n_tok ? pos[t * DIM + c] : 0.f;
 }
 
-bool dynamic_tiles_enabled() {    // developer A/B: AVF_FUSED_DYNAMIC_TILES=0 keeps static striding for the NCHW form too
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("AVF_FUSED_DYNAMIC_TILES");
-    v = (e != nullptr && e[0] == '0') ? 0 : 1;
-  }
-  return v != 0;
-}
-
-bool fixed_ntok_enabled() {      // developer A/B: AVF_FUSED_FIXED_NTOK=0 keeps the run-time-geometry instantiation for the SFormer too
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("AVF_FUSED_FIXED_NTOK");
-    v = (e != nullptr && e[0] == '0') ? 0 : 1;
-  }
-  return v != 0;
-}
-
 int sm_count_cached() { return sm_count_of_current_device(); }
 
 }  // namespace
@@ -1273,9 +1133,9 @@ int encoder_fused(int io_kind, const avf_stack_shape* s, const avf_layer_weights
   static_assert(sizeof(FusedArgs) <= 4000, "kernel parameter space");
   a.in = in; a.out = out; a.pos = pos; a.pos_t = static_cast<const float*>(scratch); a.ld_in = ld_in; a.ld_out = ld_out;
   a.w_last = w_last; a.out21 = out21; a.decisions = decisions;
-  a.tile_counter = nullptr;
+  a.tile_counter = nullptr;     // fp32 rows: static striding
   if (io_kind == IO_NCHW_BF16) {
-    if (dynamic_tiles_enabled()) a.tile_counter = reinterpret_cast<int*>(static_cast<uint8_t*>(scratch) + size_t(DIM) * POS_LD * sizeof(float));
+    a.tile_counter = reinterpret_cast<int*>(static_cast<uint8_t*>(scratch) + size_t(DIM) * POS_LD * sizeof(float));
     launch_pdl(pos_transpose_kernel, DIM / 4, 256, 0, st, pos, static_cast<float*>(scratch), s->n_tok, a.tile_counter);
     AVF_LAUNCH_CHECK("pos_transpose_kernel");
   }
@@ -1305,7 +1165,7 @@ int encoder_fused(int io_kind, const avf_stack_shape* s, const avf_layer_weights
   }
   const int cap = sm_cap();
   const int grid = min(a.n_tiles, cap > 0 ? min(cap, sm_count_cached()) : sm_count_cached());
-  if (io_kind == IO_NCHW_BF16 && a.n_tok == 49 && NSPLIT == 2 && fixed_ntok_enabled())     // the SFormer's 7 x 7 maps: compile-time geometry
+  if (io_kind == IO_NCHW_BF16 && a.n_tok == 49)     // the SFormer's 7 x 7 maps: compile-time geometry
     launch_pdl(encoder_fused_kernel<IO_NCHW_BF16, 49, 256>, grid, NUM_THREADS, SMEM_ALLOC, st, a);
   else if (io_kind == IO_NCHW_BF16)
     launch_pdl(encoder_fused_kernel<IO_NCHW_BF16, 0, 256>, grid, NUM_THREADS, SMEM_ALLOC, st, a);

@@ -335,12 +335,6 @@ def set_fused_enabled(enabled: bool) -> bool:
     return bool(_lib.lib().avf_set_fused_enabled(1 if enabled else 0))
 
 
-def set_fused_small_enabled(enabled: bool) -> bool:
-    """Developer A/B (also AVF_FUSED_SMALL=0): False runs dim-128 stacks kernel per operation and keeps the positional adds and AU
-    logits of token_stack_fwd_ in their own kernels; returns the previous setting."""
-    return bool(_lib.lib().avf_set_fused_small_enabled(1 if enabled else 0))
-
-
 def encoder_fused_supported(shape: StackShape, precision="bf16") -> bool:
     return bool(_lib.lib().avf_encoder_fused_supported(ctypes.byref(shape), _mode(precision)))
 

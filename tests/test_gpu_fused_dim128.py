@@ -1,6 +1,6 @@
 """The fused encoder kernel at model width 128 (AU_formers, VA_former) and the positional add / AU logits folded into its input and
-output sweeps: against the fp64 oracle, and against the kernel-per-operation sequence the developer switch
-(set_fused_small_enabled(False), AVF_FUSED_SMALL=0) restores."""
+output sweeps: against the fp64 oracle, and against the kernel-per-operation path (set_fused_enabled(False)), which runs the
+positional add and the AU logits as kernels of their own."""
 import pytest
 import torch
 
@@ -60,9 +60,9 @@ def _model(seed):
     return m.cuda().eval().set_precision("bf16")
 
 
-def _chain(m, cls, audio, fused_small):
+def _chain(m, cls, audio, fused):
     """Both AU_formers into the [B*12, 256] fusion input, then the fusion head, with the fused path on or off."""
-    prev = AF.set_fused_small_enabled(fused_small)
+    prev = AF.set_fused_enabled(fused)
     try:
         n = cls.shape[0]
         tokens = torch.empty((n * 12, 256), dtype=torch.float32, device="cuda")
@@ -72,10 +72,10 @@ def _chain(m, cls, audio, fused_small):
             out21, dec = m.au_head.logits21_(tokens.clone(), n, True)
         return tokens, out21, dec
     finally:
-        AF.set_fused_small_enabled(prev)
+        AF.set_fused_enabled(prev)
 
 
-def test_au_formers_and_head_fused_against_switch_off_512_clips():
+def test_au_formers_and_head_fused_against_unfused_512_clips():
     seed = 4545
     m = _model(seed)
     g = torch.Generator(device="cpu").manual_seed(seed)

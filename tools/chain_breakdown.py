@@ -7,8 +7,7 @@
 
 Each stage is captured REPS times into its own CUDA graph and replayed, so the numbers are device time with the launch gaps of a
 graph, not Python launch overhead (fusion_head includes a 6 MB device copy that restores its input, which the kernel-per-operation
-path updates in place).  With AVF_FUSED_SMALL available the stages are measured with the fused dim-128 / folded head
-path off and on, alternating ROUNDS times; a build without the switch is measured as is ("default").
+path updates in place).  Each stage is timed ROUNDS times.
 Usage: python tools/chain_breakdown.py [out.json] [rounds]"""
 import json
 import os
@@ -22,7 +21,6 @@ import torch
 import avformer_b200 as A
 
 B, T, SEED, REPS, REPLAYS = 512, 16, 2024, 20, 10
-AF = A.functional
 L = A._lib.lib()
 
 
@@ -79,26 +77,18 @@ def main():
         "audio_au_former": lambda: model.audio_model.au_head.tokens_into(audio, audio.shape[1], B, out=tokens, ld_out=256),
         "fusion_head": lambda: (scratch.copy_(tokens), model.au_head.logits21_(scratch, B, True)),
     }
-    switch = getattr(AF, "set_fused_small_enabled", None)
-    states = [False, True] if switch is not None else [None]
-    graphs, counts = {}, {}
     with torch.no_grad():
-        for st in states:
-            if switch is not None:
-                switch(st)
-            key = "default" if st is None else ("fused_small_on" if st else "fused_small_off")
-            graphs[key] = {name: graph_of(fn) for name, fn in stages.items()}
-            graphs[key]["graphed_step"] = A.GraphedHotPath(model, stage3, frame, audio)
-            counts[key] = {name: launches(fn) for name, fn in stages.items()}
-            counts[key]["graphed_step"] = launches(lambda: model.hot_path(stage3, frame, audio, want_decisions=True))     # eager, same kernels
-    samples = {k: {name: [] for name in graphs[k]} for k in graphs}
+        graphs = {name: graph_of(fn) for name, fn in stages.items()}
+        graphs["graphed_step"] = A.GraphedHotPath(model, stage3, frame, audio)
+        counts = {name: launches(fn) for name, fn in stages.items()}
+        counts["graphed_step"] = launches(lambda: model.hot_path(stage3, frame, audio, want_decisions=True))     # eager, same kernels
+    samples = {name: [] for name in graphs}
     for _ in range(rounds):
-        for k, gs in graphs.items():
-            for name, gr in gs.items():
-                if name == "graphed_step":
-                    samples[k][name].append(time_graph_replay(gr))
-                else:
-                    samples[k][name].append(time_graph(gr, REPS))
+        for name, gr in graphs.items():
+            if name == "graphed_step":
+                samples[name].append(time_graph_replay(gr))
+            else:
+                samples[name].append(time_graph(gr, REPS))
     gpu = torch.cuda.get_device_name(0)
     try:
         smi = subprocess.run(["nvidia-smi", "--query-gpu=power.limit,clocks.sm,clocks.max.sm,clocks_throttle_reasons.active", "--format=csv,noheader"],
@@ -106,12 +96,11 @@ def main():
     except Exception as ex:      # the numbers stand without it; say why it is missing
         smi = f"nvidia-smi unavailable: {ex}"
     res = {"gpu": gpu, "nvidia_smi_after": smi, "clips": B, "frames": T, "rounds": rounds, "graph_reps_per_stage": REPS,
-           "ms": {k: {n: {"median": statistics.median(v), "min": min(v), "max": max(v), "samples": v} for n, v in s.items()} for k, s in samples.items()},
+           "ms": {n: {"median": statistics.median(v), "min": min(v), "max": max(v), "samples": v} for n, v in samples.items()},
            "launches": counts}
     with open(out_path, "w") as f:
         json.dump(res, f, indent=1)
-    for k, s in res["ms"].items():
-        print(k, {n: round(v["median"], 4) for n, v in s.items()}, counts[k])
+    print({n: round(v["median"], 4) for n, v in res["ms"].items()}, counts)
 
 
 def time_graph_replay(graphed):
