@@ -129,6 +129,7 @@ int avf_token_stack_fwd(int mode, const avf_stack_shape* s, const avf_layer_weig
                         float* out, int32_t ld_out, const float* w_last, float* out21, int32_t* decisions,
                         void* workspace, size_t workspace_bytes, void* stream);
 
+
 /* Building blocks (exposed for tests and for callers that fuse differently). */
 /* y[r,:] = LayerNorm(x[r,:]) * gamma + beta, eps 1e-5; y is bf16 (mode BF16) or fp32. */
 int avf_layernorm_fwd(int out_mode, const float* x, int32_t ld_x, const float* gamma, const float* beta,
@@ -342,6 +343,33 @@ int avf_au_logits_bwd(const float* dlogits, int32_t ld_dlogits, const float* x, 
 int avf_adam_step(float* params, const float* grads, float* exp_avg, float* exp_avg_sq, void* bf16_shadow, size_t n,
                   float lr, float beta1, float beta2, float eps, float weight_decay, int32_t step, int decoupled,
                   float grad_scale, void* stream);
+
+/* ---- attention masks (the `mask` of Transformer.forward, models/heads.py:225-232) ---------------
+ * keep [n_seq, n_tok] DEVICE uint8, 1 = keep.  Score (i, j) of every head of sequence b survives iff keep[b, i] and keep[b, j]; the
+ * other scores are filled with the same very negative value before the softmax.  So a kept query attends only to kept keys (dropped
+ * keys get probability exactly 0), and a dropped query attends uniformly to all n_tok tokens (its output is the mean of V, never NaN).
+ * The mask is generic: a caller that wants a token kept always (the cls slot) sets its byte.  n_tok <= 64.  keep == NULL is exactly
+ * the unmasked call.  A masked stack never takes the fused kernel (it runs kernel by kernel); the backward must be given the keep
+ * array of its forward.  Same workspace / tape sizes as the unmasked calls. */
+int avf_attention_fwd_masked(int io_mode, const void* qkv, void* out, int32_t n_seq, int32_t n_tok,
+                             int32_t heads, int32_t dim_head, const uint8_t* keep, void* stream);
+int avf_attention_bwd_masked(int io_mode, const void* qkv, const void* dout, void* dqkv, int32_t n_seq, int32_t n_tok,
+                             int32_t heads, int32_t dim_head, const uint8_t* keep, void* stream);
+int avf_encoder_stack_fwd_masked(int mode, const avf_stack_shape* s, const avf_layer_weights* layers, const uint8_t* keep,
+                                 float* x, int32_t ld_x, float* out, int32_t ld_out,
+                                 void* workspace, size_t workspace_bytes, void* stream);
+int avf_encoder_stack_fwd_train_masked(int mode, const avf_stack_shape* s, const avf_layer_weights* layers, const uint8_t* keep,
+                                       const float* x, int32_t ld_x, float* out, int32_t ld_out,
+                                       void* tape, size_t tape_bytes, float dropout_p, uint64_t dropout_seed,
+                                       const uint32_t* dropout_salt, void* stream);
+int avf_encoder_stack_bwd_masked(int mode, const avf_stack_shape* s, const avf_layer_weights* layers, const uint8_t* keep,
+                                 const void* tape, size_t tape_bytes, float* dx, int32_t ld_dx,
+                                 const avf_layer_grads* grads, int accumulate, void* workspace, size_t workspace_bytes,
+                                 float dropout_p, uint64_t dropout_seed, const uint32_t* dropout_salt, void* stream);
+/* avf_tformer_fwd with keep [n_clips, T+1] (row 0 of each clip is its cls token); the cls-only last layer honours it too. */
+int avf_tformer_fwd_masked(int mode, int io_mode, const avf_stack_shape* s, const avf_layer_weights* layers, const uint8_t* keep,
+                           const void* frames, const float* cls_token, const float* pos, float* cls_out,
+                           void* workspace, size_t workspace_bytes, void* stream);
 
 #ifdef __cplusplus
 }

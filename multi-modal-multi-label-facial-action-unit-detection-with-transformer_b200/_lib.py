@@ -122,6 +122,18 @@ SIGNATURES = {
                                                _c_p, _c_p, _c_p, _c_p, _i32, _i32, _i32, _c_p, _sz, _c_p]),
     "avf_au_logits_bwd": (ctypes.c_int, [_c_p, _i32, _c_p, _i32, _c_p, _c_p, _i32, _c_p, _i32, _i32, _c_p]),
     "avf_adam_step": (ctypes.c_int, [_c_p, _c_p, _c_p, _c_p, _c_p, _sz] + [ctypes.c_float] * 5 + [_i32, ctypes.c_int, ctypes.c_float, _c_p]),
+    # ---- attention masks (keep: device uint8 [n_seq, n_tok]) ----
+    "avf_attention_fwd_masked": (ctypes.c_int, [ctypes.c_int, _c_p, _c_p, _i32, _i32, _i32, _i32, _c_p, _c_p]),
+    "avf_attention_bwd_masked": (ctypes.c_int, [ctypes.c_int, _c_p, _c_p, _c_p, _i32, _i32, _i32, _i32, _c_p, _c_p]),
+    "avf_encoder_stack_fwd_masked": (ctypes.c_int, [ctypes.c_int, ctypes.POINTER(StackShape), ctypes.POINTER(LayerWeights), _c_p, _c_p, _i32,
+                                                    _c_p, _i32, _c_p, _sz, _c_p]),
+    "avf_encoder_stack_fwd_train_masked": (ctypes.c_int, [ctypes.c_int, ctypes.POINTER(StackShape), ctypes.POINTER(LayerWeights), _c_p, _c_p, _i32,
+                                                          _c_p, _i32, _c_p, _sz, ctypes.c_float, ctypes.c_uint64, _c_p, _c_p]),
+    "avf_encoder_stack_bwd_masked": (ctypes.c_int, [ctypes.c_int, ctypes.POINTER(StackShape), ctypes.POINTER(LayerWeights), _c_p, _c_p, _sz, _c_p,
+                                                    _i32, ctypes.POINTER(LayerGrads), ctypes.c_int, _c_p, _sz, ctypes.c_float, ctypes.c_uint64, _c_p,
+                                                    _c_p]),
+    "avf_tformer_fwd_masked": (ctypes.c_int, [ctypes.c_int, ctypes.c_int, ctypes.POINTER(StackShape), ctypes.POINTER(LayerWeights), _c_p, _c_p,
+                                              _c_p, _c_p, _c_p, _c_p, _sz, _c_p]),
 }
 
 _lock = threading.Lock()

@@ -82,25 +82,27 @@ def _hand_over(params, grads):
 
 
 class EncoderStackFn(torch.autograd.Function):
-    """Transformer (models/heads.py:242-256) on an fp32 token matrix [n_seq*n_tok, dim]."""
+    """Transformer (models/heads.py:242-256) on an fp32 token matrix [n_seq*n_tok, dim]; ``keep`` [n_seq, n_tok] bool (or None) is
+    the attention mask of every layer, a non-differentiable input."""
 
     @staticmethod
-    def forward(ctx, x, tr, n_seq, n_tok, *params):
+    def forward(ctx, x, tr, n_seq, n_tok, keep, *params):
         packed = tr.packed()
         shape = tr.shape(n_seq, n_tok)
         ctx.drop = tr.dropout_state()
-        y, tape = AF.encoder_stack_fwd_train(_f32_dense(x.detach()), packed, shape, *ctx.drop)
-        ctx.packed, ctx.shape_, ctx.tape, ctx.params = packed, shape, tape, params
+        y, tape = AF.encoder_stack_fwd_train(_f32_dense(x.detach()), packed, shape, *ctx.drop, keep=keep)
+        ctx.packed, ctx.shape_, ctx.tape, ctx.params, ctx.keep = packed, shape, tape, params, keep
         return y
 
     @staticmethod
     def backward(ctx, dy):
         needs = ctx.needs_input_grad
         dx = _f32_dense(dy).clone()
-        dx, grads = AF.encoder_stack_bwd_(dx, ctx.packed, ctx.shape_, ctx.tape, list(needs[4:]), *ctx.drop, into=_direct_targets(ctx.params))
-        ctx.tape = None
+        dx, grads = AF.encoder_stack_bwd_(dx, ctx.packed, ctx.shape_, ctx.tape, list(needs[5:]), *ctx.drop, into=_direct_targets(ctx.params),
+                                          keep=ctx.keep)
+        ctx.tape = ctx.keep = None
         _notify(ctx.params)
-        return (dx if needs[0] else None, None, None, None, *grads)
+        return (dx if needs[0] else None, None, None, None, None, *grads)
 
 
 class SFormerFn(torch.autograd.Function):

@@ -137,12 +137,12 @@ class TwoStreamAuralVisualFormer(nn.Module):
         emb = emb.detach().float().contiguous()
         return head.tokens_into(emb, emb.shape[1], bs)
 
-    def hot_path_train(self, stage3, frame_feat, audio_feat):
+    def hot_path_train(self, stage3, frame_feat, audio_feat, frame_mask=None):
         """hot_path() with autograd: returns (sformer_out, out21); call .backward() on a loss of either."""
         vm = self.video_model.video_model
         s_out = vm.s_former.sformer(stage3)
         n_clips = frame_feat.numel() // (vm.t_former.num_patches * vm.t_former.dim)
-        cls = vm.t_former(frame_feat)
+        cls = vm.t_former(frame_feat, frame_mask)
         tok_v = self._au_tokens(self.video_model.au_head, cls, n_clips)
         tok_a = self._au_tokens(self.audio_model.au_head, audio_feat, n_clips)
         return s_out, self.au_head.logits21_train(torch.cat([tok_a, tok_v], dim=1), n_clips)
@@ -154,15 +154,16 @@ class TwoStreamAuralVisualFormer(nn.Module):
                 m.dropout = float(p)
         return self
 
-    def hot_path(self, stage3, frame_feat, audio_feat, want_decisions=False):
+    def hot_path(self, stage3, frame_feat, audio_feat, want_decisions=False, frame_mask=None):
         """The transformer stack alone, on tensors already at its boundaries (what bench.py times and
         what SURVEY.md §8 scopes): SFormer on stage-3 maps [B*T,256,7,7] (fp32/bf16), then TFormer on frame
         features [B*T,512], the two AU_formers (video: TFormer cls rows; audio: audio_feat [B,512] fp32) and
         the fusion head.  In the full model the conv stage 4 sits between SFormer and TFormer; here the two
-        are fed independently.  Returns (sformer_out, out21 [B,21]) (+ int32 decisions [B,12])."""
+        are fed independently.  Returns (sformer_out, out21 [B,21]) (+ int32 decisions [B,12]).  ``frame_mask`` (optional): bool
+        [B, T], True = a real frame, passed to the TFormer as its attention mask (TFormer.forward)."""
         vm = self.video_model.video_model
         s_out = vm.s_former.sformer(stage3)
-        cls = vm.t_former.cls_features(frame_feat)
+        cls = vm.t_former.cls_features(frame_feat, frame_mask)
         n_clips = cls.shape[0]
         fused = torch.empty((n_clips * 12, 256), dtype=torch.float32, device=cls.device)
         a_feat = audio_feat if (audio_feat.dtype == torch.float32 and audio_feat.is_contiguous()) else audio_feat.float().contiguous()

@@ -113,13 +113,14 @@ static bool fused_rows(int mode, const avf_stack_shape* s, int ld_x, const float
          ld_x % 4 == 0 && (out == nullptr || ld_out % 4 == 0);
 }
 
+// keep (optional, [n_seq, n_tok] uint8): attention mask of every layer; the fused kernel has none, so a masked stack runs kernel by kernel.
 static int encoder_stack(int mode, const avf_stack_shape* s, const avf_layer_weights* L, float* x, int ld_x, float* out, int ld_out,
-                         void* ws, size_t ws_bytes, cudaStream_t st) {
+                         void* ws, size_t ws_bytes, cudaStream_t st, const uint8_t* keep = nullptr) {
   int e = check_shape(s);
   if (e) return e;
   AVF_REQUIRE(mode == AVF_BF16 || mode == AVF_FP32, AVF_EINVAL, "mode=%d", mode);
   AVF_REQUIRE(L != nullptr && x != nullptr && ws != nullptr, AVF_EINVAL, "null pointer argument");
-  if (fused_rows(mode, s, ld_x, out, ld_out))     // whole stack, one persistent kernel
+  if (keep == nullptr && fused_rows(mode, s, ld_x, out, ld_out))     // whole stack, one persistent kernel
     return encoder_fused(1, s, L, x, ld_x, out ? out : x, out ? ld_out : ld_x, nullptr, nullptr, nullptr, nullptr, nullptr, st);
   const EncoderWs w = carve_encoder_ws(s, mode, ws);
   AVF_REQUIRE(ws_bytes >= w.total, AVF_EWORKSPACE, "workspace too small: %zu < %zu bytes", ws_bytes, w.total);
@@ -129,7 +130,7 @@ static int encoder_stack(int mode, const avf_stack_shape* s, const avf_layer_wei
     // x + to_out(attn(to_qkv(LN(x))))                                     models/heads.py:175,185,219-239
     if ((e = layernorm(mode, x, ld_x, W.ln1_gamma, W.ln1_beta, w.ln, R, D, st))) return e;
     if ((e = linear(mode, w.ln, D, W.w_qkv, nullptr, nullptr, 0, w.qkv, 3 * I, mode, R, 3 * I, D, 0, st))) return e;
-    if ((e = attention_small(mode, w.qkv, w.attn, s->n_seq, s->n_tok, s->heads, s->dim_head, st))) return e;
+    if ((e = attention_small(mode, w.qkv, w.attn, s->n_seq, s->n_tok, s->heads, s->dim_head, st, keep))) return e;
     if ((e = linear(mode, w.attn, I, W.w_out, W.b_out, x, ld_x, x, ld_x, AVF_FP32, R, D, I, AVF_EPI_BIAS | AVF_EPI_RESIDUAL, st))) return e;
     // x + W2 gelu(W1 LN(x) + b1) + b2                                     models/heads.py:188-200
     if ((e = layernorm(mode, x, ld_x, W.ln2_gamma, W.ln2_beta, w.ln, R, D, st))) return e;
@@ -140,6 +141,48 @@ static int encoder_stack(int mode, const avf_stack_shape* s, const avf_layer_wei
       return e;
   }
   return 0;
+}
+
+static int tformer_fwd(int mode, int io_mode, const avf_stack_shape* s, const avf_layer_weights* layers, const void* frames, const float* cls_token,
+                       const float* pos, float* cls_out, void* workspace, size_t workspace_bytes, const uint8_t* keep, cudaStream_t st) {
+  int e = check_shape(s);
+  if (e) return e;
+  AVF_REQUIRE(layers && frames && cls_token && pos && cls_out && workspace, AVF_EINVAL, "tformer_fwd: null pointer");
+  AVF_REQUIRE(s->n_tok >= 2, AVF_EINVAL, "tformer_fwd: n_tok=%d (cls + at least one frame)", s->n_tok);
+  const size_t need = avf_tformer_workspace_bytes(s, mode);
+  AVF_REQUIRE(workspace_bytes >= need, AVF_EWORKSPACE, "workspace too small: %zu < %zu bytes", workspace_bytes, need);
+  const int B = s->n_seq, N = s->n_tok, R = B * N, D = s->dim, I = s->heads * s->dim_head, M = s->mlp_dim;
+  uint8_t* p = static_cast<uint8_t*>(workspace);
+  float* x = reinterpret_cast<float*>(p);   p += align_up(size_t(R) * D * 4);
+  void* enc_ws = p;
+  const EncoderWs w = carve_encoder_ws(s, mode, enc_ws);
+  p += w.total;
+  float* xc = reinterpret_cast<float*>(p);  p += align_up(size_t(B) * D * 4);
+  void* lnc = p;                            p += align_up(size_t(B) * D * elt(mode));
+  void* oc = p;                             p += align_up(size_t(B) * I * elt(mode));
+  void* hc = p;
+  if ((e = tformer_embed(io_mode, frames, cls_token, pos, x, B, N - 1, D, st))) return e;
+  if (s->depth > 1) {
+    avf_stack_shape head = *s;
+    head.depth = s->depth - 1;
+    if ((e = encoder_stack(mode, &head, layers, x, D, nullptr, 0, enc_ws, w.total, st, keep))) return e;
+  }
+  // Last layer (models/vformer.py:288-290 returns x[:, 0] only): keys / values need every row, everything after the softmax only
+  // the cls row of each clip — out-projection, LayerNorm, MLP run on [n_clips, dim] instead of [n_clips * (T+1), dim].
+  const avf_layer_weights& W = layers[s->depth - 1];
+  if ((e = layernorm(mode, x, D, W.ln1_gamma, W.ln1_beta, w.ln, R, D, st))) return e;
+  if ((e = linear(mode, w.ln, D, W.w_qkv, nullptr, nullptr, 0, w.qkv, 3 * I, mode, R, 3 * I, D, 0, st))) return e;
+  if (mode == AVF_BF16) {
+    if ((e = attention_mma_bf16(w.qkv, oc, B, N, s->heads, s->dim_head, st, 1, keep))) return e;
+  } else {
+    if ((e = attention_small(mode, w.qkv, w.attn, B, N, s->heads, s->dim_head, st, keep))) return e;
+    AVF_CUDA(cudaMemcpy2DAsync(oc, size_t(I) * 4, w.attn, size_t(N) * I * 4, size_t(I) * 4, B, cudaMemcpyDeviceToDevice, st));
+  }
+  if ((e = rows_gather(x, size_t(N) * D, xc, B, D, st))) return e;
+  if ((e = linear(mode, oc, I, W.w_out, W.b_out, xc, D, xc, D, AVF_FP32, B, D, I, AVF_EPI_BIAS | AVF_EPI_RESIDUAL, st))) return e;
+  if ((e = layernorm(mode, xc, D, W.ln2_gamma, W.ln2_beta, lnc, B, D, st))) return e;
+  if ((e = linear(mode, lnc, D, W.w_ff1, W.b_ff1, nullptr, 0, hc, M, mode, B, M, D, AVF_EPI_BIAS | AVF_EPI_GELU, st))) return e;
+  return linear(mode, hc, M, W.w_ff2, W.b_ff2, xc, D, cls_out, D, AVF_FP32, B, D, M, AVF_EPI_BIAS | AVF_EPI_RESIDUAL, st);
 }
 
 }  // namespace avf
@@ -206,6 +249,13 @@ int avf_encoder_stack_fwd(int mode, const avf_stack_shape* s, const avf_layer_we
   return encoder_stack(mode, s, layers, x, ld_x, out, ld_out, workspace, workspace_bytes, static_cast<cudaStream_t>(stream));
 }
 
+int avf_encoder_stack_fwd_masked(int mode, const avf_stack_shape* s, const avf_layer_weights* layers, const uint8_t* keep, float* x, int32_t ld_x,
+                                 float* out, int32_t ld_out, void* workspace, size_t workspace_bytes, void* stream) {
+  int e = require_device();
+  if (e) return e;
+  return encoder_stack(mode, s, layers, x, ld_x, out, ld_out, workspace, workspace_bytes, static_cast<cudaStream_t>(stream), keep);
+}
+
 int avf_token_stack_fwd(int mode, const avf_stack_shape* s, const avf_layer_weights* layers, float* x, int32_t ld_x, const float* pos, float* out,
                         int32_t ld_out, const float* w_last, float* out21, int32_t* decisions, void* workspace, size_t workspace_bytes, void* stream) {
   int e = require_device();
@@ -245,6 +295,14 @@ int avf_attention_fwd(int io_mode, const void* qkv, void* out, int32_t n_seq, in
   if (e) return e;
   AVF_REQUIRE(qkv && out, AVF_EINVAL, "attention: null pointer");
   return attention_small(io_mode, qkv, out, n_seq, n_tok, heads, dim_head, static_cast<cudaStream_t>(stream));
+}
+
+int avf_attention_fwd_masked(int io_mode, const void* qkv, void* out, int32_t n_seq, int32_t n_tok, int32_t heads, int32_t dim_head, const uint8_t* keep,
+                             void* stream) {
+  int e = require_device();
+  if (e) return e;
+  AVF_REQUIRE(qkv && out, AVF_EINVAL, "attention: null pointer");
+  return attention_small(io_mode, qkv, out, n_seq, n_tok, heads, dim_head, static_cast<cudaStream_t>(stream), keep);
 }
 
 int avf_sformer_tokens_pack(int io_mode, const void* fmap, const float* pos, float* x, int32_t n_frames, int32_t dim, int32_t hw, void* stream) {
@@ -303,44 +361,14 @@ int avf_tformer_fwd(int mode, int io_mode, const avf_stack_shape* s, const avf_l
                     const float* cls_token, const float* pos, float* cls_out, void* workspace, size_t workspace_bytes, void* stream) {
   int e = require_device();
   if (e) return e;
-  if ((e = check_shape(s))) return e;
-  AVF_REQUIRE(layers && frames && cls_token && pos && cls_out && workspace, AVF_EINVAL, "tformer_fwd: null pointer");
-  AVF_REQUIRE(s->n_tok >= 2, AVF_EINVAL, "tformer_fwd: n_tok=%d (cls + at least one frame)", s->n_tok);
-  const size_t need = avf_tformer_workspace_bytes(s, mode);
-  AVF_REQUIRE(workspace_bytes >= need, AVF_EWORKSPACE, "workspace too small: %zu < %zu bytes", workspace_bytes, need);
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const int B = s->n_seq, N = s->n_tok, R = B * N, D = s->dim, I = s->heads * s->dim_head, M = s->mlp_dim;
-  uint8_t* p = static_cast<uint8_t*>(workspace);
-  float* x = reinterpret_cast<float*>(p);   p += align_up(size_t(R) * D * 4);
-  void* enc_ws = p;
-  const EncoderWs w = carve_encoder_ws(s, mode, enc_ws);
-  p += w.total;
-  float* xc = reinterpret_cast<float*>(p);  p += align_up(size_t(B) * D * 4);
-  void* lnc = p;                            p += align_up(size_t(B) * D * elt(mode));
-  void* oc = p;                             p += align_up(size_t(B) * I * elt(mode));
-  void* hc = p;
-  if ((e = tformer_embed(io_mode, frames, cls_token, pos, x, B, N - 1, D, st))) return e;
-  if (s->depth > 1) {
-    avf_stack_shape head = *s;
-    head.depth = s->depth - 1;
-    if ((e = encoder_stack(mode, &head, layers, x, D, nullptr, 0, enc_ws, w.total, st))) return e;
-  }
-  // Last layer (models/vformer.py:288-290 returns x[:, 0] only): keys / values need every row, everything after the softmax only
-  // the cls row of each clip — out-projection, LayerNorm, MLP run on [n_clips, dim] instead of [n_clips * (T+1), dim].
-  const avf_layer_weights& W = layers[s->depth - 1];
-  if ((e = layernorm(mode, x, D, W.ln1_gamma, W.ln1_beta, w.ln, R, D, st))) return e;
-  if ((e = linear(mode, w.ln, D, W.w_qkv, nullptr, nullptr, 0, w.qkv, 3 * I, mode, R, 3 * I, D, 0, st))) return e;
-  if (mode == AVF_BF16) {
-    if ((e = attention_mma_bf16(w.qkv, oc, B, N, s->heads, s->dim_head, st, 1))) return e;
-  } else {
-    if ((e = attention_small(mode, w.qkv, w.attn, B, N, s->heads, s->dim_head, st))) return e;
-    AVF_CUDA(cudaMemcpy2DAsync(oc, size_t(I) * 4, w.attn, size_t(N) * I * 4, size_t(I) * 4, B, cudaMemcpyDeviceToDevice, st));
-  }
-  if ((e = rows_gather(x, size_t(N) * D, xc, B, D, st))) return e;
-  if ((e = linear(mode, oc, I, W.w_out, W.b_out, xc, D, xc, D, AVF_FP32, B, D, I, AVF_EPI_BIAS | AVF_EPI_RESIDUAL, st))) return e;
-  if ((e = layernorm(mode, xc, D, W.ln2_gamma, W.ln2_beta, lnc, B, D, st))) return e;
-  if ((e = linear(mode, lnc, D, W.w_ff1, W.b_ff1, nullptr, 0, hc, M, mode, B, M, D, AVF_EPI_BIAS | AVF_EPI_GELU, st))) return e;
-  return linear(mode, hc, M, W.w_ff2, W.b_ff2, xc, D, cls_out, D, AVF_FP32, B, D, M, AVF_EPI_BIAS | AVF_EPI_RESIDUAL, st);
+  return tformer_fwd(mode, io_mode, s, layers, frames, cls_token, pos, cls_out, workspace, workspace_bytes, nullptr, static_cast<cudaStream_t>(stream));
+}
+
+int avf_tformer_fwd_masked(int mode, int io_mode, const avf_stack_shape* s, const avf_layer_weights* layers, const uint8_t* keep, const void* frames,
+                           const float* cls_token, const float* pos, float* cls_out, void* workspace, size_t workspace_bytes, void* stream) {
+  int e = require_device();
+  if (e) return e;
+  return tformer_fwd(mode, io_mode, s, layers, frames, cls_token, pos, cls_out, workspace, workspace_bytes, keep, static_cast<cudaStream_t>(stream));
 }
 
 int avf_tformer_cls_extract(const float* x, float* cls, int32_t n_clips, int32_t n_tok, int32_t dim, void* stream) {

@@ -35,9 +35,27 @@ __device__ __forceinline__ void quad_transpose32(uint32_t (&p)[4], int lane) {
   r = __shfl_xor_sync(0xffffffffu, b1 ? p[1] : p[3], 2); if (b1) p[1] = r; else p[3] = r;
 }
 
-template <int DH, int NP>    // NP = tokens padded to a multiple of 16 (16 / 32 / 48 / 64)
+// Keep bits of one sequence (bit j = token j is kept; bits >= n_tok are 0) from its keep row of <= 64 bytes: two ballots of the warp.
+__device__ __forceinline__ uint64_t keep_bits(const uint8_t* __restrict__ row, int n_tok, int lane) {
+  const uint32_t lo = __ballot_sync(0xffffffffu, lane < n_tok && row[lane] != 0);
+  const uint32_t hi = __ballot_sync(0xffffffffu, lane + 32 < n_tok && row[lane + 32] != 0);
+  return (uint64_t(hi) << 32) | lo;
+}
+
+// Masked score (query kept: row_kept, key column c): a kept query keeps the scores of kept keys and gets -INF on dropped keys, like on
+// the padding columns c >= n_tok; a dropped query gets the same score 0 on every real key, i.e. the uniform row that masked_fill with
+// -finfo.max gives (and no -INF - (-INF) in the exp).
+__device__ __forceinline__ float mask_score(float s, bool row_kept, uint64_t km, int c, int n_tok) {
+  if (c >= n_tok) return -INFINITY;
+  if (!row_kept) return 0.f;
+  return ((km >> c) & 1) ? s : -INFINITY;
+}
+
+// MASKED: keep [n_seq, n_tok] uint8 (1 = keep) masks score (i, j) unless tokens i and j are both kept (mask_score).
+template <int DH, int NP, bool MASKED>    // NP = tokens padded to a multiple of 16 (16 / 32 / 48 / 64)
 __global__ void __launch_bounds__(DH == 32 ? 128 : 64) attention_mma_kernel(const __nv_bfloat16* __restrict__ qkv, __nv_bfloat16* __restrict__ out,
-                                                            int n_problems, int n_tok, int heads, float scale_log2e, int q_rows) {
+                                                            int n_problems, int n_tok, int heads, float scale_log2e, int q_rows,
+                                                            const uint8_t* __restrict__ keep) {
   pdl_wait();      // programmatic dependent launch: everything above is launch overhead hidden behind the previous kernel
   pdl_trigger();
   // q_rows: only the first q_rows query rows of every sequence are computed and written (compactly: out [n_seq * q_rows, inner]);
@@ -54,6 +72,8 @@ __global__ void __launch_bounds__(DH == 32 ? 128 : 64) attention_mma_kernel(cons
   const __nv_bfloat16* base = qkv + row0 * (3 * inner) + head * DH;
   __nv_bfloat16 (*Ks)[PITCH] = smem[warp][0];
   __nv_bfloat16 (*Vs)[PITCH] = smem[warp][1];
+  uint64_t km = 0;
+  if constexpr (MASKED) km = keep_bits(keep + row0, n_tok, lane);
 
   // stage K and V (zero rows beyond n_tok: 0 * garbage must not become NaN in P*V)
   constexpr int CH = DH / 8;                          // 16-byte chunks per row
@@ -123,11 +143,17 @@ __global__ void __launch_bounds__(DH == 32 ? 128 : 64) attention_mma_kernel(cons
     }
     // softmax over keys, rows r_lo (regs 0,1) and r_hi (regs 2,3); columns >= n_tok masked
     float m_lo = -INFINITY, m_hi = -INFINITY;
+    const bool k_lo = (km >> r_lo) & 1, k_hi = (km >> r_hi) & 1;
 #pragma unroll
     for (int nt = 0; nt < NP / 8; ++nt) {
       const int c = nt * 8 + 2 * t;
-      if (c >= n_tok) { s[nt][0] = -INFINITY; s[nt][2] = -INFINITY; }
-      if (c + 1 >= n_tok) { s[nt][1] = -INFINITY; s[nt][3] = -INFINITY; }
+      if constexpr (MASKED) {
+        s[nt][0] = mask_score(s[nt][0], k_lo, km, c, n_tok); s[nt][1] = mask_score(s[nt][1], k_lo, km, c + 1, n_tok);
+        s[nt][2] = mask_score(s[nt][2], k_hi, km, c, n_tok); s[nt][3] = mask_score(s[nt][3], k_hi, km, c + 1, n_tok);
+      } else {
+        if (c >= n_tok) { s[nt][0] = -INFINITY; s[nt][2] = -INFINITY; }
+        if (c + 1 >= n_tok) { s[nt][1] = -INFINITY; s[nt][3] = -INFINITY; }
+      }
       m_lo = fmaxf(m_lo, fmaxf(s[nt][0], s[nt][1]));
       m_hi = fmaxf(m_hi, fmaxf(s[nt][2], s[nt][3]));
     }
@@ -187,13 +213,13 @@ __global__ void __launch_bounds__(DH == 32 ? 128 : 64) attention_mma_kernel(cons
   }
 }
 
-template <int DH, int NP>
-int launch(const void* qkv, void* out, int n_seq, int n_tok, int heads, int q_rows, cudaStream_t st) {
+template <int DH, int NP, bool MASKED>
+int launch(const void* qkv, void* out, int n_seq, int n_tok, int heads, int q_rows, const uint8_t* keep, cudaStream_t st) {
   const int n_problems = n_seq * heads;
   const float scale_log2e = 1.4426950408889634f / sqrtf(float(DH));
   constexpr int kWarps = DH == 32 ? 4 : 2;
-  launch_pdl(attention_mma_kernel<DH, NP>, ceil_div(n_problems, kWarps), kWarps * 32, 0, st, static_cast<const __nv_bfloat16*>(qkv), static_cast<__nv_bfloat16*>(out),
-                                                                      n_problems, n_tok, heads, scale_log2e, q_rows);
+  launch_pdl(attention_mma_kernel<DH, NP, MASKED>, ceil_div(n_problems, kWarps), kWarps * 32, 0, st, static_cast<const __nv_bfloat16*>(qkv), static_cast<__nv_bfloat16*>(out),
+                                                                      n_problems, n_tok, heads, scale_log2e, q_rows, keep);
   AVF_LAUNCH_CHECK("attention_mma_kernel");
   return 0;
 }
@@ -214,11 +240,14 @@ struct BwdCfg {
   static constexpr int WARPS = SLAB_BYTES * 2 <= 46 * 1024 ? 2 : 1;
 };
 
-template <int DH, int NP>
+// MASKED: the scores are masked as in the forward (mask_score); dS is 0 wherever a score was filled, and the uniform P of a dropped
+// query still carries its dO into dV.
+template <int DH, int NP, bool MASKED>
 __global__ void __launch_bounds__(BwdCfg<DH, NP>::WARPS * 32) attention_bwd_mma_kernel(const __nv_bfloat16* __restrict__ qkv,
                                                                                        const __nv_bfloat16* __restrict__ dout,
                                                                                        __nv_bfloat16* __restrict__ dqkv, int n_problems,
-                                                                                       int n_tok, int heads, float scale) {
+                                                                                       int n_tok, int heads, float scale,
+                                                                                       const uint8_t* __restrict__ keep) {
   pdl_wait();      // programmatic dependent launch: everything above is launch overhead hidden behind the previous kernel
   pdl_trigger();
   using Cfg = BwdCfg<DH, NP>;
@@ -242,6 +271,8 @@ __global__ void __launch_bounds__(BwdCfg<DH, NP>::WARPS * 32) attention_bwd_mma_
   float* st_il = stats[warp][1];
   float* st_d = stats[warp][2];
   const float scale_log2e = scale * 1.4426950408889634f;
+  uint64_t km = 0;
+  if constexpr (MASKED) km = keep_bits(keep + row0, n_tok, lane);
 
   constexpr int CH = DH / 8;
   for (int i = lane; i < NP * CH; i += 32) {
@@ -325,11 +356,17 @@ __global__ void __launch_bounds__(BwdCfg<DH, NP>::WARPS * 32) attention_bwd_mma_
     load_a(af, Os, r_lo);
     mma_abt(dp, af, Vs);
     float m_lo = -INFINITY, m_hi = -INFINITY;
+    const bool k_lo = (km >> r_lo) & 1, k_hi = (km >> (r_lo + 8)) & 1;
 #pragma unroll
     for (int nt = 0; nt < NP / 8; ++nt) {
       const int c = nt * 8 + 2 * t;
-      if (c >= n_tok) { s[nt][0] = -INFINITY; s[nt][2] = -INFINITY; }
-      if (c + 1 >= n_tok) { s[nt][1] = -INFINITY; s[nt][3] = -INFINITY; }
+      if constexpr (MASKED) {
+        s[nt][0] = mask_score(s[nt][0], k_lo, km, c, n_tok); s[nt][1] = mask_score(s[nt][1], k_lo, km, c + 1, n_tok);
+        s[nt][2] = mask_score(s[nt][2], k_hi, km, c, n_tok); s[nt][3] = mask_score(s[nt][3], k_hi, km, c + 1, n_tok);
+      } else {
+        if (c >= n_tok) { s[nt][0] = -INFINITY; s[nt][2] = -INFINITY; }
+        if (c + 1 >= n_tok) { s[nt][1] = -INFINITY; s[nt][3] = -INFINITY; }
+      }
       m_lo = fmaxf(m_lo, fmaxf(s[nt][0], s[nt][1]));
       m_hi = fmaxf(m_hi, fmaxf(s[nt][2], s[nt][3]));
     }
@@ -372,6 +409,10 @@ __global__ void __launch_bounds__(BwdCfg<DH, NP>::WARPS * 32) attention_bwd_mma_
     for (int nt = 0; nt < NP / 8; ++nt) {      // dS (the 1/sqrt(dh) is applied once when dQ is stored)
       s[nt][0] *= dp[nt][0] - d_lo; s[nt][1] *= dp[nt][1] - d_lo;
       s[nt][2] *= dp[nt][2] - d_hi; s[nt][3] *= dp[nt][3] - d_hi;
+      if constexpr (MASKED) {                  // every score of a dropped query was filled
+        if (!k_lo) s[nt][0] = s[nt][1] = 0.f;
+        if (!k_hi) s[nt][2] = s[nt][3] = 0.f;
+      }
     }
     float dq[DH / 8][4];
     mma_xm(dq, s, Ks);
@@ -391,6 +432,7 @@ __global__ void __launch_bounds__(BwdCfg<DH, NP>::WARPS * 32) attention_bwd_mma_
     load_a(af, Vs, r_lo);
     mma_abt(dp, af, Os);                      // dP^T[key][query]
     float ds[NP / 8][4];
+    const bool k_lo = (km >> r_lo) & 1, k_hi = (km >> (r_lo + 8)) & 1;
 #pragma unroll
     for (int nt = 0; nt < NP / 8; ++nt) {
 #pragma unroll
@@ -398,12 +440,21 @@ __global__ void __launch_bounds__(BwdCfg<DH, NP>::WARPS * 32) attention_bwd_mma_
         const int qi = nt * 8 + 2 * t + e;    // query index of elements e (row r_lo) and e + 2 (row r_lo + 8)
         const bool ok = qi < n_tok;
         const float m = ok ? st_m[qi] : 0.f, il = ok ? st_il[qi] : 0.f, dl = ok ? st_d[qi] : 0.f;
-        const float p0 = ok ? exp2f(fmaf(p[nt][e], scale_log2e, -m)) * il : 0.f;
-        const float p1 = ok ? exp2f(fmaf(p[nt][e + 2], scale_log2e, -m)) * il : 0.f;
+        float p0, p1;
+        if constexpr (MASKED) {               // dropped query: its uniform row 1 / n_tok (= il of pass 1) and dS = 0
+          const bool qk = (km >> qi) & 1;
+          p0 = ok ? exp2f(fmaf(qk ? (k_lo ? p[nt][e] : -INFINITY) : 0.f, scale_log2e, -m)) * il : 0.f;       // m = 0 on a dropped row
+          p1 = ok ? exp2f(fmaf(qk ? (k_hi ? p[nt][e + 2] : -INFINITY) : 0.f, scale_log2e, -m)) * il : 0.f;
+          ds[nt][e] = qk ? p0 * (dp[nt][e] - dl) : 0.f;
+          ds[nt][e + 2] = qk ? p1 * (dp[nt][e + 2] - dl) : 0.f;
+        } else {
+          p0 = ok ? exp2f(fmaf(p[nt][e], scale_log2e, -m)) * il : 0.f;
+          p1 = ok ? exp2f(fmaf(p[nt][e + 2], scale_log2e, -m)) * il : 0.f;
+          ds[nt][e] = p0 * (dp[nt][e] - dl);
+          ds[nt][e + 2] = p1 * (dp[nt][e + 2] - dl);
+        }
         p[nt][e] = p0;
         p[nt][e + 2] = p1;
-        ds[nt][e] = p0 * (dp[nt][e] - dl);
-        ds[nt][e + 2] = p1 * (dp[nt][e + 2] - dl);
       }
     }
     float acc[DH / 8][4];
@@ -414,23 +465,26 @@ __global__ void __launch_bounds__(BwdCfg<DH, NP>::WARPS * 32) attention_bwd_mma_
   }
 }
 
-template <int DH, int NP>
-int launch_bwd(const void* qkv, const void* dout, void* dqkv, int n_seq, int n_tok, int heads, cudaStream_t st) {
+template <int DH, int NP, bool MASKED>
+int launch_bwd(const void* qkv, const void* dout, void* dqkv, int n_seq, int n_tok, int heads, const uint8_t* keep, cudaStream_t st) {
   const int n_problems = n_seq * heads;
   constexpr int kWarps = BwdCfg<DH, NP>::WARPS;
-  launch_pdl(attention_bwd_mma_kernel<DH, NP>, ceil_div(n_problems, kWarps), kWarps * 32, 0, st, static_cast<const __nv_bfloat16*>(qkv), static_cast<const __nv_bfloat16*>(dout), static_cast<__nv_bfloat16*>(dqkv), n_problems, n_tok, heads,
-      1.0f / sqrtf(float(DH)));
+  launch_pdl(attention_bwd_mma_kernel<DH, NP, MASKED>, ceil_div(n_problems, kWarps), kWarps * 32, 0, st, static_cast<const __nv_bfloat16*>(qkv), static_cast<const __nv_bfloat16*>(dout), static_cast<__nv_bfloat16*>(dqkv), n_problems, n_tok, heads,
+      1.0f / sqrtf(float(DH)), keep);
   AVF_LAUNCH_CHECK("attention_bwd_mma_kernel");
   return 0;
 }
 
 }  // namespace
 
-int attention_mma_bf16(const void* qkv, void* out, int n_seq, int n_tok, int heads, int dim_head, cudaStream_t st, int q_rows) {
+int attention_mma_bf16(const void* qkv, void* out, int n_seq, int n_tok, int heads, int dim_head, cudaStream_t st, int q_rows, const uint8_t* keep) {
   AVF_REQUIRE(n_tok >= 1 && n_tok <= 64, AVF_EUNSUPPORTED, "attention: n_tok=%d (1..64)", n_tok);
   if (q_rows <= 0 || q_rows > n_tok) q_rows = n_tok;
   const int np = (n_tok + 15) / 16 * 16;
-#define AVF_ATT(D, P) if (dim_head == D && np == P) return launch<D, P>(qkv, out, n_seq, n_tok, heads, q_rows, st);
+#define AVF_ATT(D, P)                                                                                   \
+  if (dim_head == D && np == P)                                                                         \
+    return keep ? launch<D, P, true>(qkv, out, n_seq, n_tok, heads, q_rows, keep, st)                   \
+                : launch<D, P, false>(qkv, out, n_seq, n_tok, heads, q_rows, nullptr, st);
   AVF_ATT(32, 16) AVF_ATT(32, 32) AVF_ATT(32, 48) AVF_ATT(32, 64)
   AVF_ATT(64, 16) AVF_ATT(64, 32) AVF_ATT(64, 48) AVF_ATT(64, 64)
 #undef AVF_ATT
@@ -441,10 +495,14 @@ int attention_mma_bf16(const void* qkv, void* out, int n_seq, int n_tok, int hea
 }  // namespace avf
 
 namespace avf {
-int attention_bwd_mma_bf16(const void* qkv, const void* dout, void* dqkv, int n_seq, int n_tok, int heads, int dim_head, cudaStream_t st) {
+int attention_bwd_mma_bf16(const void* qkv, const void* dout, void* dqkv, int n_seq, int n_tok, int heads, int dim_head, cudaStream_t st,
+                           const uint8_t* keep) {
   AVF_REQUIRE(n_tok >= 1 && n_tok <= 64, AVF_EUNSUPPORTED, "attention_bwd: n_tok=%d (1..64)", n_tok);
   const int np = (n_tok + 15) / 16 * 16;
-#define AVF_ATT(D, P) if (dim_head == D && np == P) return launch_bwd<D, P>(qkv, dout, dqkv, n_seq, n_tok, heads, st);
+#define AVF_ATT(D, P)                                                                                   \
+  if (dim_head == D && np == P)                                                                         \
+    return keep ? launch_bwd<D, P, true>(qkv, dout, dqkv, n_seq, n_tok, heads, keep, st)                \
+                : launch_bwd<D, P, false>(qkv, dout, dqkv, n_seq, n_tok, heads, nullptr, st);
   AVF_ATT(32, 16) AVF_ATT(32, 32) AVF_ATT(32, 48) AVF_ATT(32, 64)
   AVF_ATT(64, 16) AVF_ATT(64, 32) AVF_ATT(64, 48) AVF_ATT(64, 64)
 #undef AVF_ATT

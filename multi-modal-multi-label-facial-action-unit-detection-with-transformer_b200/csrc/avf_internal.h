@@ -35,7 +35,9 @@ int au_confusion(const float* pred, int ld_pred, float thresh, const float* labe
 // avf_simt.cu
 int linear_f32(const float* a, int lda, const float* w, const float* bias, const float* res, int ld_res, void* c, int ldc,
                int c_mode, int m, int n, int k, int flags, cudaStream_t st);
-int attention_small(int io_mode, const void* qkv, void* out, int n_seq, int n_tok, int heads, int dim_head, cudaStream_t st);
+// keep (optional): [n_seq, n_tok] uint8, 1 = keep; score (i, j) survives only when tokens i and j are both kept (include/avformer_b200.h).
+int attention_small(int io_mode, const void* qkv, void* out, int n_seq, int n_tok, int heads, int dim_head, cudaStream_t st,
+                    const uint8_t* keep = nullptr);
 
 int gemm_f32(int trans_a, int trans_b, const float* a, int lda, const float* w, int ldw, const float* bias, const float* res, int ld_res,
              float* aux, int ld_aux, void* c, int ldc, int c_mode, int m, int n, int k, int flags, cudaStream_t st, DropSpec drop = DropSpec{});
@@ -53,7 +55,8 @@ int layernorm_bwd(const float* x, int ld_x, const float* gamma, const float* dyn
 // y = x * mask(drop) as bf16 / fp32 (dense [rows, dim]); without dropout a plain cast / copy
 int masked_copy(const float* x, void* y, int y_mode, int rows, int dim, DropSpec drop, cudaStream_t st);
 int dropout_mask(float* out, int rows, int cols, DropSpec drop, cudaStream_t st);
-int attention_bwd(int io_mode, const void* qkv, const void* dout, void* dqkv, int n_seq, int n_tok, int heads, int dim_head, cudaStream_t st);
+int attention_bwd(int io_mode, const void* qkv, const void* dout, void* dqkv, int n_seq, int n_tok, int heads, int dim_head, cudaStream_t st,
+                  const uint8_t* keep = nullptr);
 int au_logits_bwd(const float* dl, int ld_dl, const float* x, int ld_x, const float* w_last, float* dx, int ld_dx, float* dw, int n_clips,
                   int dim, cudaStream_t st);
 int bn_train_fwd(int out_mode, const float* x, int ld_x, const float* g, const float* b, float* run_mean, float* run_var, float momentum,
@@ -64,8 +67,10 @@ int adam_step(float* p, const float* g, float* m, float* v, void* shadow, size_t
               int decoupled, float grad_scale, cudaStream_t st);
 
 // avf_attention_mma.cu
-int attention_mma_bf16(const void* qkv, void* out, int n_seq, int n_tok, int heads, int dim_head, cudaStream_t st, int q_rows = 0);
-int attention_bwd_mma_bf16(const void* qkv, const void* dout, void* dqkv, int n_seq, int n_tok, int heads, int dim_head, cudaStream_t st);
+int attention_mma_bf16(const void* qkv, void* out, int n_seq, int n_tok, int heads, int dim_head, cudaStream_t st, int q_rows = 0,
+                       const uint8_t* keep = nullptr);
+int attention_bwd_mma_bf16(const void* qkv, const void* dout, void* dqkv, int n_seq, int n_tok, int heads, int dim_head, cudaStream_t st,
+                           const uint8_t* keep = nullptr);
 
 // avf_layer_fused.cu: whole encoder stack in one persistent tcgen05 kernel (dim 256 or 128, 8 heads x 32)
 bool encoder_fused_supported(const avf_stack_shape* s);

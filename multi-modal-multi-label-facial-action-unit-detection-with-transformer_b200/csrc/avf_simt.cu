@@ -163,10 +163,13 @@ __device__ __forceinline__ void store_frag(T* __restrict__ p, const float (&src)
 // Small-sequence attention, models/heads.py:221-237.  qkv [rows, 3*H*dh] (columns q|k|v, head-major),
 // out [rows, H*dh].  A CTA stages K and V of `spb` sequences in shared memory; each thread owns one
 // (sequence, head, query) row and runs an online softmax in base 2 over the <= 64 keys.
+// MASKED: keep [n_seq, n_tok] uint8 (1 = keep); one warp per staged sequence turns its row into 64 keep bits (behind K|V in shared
+// memory).  A kept query skips the dropped keys; a dropped query attends uniformly to all n_tok keys (every score filled alike), so
+// its running max starts from a real score and never meets -INF - (-INF).
 // ---------------------------------------------------------------------------------------------
-template <typename T, int DH>
+template <typename T, int DH, bool MASKED>
 __global__ void __launch_bounds__(DH == 32 ? 512 : 256) attention_small_kernel(const T* __restrict__ qkv, T* __restrict__ out, int n_seq, int n_tok,
-                                                              int heads, int spb, int hpb, float scale_log2e) {
+                                                              int heads, int spb, int hpb, float scale_log2e, const uint8_t* __restrict__ keep) {
   pdl_wait();      // programmatic dependent launch: everything above is launch overhead hidden behind the previous kernel
   pdl_trigger();
   extern __shared__ uint8_t smem_attn[];
@@ -186,6 +189,16 @@ __global__ void __launch_bounds__(DH == 32 ? 512 : 256) attention_small_kernel(c
     const uint4 v = *reinterpret_cast<const uint4*>(qkv + (size_t(seq0) * n_tok + r) * (3 * inner) + size_t(1 + part) * inner + h0 * DH + col);
     *reinterpret_cast<uint4*>(kv + size_t(r) * 2 * w + c) = v;
   }
+  uint64_t* kmask = reinterpret_cast<uint64_t*>(kv + size_t(spb) * n_tok * 2 * w);     // [spb] keep bits (MASKED only)
+  if constexpr (MASKED) {
+    const int lane = threadIdx.x & 31;
+    for (int sl = threadIdx.x >> 5; sl < nseq_here; sl += blockDim.x >> 5) {
+      const uint8_t* row = keep + size_t(seq0 + sl) * n_tok;
+      const uint32_t lo = __ballot_sync(0xffffffffu, lane < n_tok && row[lane] != 0);
+      const uint32_t hi = __ballot_sync(0xffffffffu, lane + 32 < n_tok && row[lane + 32] != 0);
+      if (lane == 0) kmask[sl] = (uint64_t(hi) << 32) | lo;
+    }
+  }
   __syncthreads();
   const int items = nseq_here * nh * n_tok;
   for (int it = threadIdx.x; it < items; it += blockDim.x) {
@@ -201,13 +214,18 @@ __global__ void __launch_bounds__(DH == 32 ? 512 : 256) attention_small_kernel(c
 #pragma unroll
     for (int d = 0; d < DH; ++d) acc[d] = 0.f;
     const T* kbase = kv + size_t(sl) * n_tok * 2 * w + hl * DH;
+    const uint64_t km = MASKED ? kmask[sl] : 0;
+    const bool row_kept = !MASKED || ((km >> qi) & 1);
     for (int j = 0; j < n_tok; ++j) {
+      if (MASKED && row_kept && !((km >> j) & 1)) continue;
       const T* kp = kbase + size_t(j) * 2 * w;
       float kf[DH];
       load_frag<T, DH>(kp, kf);
       float s = 0.f;
+      if (row_kept) {
 #pragma unroll
-      for (int d = 0; d < DH; ++d) s = fmaf(q[d], kf[d], s);
+        for (int d = 0; d < DH; ++d) s = fmaf(q[d], kf[d], s);
+      }
       if (s > m) {
         const float corr = exp2f(m - s);
         l *= corr;
@@ -257,8 +275,8 @@ int gemm_f32(int trans_a, int trans_b, const float* a, int lda, const float* w, 
   return 0;
 }
 
-template <typename T, int DH>
-static int launch_attention(const void* qkv, void* out, int n_seq, int n_tok, int heads, cudaStream_t st) {
+template <typename T, int DH, bool MASKED>
+static int launch_attention(const void* qkv, void* out, int n_seq, int n_tok, int heads, const uint8_t* keep, cudaStream_t st) {
   const int inner = heads * DH;
   int hpb = heads;                                        // heads staged per block: all of them unless K|V of a sequence exceed 96 KB
   while (hpb > 1 && size_t(n_tok) * 2 * hpb * DH * sizeof(T) > 96 * 1024) hpb = (hpb + 1) / 2;
@@ -267,27 +285,31 @@ static int launch_attention(const void* qkv, void* out, int n_seq, int n_tok, in
   constexpr int kMaxThreads = DH == 32 ? 512 : 256;
   int spb = max(1, min(kMaxThreads / threads_per_seq, int((96 * 1024) / per_seq)));
   spb = min(spb, n_seq);
-  const size_t smem = per_seq * spb;
+  const size_t smem = per_seq * spb + (MASKED ? spb * sizeof(uint64_t) : 0);
   AVF_REQUIRE(smem <= 200 * 1024, AVF_EUNSUPPORTED, "attention: %d tokens x %d inner does not fit shared memory", n_tok, inner);
   int threads = min(kMaxThreads, ceil_div(threads_per_seq * spb, 32) * 32);
-  auto kern = attention_small_kernel<T, DH>;
+  auto kern = attention_small_kernel<T, DH, MASKED>;
   static PerDeviceOnce once;
   if (once.first()) {
     AVF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
   }
   const float scale_log2e = 1.4426950408889634f / sqrtf(float(DH));
   launch_pdl(kern, dim3(ceil_div(n_seq, spb), ceil_div(heads, hpb)), threads, smem, st, static_cast<const T*>(qkv), static_cast<T*>(out), n_seq, n_tok, heads, spb, hpb,
-                                                                               scale_log2e);
+                                                                               scale_log2e, keep);
   AVF_LAUNCH_CHECK("attention_small_kernel");
   return 0;
 }
 
-int attention_small(int io_mode, const void* qkv, void* out, int n_seq, int n_tok, int heads, int dim_head, cudaStream_t st) {
+int attention_small(int io_mode, const void* qkv, void* out, int n_seq, int n_tok, int heads, int dim_head, cudaStream_t st, const uint8_t* keep) {
   AVF_REQUIRE(n_seq > 0 && n_tok > 0 && heads > 0, AVF_EINVAL, "attention: n_seq=%d n_tok=%d heads=%d", n_seq, n_tok, heads);
   AVF_REQUIRE(dim_head == 32 || dim_head == 64, AVF_EUNSUPPORTED, "attention: dim_head=%d (supported: 32, 64)", dim_head);
-  if (io_mode == AVF_BF16) return attention_mma_bf16(qkv, out, n_seq, n_tok, heads, dim_head, st);   // tensor cores
-  return dim_head == 32 ? launch_attention<float, 32>(qkv, out, n_seq, n_tok, heads, st)
-                        : launch_attention<float, 64>(qkv, out, n_seq, n_tok, heads, st);
+  AVF_REQUIRE(keep == nullptr || n_tok <= 64, AVF_EUNSUPPORTED, "attention: a keep mask needs n_tok <= 64 (n_tok=%d)", n_tok);
+  if (io_mode == AVF_BF16) return attention_mma_bf16(qkv, out, n_seq, n_tok, heads, dim_head, st, 0, keep);   // tensor cores
+  if (keep != nullptr)
+    return dim_head == 32 ? launch_attention<float, 32, true>(qkv, out, n_seq, n_tok, heads, keep, st)
+                          : launch_attention<float, 64, true>(qkv, out, n_seq, n_tok, heads, keep, st);
+  return dim_head == 32 ? launch_attention<float, 32, false>(qkv, out, n_seq, n_tok, heads, nullptr, st)
+                        : launch_attention<float, 64, false>(qkv, out, n_seq, n_tok, heads, nullptr, st);
 }
 
 }  // namespace avf

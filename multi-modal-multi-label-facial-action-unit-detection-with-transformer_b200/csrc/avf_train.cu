@@ -267,10 +267,12 @@ __global__ void __launch_bounds__(256) dropout_mask_kernel(float* __restrict__ o
 // Attention backward (models/heads.py:221-237) for one (sequence, head) per CTA.  P is recomputed from q, k.
 //   dV = P^T dO;  dP = dO V^T;  dS = P o (dP - rowsum(P o dP));  dQ = scale dS K;  dK = scale dS^T Q
 // Sequences are 12 / 17 / 49 tokens: everything of one head lives in shared memory as fp32.
+// MASKED: keep [n_seq, n_tok] uint8 (1 = keep), turned into 64 keep bits by two ballots of every warp.  Scores of a kept query on
+// dropped keys are -INF (P = 0); a dropped query's scores are all equal (uniform P); dS = 0 on every filled score.
 // ---------------------------------------------------------------------------------------------
-template <typename T, int DH>
+template <typename T, int DH, bool MASKED>
 __global__ void __launch_bounds__(128) attention_bwd_kernel(const T* __restrict__ qkv, const T* __restrict__ dout, T* __restrict__ dqkv,
-                                                            int n_tok, int heads, float scale) {
+                                                            int n_tok, int heads, float scale, const uint8_t* __restrict__ keep) {
   pdl_wait();      // programmatic dependent launch: everything above is launch overhead hidden behind the previous kernel
   pdl_trigger();
   extern __shared__ float sm[];
@@ -285,6 +287,13 @@ __global__ void __launch_bounds__(128) attention_bwd_kernel(const T* __restrict_
   const int seq = blockIdx.x / heads, h = blockIdx.x - seq * heads;
   const int inner = heads * DH;
   const size_t row0 = size_t(seq) * N;
+  uint64_t km = 0;
+  if constexpr (MASKED) {
+    const int lane = threadIdx.x & 31;
+    const uint32_t lo = __ballot_sync(0xffffffffu, lane < N && keep[row0 + lane] != 0);
+    const uint32_t hi = __ballot_sync(0xffffffffu, lane + 32 < N && keep[row0 + lane + 32] != 0);
+    km = (uint64_t(hi) << 32) | lo;
+  }
   for (int i = threadIdx.x; i < N * DH; i += blockDim.x) {
     const int t = i / DH, d = i - t * DH;
     const T* qp = qkv + (row0 + t) * size_t(3 * inner) + h * DH + d;
@@ -302,7 +311,9 @@ __global__ void __launch_bounds__(128) attention_bwd_kernel(const T* __restrict_
       s = fmaf(sq[a * P + d], sk[b * P + d], s);
       dp = fmaf(sdo[a * P + d], sv[b * P + d], dp);
     }
-    sp[a * NP + b] = s * scale;
+    float v = s * scale;
+    if constexpr (MASKED) v = !((km >> a) & 1) ? 0.f : ((km >> b) & 1) ? v : -INFINITY;
+    sp[a * NP + b] = v;
     sds[a * NP + b] = dp;
   }
   __syncthreads();
@@ -326,7 +337,8 @@ __global__ void __launch_bounds__(128) attention_bwd_kernel(const T* __restrict_
       delta += p * sds[a * NP + b];
     }
     delta = warp_sum(delta);
-    for (int b = lane; b < N; b += 32) sds[a * NP + b] = sp[a * NP + b] * (sds[a * NP + b] - delta) * scale;
+    const bool filled_row = MASKED && !((km >> a) & 1);
+    for (int b = lane; b < N; b += 32) sds[a * NP + b] = filled_row ? 0.f : sp[a * NP + b] * (sds[a * NP + b] - delta) * scale;
   }
   __syncthreads();
   for (int i = threadIdx.x; i < N * DH; i += blockDim.x) {
@@ -595,27 +607,31 @@ int dropout_mask(float* out, int rows, int cols, DropSpec drop, cudaStream_t st)
   return 0;
 }
 
-template <typename T, int DH>
-static int launch_attention_bwd(const void* qkv, const void* dout, void* dqkv, int n_seq, int n_tok, int heads, cudaStream_t st) {
+template <typename T, int DH, bool MASKED>
+static int launch_attention_bwd(const void* qkv, const void* dout, void* dqkv, int n_seq, int n_tok, int heads, const uint8_t* keep, cudaStream_t st) {
   const size_t smem = (size_t(4) * n_tok * (DH + 1) + size_t(2) * n_tok * (n_tok + 1)) * sizeof(float);
   AVF_REQUIRE(smem <= 200 * 1024, AVF_EUNSUPPORTED, "attention_bwd: %d tokens x %d do not fit shared memory", n_tok, DH);
-  auto kern = attention_bwd_kernel<T, DH>;
+  auto kern = attention_bwd_kernel<T, DH, MASKED>;
   static PerDeviceOnce once;
   if (once.first()) {
     AVF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
   }
   launch_pdl(kern, n_seq * heads, 128, smem, st, static_cast<const T*>(qkv), static_cast<const T*>(dout), static_cast<T*>(dqkv), n_tok, heads,
-                                         rsqrtf(float(DH)));
+                                         rsqrtf(float(DH)), keep);
   AVF_LAUNCH_CHECK("attention_bwd_kernel");
   return 0;
 }
 
-int attention_bwd(int io_mode, const void* qkv, const void* dout, void* dqkv, int n_seq, int n_tok, int heads, int dim_head, cudaStream_t st) {
+int attention_bwd(int io_mode, const void* qkv, const void* dout, void* dqkv, int n_seq, int n_tok, int heads, int dim_head, cudaStream_t st,
+                  const uint8_t* keep) {
   AVF_REQUIRE(n_seq > 0 && n_tok > 0 && n_tok <= 64 && heads > 0, AVF_EINVAL, "attention_bwd: n_seq=%d n_tok=%d heads=%d", n_seq, n_tok, heads);
   AVF_REQUIRE(dim_head == 32 || dim_head == 64, AVF_EUNSUPPORTED, "attention_bwd: dim_head=%d (supported: 32, 64)", dim_head);
-  if (io_mode == AVF_BF16) return attention_bwd_mma_bf16(qkv, dout, dqkv, n_seq, n_tok, heads, dim_head, st);      // tensor cores
-  return dim_head == 32 ? launch_attention_bwd<float, 32>(qkv, dout, dqkv, n_seq, n_tok, heads, st)
-                        : launch_attention_bwd<float, 64>(qkv, dout, dqkv, n_seq, n_tok, heads, st);
+  if (io_mode == AVF_BF16) return attention_bwd_mma_bf16(qkv, dout, dqkv, n_seq, n_tok, heads, dim_head, st, keep);      // tensor cores
+  if (keep != nullptr)
+    return dim_head == 32 ? launch_attention_bwd<float, 32, true>(qkv, dout, dqkv, n_seq, n_tok, heads, keep, st)
+                          : launch_attention_bwd<float, 64, true>(qkv, dout, dqkv, n_seq, n_tok, heads, keep, st);
+  return dim_head == 32 ? launch_attention_bwd<float, 32, false>(qkv, dout, dqkv, n_seq, n_tok, heads, nullptr, st)
+                        : launch_attention_bwd<float, 64, false>(qkv, dout, dqkv, n_seq, n_tok, heads, nullptr, st);
 }
 
 int au_logits_bwd(const float* dl, int ld_dl, const float* x, int ld_x, const float* w_last, float* dx, int ld_dx, float* dw, int n_clips,

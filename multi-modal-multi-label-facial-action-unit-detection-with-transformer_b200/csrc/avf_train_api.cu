@@ -85,9 +85,11 @@ static int copy_rows(float* dst, int ld_dst, const float* src, int ld_src, int r
 
 // ---------------------------------------------------------------------------------------------
 // forward with tape:  the residual stream walks x_in(0) -> x_mid(0) -> x_in(1) -> ... -> out
+// keep (optional, [n_seq, n_tok] uint8): attention mask of every layer; the backward needs the same one
 // ---------------------------------------------------------------------------------------------
 static int encoder_fwd_train(int mode, const avf_stack_shape* s, const avf_layer_weights* L, const float* x, int ld_x, float* out, int ld_out,
-                             void* tape, size_t tape_bytes, float p_drop, uint64_t seed, const uint32_t* salt, cudaStream_t st) {
+                             void* tape, size_t tape_bytes, float p_drop, uint64_t seed, const uint32_t* salt, cudaStream_t st,
+                             const uint8_t* keep = nullptr) {
   int e = check_train_shape(s);
   if (e) return e;
   AVF_REQUIRE(p_drop >= 0.f && p_drop < 1.f, AVF_EINVAL, "dropout p=%f", p_drop);
@@ -106,7 +108,7 @@ static int encoder_fwd_train(int mode, const avf_stack_shape* s, const avf_layer
     const int ld_next = last ? ld_out : D;
     if ((e = layernorm(mode, t.x_in, D, W.ln1_gamma, W.ln1_beta, t.xn1, R, D, st))) return e;
     if ((e = gemm(mode, 0, 0, t.xn1, D, W.w_qkv, D, nullptr, nullptr, 0, nullptr, 0, t.qkv, 3 * I, mode, R, 3 * I, D, 0, nullptr, 0, st))) return e;
-    if ((e = attention_small(mode, t.qkv, t.o, s->n_seq, s->n_tok, s->heads, s->dim_head, st))) return e;
+    if ((e = attention_small(mode, t.qkv, t.o, s->n_seq, s->n_tok, s->heads, s->dim_head, st, keep))) return e;
     if ((e = gemm(mode, 0, 0, t.o, I, W.w_out, I, W.b_out, t.x_in, D, nullptr, 0, t.x_mid, D, AVF_FP32, R, D, I, AVF_EPI_BIAS | AVF_EPI_RESIDUAL,
                   nullptr, 0, st, drop_site(p_drop, seed, salt, l, 0))))
       return e;
@@ -159,7 +161,7 @@ static BwdWs carve_bwd_ws(const avf_stack_shape* s, int mode, void* base) {
 
 static int encoder_bwd(int mode, const avf_stack_shape* s, const avf_layer_weights* L, const void* tape, size_t tape_bytes, float* dx, int ld_dx,
                        const avf_layer_grads* G, int accumulate, void* ws, size_t ws_bytes, float p_drop, uint64_t seed, const uint32_t* salt,
-                       cudaStream_t st) {
+                       cudaStream_t st, const uint8_t* keep = nullptr) {
   int e = check_train_shape(s);
   if (e) return e;
   AVF_REQUIRE(p_drop >= 0.f && p_drop < 1.f, AVF_EINVAL, "dropout p=%f", p_drop);
@@ -202,7 +204,7 @@ static int encoder_bwd(int mode, const avf_stack_shape* s, const avf_layer_weigh
     // ---- attention sub-layer:  x_mid = x_in + Wo attn(Wqkv LN1(x_in)) + bo -----------------------------------
     if (g.w_out && (e = gemm(mode, 1, 1, dyb, ld_dyb, t.o, I, nullptr, nullptr, 0, nullptr, 0, g.w_out, I, AVF_FP32, D, I, R, wg, w.red, w.red_bytes, st))) return e;
     if ((e = gemm(mode, 0, 1, dyb, ld_dyb, W.w_out, I, nullptr, nullptr, 0, nullptr, 0, w.dob, I, mode, R, I, D, 0, nullptr, 0, st))) return e;
-    if ((e = attention_bwd(mode, t.qkv, w.dob, w.big, s->n_seq, s->n_tok, s->heads, s->dim_head, st))) return e;
+    if ((e = attention_bwd(mode, t.qkv, w.dob, w.big, s->n_seq, s->n_tok, s->heads, s->dim_head, st, keep))) return e;
     if (g.w_qkv && (e = gemm(mode, 1, 1, w.big, 3 * I, t.xn1, D, nullptr, nullptr, 0, nullptr, 0, g.w_qkv, D, AVF_FP32, 3 * I, D, R, wg, w.red, w.red_bytes, st))) return e;
     if ((e = gemm(mode, 0, 1, w.big, 3 * I, W.w_qkv, D, nullptr, nullptr, 0, nullptr, 0, w.dxn, D, AVF_FP32, R, D, 3 * I, 0, nullptr, 0, st))) return e;
     if ((e = layernorm_bwd(t.x_in, D, W.ln1_gamma, w.dxn, dx, ld_dx, dxb_out, mode, g.ln1_gamma, g.ln1_beta, g.b_out, beta, R, D, w.red, w.red_bytes, st,
@@ -255,6 +257,24 @@ int avf_encoder_stack_bwd(int mode, const avf_stack_shape* s, const avf_layer_we
                      static_cast<cudaStream_t>(stream));
 }
 
+int avf_encoder_stack_fwd_train_masked(int mode, const avf_stack_shape* s, const avf_layer_weights* layers, const uint8_t* keep, const float* x,
+                                       int32_t ld_x, float* out, int32_t ld_out, void* tape, size_t tape_bytes, float dropout_p, uint64_t dropout_seed,
+                                       const uint32_t* dropout_salt, void* stream) {
+  int e = require_device_train();
+  if (e) return e;
+  return encoder_fwd_train(mode, s, layers, x, ld_x, out, ld_out, tape, tape_bytes, dropout_p, dropout_seed, dropout_salt, static_cast<cudaStream_t>(stream),
+                           keep);
+}
+
+int avf_encoder_stack_bwd_masked(int mode, const avf_stack_shape* s, const avf_layer_weights* layers, const uint8_t* keep, const void* tape,
+                                 size_t tape_bytes, float* dx, int32_t ld_dx, const avf_layer_grads* grads, int accumulate, void* workspace,
+                                 size_t workspace_bytes, float dropout_p, uint64_t dropout_seed, const uint32_t* dropout_salt, void* stream) {
+  int e = require_device_train();
+  if (e) return e;
+  return encoder_bwd(mode, s, layers, tape, tape_bytes, dx, ld_dx, grads, accumulate, workspace, workspace_bytes, dropout_p, dropout_seed, dropout_salt,
+                     static_cast<cudaStream_t>(stream), keep);
+}
+
 int avf_dropout_mask(float dropout_p, uint64_t dropout_seed, const uint32_t* dropout_salt, int32_t layer, int32_t site, int32_t rows,
                      int32_t cols, float* out, void* stream) {
   int e = require_device_train();
@@ -303,6 +323,14 @@ int avf_attention_bwd(int io_mode, const void* qkv, const void* dout, void* dqkv
   if (e) return e;
   AVF_REQUIRE(qkv && dout && dqkv, AVF_EINVAL, "attention_bwd: null pointer");
   return attention_bwd(io_mode, qkv, dout, dqkv, n_seq, n_tok, heads, dim_head, static_cast<cudaStream_t>(stream));
+}
+
+int avf_attention_bwd_masked(int io_mode, const void* qkv, const void* dout, void* dqkv, int32_t n_seq, int32_t n_tok, int32_t heads, int32_t dim_head,
+                             const uint8_t* keep, void* stream) {
+  int e = require_device_train();
+  if (e) return e;
+  AVF_REQUIRE(qkv && dout && dqkv, AVF_EINVAL, "attention_bwd: null pointer");
+  return attention_bwd(io_mode, qkv, dout, dqkv, n_seq, n_tok, heads, dim_head, static_cast<cudaStream_t>(stream), keep);
 }
 
 /* ---- AU_former front end with tape ------------------------------------------------------------------------- */

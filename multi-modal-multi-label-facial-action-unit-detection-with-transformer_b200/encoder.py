@@ -109,15 +109,15 @@ class Attention(nn.Module):
         self.to_out = nn.Sequential(nn.Linear(inner, dim), nn.Dropout(dropout)) if project_out else nn.Identity()
 
     def forward(self, x, mask=None):
-        if mask is not None:
-            raise NotImplementedError("attention masks are never passed on the AVFormer path (models/heads.py:225-232 is dead code)")
+        """x [b, n, dim]; ``mask`` (optional) bool [b, n - 1], True = keep: see Transformer.forward."""
         prec = default_precision()
         cast = AF.to_bf16 if prec == "bf16" else (lambda t: t.detach().float())
         b, n, _ = x.shape
+        keep = None if mask is None else AF.keep_from_mask(mask, b, n)
         a = x.reshape(b * n, -1)
         a = a if a.dtype == (torch.bfloat16 if prec == "bf16" else torch.float32) else cast(a)
         qkv = AF.linear_fwd(a, cast(self.to_qkv.weight), out_dtype=a.dtype, precision=prec)
-        o = AF.attention_fwd(qkv, b, n, self.heads, self.dim_head)
+        o = AF.attention_fwd(qkv, b, n, self.heads, self.dim_head, keep)
         if isinstance(self.to_out, nn.Identity):
             return AF.to_f32(o).view(b, n, -1) if o.dtype != torch.float32 else o.view(b, n, -1)
         y = AF.linear_fwd(o, cast(self.to_out[0].weight), self.to_out[0].bias, out_dtype=torch.float32, precision=prec)
@@ -180,33 +180,41 @@ class Transformer(nn.Module):
 
     # -- forward -------------------------------------------------------------------------------
     def forward_(self, x2d: torch.Tensor, n_seq: int, n_tok: int, out: Optional[torch.Tensor] = None, ld_out: int = 0,
-                 pos: Optional[torch.Tensor] = None) -> torch.Tensor:
+                 pos: Optional[torch.Tensor] = None, keep: Optional[torch.Tensor] = None) -> torch.Tensor:
         """Inference kernels, in place on an fp32 residual stream [n_seq*n_tok, dim] (+ pos [n_tok, dim] first, if given).  In
         train() mode with dropout > 0 (a frozen sub-model inside a training loop, models/avformer.py:78-85 + train.py:327) the
-        tape-keeping kernels run instead, because they are the ones that apply dropout."""
+        tape-keeping kernels run instead, because they are the ones that apply dropout.  ``keep`` [n_seq, n_tok] bool: attention
+        mask of every layer (AF.keep_from_mask); a masked stack runs kernel by kernel, never as the fused kernel."""
         p, seed, salt = self.dropout_state()
         if p > 0.0:
             if pos is not None:
                 AF.add_row_periodic_(x2d, pos, n_tok)
-            y, _ = AF.encoder_stack_fwd_train(x2d, self.packed(), self.shape(n_seq, n_tok), p, seed, salt)
+            y, _ = AF.encoder_stack_fwd_train(x2d, self.packed(), self.shape(n_seq, n_tok), p, seed, salt, keep=keep)
             if out is None:
                 x2d.copy_(y)
                 return x2d
             torch.as_strided(out, (y.shape[0], y.shape[1]), (ld_out, 1)).copy_(y)
             return out
-        return AF.token_stack_fwd_(x2d, self.packed(), self.shape(n_seq, n_tok), pos, out, ld_out)
+        if keep is None:
+            return AF.token_stack_fwd_(x2d, self.packed(), self.shape(n_seq, n_tok), pos, out, ld_out)
+        if pos is not None:
+            AF.add_row_periodic_(x2d, pos, n_tok)
+        return AF.encoder_stack_fwd_(x2d, self.packed(), self.shape(n_seq, n_tok), out, ld_out, keep=keep)
 
-    def forward_train(self, x2d: torch.Tensor, n_seq: int, n_tok: int) -> torch.Tensor:
+    def forward_train(self, x2d: torch.Tensor, n_seq: int, n_tok: int, keep: Optional[torch.Tensor] = None) -> torch.Tensor:
         """Autograd-visible forward on an fp32 token matrix [n_seq*n_tok, dim] (activation tape kept for backward)."""
         from .autograd import EncoderStackFn
-        return EncoderStackFn.apply(x2d, self, n_seq, n_tok, *self.param_list())
+        return EncoderStackFn.apply(x2d, self, n_seq, n_tok, keep, *self.param_list())
 
     def forward(self, x: torch.Tensor, mask=None) -> torch.Tensor:
-        if mask is not None:
-            raise NotImplementedError("attention masks are never passed on the AVFormer path (models/heads.py:225-232 is dead code)")
+        """x [b, n, dim].  ``mask`` (optional): bool [b, n - 1] on x's device, True = keep; the first (cls) token is always kept.  Score
+        (i, j) of every head of sequence b survives iff tokens i and j are both kept, in every layer: a kept token attends only to
+        kept tokens, a dropped token attends uniformly to all n tokens (models/heads.py:225-234 in its ViT form).  Any other mask
+        shape raises NotImplementedError, a non-bool mask TypeError, a mask off the input's CUDA device RuntimeError."""
         AF._cuda(x, "x")
         b, n, d = x.shape
+        keep = None if mask is None else AF.keep_from_mask(mask, b, n)
         if needs_grad(self, x):
-            return self.forward_train(x.reshape(b * n, d), b, n).view(b, n, d)
+            return self.forward_train(x.reshape(b * n, d), b, n, keep).view(b, n, d)
         y = x.detach().float().reshape(b * n, d).clone()
-        return self.forward_(y, b, n).view(b, n, d)
+        return self.forward_(y, b, n, keep=keep).view(b, n, d)

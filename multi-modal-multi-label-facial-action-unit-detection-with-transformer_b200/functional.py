@@ -52,6 +52,27 @@ def _stream():
     return ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)
 
 
+def keep_from_mask(mask, n_seq: int, n_tok: int) -> torch.Tensor:
+    """The attention ``mask`` of Transformer.forward (models/heads.py:225-232): bool [n_seq, n_tok - 1], True = keep, on the input's
+    CUDA device.  Returns the keep rows of the C ABI, bool [n_seq, n_tok] with the first (cls) token always kept; a bool tensor is one
+    byte per element, so it is passed to the library as is."""
+    shape = tuple(mask.shape) if torch.is_tensor(mask) else type(mask).__name__
+    if shape != (n_seq, n_tok - 1):
+        raise NotImplementedError(f"attention mask of shape {shape} for {n_seq} sequences of {n_tok} tokens: only the per-sequence keep mask "
+                                  f"[{n_seq}, {n_tok - 1}] (bool, True = keep; the first token is always kept) is implemented")
+    if mask.dtype != torch.bool:
+        raise TypeError(f"avformer_b200: the attention mask must be a bool tensor (True = keep), got {mask.dtype}")
+    _cuda(mask, "mask")
+    return torch.nn.functional.pad(mask, (1, 0), value=True)
+
+
+def _keep_ptr(keep: Optional[torch.Tensor], n_seq: int, n_tok: int):
+    """Pointer of a keep array [n_seq, n_tok] (bool or uint8, 1 = keep) for the *_masked entry points."""
+    if keep.dtype not in (torch.bool, torch.uint8) or tuple(keep.shape) != (n_seq, n_tok) or not keep.is_contiguous():
+        raise ValueError(f"avformer_b200: keep must be a contiguous bool / uint8 tensor [{n_seq}, {n_tok}], got {keep.dtype} {tuple(keep.shape)}")
+    return _ptr(_cuda(keep, "keep"))
+
+
 def _f32c(t: torch.Tensor) -> torch.Tensor:
     t = t.detach()
     return t if (t.dtype == torch.float32 and t.is_contiguous()) else t.float().contiguous()
@@ -144,17 +165,22 @@ def make_shape(n_seq, n_tok, dim, heads, dim_head, mlp_dim, depth) -> StackShape
 
 
 def encoder_stack_fwd_(x: torch.Tensor, packed: PackedStack, shape: StackShape, out: Optional[torch.Tensor] = None,
-                       ld_out: int = 0) -> torch.Tensor:
+                       ld_out: int = 0, keep: Optional[torch.Tensor] = None) -> torch.Tensor:
     """In-place encoder stack on the fp32 residual stream x [n_seq*n_tok, dim] (row stride = x.stride(0)).
-    If ``out`` is given the last layer writes there (row stride ld_out) instead."""
+    If ``out`` is given the last layer writes there (row stride ld_out) instead.  ``keep`` [n_seq, n_tok] (bool / uint8, 1 = keep):
+    attention mask of every layer (avf_encoder_stack_fwd_masked)."""
     _cuda(x, "x")
     if x.dtype != torch.float32 or x.stride(-1) != 1:
         raise TypeError("encoder_stack_fwd_: x must be a float32 residual stream with unit column stride")
     L = _lib.lib()
     need = L.avf_encoder_workspace_bytes(ctypes.byref(shape), packed.mode)
     ws = workspace(need, x.device)
-    check(L.avf_encoder_stack_fwd(packed.mode, ctypes.byref(shape), packed.array, _ptr(x), x.stride(0), _ptr(out), ld_out,
-                                  _ptr(ws), ws.numel(), _stream()), "encoder_stack_fwd")
+    if keep is None:
+        check(L.avf_encoder_stack_fwd(packed.mode, ctypes.byref(shape), packed.array, _ptr(x), x.stride(0), _ptr(out), ld_out,
+                                      _ptr(ws), ws.numel(), _stream()), "encoder_stack_fwd")
+    else:
+        check(L.avf_encoder_stack_fwd_masked(packed.mode, ctypes.byref(shape), packed.array, _keep_ptr(keep, shape.n_seq, shape.n_tok), _ptr(x),
+                                             x.stride(0), _ptr(out), ld_out, _ptr(ws), ws.numel(), _stream()), "encoder_stack_fwd_masked")
     return x if out is None else out
 
 
@@ -211,10 +237,15 @@ def linear_fwd(a: torch.Tensor, w: torch.Tensor, bias: Optional[torch.Tensor] = 
     return c
 
 
-def attention_fwd(qkv: torch.Tensor, n_seq: int, n_tok: int, heads: int, dim_head: int) -> torch.Tensor:
+def attention_fwd(qkv: torch.Tensor, n_seq: int, n_tok: int, heads: int, dim_head: int, keep: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """softmax(q k^T / sqrt(dh)) v per (sequence, head); ``keep`` [n_seq, n_tok] (bool / uint8, 1 = keep) masks the scores."""
     qkv = _cuda(qkv, "qkv").contiguous()
     out = torch.empty((n_seq * n_tok, heads * dim_head), dtype=qkv.dtype, device=qkv.device)
-    check(_lib.lib().avf_attention_fwd(_io_mode(qkv), _ptr(qkv), _ptr(out), n_seq, n_tok, heads, dim_head, _stream()), "attention_fwd")
+    if keep is None:
+        check(_lib.lib().avf_attention_fwd(_io_mode(qkv), _ptr(qkv), _ptr(out), n_seq, n_tok, heads, dim_head, _stream()), "attention_fwd")
+    else:
+        check(_lib.lib().avf_attention_fwd_masked(_io_mode(qkv), _ptr(qkv), _ptr(out), n_seq, n_tok, heads, dim_head, _keep_ptr(keep, n_seq, n_tok),
+                                                  _stream()), "attention_fwd_masked")
     return out
 
 
@@ -249,14 +280,21 @@ def tformer_embed(frames: torch.Tensor, cls_token: torch.Tensor, pos: torch.Tens
     return x
 
 
-def tformer_fwd(frames: torch.Tensor, cls_token: torch.Tensor, pos: torch.Tensor, packed: PackedStack, shape: StackShape) -> torch.Tensor:
-    """Inference TFormer in one call: frames [n_clips*T, dim] -> cls features [n_clips, dim] fp32 (last layer on the cls rows only)."""
+def tformer_fwd(frames: torch.Tensor, cls_token: torch.Tensor, pos: torch.Tensor, packed: PackedStack, shape: StackShape,
+                keep: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """Inference TFormer in one call: frames [n_clips*T, dim] -> cls features [n_clips, dim] fp32 (last layer on the cls rows only).
+    ``keep`` [n_clips, T+1] (bool / uint8, 1 = keep; column 0 is the cls token): attention mask of every layer."""
     frames = _cuda(frames, "frames").contiguous()
     cls = torch.empty((shape.n_seq, shape.dim), dtype=torch.float32, device=frames.device)
     L = _lib.lib()
     ws = workspace(L.avf_tformer_workspace_bytes(ctypes.byref(shape), packed.mode), frames.device)
-    check(L.avf_tformer_fwd(packed.mode, _io_mode(frames), ctypes.byref(shape), packed.array, _ptr(frames), _ptr(_f32c(cls_token)), _ptr(_f32c(pos)),
-                            _ptr(cls), _ptr(ws), ws.numel(), _stream()), "tformer_fwd")
+    if keep is None:
+        check(L.avf_tformer_fwd(packed.mode, _io_mode(frames), ctypes.byref(shape), packed.array, _ptr(frames), _ptr(_f32c(cls_token)), _ptr(_f32c(pos)),
+                                _ptr(cls), _ptr(ws), ws.numel(), _stream()), "tformer_fwd")
+    else:
+        check(L.avf_tformer_fwd_masked(packed.mode, _io_mode(frames), ctypes.byref(shape), packed.array, _keep_ptr(keep, shape.n_seq, shape.n_tok),
+                                       _ptr(frames), _ptr(_f32c(cls_token)), _ptr(_f32c(pos)), _ptr(cls), _ptr(ws), ws.numel(), _stream()),
+              "tformer_fwd_masked")
     return cls
 
 
@@ -398,38 +436,50 @@ def layernorm_bwd_(x: torch.Tensor, gamma: torch.Tensor, dy_norm: torch.Tensor, 
     return dres, xb, dg, db, dbias
 
 
-def attention_bwd(qkv: torch.Tensor, dout: torch.Tensor, n_seq: int, n_tok: int, heads: int, dim_head: int) -> torch.Tensor:
+def attention_bwd(qkv: torch.Tensor, dout: torch.Tensor, n_seq: int, n_tok: int, heads: int, dim_head: int,
+                  keep: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """dqkv of attention_fwd (softmax recomputed); ``keep`` must be the mask of the forward."""
     qkv, dout = _cuda(qkv, "qkv").contiguous(), dout.contiguous()
     dqkv = torch.empty_like(qkv)
-    check(_lib.lib().avf_attention_bwd(_io_mode(qkv), _ptr(qkv), _ptr(dout), _ptr(dqkv), n_seq, n_tok, heads, dim_head, _stream()), "attention_bwd")
+    if keep is None:
+        check(_lib.lib().avf_attention_bwd(_io_mode(qkv), _ptr(qkv), _ptr(dout), _ptr(dqkv), n_seq, n_tok, heads, dim_head, _stream()), "attention_bwd")
+    else:
+        check(_lib.lib().avf_attention_bwd_masked(_io_mode(qkv), _ptr(qkv), _ptr(dout), _ptr(dqkv), n_seq, n_tok, heads, dim_head,
+                                                  _keep_ptr(keep, n_seq, n_tok), _stream()), "attention_bwd_masked")
     return dqkv
 
 
 def encoder_stack_fwd_train(x: torch.Tensor, packed: PackedStack, shape: StackShape, dropout_p: float = 0.0, dropout_seed: int = 0,
-                            dropout_salt: Optional[torch.Tensor] = None):
+                            dropout_salt: Optional[torch.Tensor] = None, keep: Optional[torch.Tensor] = None):
     """Forward of a whole stack that keeps the activations the backward needs.  x [n_seq*n_tok, dim] fp32 is left
     untouched; returns (y, tape).  dropout_p > 0 applies the reference's three dropout sites per layer with masks derived from
-    dropout_seed (give the same pair to encoder_stack_bwd_)."""
+    dropout_seed (give the same pair to encoder_stack_bwd_).  ``keep`` [n_seq, n_tok] (bool / uint8, 1 = keep): attention mask of
+    every layer; give the same tensor to encoder_stack_bwd_."""
     _cuda(x, "x")
     if x.dtype != torch.float32 or x.stride(-1) != 1:
         raise TypeError("encoder_stack_fwd_train: x must be a float32 residual stream with unit column stride")
     L = _lib.lib()
     tape = torch.empty(L.avf_encoder_tape_bytes(ctypes.byref(shape), packed.mode), dtype=torch.uint8, device=x.device)
     y = torch.empty((x.shape[0], shape.dim), dtype=torch.float32, device=x.device)
-    check(L.avf_encoder_stack_fwd_train(packed.mode, ctypes.byref(shape), packed.array, _ptr(x), x.stride(0), _ptr(y), shape.dim, _ptr(tape),
-                                        tape.numel(), float(dropout_p), int(dropout_seed), _ptr(dropout_salt), _stream()), "encoder_stack_fwd_train")
+    if keep is None:
+        check(L.avf_encoder_stack_fwd_train(packed.mode, ctypes.byref(shape), packed.array, _ptr(x), x.stride(0), _ptr(y), shape.dim, _ptr(tape),
+                                            tape.numel(), float(dropout_p), int(dropout_seed), _ptr(dropout_salt), _stream()), "encoder_stack_fwd_train")
+    else:
+        check(L.avf_encoder_stack_fwd_train_masked(packed.mode, ctypes.byref(shape), packed.array, _keep_ptr(keep, shape.n_seq, shape.n_tok), _ptr(x),
+                                                   x.stride(0), _ptr(y), shape.dim, _ptr(tape), tape.numel(), float(dropout_p), int(dropout_seed),
+                                                   _ptr(dropout_salt), _stream()), "encoder_stack_fwd_train_masked")
     return y, tape
 
 
 def encoder_stack_bwd_(dx: torch.Tensor, packed: PackedStack, shape: StackShape, tape: torch.Tensor, want: Sequence[bool],
                        dropout_p: float = 0.0, dropout_seed: int = 0, dropout_salt: Optional[torch.Tensor] = None,
-                       into: Optional[Sequence[Optional[torch.Tensor]]] = None):
+                       into: Optional[Sequence[Optional[torch.Tensor]]] = None, keep: Optional[torch.Tensor] = None):
     """dx [rows, dim] fp32 dense: dL/dy on entry, dL/dx on return.  ``want`` has 11*depth flags in avf_layer_weights
     order; returns the matching list of fp32 gradient tensors (None where not wanted).
 
     ``into`` (optional, same order): existing fp32 contiguous gradient buffers — typically the ``p.grad`` views of the
     optimiser's flat bucket.  When every wanted gradient has one, the kernels ACCUMULATE straight into them and the returned
-    list holds None throughout (nothing left for autograd to add)."""
+    list holds None throughout (nothing left for autograd to add).  ``keep``: the attention mask of the forward, if it had one."""
     from ._lib import LayerGrads
     names = [n for n, _ in LayerWeights._fields_]
     n_par = packed.depth * len(names)
@@ -447,9 +497,14 @@ def encoder_stack_bwd_(dx: torch.Tensor, packed: PackedStack, shape: StackShape,
             setattr(arr[l], name, g.data_ptr() if g is not None else None)
     L = _lib.lib()
     ws = workspace(L.avf_encoder_bwd_workspace_bytes(ctypes.byref(shape), packed.mode), dx.device)
-    check(L.avf_encoder_stack_bwd(packed.mode, ctypes.byref(shape), packed.array, _ptr(tape), tape.numel(), _ptr(dx), dx.stride(0), arr,
-                                  1 if direct else 0, _ptr(ws), ws.numel(), float(dropout_p), int(dropout_seed), _ptr(dropout_salt), _stream()),
-          "encoder_stack_bwd")
+    if keep is None:
+        check(L.avf_encoder_stack_bwd(packed.mode, ctypes.byref(shape), packed.array, _ptr(tape), tape.numel(), _ptr(dx), dx.stride(0), arr,
+                                      1 if direct else 0, _ptr(ws), ws.numel(), float(dropout_p), int(dropout_seed), _ptr(dropout_salt), _stream()),
+              "encoder_stack_bwd")
+    else:
+        check(L.avf_encoder_stack_bwd_masked(packed.mode, ctypes.byref(shape), packed.array, _keep_ptr(keep, shape.n_seq, shape.n_tok), _ptr(tape),
+                                             tape.numel(), _ptr(dx), dx.stride(0), arr, 1 if direct else 0, _ptr(ws), ws.numel(), float(dropout_p),
+                                             int(dropout_seed), _ptr(dropout_salt), _stream()), "encoder_stack_bwd_masked")
     return dx, grads
 
 

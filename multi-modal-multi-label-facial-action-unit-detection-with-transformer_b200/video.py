@@ -137,38 +137,44 @@ class TFormer(nn.Module):
         self.pos_embedding = nn.Parameter(torch.randn(1, num_patches + 1, dim))
         self.spatial_transformer = Transformer(dim, depth, heads, dim_head, mlp_dim, dropout)
 
-    def tokens(self, x):
-        """Embedded + encoded tokens [n_clips*(T+1), dim] (fp32) and n_clips; the cls rows are rows c*(T+1)."""
+    def _n_clips(self, x) -> int:
         AF._cuda(x, "x")
         if x.numel() % (self.num_patches * self.dim) != 0:
             raise ValueError(f"TFormer(num_patches={self.num_patches}): input of {tuple(x.shape)} is not a whole number of clips")
-        n_clips = x.numel() // (self.num_patches * self.dim)
+        return x.numel() // (self.num_patches * self.dim)
+
+    def tokens(self, x, mask=None):
+        """Embedded + encoded tokens [n_clips*(T+1), dim] (fp32) and n_clips; the cls rows are rows c*(T+1).  ``mask`` (optional):
+        frames kept, bool [n_clips, T] (True = a real frame), the attention mask of every layer (Transformer.forward)."""
+        n_clips = self._n_clips(x)
+        keep = None if mask is None else AF.keep_from_mask(mask, n_clips, self.num_patches + 1)
         if needs_grad(self, x):
             from .autograd import TFormerEmbedFn
             tok = TFormerEmbedFn.apply(x, self.cls_token, self.pos_embedding, self.num_patches)
-            return self.spatial_transformer.forward_train(tok, n_clips, self.num_patches + 1), n_clips
+            return self.spatial_transformer.forward_train(tok, n_clips, self.num_patches + 1, keep), n_clips
         tok = AF.tformer_embed(x.detach(), self.cls_token.view(-1), self.pos_embedding[0], self.num_patches)
-        self.spatial_transformer.forward_(tok, n_clips, self.num_patches + 1)
+        self.spatial_transformer.forward_(tok, n_clips, self.num_patches + 1, keep=keep)
         return tok, n_clips
 
-    def cls_features(self, x):
+    def cls_features(self, x, mask=None):
         """Inference: cls features [n_clips, dim] fp32 in one library call; the last layer runs its post-softmax part on the cls rows
-        only (the other rows never leave the module, models/vformer.py:290)."""
-        AF._cuda(x, "x")
-        if x.numel() % (self.num_patches * self.dim) != 0:
-            raise ValueError(f"TFormer(num_patches={self.num_patches}): input of {tuple(x.shape)} is not a whole number of clips")
-        n_clips = x.numel() // (self.num_patches * self.dim)
+        only (the other rows never leave the module, models/vformer.py:290).  ``mask``: frames kept, as in tokens()."""
+        n_clips = self._n_clips(x)
         st = self.spatial_transformer
         if st.dropout_state()[0] > 0.0:                 # train() with dropout: the tape-keeping kernels apply it
-            tok, _ = self.tokens(x)
+            tok, _ = self.tokens(x, mask)
             return AF.tformer_cls_extract(tok, n_clips, self.num_patches + 1)
-        return AF.tformer_fwd(x.detach(), self.cls_token.view(-1), self.pos_embedding[0], st.packed(), st.shape(n_clips, self.num_patches + 1))
+        keep = None if mask is None else AF.keep_from_mask(mask, n_clips, self.num_patches + 1)
+        return AF.tformer_fwd(x.detach(), self.cls_token.view(-1), self.pos_embedding[0], st.packed(), st.shape(n_clips, self.num_patches + 1),
+                              keep)
 
-    def forward(self, x):
+    def forward(self, x, mask=None):
+        """x [n_clips*T, dim] frame features -> cls features [n_clips, dim].  ``mask`` (optional): bool [n_clips, T], True = a real
+        frame; clips with fewer real frames can share a batch with full ones (the padding frames' values do not matter)."""
         if needs_grad(self, x):
-            tok, n_clips = self.tokens(x)
+            tok, n_clips = self.tokens(x, mask)
             return tok.view(n_clips, self.num_patches + 1, self.dim)[:, 0]          # cls rows (a view: data movement only)
-        return self.cls_features(x)
+        return self.cls_features(x, mask)
 
 
 class VideoModel(nn.Module):
