@@ -371,6 +371,20 @@ int avf_tformer_fwd_masked(int mode, int io_mode, const avf_stack_shape* s, cons
                            const void* frames, const float* cls_token, const float* pos, float* cls_out,
                            void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---- whole-video inference: TFormer clips gathered from a per-video frame bank (models/vformer.py:280-290) --------------------
+ * bank [n_bank, dim] DEVICE, contiguous, fp32 or bf16 per io_mode (16- / 8-byte aligned): the frame features of one video, each
+ * frame computed once.  index [n_clips, T] DEVICE int32: clip c's slot t is frame index[c*T + t].  s->n_seq = n_clips,
+ * s->n_tok = T+1.  An entry outside [0, n_bank) is a MISSING frame: its token is pos[1+t] alone and it is masked out of every layer
+ * (keep of avf_tformer_fwd_masked, with the cls slot kept); the bank is never read outside [0, n_bank), whatever the index holds.
+ * The gather, the keep rows and the embed are one launch; the layers always run masked, so the result equals avf_tformer_fwd_masked
+ * on the gathered frames (any value in the missing slots) with keep = (0 <= index < n_bank).  Inference only; the workspace is
+ * avf_tformer_workspace_bytes plus the keep rows. */
+size_t avf_tformer_indexed_workspace_bytes(const avf_stack_shape* s, int mode);
+int avf_tformer_fwd_indexed(int mode, int io_mode, const avf_stack_shape* s, const avf_layer_weights* layers,
+                            const void* bank, int32_t n_bank, const int32_t* index,
+                            const float* cls_token, const float* pos, float* cls_out,
+                            void* workspace, size_t workspace_bytes, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

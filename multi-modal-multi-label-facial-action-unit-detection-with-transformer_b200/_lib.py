@@ -134,6 +134,10 @@ SIGNATURES = {
                                                     _c_p]),
     "avf_tformer_fwd_masked": (ctypes.c_int, [ctypes.c_int, ctypes.c_int, ctypes.POINTER(StackShape), ctypes.POINTER(LayerWeights), _c_p, _c_p,
                                               _c_p, _c_p, _c_p, _c_p, _sz, _c_p]),
+    # ---- whole-video inference: TFormer clips gathered from a frame bank ----
+    "avf_tformer_indexed_workspace_bytes": (_sz, [ctypes.POINTER(StackShape), ctypes.c_int]),
+    "avf_tformer_fwd_indexed": (ctypes.c_int, [ctypes.c_int, ctypes.c_int, ctypes.POINTER(StackShape), ctypes.POINTER(LayerWeights), _c_p, _i32, _c_p,
+                                               _c_p, _c_p, _c_p, _c_p, _sz, _c_p]),
 }
 
 _lock = threading.Lock()

@@ -143,14 +143,21 @@ static int encoder_stack(int mode, const avf_stack_shape* s, const avf_layer_wei
   return 0;
 }
 
-static int tformer_fwd(int mode, int io_mode, const avf_stack_shape* s, const avf_layer_weights* layers, const void* frames, const float* cls_token,
-                       const float* pos, float* cls_out, void* workspace, size_t workspace_bytes, const uint8_t* keep, cudaStream_t st) {
+// Checks shared by the TFormer entry points; `in` is the frames or the frame bank, `need` the workspace the entry point carves.
+static int tformer_check(const avf_stack_shape* s, const avf_layer_weights* layers, const void* in, const float* cls_token, const float* pos,
+                         const float* cls_out, const void* workspace, size_t workspace_bytes, size_t need) {
   int e = check_shape(s);
   if (e) return e;
-  AVF_REQUIRE(layers && frames && cls_token && pos && cls_out && workspace, AVF_EINVAL, "tformer_fwd: null pointer");
+  AVF_REQUIRE(layers && in && cls_token && pos && cls_out && workspace, AVF_EINVAL, "tformer_fwd: null pointer");
   AVF_REQUIRE(s->n_tok >= 2, AVF_EINVAL, "tformer_fwd: n_tok=%d (cls + at least one frame)", s->n_tok);
-  const size_t need = avf_tformer_workspace_bytes(s, mode);
   AVF_REQUIRE(workspace_bytes >= need, AVF_EWORKSPACE, "workspace too small: %zu < %zu bytes", workspace_bytes, need);
+  return 0;
+}
+
+// The layers of the TFormer on the embedded tokens x [n_seq*n_tok, dim] fp32 that start the workspace -> cls_out.
+static int tformer_layers(int mode, const avf_stack_shape* s, const avf_layer_weights* layers, void* workspace, float* cls_out, const uint8_t* keep,
+                          cudaStream_t st) {
+  int e = 0;
   const int B = s->n_seq, N = s->n_tok, R = B * N, D = s->dim, I = s->heads * s->dim_head, M = s->mlp_dim;
   uint8_t* p = static_cast<uint8_t*>(workspace);
   float* x = reinterpret_cast<float*>(p);   p += align_up(size_t(R) * D * 4);
@@ -161,7 +168,6 @@ static int tformer_fwd(int mode, int io_mode, const avf_stack_shape* s, const av
   void* lnc = p;                            p += align_up(size_t(B) * D * elt(mode));
   void* oc = p;                             p += align_up(size_t(B) * I * elt(mode));
   void* hc = p;
-  if ((e = tformer_embed(io_mode, frames, cls_token, pos, x, B, N - 1, D, st))) return e;
   if (s->depth > 1) {
     avf_stack_shape head = *s;
     head.depth = s->depth - 1;
@@ -183,6 +189,28 @@ static int tformer_fwd(int mode, int io_mode, const avf_stack_shape* s, const av
   if ((e = layernorm(mode, xc, D, W.ln2_gamma, W.ln2_beta, lnc, B, D, st))) return e;
   if ((e = linear(mode, lnc, D, W.w_ff1, W.b_ff1, nullptr, 0, hc, M, mode, B, M, D, AVF_EPI_BIAS | AVF_EPI_GELU, st))) return e;
   return linear(mode, hc, M, W.w_ff2, W.b_ff2, xc, D, cls_out, D, AVF_FP32, B, D, M, AVF_EPI_BIAS | AVF_EPI_RESIDUAL, st);
+}
+
+static int tformer_fwd(int mode, int io_mode, const avf_stack_shape* s, const avf_layer_weights* layers, const void* frames, const float* cls_token,
+                       const float* pos, float* cls_out, void* workspace, size_t workspace_bytes, const uint8_t* keep, cudaStream_t st) {
+  int e = tformer_check(s, layers, frames, cls_token, pos, cls_out, workspace, workspace_bytes, avf_tformer_workspace_bytes(s, mode));
+  if (e) return e;
+  if ((e = tformer_embed(io_mode, frames, cls_token, pos, static_cast<float*>(workspace), s->n_seq, s->n_tok - 1, s->dim, st))) return e;
+  return tformer_layers(mode, s, layers, workspace, cls_out, keep, st);
+}
+
+// Clips described by frame indices into a bank: gather, keep rows and embed in one launch, then the masked layers.  The keep rows
+// follow the workspace of avf_tformer_fwd.
+static int tformer_fwd_indexed(int mode, int io_mode, const avf_stack_shape* s, const avf_layer_weights* layers, const void* bank, int n_bank,
+                               const int32_t* index, const float* cls_token, const float* pos, float* cls_out, void* workspace, size_t workspace_bytes,
+                               cudaStream_t st) {
+  int e = tformer_check(s, layers, index, cls_token, pos, cls_out, workspace, workspace_bytes, avf_tformer_indexed_workspace_bytes(s, mode));
+  if (e) return e;
+  AVF_REQUIRE(n_bank >= 0 && (bank != nullptr || n_bank == 0), AVF_EINVAL, "tformer_fwd_indexed: bank of %d frames at %p", n_bank, bank);
+  uint8_t* keep = static_cast<uint8_t*>(workspace) + avf_tformer_workspace_bytes(s, mode);
+  if ((e = tformer_embed_indexed(io_mode, bank, n_bank, index, cls_token, pos, static_cast<float*>(workspace), keep, s->n_seq, s->n_tok - 1, s->dim, st)))
+    return e;
+  return tformer_layers(mode, s, layers, workspace, cls_out, keep, st);
 }
 
 }  // namespace avf
@@ -369,6 +397,20 @@ int avf_tformer_fwd_masked(int mode, int io_mode, const avf_stack_shape* s, cons
   int e = require_device();
   if (e) return e;
   return tformer_fwd(mode, io_mode, s, layers, frames, cls_token, pos, cls_out, workspace, workspace_bytes, keep, static_cast<cudaStream_t>(stream));
+}
+
+size_t avf_tformer_indexed_workspace_bytes(const avf_stack_shape* s, int mode) {
+  if (s == nullptr || s->n_seq <= 0 || s->n_tok <= 0) return 0;
+  return avf_tformer_workspace_bytes(s, mode) + align_up(size_t(s->n_seq) * s->n_tok);
+}
+
+int avf_tformer_fwd_indexed(int mode, int io_mode, const avf_stack_shape* s, const avf_layer_weights* layers, const void* bank, int32_t n_bank,
+                            const int32_t* index, const float* cls_token, const float* pos, float* cls_out, void* workspace, size_t workspace_bytes,
+                            void* stream) {
+  int e = require_device();
+  if (e) return e;
+  return tformer_fwd_indexed(mode, io_mode, s, layers, bank, n_bank, index, cls_token, pos, cls_out, workspace, workspace_bytes,
+                             static_cast<cudaStream_t>(stream));
 }
 
 int avf_tformer_cls_extract(const float* x, float* cls, int32_t n_clips, int32_t n_tok, int32_t dim, void* stream) {

@@ -202,6 +202,45 @@ __global__ void tformer_embed_kernel(const InT* __restrict__ frames, const float
   reinterpret_cast<float4*>(x)[idx] = make_float4(v.x + p.x, v.y + p.y, v.z + p.z, v.w + p.w);
 }
 
+// The same embed with the frames gathered from a per-video frame bank (models/vformer.py:280-290 on clips described by frame indices):
+// i = index[c*T + t]; x[c, t+1, :] = bank[i, :] + pos[t+1] when 0 <= i < n_bank, else pos[t+1] alone (a missing frame, value 0).
+// keep[c, 0] = 1 and keep[c, t+1] = (0 <= i < n_bank): the attention mask of the layers that follow.  The bank is never read outside
+// [0, n_bank), whatever the index holds.
+template <typename InT>
+__global__ void tformer_embed_indexed_kernel(const InT* __restrict__ bank, int n_bank, const int* __restrict__ index, const float* __restrict__ cls,
+                                             const float* __restrict__ pos, float* __restrict__ x, uint8_t* __restrict__ keep, int n_clips, int T, int dim) {
+  pdl_wait();      // programmatic dependent launch: everything above is launch overhead hidden behind the previous kernel
+  pdl_trigger();
+  const size_t idx = size_t(blockIdx.x) * blockDim.x + threadIdx.x;      // over float4 groups
+  const int d4 = dim >> 2;
+  const size_t total = size_t(n_clips) * (T + 1) * d4;
+  if (idx >= total) return;
+  const int c4 = int(idx % d4);
+  const size_t r = idx / d4;
+  const int tok = int(r % (T + 1));
+  const size_t clip = r / (T + 1);
+  float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+  bool real = true;
+  if (tok == 0) {
+    v = __ldg(reinterpret_cast<const float4*>(cls) + c4);
+  } else {
+    const int i = __ldg(index + clip * T + (tok - 1));
+    real = unsigned(i) < unsigned(n_bank);
+    if (real) {
+      const InT* fp = bank + size_t(i) * dim + c4 * 4;
+      if constexpr (sizeof(InT) == 4) {
+        v = __ldg(reinterpret_cast<const float4*>(fp));
+      } else {
+        const uint2 q = __ldg(reinterpret_cast<const uint2*>(fp));
+        v = make_float4(__uint_as_float(q.x << 16), __uint_as_float(q.x & 0xffff0000u), __uint_as_float(q.y << 16), __uint_as_float(q.y & 0xffff0000u));
+      }
+    }
+  }
+  const float4 p = __ldg(reinterpret_cast<const float4*>(pos + size_t(tok) * dim) + c4);
+  reinterpret_cast<float4*>(x)[idx] = make_float4(v.x + p.x, v.y + p.y, v.z + p.z, v.w + p.w);
+  if (c4 == 0) keep[r] = real ? 1 : 0;
+}
+
 __global__ void rows_gather_kernel(const float* __restrict__ x, size_t src_row_stride, float* __restrict__ y, int rows, int dim) {
   pdl_wait();      // programmatic dependent launch: everything above is launch overhead hidden behind the previous kernel
   pdl_trigger();
@@ -421,6 +460,23 @@ int tformer_embed(int io_mode, const void* frames, const float* cls, const float
   if (io_mode == AVF_BF16) launch_pdl(tformer_embed_kernel<__nv_bfloat16>, grid, 256, 0, st, static_cast<const __nv_bfloat16*>(frames), cls, pos, x, n_clips, T, dim);
   else launch_pdl(tformer_embed_kernel<float>, grid, 256, 0, st, static_cast<const float*>(frames), cls, pos, x, n_clips, T, dim);
   AVF_LAUNCH_CHECK("tformer_embed_kernel");
+  return 0;
+}
+
+int tformer_embed_indexed(int io_mode, const void* bank, int n_bank, const int* index, const float* cls, const float* pos, float* x, uint8_t* keep,
+                          int n_clips, int T, int dim, cudaStream_t st) {
+  AVF_REQUIRE(n_clips > 0 && T > 0 && dim % 4 == 0 && n_bank >= 0, AVF_EINVAL, "tformer_embed_indexed: n_clips=%d T=%d dim=%d n_bank=%d", n_clips, T,
+              dim, n_bank);
+  AVF_REQUIRE((reinterpret_cast<uintptr_t>(bank) & (io_mode == AVF_BF16 ? 7 : 15)) == 0, AVF_EINVAL,
+              "tformer_embed_indexed: the bank must be %d-byte aligned", io_mode == AVF_BF16 ? 8 : 16);
+  const size_t total = size_t(n_clips) * (T + 1) * (dim / 4);
+  const unsigned grid = unsigned((total + 255) / 256);
+  if (io_mode == AVF_BF16)
+    launch_pdl(tformer_embed_indexed_kernel<__nv_bfloat16>, grid, 256, 0, st, static_cast<const __nv_bfloat16*>(bank), n_bank, index, cls, pos, x, keep,
+               n_clips, T, dim);
+  else
+    launch_pdl(tformer_embed_indexed_kernel<float>, grid, 256, 0, st, static_cast<const float*>(bank), n_bank, index, cls, pos, x, keep, n_clips, T, dim);
+  AVF_LAUNCH_CHECK("tformer_embed_indexed_kernel");
   return 0;
 }
 

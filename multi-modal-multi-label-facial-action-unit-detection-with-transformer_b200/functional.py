@@ -298,6 +298,24 @@ def tformer_fwd(frames: torch.Tensor, cls_token: torch.Tensor, pos: torch.Tensor
     return cls
 
 
+def tformer_fwd_indexed(bank: torch.Tensor, index: torch.Tensor, cls_token: torch.Tensor, pos: torch.Tensor, packed: PackedStack,
+                        shape: StackShape) -> torch.Tensor:
+    """Inference TFormer on clips gathered from a frame bank in one call (avf_tformer_fwd_indexed): bank [n_bank, dim] fp32 / bf16,
+    index [n_clips, T] int32 contiguous on the bank's device, an entry outside [0, n_bank) = a missing frame, masked out of every
+    layer -> cls features [n_clips, dim] fp32."""
+    bank = _cuda(bank, "bank").contiguous()
+    if index.dtype != torch.int32 or not index.is_contiguous() or tuple(index.shape) != (shape.n_seq, shape.n_tok - 1):
+        raise ValueError(f"tformer_fwd_indexed: index must be a contiguous int32 tensor [{shape.n_seq}, {shape.n_tok - 1}], "
+                         f"got {index.dtype} {tuple(index.shape)}")
+    _cuda(index, "index")
+    cls = torch.empty((shape.n_seq, shape.dim), dtype=torch.float32, device=bank.device)
+    L = _lib.lib()
+    ws = workspace(L.avf_tformer_indexed_workspace_bytes(ctypes.byref(shape), packed.mode), bank.device)
+    check(L.avf_tformer_fwd_indexed(packed.mode, _io_mode(bank), ctypes.byref(shape), packed.array, _ptr(bank), bank.shape[0], _ptr(index),
+                                    _ptr(_f32c(cls_token)), _ptr(_f32c(pos)), _ptr(cls), _ptr(ws), ws.numel(), _stream()), "tformer_fwd_indexed")
+    return cls
+
+
 def tformer_cls_extract(x: torch.Tensor, n_clips: int, n_tok: int) -> torch.Tensor:
     dim = x.shape[-1]
     cls = torch.empty((n_clips, dim), dtype=torch.float32, device=x.device)

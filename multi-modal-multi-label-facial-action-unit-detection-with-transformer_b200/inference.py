@@ -10,6 +10,11 @@ torch / cuDNN — prepared the way a B200 wants them, without touching the model
     eng = InferenceEngine(model, backbone_dtype=torch.bfloat16)
     out21 = eng({"clip": clip, "audio_features": mel})          # [B,21] like model(x), models/avformer.py:93-106
 
+A whole video runs each frame through the video trunk once instead of once per clip that contains it (eager, no graph):
+
+    bank = torch.cat([eng.frame_features(frames[i:i + 256]) for i in range(0, len(frames), 256)])   # [F,512]
+    out21, decisions = eng.clips(bank, index, mel)              # index [n,T] frame numbers, -1 = missing; mel [n,1,64,1001]
+
 ``backbone_dtype=torch.float32`` reproduces ``model(x)`` up to the re-association of the BN fold (checked at 1e-3 in the
 tests); bf16 backbones trade ~1e-1 absolute on the logits for tensor-core convolutions and are therefore opt-in.
 """
@@ -90,40 +95,81 @@ class InferenceEngine:
         self._graphs: Dict[tuple, tuple] = {}
         self._sig = weights_signature(model)
 
-    # -- eager forward (also what gets captured) ---------------------------------------------------------------
+    # -- eager pieces (the forward below is also what gets captured) --------------------------------------------
+    def _audio_tokens_into(self, audio: torch.Tensor, fused: torch.Tensor) -> None:
+        """audio [B,1,64,1001]: ResNet-18 trunk -> global average pool -> [B,512] fp32 -> AU_former into columns [0,128) of fused."""
+        a = self.audio.to_stage(self.audio.stem_fwd(audio), 1, 4)
+        a_feat = a.float().mean(dim=(2, 3))
+        self.model.audio_model.au_head.tokens_into(a_feat, a_feat.shape[1], audio.shape[0], out=fused, ld_out=256)
+
+    def _frame_features(self, frames: torch.Tensor) -> torch.Tensor:
+        """frames [F,C,H,W] -> stem..stage 3 -> SFormer -> stage 4 -> pool -> [F,512] fp32; every step works frame by frame."""
+        vm = self.model.video_model.video_model
+        s3 = self.video.to_stage(self.video.stem_fwd(frames), 1, 3)
+        s3 = s3.to(torch.bfloat16 if AF._mode(vm.s_former.spatial_transformer.precision or default_precision()) == AF.AVF_BF16 else torch.float32)
+        s3 = vm.s_former.sformer(s3.contiguous())                      # NCHW-contiguous map in, same out (models/vformer.py:245-259)
+        f = self.video.to_stage(s3.to(self.dtype).contiguous(memory_format=torch.channels_last), 4, 4)
+        return f.float().mean(dim=(2, 3))                               # AdaptiveAvgPool2d((1,1)) + flatten
+
     @torch.no_grad()
     def _forward(self, clip: torch.Tensor, audio: torch.Tensor) -> torch.Tensor:
         m = self.model
         vm = m.video_model.video_model
         bs, _, T, H, W = clip.shape
-        # audio: ResNet-18 trunk -> global average pool -> [B,512] fp32 -> AU_former
-        a = self.audio.to_stage(self.audio.stem_fwd(audio), 1, 4)
-        a_feat = a.float().mean(dim=(2, 3))
         fused = torch.empty((bs * 12, 256), dtype=torch.float32, device=clip.device)
-        m.audio_model.au_head.tokens_into(a_feat, a_feat.shape[1], bs, out=fused, ld_out=256)
-        # video: [B,C,T,H,W] -> frames [B*T,C,H,W] -> stem..stage 3 -> SFormer -> stage 4 -> pool -> TFormer -> AU_former
+        self._audio_tokens_into(audio, fused)
+        # video: [B,C,T,H,W] -> frames [B*T,C,H,W] -> per-frame features -> TFormer -> AU_former into columns [128,256)
         frames = clip[:, -self.num_channels:].permute(0, 2, 1, 3, 4).reshape(bs * T, self.num_channels, H, W)
-        s3 = self.video.to_stage(self.video.stem_fwd(frames), 1, 3)
-        s3 = s3.to(torch.bfloat16 if AF._mode(vm.s_former.spatial_transformer.precision or default_precision()) == AF.AVF_BF16 else torch.float32)
-        s3 = vm.s_former.sformer(s3.contiguous())                      # NCHW-contiguous map in, same out (models/vformer.py:245-259)
-        f = self.video.to_stage(s3.to(self.dtype).contiguous(memory_format=torch.channels_last), 4, 4)
-        frame_feat = f.float().mean(dim=(2, 3))                         # AdaptiveAvgPool2d((1,1)) + flatten
-        cls = vm.t_former.cls_features(frame_feat)
+        cls = vm.t_former.cls_features(self._frame_features(frames))
         m.video_model.au_head.tokens_into(cls, cls.shape[1], cls.shape[0], out=fused[:, 128:], ld_out=256)
         if m.task != "AU":
             return torch.zeros(bs, 21, device=clip.device)
         return m.au_head.logits21_(fused, bs)
 
-    def __call__(self, x: Dict[str, torch.Tensor]) -> torch.Tensor:
-        clip, audio = x["clip"], x["audio_features"]
-        AF._cuda(clip, "x['clip']")
-        AF._cuda(audio, "x['audio_features']")
-        from .graphs import weights_signature, _packed_refs
+    def _refresh(self) -> None:
+        from .graphs import weights_signature
         if weights_signature(self.model) != self._sig:        # load_state_dict / optimizer.step() / in-place edits since the fold
             if self.model.training:
                 raise RuntimeError("InferenceEngine folds the eval-mode BatchNorm statistics: call model.eval() first")
             self.refolds += 1
             self._fold()
+
+    # -- whole videos: each frame through the video trunk once, clips gathered from the frame bank ------------------------
+    @torch.no_grad()
+    def frame_features(self, frames: torch.Tensor) -> torch.Tensor:
+        """frames [F,C,H,W] (C = the model's num_channels) -> frame features [F,512] fp32: the per-frame part of a forward.  The rows of
+        one video, concatenated over frame chunks, are the bank that ``clips`` gathers from.  Eager (no graph capture)."""
+        AF._cuda(frames, "frames")
+        if frames.dim() != 4 or frames.shape[1] != self.num_channels:
+            raise ValueError(f"InferenceEngine.frame_features: frames must be [F, {self.num_channels}, H, W], got {tuple(frames.shape)}")
+        self._refresh()
+        return self._frame_features(frames)
+
+    @torch.no_grad()
+    def clips(self, bank: torch.Tensor, index: torch.Tensor, audio_features: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
+        """Clips described by frame indices into ``bank`` (frame_features of one video): index integer [n, T], -1 = a missing frame
+        (masked out of the TFormer), audio_features [n,1,64,1001] one mel window per clip.  Returns (out21 [n,21] like model(x),
+        decisions [n,12] int32 = out21[:, :12] > 0).  Eager (no graph capture)."""
+        AF._cuda(audio_features, "audio_features")
+        m = self.model
+        if torch.is_tensor(index) and index.dim() == 2 and audio_features.shape[0] != index.shape[0]:
+            raise ValueError(f"InferenceEngine.clips: {audio_features.shape[0]} audio windows for {index.shape[0]} clips: one window per clip")
+        self._refresh()
+        cls = m.video_model.video_model.t_former.cls_features_indexed(bank, index)      # checks the index itself
+        n = cls.shape[0]
+        fused = torch.empty((n * 12, 256), dtype=torch.float32, device=bank.device)
+        self._audio_tokens_into(audio_features, fused)
+        m.video_model.au_head.tokens_into(cls, cls.shape[1], n, out=fused[:, 128:], ld_out=256)
+        if m.task != "AU":
+            return torch.zeros(n, 21, device=bank.device), torch.zeros(n, 12, dtype=torch.int32, device=bank.device)
+        return m.au_head.logits21_(fused, n, want_decisions=True)
+
+    def __call__(self, x: Dict[str, torch.Tensor]) -> torch.Tensor:
+        clip, audio = x["clip"], x["audio_features"]
+        AF._cuda(clip, "x['clip']")
+        AF._cuda(audio, "x['audio_features']")
+        from .graphs import _packed_refs
+        self._refresh()
         if not self.use_graphs:
             return self._forward(clip, audio)
         key = (tuple(clip.shape), clip.dtype, tuple(audio.shape), audio.dtype)

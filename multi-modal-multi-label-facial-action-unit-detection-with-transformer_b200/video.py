@@ -168,6 +168,40 @@ class TFormer(nn.Module):
         return AF.tformer_fwd(x.detach(), self.cls_token.view(-1), self.pos_embedding[0], st.packed(), st.shape(n_clips, self.num_patches + 1),
                               keep)
 
+    def cls_features_indexed(self, bank, index):
+        """Inference on clips described by frame indices: cls features [n_clips, dim] fp32, equal to
+        ``cls_features(bank[index.clamp(min=0)].reshape(-1, dim), mask=index >= 0)`` without the gathered copy (gather, mask and embed
+        are one launch).  ``bank`` [n_bank, dim] fp32 / bf16 on CUDA: the frame features of one video, each frame computed once.
+        ``index`` integer [n_clips, num_patches], on the host or the bank's device; -1 = a missing frame (masked out of every layer)."""
+        AF._cuda(bank, "bank")
+        st = self.spatial_transformer
+        if st.dropout_state()[0] > 0.0:
+            raise RuntimeError("TFormer.cls_features_indexed is inference only: this TFormer applies dropout (train() with dropout > 0), which "
+                               "only the tape-keeping kernels of cls_features implement; call eval() first")
+        if bank.dim() != 2 or bank.shape[1] != self.dim:
+            raise ValueError(f"TFormer.cls_features_indexed: bank must be [n_bank, {self.dim}], got {tuple(bank.shape)}")
+        if not torch.is_tensor(index):
+            raise TypeError(f"TFormer.cls_features_indexed: index must be an integer tensor, got {type(index).__name__}")
+        if index.dtype.is_floating_point or index.dtype.is_complex or index.dtype == torch.bool:
+            raise TypeError(f"TFormer.cls_features_indexed: index must be an integer tensor, got {index.dtype}")
+        if index.dim() != 2 or index.shape[0] == 0 or index.shape[1] != self.num_patches:
+            raise ValueError(f"TFormer.cls_features_indexed: index must be [n_clips, {self.num_patches}] (num_patches frames per clip), got "
+                             f"{tuple(index.shape)}")
+        # Checked where the table lives: on the host for free, on the device at the cost of one stream synchronisation.  While a graph
+        # is captured neither that synchronisation nor a host-to-device copy is possible: the index must already be on the device, and
+        # the kernel's bounds guard alone holds.
+        if torch.cuda.is_current_stream_capturing():
+            if not index.is_cuda:
+                raise RuntimeError("TFormer.cls_features_indexed: while a CUDA graph is being captured the index must already be on the "
+                                   f"bank's device ({bank.device}); it is on {index.device}")
+        else:
+            lo, hi = (int(v) for v in torch.aminmax(index))
+            if lo < -1 or hi >= bank.shape[0]:
+                raise ValueError(f"TFormer.cls_features_indexed: index entries must lie in [-1, {bank.shape[0]}) (-1 = missing frame), got "
+                                 f"[{lo}, {hi}]")
+        return AF.tformer_fwd_indexed(bank.detach(), index.to(device=bank.device, dtype=torch.int32).contiguous(), self.cls_token.view(-1), self.pos_embedding[0],
+                                      st.packed(), st.shape(index.shape[0], self.num_patches + 1))
+
     def forward(self, x, mask=None):
         """x [n_clips*T, dim] frame features -> cls features [n_clips, dim].  ``mask`` (optional): bool [n_clips, T], True = a real
         frame; clips with fewer real frames can share a batch with full ones (the padding frames' values do not matter)."""
