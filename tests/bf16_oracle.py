@@ -67,7 +67,9 @@ def _gelu_fused(h):
     return bf(hx * bf(torch.tanh(u)) + hx)
 
 
-def _attention(x, p, pre, heads, path, bug):
+def _attention(x, p, pre, heads, path, bug, keep=None, tape=None):
+    """``keep`` [B, N] bool (True = kept): the mask of mask_score (avf_attention_mma.cu:48-52); ``tape`` (a dict) receives the
+    bf16 qkv and merged-head o that the training forward stores (avf_train_api.cu:110-111)."""
     B, N, _ = x.shape
     r = bf if path else (lambda t: t)
     wqkv = p[pre + "fn.fn.to_qkv.weight"]
@@ -77,6 +79,8 @@ def _attention(x, p, pre, heads, path, bug):
     qkv = r(x @ r(wqkv).t())
     q, k, v = (t.reshape(B, N, heads, dh).permute(0, 2, 1, 3) for t in qkv.split(inner, dim=-1))
     s = torch.matmul(q, k.transpose(-1, -2))
+    if keep is not None:                             # kept query: -inf on dropped keys; dropped query: the same score on every key
+        s = s.masked_fill(~keep[:, None, None, :], -math.inf).masked_fill(~keep[:, None, :, None], 0.0)
     if bug == "drop_last_key":
         s[..., -1] = -math.inf
     elif bug == "head_uniform":
@@ -104,10 +108,13 @@ def _attention(x, p, pre, heads, path, bug):
         e = torch.exp2(arg)
         o = torch.matmul(e, v) / e.sum(dim=-1, keepdim=True)
     o = o.permute(0, 2, 1, 3).reshape(B, N, inner)
+    if tape is not None:
+        tape.update(qkv=qkv, o=o)
     return o @ r(p[pre + "fn.fn.to_out.0.weight"]).t() + p[pre + "fn.fn.to_out.0.bias"]
 
 
-def _feed_forward(x, p, pre, path):
+def _feed_forward(x, p, pre, path, tape=None):
+    """``tape`` (a dict) receives the fp32 pre-activation h (the training forward stores bf16(h), avf_gemm_umma.cu:113-124) and g."""
     r = bf if path else (lambda t: t)
     h = x @ r(p[pre + "fn.fn.net.0.weight"]).t() + p[pre + "fn.fn.net.0.bias"]
     if path == "fused":
@@ -116,6 +123,8 @@ def _feed_forward(x, p, pre, path):
         g = bf(O.gelu_tanh(h))                       # avf_gemm_umma.cu:127: fp32 tanh-GELU in the epilogue, stored as bf16
     else:
         g = O.gelu_tanh(h)
+    if tape is not None:
+        tape.update(h=h, g=g)
     return g @ r(p[pre + "fn.fn.net.3.weight"]).t() + p[pre + "fn.fn.net.3.bias"]
 
 
