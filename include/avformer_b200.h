@@ -385,6 +385,22 @@ int avf_tformer_fwd_indexed(int mode, int io_mode, const avf_stack_shape* s, con
                             const float* cls_token, const float* pos, float* cls_out,
                             void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---- training over a frame bank: the indexed embed and its backward (models/vformer.py:280-290) ------------------------------
+ * avf_tformer_embed_indexed: the gather + embed step of avf_tformer_fwd_indexed alone.  bank / index as there; writes the fp32 token
+ * matrix x [n_clips*(T+1), dim] (T = n_frames) and keep [n_clips, T+1] uint8 (1 = kept, the cls slot always), the input and the
+ * mask of the tape-keeping avf_encoder_stack_fwd_train_masked.
+ * avf_tformer_embed_indexed_bwd: dbank [n_bank, dim] (fp32, or bf16 for a bf16 bank: out_mode) =
+ *   dbank[i] = sum of dtok[c*(T+1) + 1 + t] over every slot s = c*T + t with index[s] == i,
+ * each column one fp32 chain over the slots in ascending s starting from +0.0 (bf16: that sum rounded once), so the result is
+ * bit-reproducible and independent of the grid.  No float atomics.  Every row is written (+0.0 where no slot points); an entry
+ * outside [0, n_bank) contributes nowhere, and nothing outside dbank is written.  dtok 16-byte aligned, dbank 16- (fp32) or 8-byte
+ * (bf16) aligned.  The gradients of cls_token and pos are avf_colsum over dtok, as for avf_tformer_embed.  Three launches. */
+int avf_tformer_embed_indexed(int io_mode, const void* bank, int32_t n_bank, const int32_t* index, const float* cls_token,
+                              const float* pos, float* x, uint8_t* keep, int32_t n_clips, int32_t n_frames, int32_t dim, void* stream);
+size_t avf_tformer_embed_indexed_bwd_workspace_bytes(int32_t n_clips, int32_t n_frames, int32_t n_bank);
+int avf_tformer_embed_indexed_bwd(int out_mode, const float* dtok, const int32_t* index, int32_t n_clips, int32_t n_frames,
+                                  int32_t dim, int32_t n_bank, void* dbank, void* workspace, size_t workspace_bytes, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

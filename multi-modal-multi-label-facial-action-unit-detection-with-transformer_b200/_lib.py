@@ -138,6 +138,10 @@ SIGNATURES = {
     "avf_tformer_indexed_workspace_bytes": (_sz, [ctypes.POINTER(StackShape), ctypes.c_int]),
     "avf_tformer_fwd_indexed": (ctypes.c_int, [ctypes.c_int, ctypes.c_int, ctypes.POINTER(StackShape), ctypes.POINTER(LayerWeights), _c_p, _i32, _c_p,
                                                _c_p, _c_p, _c_p, _c_p, _sz, _c_p]),
+    # ---- training over a frame bank: the indexed embed and its backward ----
+    "avf_tformer_embed_indexed": (ctypes.c_int, [ctypes.c_int, _c_p, _i32, _c_p, _c_p, _c_p, _c_p, _c_p, _i32, _i32, _i32, _c_p]),
+    "avf_tformer_embed_indexed_bwd_workspace_bytes": (_sz, [_i32, _i32, _i32]),
+    "avf_tformer_embed_indexed_bwd": (ctypes.c_int, [ctypes.c_int, _c_p, _c_p, _i32, _i32, _i32, _i32, _c_p, _c_p, _sz, _c_p]),
 }
 
 _lock = threading.Lock()

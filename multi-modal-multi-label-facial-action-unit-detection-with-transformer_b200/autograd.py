@@ -154,16 +154,51 @@ class TFormerEmbedFn(torch.autograd.Function):
         dtok = _f32_dense(dtok)
         dim = dtok.shape[1]
         n_clips = dtok.shape[0] // (T + 1)
-        dframes = dcls = dpos = None
+        dframes = None
         if needs[0]:
             dframes = dtok.view(n_clips, T + 1, dim)[:, 1:].reshape(fshape).to(fdtype)
-        if needs[1] or needs[2]:
-            s = AF.colsum(dtok.view(n_clips, (T + 1) * dim))
-            dpos = s.view(pshape) if needs[2] else None
-            dcls = s[:dim].clone().view(cshape) if needs[1] else None
-        dcls, dpos = _hand_over(ctx.params, (dcls, dpos))
-        _notify(ctx.params)
+        dcls, dpos = _embed_param_grads(ctx.params, dtok, n_clips, T, needs[1], needs[2], cshape, pshape)
         return dframes, dcls, dpos, None
+
+
+def _embed_param_grads(params, dtok, n_clips, T, need_cls, need_pos, cshape, pshape):
+    """Gradients of (cls_token, pos) of a TFormer embed from the fp32 token gradient dtok [n_clips*(T+1), dim]: one column sum over
+    the clips gives dpos, and its row 0 is dcls; handed over and reported like every parameter gradient of this module."""
+    dim = dtok.shape[1]
+    dcls = dpos = None
+    if need_cls or need_pos:
+        s = AF.colsum(dtok.view(n_clips, (T + 1) * dim))
+        dpos = s.view(pshape) if need_pos else None
+        dcls = s[:dim].clone().view(cshape) if need_cls else None
+    dcls, dpos = _hand_over(params, (dcls, dpos))
+    _notify(params)
+    return dcls, dpos
+
+
+class TFormerEmbedIndexedFn(torch.autograd.Function):
+    """TFormerEmbedFn on clips gathered from a frame bank: bank [n_bank, dim] (fp32 / bf16), index [n_clips, T] int32 on the bank's
+    device (outside [0, n_bank) = a missing frame) -> (tokens [n_clips*(T+1), dim] fp32, keep [n_clips, T+1] bool, not
+    differentiable).  The bank's gradient is the scatter-add of the frame-token gradients (avf_tformer_embed_indexed_bwd: each row
+    one ascending fp32 chain, no float atomics), so a frame shared by several clips costs one trunk backward."""
+
+    @staticmethod
+    def forward(ctx, bank, index, cls_token, pos, n_frames):
+        tok, keep = AF.tformer_embed_indexed(bank.detach(), index, cls_token.detach().reshape(-1), pos.detach()[0], n_frames)
+        ctx.mark_non_differentiable(keep)
+        ctx.meta = (bank.shape[0], bank.dtype, n_frames, cls_token.shape, pos.shape)
+        ctx.index = index
+        ctx.params = (cls_token, pos)
+        return tok, keep
+
+    @staticmethod
+    def backward(ctx, dtok, _dkeep):
+        n_bank, bdtype, T, cshape, pshape = ctx.meta
+        needs = ctx.needs_input_grad
+        dtok = _f32_dense(dtok)
+        n_clips = dtok.shape[0] // (T + 1)
+        dbank = AF.tformer_embed_indexed_bwd(dtok, ctx.index, n_bank, T, bdtype) if needs[0] else None
+        dcls, dpos = _embed_param_grads(ctx.params, dtok, n_clips, T, needs[2], needs[3], cshape, pshape)
+        return dbank, None, dcls, dpos, None
 
 
 class AUFrontFn(torch.autograd.Function):

@@ -130,6 +130,43 @@ class TwoStreamAuralVisualFormer(nn.Module):
             return torch.zeros(bs, 21, device=clip.device)
         return self.au_head.logits21_train(fused, bs)
 
+    def forward_indexed(self, frames, index, audio_features):
+        """forward() over clips described by frame indices into one video's frames, each frame through the video trunk once.
+
+        ``frames`` [F, C, H, W] (the processed frames; the last ``num_channels`` channels are used, as of x['clip']), ``index``
+        integer [n_clips, T] into them (-1 = a missing frame, masked out of the TFormer), ``audio_features`` [n_clips, 1, 64, 1001]
+        (one mel window per clip).  Returns float32 [n_clips, 21] like forward().  The ResNet stem, stages 1-3, the SFormer, stage 4
+        and the pool run on the F frames (a bank [F, 512]); the TFormer gathers its clips from that bank (TFormer.forward_indexed),
+        and with autograd the trunk's backward runs once per frame on the summed gradient of every slot that uses it.  With BatchNorm
+        in eval() this equals forward() on the gathered clips; in train() BatchNorm2d takes its batch statistics over the F frames."""
+        vm = self.video_model.video_model
+        tf = vm.t_former
+        AF._cuda(frames, "frames")
+        AF._cuda(audio_features, "audio_features")
+        if frames.dim() != 4 or frames.shape[0] == 0 or frames.shape[1] < vm.num_channels:
+            raise ValueError(f"forward_indexed: frames must be [F, C >= {vm.num_channels}, H, W], got {tuple(frames.shape)}")
+        index = tf.bank_index((frames.shape[0], tf.dim), frames.device, index, "forward_indexed")
+        n_clips = index.shape[0]
+        if audio_features.dim() == 0 or audio_features.shape[0] != n_clips:
+            raise ValueError(f"forward_indexed: one audio window per clip: {n_clips} clips but audio_features of {tuple(audio_features.shape)}")
+        x = frames[:, -vm.num_channels:].unsqueeze(0)                  # [1, F, c, H, W]: one "clip" of all F frames
+        if needs_grad(self, frames, audio_features):
+            a_feat = self.audio_model.audio_model(audio_features)
+            tok_a = self._au_tokens(self.audio_model.au_head, a_feat, n_clips)
+            cls = tf.forward_indexed_checked(vm.s_former(x), index)
+            tok_v = self._au_tokens(self.video_model.au_head, cls, n_clips)
+            if self.task != "AU":
+                return torch.zeros(n_clips, 21, device=frames.device)
+            return self.au_head.logits21_train(torch.cat([tok_a, tok_v], dim=1), n_clips)
+        fused = torch.empty((n_clips * 12, 256), dtype=torch.float32, device=frames.device)
+        a_feat = self.audio_model.audio_model(audio_features).float().contiguous()
+        self.audio_model.au_head.tokens_into(a_feat, a_feat.shape[1], n_clips, out=fused, ld_out=256)
+        cls = tf.forward_indexed_checked(vm.s_former(x), index).contiguous()     # a strided view of the tokens under dropout
+        self.video_model.au_head.tokens_into(cls, cls.shape[1], n_clips, out=fused[:, 128:], ld_out=256)
+        if self.task != "AU":
+            return torch.zeros(n_clips, 21, device=frames.device)
+        return self.au_head.logits21_(fused, n_clips)
+
     @staticmethod
     def _au_tokens(head, emb, bs):
         if needs_grad(head, emb):

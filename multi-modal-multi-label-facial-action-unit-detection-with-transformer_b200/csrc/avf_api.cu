@@ -413,6 +413,15 @@ int avf_tformer_fwd_indexed(int mode, int io_mode, const avf_stack_shape* s, con
                              static_cast<cudaStream_t>(stream));
 }
 
+int avf_tformer_embed_indexed(int io_mode, const void* bank, int32_t n_bank, const int32_t* index, const float* cls_token, const float* pos, float* x,
+                              uint8_t* keep, int32_t n_clips, int32_t n_frames, int32_t dim, void* stream) {
+  int e = require_device();
+  if (e) return e;
+  AVF_REQUIRE(index && cls_token && pos && x && keep, AVF_EINVAL, "tformer_embed_indexed: null pointer");
+  AVF_REQUIRE(bank != nullptr || n_bank == 0, AVF_EINVAL, "tformer_embed_indexed: bank of %d frames at %p", n_bank, bank);
+  return tformer_embed_indexed(io_mode, bank, n_bank, index, cls_token, pos, x, keep, n_clips, n_frames, dim, static_cast<cudaStream_t>(stream));
+}
+
 int avf_tformer_cls_extract(const float* x, float* cls, int32_t n_clips, int32_t n_tok, int32_t dim, void* stream) {
   int e = require_device();
   if (e) return e;

@@ -17,6 +17,9 @@ int sformer_unpack(int io_mode, const float* x, void* fmap, int n_frames, int di
 int tformer_embed(int io_mode, const void* frames, const float* cls, const float* pos, float* x, int n_clips, int T, int dim, cudaStream_t st);
 int tformer_embed_indexed(int io_mode, const void* bank, int n_bank, const int* index, const float* cls, const float* pos, float* x, uint8_t* keep,
                           int n_clips, int T, int dim, cudaStream_t st);
+size_t tformer_embed_indexed_bwd_workspace_bytes(int n_clips, int T, int n_bank);
+int tformer_embed_indexed_bwd(int out_mode, const float* dtok, const int* index, int n_clips, int T, int dim, int n_bank, void* dbank, void* ws,
+                              size_t ws_bytes, cudaStream_t st);
 int rows_gather(const float* x, size_t src_row_stride, float* y, int rows, int dim, cudaStream_t st);
 int add_row_periodic(float* x, int ld_x, const float* pos, int rows, int dim, int period, cudaStream_t st);
 int cast_f32_bf16(const float* s, void* d, size_t n, cudaStream_t st);

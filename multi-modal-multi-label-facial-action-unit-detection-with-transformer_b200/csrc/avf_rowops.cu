@@ -241,6 +241,116 @@ __global__ void tformer_embed_indexed_kernel(const InT* __restrict__ bank, int n
   if (c4 == 0) keep[r] = real ? 1 : 0;
 }
 
+// Backward of that gather (models/vformer.py:280-290): a bank row receives the token gradients of every slot that points at it,
+//   dbank[i, :] = sum over slots s = c*T + t with index[s] == i, in ascending s, of dtok[c*(T+1) + 1 + t, :],
+// each column one sequential fp32 chain that starts from +0.0.  Training reductions here are deterministic and free of float atomics,
+// so the sum never depends on timing or grid size.  Three launches:
+//   1. bank_slots_build_kernel (one block): per-row slot counts with integer atomics (order-free), their exclusive scan into row
+//      offsets, and every valid slot placed inside its row's segment -- in the order the atomics happened to run;
+//   2. bank_slots_order_kernel (one thread per placed slot): its rank = the number of smaller slots in its segment, so the segment
+//      comes out ascending whatever that order was;
+//   3. tformer_embed_indexed_bwd_kernel (one thread per bank row and float4 column group): the ordered chain.  Every row is written,
+//      so a row no slot references is exactly +0.0 and no memset is needed.
+// An index entry outside [0, n_bank) (a missing frame) contributes to no row, and nothing outside dbank is written.  A row is never
+// split into parallel partial sums (that would change its bits), so a frame that many slots share -- the clamped edge frame of a
+// video, up to T/2 of a dense window's slots -- is one long serial chain, and ranking its segment costs its length squared over as
+// many threads.  That cost is accepted for determinism.
+// Workspace (ints): offsets [n_bank + 1], placed slots [S], ordered slots [S] (which the build kernel also uses for the ranks).
+__global__ void __launch_bounds__(1024) bank_slots_build_kernel(const int* __restrict__ index, int n_slots, int n_bank, int* __restrict__ offs,
+                                                                 int* __restrict__ placed, int* __restrict__ rank) {
+  pdl_wait();      // programmatic dependent launch: everything above is launch overhead hidden behind the previous kernel
+  pdl_trigger();
+  __shared__ int warp_tot[32];
+  __shared__ int carry;
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nthr = blockDim.x;
+  for (int i = tid; i < n_bank; i += nthr) offs[i] = 0;
+  __syncthreads();
+  for (int s = tid; s < n_slots; s += nthr) {
+    const int i = __ldg(index + s);
+    if (unsigned(i) < unsigned(n_bank)) rank[s] = atomicAdd(offs + i, 1);
+  }
+  __syncthreads();
+  // in-place exclusive scan of the counts, nthr rows per round
+  if (tid == 0) carry = 0;
+  __syncthreads();
+  for (int base = 0; base < n_bank; base += nthr) {
+    const int i = base + tid;
+    const int v = i < n_bank ? offs[i] : 0;
+    int incl = v;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const int u = __shfl_up_sync(0xffffffffu, incl, o);
+      if (lane >= o) incl += u;
+    }
+    if (lane == 31) warp_tot[warp] = incl;
+    __syncthreads();
+    if (warp == 0) {
+      const int nw = nthr >> 5;
+      int w = lane < nw ? warp_tot[lane] : 0;
+#pragma unroll
+      for (int o = 1; o < 32; o <<= 1) {
+        const int u = __shfl_up_sync(0xffffffffu, w, o);
+        if (lane >= o) w += u;
+      }
+      if (lane < nw) warp_tot[lane] = w;      // inclusive over warps
+    }
+    __syncthreads();
+    const int before = carry + (warp > 0 ? warp_tot[warp - 1] : 0) + incl - v;
+    if (i < n_bank) offs[i] = before;
+    __syncthreads();
+    if (tid == nthr - 1) carry = before + v;
+    __syncthreads();
+  }
+  if (tid == 0) offs[n_bank] = carry;
+  __syncthreads();
+  for (int s = tid; s < n_slots; s += nthr) {
+    const int i = __ldg(index + s);
+    if (unsigned(i) < unsigned(n_bank)) placed[offs[i] + rank[s]] = s;
+  }
+}
+
+__global__ void bank_slots_order_kernel(const int* __restrict__ index, int n_slots, int n_bank, const int* __restrict__ offs,
+                                        const int* __restrict__ placed, int* __restrict__ ordered) {
+  pdl_wait();
+  pdl_trigger();
+  const int p = blockIdx.x * blockDim.x + threadIdx.x;
+  if (p >= n_slots || p >= offs[n_bank]) return;
+  const int s = placed[p];
+  const int i = __ldg(index + s);           // a placed slot's entry is in [0, n_bank)
+  const int lo = offs[i], hi = offs[i + 1];
+  int r = 0;
+  for (int q = lo; q < hi; ++q) r += placed[q] < s;
+  ordered[lo + r] = s;
+}
+
+template <typename OutT>
+__global__ void tformer_embed_indexed_bwd_kernel(const float* __restrict__ dtok, const int* __restrict__ offs, const int* __restrict__ ordered,
+                                                 OutT* __restrict__ dbank, int n_bank, int T, int dim) {
+  pdl_wait();
+  pdl_trigger();
+  const size_t idx = size_t(blockIdx.x) * blockDim.x + threadIdx.x;      // over float4 groups of the bank
+  const int d4 = dim >> 2;
+  if (idx >= size_t(n_bank) * d4) return;
+  const int c4 = int(idx % d4);
+  const int i = int(idx / d4);
+  float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
+  const int hi = offs[i + 1];
+  for (int q = offs[i]; q < hi; ++q) {
+    const int s = ordered[q];
+    const size_t row = size_t(s / T) * (T + 1) + 1 + s % T;
+    const float4 g = __ldg(reinterpret_cast<const float4*>(dtok + row * dim) + c4);
+    acc.x = __fadd_rn(acc.x, g.x);
+    acc.y = __fadd_rn(acc.y, g.y);
+    acc.z = __fadd_rn(acc.z, g.z);
+    acc.w = __fadd_rn(acc.w, g.w);
+  }
+  if constexpr (sizeof(OutT) == 4) {
+    reinterpret_cast<float4*>(dbank)[idx] = acc;
+  } else {
+    reinterpret_cast<uint2*>(dbank)[idx] = make_uint2(pack_bf16x2(acc.x, acc.y), pack_bf16x2(acc.z, acc.w));
+  }
+}
+
 __global__ void rows_gather_kernel(const float* __restrict__ x, size_t src_row_stride, float* __restrict__ y, int rows, int dim) {
   pdl_wait();      // programmatic dependent launch: everything above is launch overhead hidden behind the previous kernel
   pdl_trigger();
@@ -477,6 +587,45 @@ int tformer_embed_indexed(int io_mode, const void* bank, int n_bank, const int* 
   else
     launch_pdl(tformer_embed_indexed_kernel<float>, grid, 256, 0, st, static_cast<const float*>(bank), n_bank, index, cls, pos, x, keep, n_clips, T, dim);
   AVF_LAUNCH_CHECK("tformer_embed_indexed_kernel");
+  return 0;
+}
+
+static inline size_t align_up(size_t v, size_t a = 256) { return (v + a - 1) / a * a; }
+
+size_t tformer_embed_indexed_bwd_workspace_bytes(int n_clips, int T, int n_bank) {
+  const size_t slots = size_t(n_clips) * T;
+  return align_up((size_t(n_bank) + 1) * 4) + 2 * align_up(slots * 4);
+}
+
+int tformer_embed_indexed_bwd(int out_mode, const float* dtok, const int* index, int n_clips, int T, int dim, int n_bank, void* dbank, void* ws,
+                              size_t ws_bytes, cudaStream_t st) {
+  AVF_REQUIRE(n_clips > 0 && T > 0 && dim > 0 && dim % 4 == 0 && n_bank > 0, AVF_EINVAL,
+              "tformer_embed_indexed_bwd: n_clips=%d T=%d dim=%d n_bank=%d", n_clips, T, dim, n_bank);
+  AVF_REQUIRE(size_t(n_clips) * T <= size_t(INT32_MAX), AVF_EINVAL, "tformer_embed_indexed_bwd: %d clips of %d slots is too many", n_clips, T);
+  AVF_REQUIRE(out_mode == AVF_FP32 || out_mode == AVF_BF16, AVF_EINVAL, "tformer_embed_indexed_bwd: out_mode=%d", out_mode);
+  AVF_REQUIRE((reinterpret_cast<uintptr_t>(dtok) & 15) == 0 && (reinterpret_cast<uintptr_t>(dbank) & (out_mode == AVF_BF16 ? 7 : 15)) == 0,
+              AVF_EINVAL, "tformer_embed_indexed_bwd: dtok must be 16-byte and dbank %d-byte aligned", out_mode == AVF_BF16 ? 8 : 16);
+  const size_t need = tformer_embed_indexed_bwd_workspace_bytes(n_clips, T, n_bank);
+  AVF_REQUIRE(ws != nullptr && ws_bytes >= need, AVF_EWORKSPACE, "tformer_embed_indexed_bwd: workspace too small (%zu < %zu bytes)", ws_bytes, need);
+  const int S = n_clips * T;
+  uint8_t* p = static_cast<uint8_t*>(ws);
+  int* offs = reinterpret_cast<int*>(p);     p += align_up((size_t(n_bank) + 1) * 4);
+  int* placed = reinterpret_cast<int*>(p);   p += align_up(size_t(S) * 4);
+  int* ordered = reinterpret_cast<int*>(p);
+  launch_pdl(bank_slots_build_kernel, 1, 1024, 0, st, index, S, n_bank, offs, placed, ordered);
+  AVF_LAUNCH_CHECK("bank_slots_build_kernel");
+  launch_pdl(bank_slots_order_kernel, ceil_div(S, 256), 256, 0, st, index, S, n_bank, static_cast<const int*>(offs), static_cast<const int*>(placed),
+             ordered);
+  AVF_LAUNCH_CHECK("bank_slots_order_kernel");
+  const size_t groups = size_t(n_bank) * (dim / 4);
+  const unsigned grid = unsigned((groups + 255) / 256);
+  if (out_mode == AVF_BF16)
+    launch_pdl(tformer_embed_indexed_bwd_kernel<__nv_bfloat16>, grid, 256, 0, st, dtok, static_cast<const int*>(offs), static_cast<const int*>(ordered),
+               static_cast<__nv_bfloat16*>(dbank), n_bank, T, dim);
+  else
+    launch_pdl(tformer_embed_indexed_bwd_kernel<float>, grid, 256, 0, st, dtok, static_cast<const int*>(offs), static_cast<const int*>(ordered),
+               static_cast<float*>(dbank), n_bank, T, dim);
+  AVF_LAUNCH_CHECK("tformer_embed_indexed_bwd_kernel");
   return 0;
 }
 

@@ -299,6 +299,19 @@ int avf_gemm(int mode, int trans_a, int trans_b, const void* a, int32_t lda, con
               workspace_bytes, static_cast<cudaStream_t>(stream));
 }
 
+size_t avf_tformer_embed_indexed_bwd_workspace_bytes(int32_t n_clips, int32_t n_frames, int32_t n_bank) {
+  return n_clips > 0 && n_frames > 0 && n_bank >= 0 ? tformer_embed_indexed_bwd_workspace_bytes(n_clips, n_frames, n_bank) : 0;
+}
+
+int avf_tformer_embed_indexed_bwd(int out_mode, const float* dtok, const int32_t* index, int32_t n_clips, int32_t n_frames, int32_t dim, int32_t n_bank,
+                                  void* dbank, void* workspace, size_t workspace_bytes, void* stream) {
+  int e = require_device_train();
+  if (e) return e;
+  AVF_REQUIRE(dtok && index && dbank, AVF_EINVAL, "tformer_embed_indexed_bwd: null pointer");
+  return tformer_embed_indexed_bwd(out_mode, dtok, index, n_clips, n_frames, dim, n_bank, dbank, workspace, workspace_bytes,
+                                   static_cast<cudaStream_t>(stream));
+}
+
 size_t avf_colsum_workspace_bytes(int32_t rows, int32_t cols) { return rows > 0 && cols > 0 ? colsum_workspace_bytes(rows, cols) : 0; }
 
 int avf_colsum(int in_mode, const void* x, size_t ld, int32_t rows, int32_t cols, float* out, void* workspace, size_t workspace_bytes, void* stream) {

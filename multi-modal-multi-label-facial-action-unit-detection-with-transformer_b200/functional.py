@@ -316,6 +316,48 @@ def tformer_fwd_indexed(bank: torch.Tensor, index: torch.Tensor, cls_token: torc
     return cls
 
 
+def _index_i32(index: torch.Tensor, n_clips: int, n_frames: int, who: str) -> torch.Tensor:
+    if index.dtype != torch.int32 or not index.is_contiguous() or tuple(index.shape) != (n_clips, n_frames):
+        raise ValueError(f"{who}: index must be a contiguous int32 tensor [{n_clips}, {n_frames}], got {index.dtype} {tuple(index.shape)}")
+    return _cuda(index, "index")
+
+
+def tformer_embed_indexed(bank: torch.Tensor, index: torch.Tensor, cls_token: torch.Tensor, pos: torch.Tensor,
+                          n_frames: int) -> Tuple[torch.Tensor, torch.Tensor]:
+    """The gather + embed step of tformer_fwd_indexed alone (avf_tformer_embed_indexed): bank [n_bank, dim] fp32 / bf16, index
+    [n_clips, T] int32 on the bank's device -> (tokens [n_clips*(T+1), dim] fp32, keep [n_clips, T+1] bool), the input and the
+    attention mask of the tape-keeping encoder stack."""
+    bank = _cuda(bank, "bank").contiguous()
+    dim = bank.shape[1]
+    index = _index_i32(index, index.shape[0] if index.dim() == 2 else -1, n_frames, "tformer_embed_indexed")
+    n_clips = index.shape[0]
+    x = torch.empty((n_clips * (n_frames + 1), dim), dtype=torch.float32, device=bank.device)
+    keep = torch.empty((n_clips, n_frames + 1), dtype=torch.bool, device=bank.device)
+    check(_lib.lib().avf_tformer_embed_indexed(_io_mode(bank), _ptr(bank), bank.shape[0], _ptr(index), _ptr(_f32c(cls_token)), _ptr(_f32c(pos)),
+                                               _ptr(x), _ptr(keep), n_clips, n_frames, dim, _stream()), "tformer_embed_indexed")
+    return x, keep
+
+
+def tformer_embed_indexed_bwd(dtok: torch.Tensor, index: torch.Tensor, n_bank: int, n_frames: int,
+                              out_dtype: torch.dtype = torch.float32) -> torch.Tensor:
+    """Backward of tformer_embed_indexed into the bank (avf_tformer_embed_indexed_bwd): dtok [n_clips*(T+1), dim] fp32 -> dbank
+    [n_bank, dim] of ``out_dtype`` (fp32 / bf16), row i = the sum of the token gradients of every slot that points at frame i, in
+    ascending slot order (bit-reproducible); +0.0 where no slot does."""
+    dtok = _cuda(dtok, "dtok")
+    if dtok.dtype != torch.float32 or dtok.dim() != 2 or dtok.shape[0] % (n_frames + 1) != 0:
+        raise ValueError(f"tformer_embed_indexed_bwd: dtok must be fp32 [n_clips*(T+1), dim], got {dtok.dtype} {tuple(dtok.shape)}")
+    dtok = dtok.contiguous()
+    dim = dtok.shape[1]
+    index = _index_i32(index, dtok.shape[0] // (n_frames + 1), n_frames, "tformer_embed_indexed_bwd")
+    n_clips = index.shape[0]
+    dbank = torch.empty((n_bank, dim), dtype=out_dtype, device=dtok.device)
+    L = _lib.lib()
+    ws = workspace(L.avf_tformer_embed_indexed_bwd_workspace_bytes(n_clips, n_frames, n_bank), dtok.device)
+    check(L.avf_tformer_embed_indexed_bwd(_io_mode(dbank), _ptr(dtok), _ptr(index), n_clips, n_frames, dim, n_bank, _ptr(dbank), _ptr(ws), ws.numel(),
+                                          _stream()), "tformer_embed_indexed_bwd")
+    return dbank
+
+
 def tformer_cls_extract(x: torch.Tensor, n_clips: int, n_tok: int) -> torch.Tensor:
     dim = x.shape[-1]
     cls = torch.empty((n_clips, dim), dtype=torch.float32, device=x.device)

@@ -178,29 +178,59 @@ class TFormer(nn.Module):
         if st.dropout_state()[0] > 0.0:
             raise RuntimeError("TFormer.cls_features_indexed is inference only: this TFormer applies dropout (train() with dropout > 0), which "
                                "only the tape-keeping kernels of cls_features implement; call eval() first")
-        if bank.dim() != 2 or bank.shape[1] != self.dim:
-            raise ValueError(f"TFormer.cls_features_indexed: bank must be [n_bank, {self.dim}], got {tuple(bank.shape)}")
+        return self._cls_indexed(bank, self.bank_index(bank.shape, bank.device, index, "cls_features_indexed"))
+
+    def _cls_indexed(self, bank, index_i32):
+        st = self.spatial_transformer
+        return AF.tformer_fwd_indexed(bank.detach(), index_i32, self.cls_token.view(-1), self.pos_embedding[0], st.packed(),
+                                      st.shape(index_i32.shape[0], self.num_patches + 1))
+
+    def forward_indexed(self, bank, index):
+        """forward() on clips described by frame indices: cls features [n_clips, dim], equal bit for bit to
+        ``self(bank[index.clamp(min=0)].reshape(-1, dim), mask=index >= 0)`` -- with autograd, dropout and the bank's gradient -- without
+        the gathered copy.  The bank's gradient sums the token gradients of every clip slot that points at a frame (ascending slot order,
+        bit-reproducible), so each frame costs one backward of whatever computed the bank.  ``bank`` / ``index`` as in
+        cls_features_indexed, with the same errors.  Without anything to differentiate and without dropout this is cls_features_indexed."""
+        AF._cuda(bank, "bank")
+        return self.forward_indexed_checked(bank, self.bank_index(bank.shape, bank.device, index, "forward_indexed"))
+
+    def forward_indexed_checked(self, bank, index_i32):
+        """forward_indexed() on an index that bank_index() returned."""
+        st = self.spatial_transformer
+        if not (needs_grad(self, bank) or (st.training and st.dropout > 0.0)):      # not dropout_state(): it draws the dropout seed
+            return self._cls_indexed(bank, index_i32)
+        from .autograd import TFormerEmbedIndexedFn
+        n_clips, T = index_i32.shape[0], self.num_patches
+        tok, keep = TFormerEmbedIndexedFn.apply(bank, index_i32, self.cls_token, self.pos_embedding, T)
+        tok = st.forward_train(tok, n_clips, T + 1, keep)
+        return tok.view(n_clips, T + 1, self.dim)[:, 0]                      # cls rows (a view: data movement only)
+
+    def bank_index(self, bank_shape, device, index, who):
+        """The checks of a bank of shape ``bank_shape`` on ``device`` and its clip table, shared by the indexed entry points (error
+        messages name ``who``) -> the index as a contiguous int32 tensor on that device.  Runs no library kernel, so a caller can check
+        the table before it computes the bank."""
+        if len(bank_shape) != 2 or bank_shape[1] != self.dim:
+            raise ValueError(f"TFormer.{who}: bank must be [n_bank, {self.dim}], got {tuple(bank_shape)}")
         if not torch.is_tensor(index):
-            raise TypeError(f"TFormer.cls_features_indexed: index must be an integer tensor, got {type(index).__name__}")
+            raise TypeError(f"TFormer.{who}: index must be an integer tensor, got {type(index).__name__}")
         if index.dtype.is_floating_point or index.dtype.is_complex or index.dtype == torch.bool:
-            raise TypeError(f"TFormer.cls_features_indexed: index must be an integer tensor, got {index.dtype}")
+            raise TypeError(f"TFormer.{who}: index must be an integer tensor, got {index.dtype}")
         if index.dim() != 2 or index.shape[0] == 0 or index.shape[1] != self.num_patches:
-            raise ValueError(f"TFormer.cls_features_indexed: index must be [n_clips, {self.num_patches}] (num_patches frames per clip), got "
+            raise ValueError(f"TFormer.{who}: index must be [n_clips, {self.num_patches}] (num_patches frames per clip), got "
                              f"{tuple(index.shape)}")
         # Checked where the table lives: on the host for free, on the device at the cost of one stream synchronisation.  While a graph
         # is captured neither that synchronisation nor a host-to-device copy is possible: the index must already be on the device, and
         # the kernel's bounds guard alone holds.
         if torch.cuda.is_current_stream_capturing():
             if not index.is_cuda:
-                raise RuntimeError("TFormer.cls_features_indexed: while a CUDA graph is being captured the index must already be on the "
-                                   f"bank's device ({bank.device}); it is on {index.device}")
+                raise RuntimeError(f"TFormer.{who}: while a CUDA graph is being captured the index must already be on the "
+                                   f"bank's device ({device}); it is on {index.device}")
         else:
             lo, hi = (int(v) for v in torch.aminmax(index))
-            if lo < -1 or hi >= bank.shape[0]:
-                raise ValueError(f"TFormer.cls_features_indexed: index entries must lie in [-1, {bank.shape[0]}) (-1 = missing frame), got "
+            if lo < -1 or hi >= bank_shape[0]:
+                raise ValueError(f"TFormer.{who}: index entries must lie in [-1, {bank_shape[0]}) (-1 = missing frame), got "
                                  f"[{lo}, {hi}]")
-        return AF.tformer_fwd_indexed(bank.detach(), index.to(device=bank.device, dtype=torch.int32).contiguous(), self.cls_token.view(-1), self.pos_embedding[0],
-                                      st.packed(), st.shape(index.shape[0], self.num_patches + 1))
+        return index.to(device=device, dtype=torch.int32).contiguous()
 
     def forward(self, x, mask=None):
         """x [n_clips*T, dim] frame features -> cls features [n_clips, dim].  ``mask`` (optional): bool [n_clips, T], True = a real
