@@ -64,7 +64,7 @@ typedef struct avf_layer_weights {
 /* Geometry of an encoder stack (SURVEY.md appendix B). */
 typedef struct avf_stack_shape {
   int32_t n_seq;      /* sequences (frames for SFormer, clips otherwise) */
-  int32_t n_tok;      /* tokens per sequence: 49 / T+1 / 12               */
+  int32_t n_tok;      /* tokens per sequence: 49 / T+1 / 12; <= 64 with 32-wide heads, <= 256 with 64-wide heads */
   int32_t dim;        /* model dim D: 256 / 512 / 128 / 256               */
   int32_t heads;      /* 8                                                */
   int32_t dim_head;   /* 32 or 64                                         */
@@ -112,7 +112,8 @@ int         avf_debug_gemm_prof(uint64_t* out16);
 size_t avf_encoder_workspace_bytes(const avf_stack_shape* s, int mode);
 
 /* ---- a1..a5: the encoder ------------------------------------------------------------------- */
-/* x [n_seq*n_tok, ld_x] fp32 residual stream, updated IN PLACE through `depth` layers
+/* x [n_seq*n_tok, ld_x] fp32 residual stream, updated IN PLACE through `depth` layers (n_tok <= 64 with dim_head 32, <= 256 with
+ * dim_head 64; longer sequences return AVF_EUNSUPPORTED)
  * (models/heads.py:252-256).  If out != NULL the LAST layer's result is written to
  * out [.., ld_out] instead of x (used to write the two AU_former outputs side by side into the
  * [B,12,256] fusion input, models/avformer.py:100). */
@@ -140,7 +141,8 @@ int avf_linear_fwd(int mode, const void* a, int32_t lda, const void* w, const fl
                    const float* residual, int32_t ld_res, void* c, int32_t ldc, int c_mode,
                    int32_t m, int32_t n, int32_t k, int epilogue_flags, void* stream);
 /* softmax(q k^T * dh^-0.5) v per (sequence, head); qkv [rows, 3*heads*dh] with columns q|k|v
- * head-major (models/heads.py:221-237); out [rows, heads*dh].  io_mode = dtype of qkv and out. */
+ * head-major (models/heads.py:221-237); out [rows, heads*dh].  io_mode = dtype of qkv and out.  n_tok 65..256 needs dh = 64
+ * (bf16: any n_tok; fp32 unmasked: n_tok with K|V of one head in shared memory). */
 int avf_attention_fwd(int io_mode, const void* qkv, void* out, int32_t n_seq, int32_t n_tok,
                       int32_t heads, int32_t dim_head, void* stream);
 
@@ -164,7 +166,8 @@ int avf_tformer_embed(int io_mode, const void* frames, const float* cls_token, c
                       int32_t n_clips, int32_t n_frames, int32_t dim, void* stream);
 /* Whole TFormer (models/vformer.py:279-290) for inference: embed, `depth` layers, cls rows -> cls_out [n_clips, dim] fp32.  s->n_seq
  * = clips, s->n_tok = T+1.  Only x[:, 0] leaves the module, so the LAST layer computes keys / values for every row but the attention
- * output, out-projection, LayerNorm and MLP for the cls row of each clip only (1/(T+1) of that work). */
+ * output, out-projection, LayerNorm and MLP for the cls row of each clip only (1/(T+1) of that work).  T <= 255 (n_tok <= 256) with
+ * 64-wide heads, T <= 63 with 32-wide heads. */
 size_t avf_tformer_workspace_bytes(const avf_stack_shape* s, int mode);
 int avf_tformer_fwd(int mode, int io_mode, const avf_stack_shape* s, const avf_layer_weights* layers, const void* frames,
                     const float* cls_token, const float* pos, float* cls_out, void* workspace, size_t workspace_bytes, void* stream);
@@ -286,7 +289,8 @@ int avf_gemm(int mode, int trans_a, int trans_b, const void* a, int32_t lda, con
  * the same (p, seed, salt) and regenerates the masks instead of storing them.  dropout_salt (optional) points to one DEVICE
  * uint32 that is hashed into the seed when the kernels start: a captured CUDA graph gets fresh masks on every replay by
  * changing that word between replays.  avf_dropout_mask writes the scaled mask
- * (0 or 1/(1-p)) of one site (0 = to_out [rows, dim], 1 = GELU [rows, mlp_dim], 2 = net.3 [rows, dim]) for tests. */
+ * (0 or 1/(1-p)) of one site (0 = to_out [rows, dim], 1 = GELU [rows, mlp_dim], 2 = net.3 [rows, dim]) for tests.
+ * n_tok <= 64 with dim_head 32, <= 256 with dim_head 64, as in avf_encoder_stack_fwd. */
 size_t avf_encoder_tape_bytes(const avf_stack_shape* s, int mode);
 size_t avf_encoder_bwd_workspace_bytes(const avf_stack_shape* s, int mode);
 int avf_encoder_stack_fwd_train(int mode, const avf_stack_shape* s, const avf_layer_weights* layers,
@@ -311,7 +315,7 @@ size_t avf_layernorm_bwd_workspace_bytes(int32_t rows, int32_t dim);
 int avf_layernorm_bwd(const float* x, int32_t ld_x, const float* gamma, const float* dy_norm, float* dres, int32_t ld_d,
                       void* dx_bf16, float* dgamma, float* dbeta, float* dbias, int32_t rows, int32_t dim,
                       void* workspace, size_t workspace_bytes, void* stream);
-/* dqkv [rows, 3*heads*dh] from qkv and dout [rows, heads*dh] (softmax recomputed). */
+/* dqkv [rows, 3*heads*dh] from qkv and dout [rows, heads*dh] (softmax recomputed).  n_tok <= 64, or <= 256 with dh = 64. */
 int avf_attention_bwd(int io_mode, const void* qkv, const void* dout, void* dqkv, int32_t n_seq, int32_t n_tok,
                       int32_t heads, int32_t dim_head, void* stream);
 
@@ -348,7 +352,8 @@ int avf_adam_step(float* params, const float* grads, float* exp_avg, float* exp_
  * keep [n_seq, n_tok] DEVICE uint8, 1 = keep.  Score (i, j) of every head of sequence b survives iff keep[b, i] and keep[b, j]; the
  * other scores are filled with the same very negative value before the softmax.  So a kept query attends only to kept keys (dropped
  * keys get probability exactly 0), and a dropped query attends uniformly to all n_tok tokens (its output is the mean of V, never NaN).
- * The mask is generic: a caller that wants a token kept always (the cls slot) sets its byte.  n_tok <= 64.  keep == NULL is exactly
+ * The mask is generic: a caller that wants a token kept always (the cls slot) sets its byte.  n_tok <= 64, or <= 256 with 64-wide
+ * heads.  keep == NULL is exactly
  * the unmasked call.  A masked stack never takes the fused kernel (it runs kernel by kernel); the backward must be given the keep
  * array of its forward.  Same workspace / tape sizes as the unmasked calls. */
 int avf_attention_fwd_masked(int io_mode, const void* qkv, void* out, int32_t n_seq, int32_t n_tok,

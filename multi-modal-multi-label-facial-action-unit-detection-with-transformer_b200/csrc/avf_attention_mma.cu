@@ -6,6 +6,7 @@
 // a per-warp padded shared-memory slab (conflict-free fragment loads / ldmatrix.trans); Q fragments come
 // straight from global memory.  qkv [rows, 3*H*dh] with columns q|k|v head-major; out [rows, H*dh].
 // (The 49-token SFormer additionally has a fully fused tcgen05 path; this kernel serves every stack.)
+// Sequences of 65..256 tokens with 64-wide heads (long TFormer clips) take the CTA-per-problem kernels further down.
 #include "avf_common.cuh"
 #include "avf_internal.h"
 
@@ -475,11 +476,373 @@ int launch_bwd(const void* qkv, const void* dout, void* dqkv, int n_seq, int n_t
   return 0;
 }
 
+// ---------------------------------------------------------------------------------------------
+// Long sequences (65..256 tokens, 64-wide heads: the TFormer of long clips).  A whole score row no longer fits a warp's registers,
+// so one CTA takes one (sequence, head): the head's operands sit in padded shared memory ([rows][72] bf16, rows padded to a
+// multiple of 64 and zero-filled), warps own 16-row tiles and sweep 64-key blocks, and no warp holds more than a 16 x 64 tile.
+// The rounding points are those of the kernels above: exact row max, exp2 against it, fp32 sums, P / dS rounded to bf16 for the
+// MMA, O scaled by 1/l before its bf16 store.  Keep bits of up to 256 tokens are four 64-bit words in shared memory.
+// ---------------------------------------------------------------------------------------------
+constexpr int kLongDH = 64, kLongPitch = kLongDH + 8, kLongWarps = 8, kLongMaxTok = 256;
+using LongRow = __nv_bfloat16[kLongPitch];
+
+__host__ __device__ __forceinline__ int long_rows(int n_tok) { return (n_tok + 63) & ~63; }
+
+// Keep bits of one sequence of up to 256 tokens into km[4] (bit j of word w = token 64 w + j is kept); warps 0..3 take a word each.
+__device__ __forceinline__ void keep_words(const uint8_t* __restrict__ row, int n_tok, uint64_t* km, int warp, int lane) {
+  if (warp < 4) {
+    const int b = warp * 64;
+    const uint64_t w = keep_bits(row + b, min(max(n_tok - b, 0), 64), lane);
+    if (lane == 0) km[warp] = w;
+  }
+}
+__device__ __forceinline__ bool keep_bit(const uint64_t* km, int i) { return (km[i >> 6] >> (i & 63)) & 1; }
+
+// rows [0, n_tok) of the head's 64 columns starting at src (row stride ld elements) -> dst [long_rows(n_tok)][72], zero-filled
+__device__ __forceinline__ void stage_rows(LongRow* dst, const __nv_bfloat16* __restrict__ src, size_t ld, int n_tok) {
+  const int n = long_rows(n_tok) * (kLongDH / 8);
+  for (int i = threadIdx.x; i < n; i += blockDim.x) {
+    const int r = i >> 3, c = (i & 7) * 8;
+    uint4 v = make_uint4(0, 0, 0, 0);
+    if (r < n_tok) v = *reinterpret_cast<const uint4*>(src + size_t(r) * ld + c);
+    *reinterpret_cast<uint4*>(&dst[r][c]) = v;
+  }
+}
+
+// A fragments (16 rows from r_lo - g, 64 columns) of a row-major shared-memory matrix
+__device__ __forceinline__ void long_load_a(uint32_t (&f)[4][4], const LongRow* M, int r_lo, int t) {
+#pragma unroll
+  for (int ks = 0; ks < 4; ++ks) {
+    f[ks][0] = *reinterpret_cast<const uint32_t*>(&M[r_lo][ks * 16 + 2 * t]);
+    f[ks][1] = *reinterpret_cast<const uint32_t*>(&M[r_lo + 8][ks * 16 + 2 * t]);
+    f[ks][2] = *reinterpret_cast<const uint32_t*>(&M[r_lo][ks * 16 + 8 + 2 * t]);
+    f[ks][3] = *reinterpret_cast<const uint32_t*>(&M[r_lo + 8][ks * 16 + 8 + 2 * t]);
+  }
+}
+// C[16 x 64] = A * M[0:64]^T  (M: the block's 64 rows, row-major)
+__device__ __forceinline__ void long_mma_abt(float (&c)[8][4], const uint32_t (&a)[4][4], const LongRow* M, int g, int t) {
+#pragma unroll
+  for (int nt = 0; nt < 8; ++nt) {
+    c[nt][0] = c[nt][1] = c[nt][2] = c[nt][3] = 0.f;
+#pragma unroll
+    for (int ks = 0; ks < 4; ++ks) {
+      const uint32_t b0 = *reinterpret_cast<const uint32_t*>(&M[nt * 8 + g][ks * 16 + 2 * t]);
+      const uint32_t b1 = *reinterpret_cast<const uint32_t*>(&M[nt * 8 + g][ks * 16 + 8 + 2 * t]);
+      mma_bf16_16816(c[nt], a[ks], b0, b1);
+    }
+  }
+}
+// D[16 x 64] += bf16(X[16 x 64]) * M[0:64]
+__device__ __forceinline__ void long_mma_xm(float (&d)[8][4], const float (&x)[8][4], const LongRow* M, int lane) {
+#pragma unroll
+  for (int kt = 0; kt < 4; ++kt) {
+    uint32_t pa[4];
+    pa[0] = pack_bf16x2(x[2 * kt][0], x[2 * kt][1]);
+    pa[1] = pack_bf16x2(x[2 * kt][2], x[2 * kt][3]);
+    pa[2] = pack_bf16x2(x[2 * kt + 1][0], x[2 * kt + 1][1]);
+    pa[3] = pack_bf16x2(x[2 * kt + 1][2], x[2 * kt + 1][3]);
+#pragma unroll
+    for (int nt = 0; nt < 8; ++nt) {
+      uint32_t b0, b1;
+      ldmatrix_x2_trans(b0, b1, &M[kt * 16 + (lane & 15)][nt * 8]);
+      mma_bf16_16816(d[nt], pa, b0, b1);
+    }
+  }
+}
+// Scores of key block kb (columns c = kb*64 + local) masked like the short kernels: mask_score on the block's keep word.
+template <bool MASKED>
+__device__ __forceinline__ void long_mask(float (&s)[8][4], bool k_lo, bool k_hi, uint64_t kw, int n_left, int t) {
+#pragma unroll
+  for (int nt = 0; nt < 8; ++nt) {
+    const int c = nt * 8 + 2 * t;
+    if constexpr (MASKED) {
+      s[nt][0] = mask_score(s[nt][0], k_lo, kw, c, n_left); s[nt][1] = mask_score(s[nt][1], k_lo, kw, c + 1, n_left);
+      s[nt][2] = mask_score(s[nt][2], k_hi, kw, c, n_left); s[nt][3] = mask_score(s[nt][3], k_hi, kw, c + 1, n_left);
+    } else {
+      if (c >= n_left) { s[nt][0] = -INFINITY; s[nt][2] = -INFINITY; }
+      if (c + 1 >= n_left) { s[nt][1] = -INFINITY; s[nt][3] = -INFINITY; }
+    }
+  }
+}
+__device__ __forceinline__ float quad_max(float v) {
+  v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, 1));
+  return fmaxf(v, __shfl_xor_sync(0xffffffffu, v, 2));
+}
+__device__ __forceinline__ float quad_sum(float v) {
+  v += __shfl_xor_sync(0xffffffffu, v, 1);
+  return v + __shfl_xor_sync(0xffffffffu, v, 2);
+}
+// 16 x 64 fp32 tile * mul -> bf16 rows r_lo, r_lo + 8 (if < n_valid) of dst (row stride ld)
+__device__ __forceinline__ void long_store(const float (&d)[8][4], __nv_bfloat16* dst, size_t ld, int r_lo, int n_valid, float mul_lo, float mul_hi,
+                                           int t) {
+  __nv_bfloat16* lo = dst + size_t(r_lo) * ld + 2 * t;
+  __nv_bfloat16* hi = lo + 8 * ld;
+#pragma unroll
+  for (int nt = 0; nt < 8; ++nt) {
+    if (r_lo < n_valid) *reinterpret_cast<uint32_t*>(lo + nt * 8) = pack_bf16x2(d[nt][0] * mul_lo, d[nt][1] * mul_lo);
+    if (r_lo + 8 < n_valid) *reinterpret_cast<uint32_t*>(hi + nt * 8) = pack_bf16x2(d[nt][2] * mul_hi, d[nt][3] * mul_hi);
+  }
+}
+
+// Forward: two sweeps over the key blocks per 16-row query tile, the first for the exact row max, the second for exp2, l and P V.
+template <bool MASKED>
+__global__ void __launch_bounds__(kLongWarps * 32) attention_long_mma_kernel(const __nv_bfloat16* __restrict__ qkv, __nv_bfloat16* __restrict__ out,
+                                                                            int n_tok, int heads, float scale_log2e, int q_rows,
+                                                                            const uint8_t* __restrict__ keep) {
+  pdl_wait();      // programmatic dependent launch: everything above is launch overhead hidden behind the previous kernel
+  pdl_trigger();
+  extern __shared__ __align__(16) uint8_t smem_long[];
+  const int NR = long_rows(n_tok);
+  LongRow* Ks = reinterpret_cast<LongRow*>(smem_long);
+  LongRow* Vs = Ks + NR;
+  uint64_t* km = reinterpret_cast<uint64_t*>(Vs + NR);
+  const int seq = blockIdx.x / heads, head = blockIdx.x - seq * heads;
+  const int inner = heads * kLongDH, warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const size_t row0 = size_t(seq) * n_tok, ld = size_t(3) * inner;
+  const __nv_bfloat16* base = qkv + row0 * ld + head * kLongDH;
+  stage_rows(Ks, base + inner, ld, n_tok);
+  stage_rows(Vs, base + 2 * inner, ld, n_tok);
+  if constexpr (MASKED) keep_words(keep + row0, n_tok, km, warp, lane);
+  __syncthreads();
+
+  const int g = lane >> 2, t = lane & 3, nkb = NR / 64;
+#pragma unroll 1
+  for (int mt = warp; mt * 16 < q_rows; mt += kLongWarps) {
+    const int r_lo = mt * 16 + g, r_hi = r_lo + 8;
+    uint32_t qf[4][4];
+#pragma unroll
+    for (int ks = 0; ks < 4; ++ks) {
+#pragma unroll
+      for (int h = 0; h < 2; ++h) {
+        const int c = ks * 16 + h * 8 + 2 * t;
+        qf[ks][2 * h] = r_lo < n_tok ? *reinterpret_cast<const uint32_t*>(base + size_t(r_lo) * ld + c) : 0u;
+        qf[ks][2 * h + 1] = r_hi < n_tok ? *reinterpret_cast<const uint32_t*>(base + size_t(r_hi) * ld + c) : 0u;
+      }
+    }
+    const bool k_lo = MASKED && keep_bit(km, r_lo), k_hi = MASKED && keep_bit(km, r_hi);
+    float s[8][4];
+    float m_lo = -INFINITY, m_hi = -INFINITY;
+#pragma unroll 1
+    for (int kb = 0; kb < nkb; ++kb) {
+      long_mma_abt(s, qf, Ks + kb * 64, g, t);
+      long_mask<MASKED>(s, k_lo, k_hi, MASKED ? km[kb] : 0, n_tok - kb * 64, t);
+#pragma unroll
+      for (int nt = 0; nt < 8; ++nt) {
+        m_lo = fmaxf(m_lo, fmaxf(s[nt][0], s[nt][1]));
+        m_hi = fmaxf(m_hi, fmaxf(s[nt][2], s[nt][3]));
+      }
+    }
+    const float o_lo = quad_max(m_lo) * scale_log2e, o_hi = quad_max(m_hi) * scale_log2e;
+    float l_lo = 0.f, l_hi = 0.f, o[8][4];
+#pragma unroll
+    for (int nt = 0; nt < 8; ++nt) o[nt][0] = o[nt][1] = o[nt][2] = o[nt][3] = 0.f;
+#pragma unroll 1
+    for (int kb = 0; kb < nkb; ++kb) {
+      long_mma_abt(s, qf, Ks + kb * 64, g, t);
+      long_mask<MASKED>(s, k_lo, k_hi, MASKED ? km[kb] : 0, n_tok - kb * 64, t);
+#pragma unroll
+      for (int nt = 0; nt < 8; ++nt) {
+        s[nt][0] = exp2f(fmaf(s[nt][0], scale_log2e, -o_lo));
+        s[nt][1] = exp2f(fmaf(s[nt][1], scale_log2e, -o_lo));
+        s[nt][2] = exp2f(fmaf(s[nt][2], scale_log2e, -o_hi));
+        s[nt][3] = exp2f(fmaf(s[nt][3], scale_log2e, -o_hi));
+        l_lo += s[nt][0] + s[nt][1];
+        l_hi += s[nt][2] + s[nt][3];
+      }
+      long_mma_xm(o, s, Vs + kb * 64, lane);
+    }
+    long_store(o, out + size_t(seq) * q_rows * inner + head * kLongDH, inner, r_lo, q_rows, 1.f / quad_sum(l_lo), 1.f / quad_sum(l_hi), t);
+  }
+}
+
+// Backward, the two passes of attention_bwd_mma_kernel with Q, K, V, dO of the (sequence, head) in shared memory:
+//   pass 1 (rows = queries): sweep 1 the row max, sweep 2 l and sum_j e_j dP_j (delta = that / l), sweep 3 dS and dQ = dS K;
+//   pass 2 (rows = keys): one sweep over 64-query blocks, P^T and dS^T from the saved statistics, dV = P^T dO, dK = dS^T Q.
+template <bool MASKED>
+__global__ void __launch_bounds__(kLongWarps * 32) attention_bwd_long_mma_kernel(const __nv_bfloat16* __restrict__ qkv,
+                                                                                const __nv_bfloat16* __restrict__ dout,
+                                                                                __nv_bfloat16* __restrict__ dqkv, int n_tok, int heads,
+                                                                                float scale, const uint8_t* __restrict__ keep) {
+  pdl_wait();      // programmatic dependent launch: everything above is launch overhead hidden behind the previous kernel
+  pdl_trigger();
+  extern __shared__ __align__(16) uint8_t smem_long[];
+  const int NR = long_rows(n_tok);
+  LongRow* Qs = reinterpret_cast<LongRow*>(smem_long);
+  LongRow* Ks = Qs + NR;
+  LongRow* Vs = Ks + NR;
+  LongRow* Os = Vs + NR;
+  float* st_m = reinterpret_cast<float*>(Os + NR);      // row max (exp2 units), 1 / row sum, delta
+  float* st_il = st_m + NR;
+  float* st_d = st_il + NR;
+  uint64_t* km = reinterpret_cast<uint64_t*>(st_d + NR);
+  const int seq = blockIdx.x / heads, head = blockIdx.x - seq * heads;
+  const int inner = heads * kLongDH, warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const size_t row0 = size_t(seq) * n_tok, ld = size_t(3) * inner;
+  const __nv_bfloat16* base = qkv + row0 * ld + head * kLongDH;
+  __nv_bfloat16* dbase = dqkv + row0 * ld + head * kLongDH;
+  stage_rows(Qs, base, ld, n_tok);
+  stage_rows(Ks, base + inner, ld, n_tok);
+  stage_rows(Vs, base + 2 * inner, ld, n_tok);
+  stage_rows(Os, dout + row0 * inner + head * kLongDH, inner, n_tok);
+  if constexpr (MASKED) keep_words(keep + row0, n_tok, km, warp, lane);
+  __syncthreads();
+  const float scale_log2e = scale * 1.4426950408889634f;
+  const int g = lane >> 2, t = lane & 3, nkb = NR / 64;
+
+  // ---- pass 1: rows = queries ------------------------------------------------------------------------------
+#pragma unroll 1
+  for (int mt = warp; mt * 16 < n_tok; mt += kLongWarps) {
+    const int r_lo = mt * 16 + g, r_hi = r_lo + 8;
+    uint32_t qf[4][4], of[4][4];
+    long_load_a(qf, Qs, r_lo, t);
+    long_load_a(of, Os, r_lo, t);
+    const bool k_lo = MASKED && keep_bit(km, r_lo), k_hi = MASKED && keep_bit(km, r_hi);
+    float s[8][4], dp[8][4];
+    float m_lo = -INFINITY, m_hi = -INFINITY;
+#pragma unroll 1
+    for (int kb = 0; kb < nkb; ++kb) {
+      long_mma_abt(s, qf, Ks + kb * 64, g, t);
+      long_mask<MASKED>(s, k_lo, k_hi, MASKED ? km[kb] : 0, n_tok - kb * 64, t);
+#pragma unroll
+      for (int nt = 0; nt < 8; ++nt) {
+        m_lo = fmaxf(m_lo, fmaxf(s[nt][0], s[nt][1]));
+        m_hi = fmaxf(m_hi, fmaxf(s[nt][2], s[nt][3]));
+      }
+    }
+    const float o_lo = quad_max(m_lo) * scale_log2e, o_hi = quad_max(m_hi) * scale_log2e;
+    float l_lo = 0.f, l_hi = 0.f, e_lo = 0.f, e_hi = 0.f;
+#pragma unroll 1
+    for (int kb = 0; kb < nkb; ++kb) {
+      long_mma_abt(s, qf, Ks + kb * 64, g, t);
+      long_mask<MASKED>(s, k_lo, k_hi, MASKED ? km[kb] : 0, n_tok - kb * 64, t);
+      long_mma_abt(dp, of, Vs + kb * 64, g, t);
+#pragma unroll
+      for (int nt = 0; nt < 8; ++nt) {
+        const float a0 = exp2f(fmaf(s[nt][0], scale_log2e, -o_lo)), a1 = exp2f(fmaf(s[nt][1], scale_log2e, -o_lo));
+        const float a2 = exp2f(fmaf(s[nt][2], scale_log2e, -o_hi)), a3 = exp2f(fmaf(s[nt][3], scale_log2e, -o_hi));
+        l_lo += a0 + a1;
+        l_hi += a2 + a3;
+        e_lo += a0 * dp[nt][0] + a1 * dp[nt][1];
+        e_hi += a2 * dp[nt][2] + a3 * dp[nt][3];
+      }
+    }
+    const float i_lo = 1.f / quad_sum(l_lo), i_hi = 1.f / quad_sum(l_hi);
+    const float d_lo = quad_sum(e_lo) * i_lo, d_hi = quad_sum(e_hi) * i_hi;
+    if (t == 0) {
+      st_m[r_lo] = o_lo; st_il[r_lo] = i_lo; st_d[r_lo] = d_lo;
+      st_m[r_hi] = o_hi; st_il[r_hi] = i_hi; st_d[r_hi] = d_hi;
+    }
+    float dq[8][4];
+#pragma unroll
+    for (int nt = 0; nt < 8; ++nt) dq[nt][0] = dq[nt][1] = dq[nt][2] = dq[nt][3] = 0.f;
+#pragma unroll 1
+    for (int kb = 0; kb < nkb; ++kb) {
+      long_mma_abt(s, qf, Ks + kb * 64, g, t);
+      long_mask<MASKED>(s, k_lo, k_hi, MASKED ? km[kb] : 0, n_tok - kb * 64, t);
+      long_mma_abt(dp, of, Vs + kb * 64, g, t);
+#pragma unroll
+      for (int nt = 0; nt < 8; ++nt) {        // dS (the 1/sqrt(dh) is applied once when dQ is stored)
+        s[nt][0] = exp2f(fmaf(s[nt][0], scale_log2e, -o_lo)) * i_lo * (dp[nt][0] - d_lo);
+        s[nt][1] = exp2f(fmaf(s[nt][1], scale_log2e, -o_lo)) * i_lo * (dp[nt][1] - d_lo);
+        s[nt][2] = exp2f(fmaf(s[nt][2], scale_log2e, -o_hi)) * i_hi * (dp[nt][2] - d_hi);
+        s[nt][3] = exp2f(fmaf(s[nt][3], scale_log2e, -o_hi)) * i_hi * (dp[nt][3] - d_hi);
+        if constexpr (MASKED) {                // every score of a dropped query was filled
+          if (!k_lo) s[nt][0] = s[nt][1] = 0.f;
+          if (!k_hi) s[nt][2] = s[nt][3] = 0.f;
+        }
+      }
+      long_mma_xm(dq, s, Ks + kb * 64, lane);
+    }
+    long_store(dq, dbase, ld, r_lo, n_tok, scale, scale, t);
+  }
+  __syncthreads();
+
+  // ---- pass 2: rows = keys ------------------------------------------------------------------------------------
+#pragma unroll 1
+  for (int mt = warp; mt * 16 < n_tok; mt += kLongWarps) {
+    const int r_lo = mt * 16 + g;
+    uint32_t kf[4][4], vf[4][4];
+    long_load_a(kf, Ks, r_lo, t);
+    long_load_a(vf, Vs, r_lo, t);
+    const bool k_lo = MASKED && keep_bit(km, r_lo), k_hi = MASKED && keep_bit(km, r_lo + 8);
+    float dv[8][4], dk[8][4];
+#pragma unroll
+    for (int nt = 0; nt < 8; ++nt) dv[nt][0] = dv[nt][1] = dv[nt][2] = dv[nt][3] = dk[nt][0] = dk[nt][1] = dk[nt][2] = dk[nt][3] = 0.f;
+#pragma unroll 1
+    for (int qb = 0; qb < nkb; ++qb) {
+      float p[8][4], ds[8][4];
+      long_mma_abt(p, kf, Qs + qb * 64, g, t);        // S^T[key][query]
+      long_mma_abt(ds, vf, Os + qb * 64, g, t);       // dP^T[key][query]
+      const uint64_t qw = MASKED ? km[qb] : 0;
+#pragma unroll
+      for (int nt = 0; nt < 8; ++nt) {
+#pragma unroll
+        for (int e = 0; e < 2; ++e) {
+          const int ql = nt * 8 + 2 * t + e, qi = qb * 64 + ql;     // query of elements e (row r_lo) and e + 2 (row r_lo + 8)
+          const bool ok = qi < n_tok;
+          const float m = ok ? st_m[qi] : 0.f, il = ok ? st_il[qi] : 0.f, dl = ok ? st_d[qi] : 0.f;
+          float p0, p1;
+          if constexpr (MASKED) {             // dropped query: its uniform row 1 / n_tok (= il of pass 1) and dS = 0
+            const bool qk = (qw >> ql) & 1;
+            p0 = ok ? exp2f(fmaf(qk ? (k_lo ? p[nt][e] : -INFINITY) : 0.f, scale_log2e, -m)) * il : 0.f;       // m = 0 on a dropped row
+            p1 = ok ? exp2f(fmaf(qk ? (k_hi ? p[nt][e + 2] : -INFINITY) : 0.f, scale_log2e, -m)) * il : 0.f;
+            ds[nt][e] = qk ? p0 * (ds[nt][e] - dl) : 0.f;
+            ds[nt][e + 2] = qk ? p1 * (ds[nt][e + 2] - dl) : 0.f;
+          } else {
+            p0 = ok ? exp2f(fmaf(p[nt][e], scale_log2e, -m)) * il : 0.f;
+            p1 = ok ? exp2f(fmaf(p[nt][e + 2], scale_log2e, -m)) * il : 0.f;
+            ds[nt][e] = p0 * (ds[nt][e] - dl);
+            ds[nt][e + 2] = p1 * (ds[nt][e + 2] - dl);
+          }
+          p[nt][e] = p0;
+          p[nt][e + 2] = p1;
+        }
+      }
+      long_mma_xm(dv, p, Os + qb * 64, lane);         // dV = P^T dO
+      long_mma_xm(dk, ds, Qs + qb * 64, lane);        // dK = dS^T Q / sqrt(dh)
+    }
+    long_store(dv, dbase + 2 * inner, ld, r_lo, n_tok, 1.f, 1.f, t);
+    long_store(dk, dbase + inner, ld, r_lo, n_tok, scale, scale, t);
+  }
+}
+
+size_t long_fwd_smem(int n_tok) { return size_t(2) * long_rows(n_tok) * kLongPitch * 2 + 4 * sizeof(uint64_t); }
+size_t long_bwd_smem(int n_tok) { return size_t(4) * long_rows(n_tok) * kLongPitch * 2 + size_t(3) * long_rows(n_tok) * 4 + 4 * sizeof(uint64_t); }
+
+template <bool MASKED>
+int launch_long(const void* qkv, void* out, int n_seq, int n_tok, int heads, int q_rows, const uint8_t* keep, cudaStream_t st) {
+  auto kern = attention_long_mma_kernel<MASKED>;
+  static PerDeviceOnce once;
+  if (once.first()) {
+    AVF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, int(long_fwd_smem(kLongMaxTok))));
+  }
+  launch_pdl(kern, n_seq * heads, kLongWarps * 32, long_fwd_smem(n_tok), st, static_cast<const __nv_bfloat16*>(qkv), static_cast<__nv_bfloat16*>(out), n_tok,
+             heads, 1.4426950408889634f / sqrtf(float(kLongDH)), q_rows, keep);
+  AVF_LAUNCH_CHECK("attention_long_mma_kernel");
+  return 0;
+}
+
+template <bool MASKED>
+int launch_bwd_long(const void* qkv, const void* dout, void* dqkv, int n_seq, int n_tok, int heads, const uint8_t* keep, cudaStream_t st) {
+  auto kern = attention_bwd_long_mma_kernel<MASKED>;
+  static PerDeviceOnce once;
+  if (once.first()) {
+    AVF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, int(long_bwd_smem(kLongMaxTok))));
+  }
+  launch_pdl(kern, n_seq * heads, kLongWarps * 32, long_bwd_smem(n_tok), st, static_cast<const __nv_bfloat16*>(qkv), static_cast<const __nv_bfloat16*>(dout),
+             static_cast<__nv_bfloat16*>(dqkv), n_tok, heads, 1.0f / sqrtf(float(kLongDH)), keep);
+  AVF_LAUNCH_CHECK("attention_bwd_long_mma_kernel");
+  return 0;
+}
+
 }  // namespace
 
 int attention_mma_bf16(const void* qkv, void* out, int n_seq, int n_tok, int heads, int dim_head, cudaStream_t st, int q_rows, const uint8_t* keep) {
-  AVF_REQUIRE(n_tok >= 1 && n_tok <= 64, AVF_EUNSUPPORTED, "attention: n_tok=%d (1..64)", n_tok);
+  AVF_REQUIRE(n_tok >= 1 && n_tok <= kLongMaxTok && (n_tok <= 64 || dim_head == kLongDH), AVF_EUNSUPPORTED,
+              "attention: n_tok=%d with dim_head=%d (1..64 tokens; 64-wide heads up to 256)", n_tok, dim_head);
   if (q_rows <= 0 || q_rows > n_tok) q_rows = n_tok;
+  if (n_tok > 64)
+    return keep ? launch_long<true>(qkv, out, n_seq, n_tok, heads, q_rows, keep, st) : launch_long<false>(qkv, out, n_seq, n_tok, heads, q_rows, nullptr, st);
   const int np = (n_tok + 15) / 16 * 16;
 #define AVF_ATT(D, P)                                                                                   \
   if (dim_head == D && np == P)                                                                         \
@@ -497,7 +860,11 @@ int attention_mma_bf16(const void* qkv, void* out, int n_seq, int n_tok, int hea
 namespace avf {
 int attention_bwd_mma_bf16(const void* qkv, const void* dout, void* dqkv, int n_seq, int n_tok, int heads, int dim_head, cudaStream_t st,
                            const uint8_t* keep) {
-  AVF_REQUIRE(n_tok >= 1 && n_tok <= 64, AVF_EUNSUPPORTED, "attention_bwd: n_tok=%d (1..64)", n_tok);
+  AVF_REQUIRE(n_tok >= 1 && n_tok <= kLongMaxTok && (n_tok <= 64 || dim_head == kLongDH), AVF_EUNSUPPORTED,
+              "attention_bwd: n_tok=%d with dim_head=%d (1..64 tokens; 64-wide heads up to 256)", n_tok, dim_head);
+  if (n_tok > 64)
+    return keep ? launch_bwd_long<true>(qkv, dout, dqkv, n_seq, n_tok, heads, keep, st)
+                : launch_bwd_long<false>(qkv, dout, dqkv, n_seq, n_tok, heads, nullptr, st);
   const int np = (n_tok + 15) / 16 * 16;
 #define AVF_ATT(D, P)                                                                                   \
   if (dim_head == D && np == P)                                                                         \

@@ -1,6 +1,7 @@
 // CUDA-core kernels: the fp32 "parity mode" GEMM (1e-4-relative agreement with the reference needs
 // true fp32 products, which the tensor cores do not offer) and the small-sequence attention
 // (N <= 64 tokens: 12 / 17 / 49) used by both modes outside the fused tcgen05 layer kernel.
+// Masked fp32 attention of 65..256 tokens (64-wide heads) has a kernel of its own.
 #include "avf_common.cuh"
 #include "avf_internal.h"
 
@@ -246,6 +247,75 @@ __global__ void __launch_bounds__(DH == 32 ? 512 : 256) attention_small_kernel(c
   }
 }
 
+// Masked fp32 attention of 65..256 tokens with 64-wide heads: one CTA per (sequence, head), K|V of the head in shared memory
+// ([n_tok][2][64], the layout of attention_small_kernel with one head per block) and the keep bits as four 64-bit words behind them.
+// Every query row runs the per-thread online softmax of attention_small_kernel in the same order, so an all-kept mask gives the
+// bits of the unmasked call.
+__global__ void __launch_bounds__(256) attention_long_f32_kernel(const float* __restrict__ qkv, float* __restrict__ out, int n_tok, int heads,
+                                                                 float scale_log2e, const uint8_t* __restrict__ keep) {
+  pdl_wait();      // programmatic dependent launch: everything above is launch overhead hidden behind the previous kernel
+  pdl_trigger();
+  constexpr int DH = 64;
+  extern __shared__ __align__(16) uint8_t smem_long_f32[];
+  float* kv = reinterpret_cast<float*>(smem_long_f32);
+  uint64_t* km = reinterpret_cast<uint64_t*>(kv + size_t(n_tok) * 2 * DH);
+  const int seq = blockIdx.x / heads, h = blockIdx.x - seq * heads;
+  const int inner = heads * DH, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const size_t row0 = size_t(seq) * n_tok;
+  for (int i = threadIdx.x; i < n_tok * 2 * DH / 4; i += blockDim.x) {
+    const int r = i / (2 * DH / 4), c = (i - r * (2 * DH / 4)) * 4;
+    const int part = c / DH, col = c - part * DH;
+    *reinterpret_cast<float4*>(kv + size_t(r) * 2 * DH + c) =
+        *reinterpret_cast<const float4*>(qkv + (row0 + r) * (3 * inner) + size_t(1 + part) * inner + h * DH + col);
+  }
+  if (warp < 4) {
+    const int b = warp * 64;
+    const uint8_t* row = keep + row0 + b;
+    const uint32_t lo = __ballot_sync(0xffffffffu, b + lane < n_tok && row[lane] != 0);
+    const uint32_t hi = __ballot_sync(0xffffffffu, b + lane + 32 < n_tok && row[lane + 32] != 0);
+    if (lane == 0) km[warp] = (uint64_t(hi) << 32) | lo;
+  }
+  __syncthreads();
+  for (int qi = threadIdx.x; qi < n_tok; qi += blockDim.x) {
+    const size_t row = row0 + qi;
+    float q[DH];
+    load_frag<float, DH>(qkv + row * (3 * inner) + h * DH, q);
+#pragma unroll
+    for (int d = 0; d < DH; ++d) q[d] *= scale_log2e;
+    float m = -INFINITY, l = 0.f, acc[DH];
+#pragma unroll
+    for (int d = 0; d < DH; ++d) acc[d] = 0.f;
+    const bool row_kept = (km[qi >> 6] >> (qi & 63)) & 1;
+    for (int j = 0; j < n_tok; ++j) {
+      if (row_kept && !((km[j >> 6] >> (j & 63)) & 1)) continue;
+      const float* kp = kv + size_t(j) * 2 * DH;
+      float kf[DH];
+      load_frag<float, DH>(kp, kf);
+      float s = 0.f;
+      if (row_kept) {
+#pragma unroll
+        for (int d = 0; d < DH; ++d) s = fmaf(q[d], kf[d], s);
+      }
+      if (s > m) {
+        const float corr = exp2f(m - s);
+        l *= corr;
+#pragma unroll
+        for (int d = 0; d < DH; ++d) acc[d] *= corr;
+        m = s;
+      }
+      const float p = exp2f(s - m);
+      l += p;
+      load_frag<float, DH>(kp + DH, kf);
+#pragma unroll
+      for (int d = 0; d < DH; ++d) acc[d] = fmaf(p, kf[d], acc[d]);
+    }
+    const float inv = 1.f / l;
+#pragma unroll
+    for (int d = 0; d < DH; ++d) acc[d] *= inv;
+    store_frag<float, DH>(out + row * inner + h * DH, acc);
+  }
+}
+
 }  // namespace
 
 int linear_f32(const float* a, int lda, const float* w, const float* bias, const float* res, int ld_res, void* c, int ldc,
@@ -303,8 +373,20 @@ static int launch_attention(const void* qkv, void* out, int n_seq, int n_tok, in
 int attention_small(int io_mode, const void* qkv, void* out, int n_seq, int n_tok, int heads, int dim_head, cudaStream_t st, const uint8_t* keep) {
   AVF_REQUIRE(n_seq > 0 && n_tok > 0 && heads > 0, AVF_EINVAL, "attention: n_seq=%d n_tok=%d heads=%d", n_seq, n_tok, heads);
   AVF_REQUIRE(dim_head == 32 || dim_head == 64, AVF_EUNSUPPORTED, "attention: dim_head=%d (supported: 32, 64)", dim_head);
-  AVF_REQUIRE(keep == nullptr || n_tok <= 64, AVF_EUNSUPPORTED, "attention: a keep mask needs n_tok <= 64 (n_tok=%d)", n_tok);
+  AVF_REQUIRE(keep == nullptr || n_tok <= 64 || (dim_head == 64 && n_tok <= 256), AVF_EUNSUPPORTED,
+              "attention: a keep mask needs n_tok <= 64, or <= 256 with 64-wide heads (n_tok=%d, dim_head=%d)", n_tok, dim_head);
   if (io_mode == AVF_BF16) return attention_mma_bf16(qkv, out, n_seq, n_tok, heads, dim_head, st, 0, keep);   // tensor cores
+  if (keep != nullptr && n_tok > 64) {
+    const size_t smem = size_t(n_tok) * 2 * 64 * sizeof(float) + 4 * sizeof(uint64_t);
+    static PerDeviceOnce once;
+    if (once.first()) {
+      AVF_CUDA(cudaFuncSetAttribute(attention_long_f32_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(256 * 2 * 64 * sizeof(float) + 32)));
+    }
+    launch_pdl(attention_long_f32_kernel, n_seq * heads, 256, smem, st, static_cast<const float*>(qkv), static_cast<float*>(out), n_tok, heads,
+               1.4426950408889634f / sqrtf(64.f), keep);
+    AVF_LAUNCH_CHECK("attention_long_f32_kernel");
+    return 0;
+  }
   if (keep != nullptr)
     return dim_head == 32 ? launch_attention<float, 32, true>(qkv, out, n_seq, n_tok, heads, keep, st)
                           : launch_attention<float, 64, true>(qkv, out, n_seq, n_tok, heads, keep, st);

@@ -357,6 +357,144 @@ __global__ void __launch_bounds__(128) attention_bwd_kernel(const T* __restrict_
 }
 
 // ---------------------------------------------------------------------------------------------
+// Attention backward of 65..256 tokens with 64-wide heads (fp32), one (sequence, head) per CTA.  Two n_tok x 64 operands fit shared
+// memory, four do not, so the CTA runs two passes, each with one warp per row and the lanes over the other side's tokens:
+//   pass 1, K | V staged, rows = queries: scores and dP, softmax statistics (max, 1/sum, delta) to shared memory, dQ = scale dS K;
+//   pass 2, Q | dO restaged, rows = keys: P and dS again from the statistics, dV = P^T dO, dK = scale dS^T Q.
+// The row's own operand pair sits in a per-warp slot (broadcast reads) and its scores in a per-warp line.  Masks as in
+// attention_bwd_kernel, with the keep bits in four 64-bit words.
+// ---------------------------------------------------------------------------------------------
+constexpr int kLongF32Pitch = 64 + 1;
+__host__ __device__ constexpr size_t attention_bwd_long_smem(int n_tok) {
+  return (size_t(2) * n_tok * kLongF32Pitch + 8 * (2 * 64 + 2 * 256) + 3 * 256) * sizeof(float) + 4 * sizeof(uint64_t);
+}
+
+template <bool MASKED>
+__global__ void __launch_bounds__(256) attention_bwd_long_f32_kernel(const float* __restrict__ qkv, const float* __restrict__ dout,
+                                                                     float* __restrict__ dqkv, int n_tok, int heads, float scale,
+                                                                     const uint8_t* __restrict__ keep) {
+  pdl_wait();      // programmatic dependent launch: everything above is launch overhead hidden behind the previous kernel
+  pdl_trigger();
+  constexpr int DH = 64, P = kLongF32Pitch;
+  extern __shared__ float sm_long[];
+  const int N = n_tok;
+  float* sa = sm_long;                  // [N][P]  K, then Q
+  float* sb = sa + N * P;               // [N][P]  V, then dO
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  float* own = sb + N * P + warp * (2 * DH + 2 * 256);      // this warp's row pair [2][DH], then its lines [2][256]
+  float* l0 = own + 2 * DH;
+  float* l1 = l0 + 256;
+  float* st_m = sb + N * P + 8 * (2 * DH + 2 * 256);       // [256] row max (exp2 units), 1 / row sum, delta
+  float* st_il = st_m + 256;
+  float* st_d = st_il + 256;
+  uint64_t* km = reinterpret_cast<uint64_t*>(st_d + 256);
+  const int seq = blockIdx.x / heads, h = blockIdx.x - seq * heads;
+  const int inner = heads * DH;
+  const size_t row0 = size_t(seq) * N;
+  const float scale_log2e = scale * 1.4426950408889634f;
+  auto kept = [&](int i) { return !MASKED || ((km[i >> 6] >> (i & 63)) & 1); };
+  auto stage = [&](const float* src_a, size_t ld_a, const float* src_b, size_t ld_b) {
+    for (int i = threadIdx.x; i < N * DH; i += blockDim.x) {
+      const int t = i / DH, d = i - t * DH;
+      sa[t * P + d] = src_a[(row0 + t) * ld_a + d];
+      sb[t * P + d] = src_b[(row0 + t) * ld_b + d];
+    }
+  };
+  const float* qbase = qkv + h * DH;
+  stage(qbase + inner, 3 * inner, qbase + 2 * inner, 3 * inner);
+  if (MASKED && warp < 4) {
+    const int b = warp * 64;
+    const uint8_t* row = keep + row0 + b;
+    const uint32_t lo = __ballot_sync(0xffffffffu, b + lane < N && row[lane] != 0);
+    const uint32_t hi = __ballot_sync(0xffffffffu, b + lane + 32 < N && row[lane + 32] != 0);
+    if (lane == 0) km[warp] = (uint64_t(hi) << 32) | lo;
+  }
+  __syncthreads();
+
+  // ---- pass 1: rows = queries, lanes over keys ----
+  for (int a = warp; a < N; a += 8) {
+    for (int d = lane; d < DH; d += 32) {
+      own[d] = qbase[(row0 + a) * (3 * inner) + d];
+      own[DH + d] = dout[(row0 + a) * size_t(inner) + h * DH + d];
+    }
+    __syncwarp();
+    const bool row_kept = kept(a);
+    float mx = -INFINITY;
+    for (int b = lane; b < N; b += 32) {
+      float s = 0.f, dp = 0.f;
+#pragma unroll 8
+      for (int d = 0; d < DH; ++d) {
+        s = fmaf(own[d], sa[b * P + d], s);
+        dp = fmaf(own[DH + d], sb[b * P + d], dp);
+      }
+      s = !row_kept ? 0.f : kept(b) ? __fmul_rn(s, scale_log2e) : -INFINITY;      // rounded product in both passes and instantiations
+      l0[b] = s;
+      l1[b] = dp;
+      mx = fmaxf(mx, s);
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
+    float sum = 0.f;
+    for (int b = lane; b < N; b += 32) sum += exp2f(l0[b] - mx);
+    const float il = 1.0f / warp_sum(sum);
+    float delta = 0.f;
+    for (int b = lane; b < N; b += 32) {
+      const float p = exp2f(l0[b] - mx) * il;
+      delta += p * l1[b];
+      l0[b] = p;
+    }
+    delta = warp_sum(delta);
+    for (int b = lane; b < N; b += 32) l1[b] = row_kept ? l0[b] * (l1[b] - delta) : 0.f;
+    if (lane == 0) { st_m[a] = mx; st_il[a] = il; st_d[a] = delta; }
+    __syncwarp();
+    for (int d = lane; d < DH; d += 32) {
+      float dq = 0.f;
+      for (int b = 0; b < N; ++b) dq = fmaf(l1[b], sa[b * P + d], dq);
+      dqkv[(row0 + a) * (3 * inner) + h * DH + d] = dq * scale;
+    }
+    __syncwarp();
+  }
+  __syncthreads();
+  stage(qbase, 3 * inner, dout + h * DH, inner);
+  __syncthreads();
+
+  // ---- pass 2: rows = keys, lanes over queries ----
+  for (int b = warp; b < N; b += 8) {
+    for (int d = lane; d < DH; d += 32) {
+      own[d] = qbase[(row0 + b) * (3 * inner) + inner + d];
+      own[DH + d] = qbase[(row0 + b) * (3 * inner) + 2 * inner + d];
+    }
+    __syncwarp();
+    const bool key_kept = kept(b);
+    for (int a = lane; a < N; a += 32) {
+      float s = 0.f, dp = 0.f;
+#pragma unroll 8
+      for (int d = 0; d < DH; ++d) {
+        s = fmaf(sa[a * P + d], own[d], s);
+        dp = fmaf(sb[a * P + d], own[DH + d], dp);
+      }
+      const bool qk = kept(a);
+      s = !qk ? 0.f : key_kept ? __fmul_rn(s, scale_log2e) : -INFINITY;
+      const float p = exp2f(s - st_m[a]) * st_il[a];
+      l0[a] = p;
+      l1[a] = qk ? p * (dp - st_d[a]) : 0.f;
+    }
+    __syncwarp();
+    for (int d = lane; d < DH; d += 32) {
+      float dk = 0.f, dv = 0.f;
+      for (int a = 0; a < N; ++a) {
+        dv = fmaf(l0[a], sb[a * P + d], dv);
+        dk = fmaf(l1[a], sa[a * P + d], dk);
+      }
+      float* op = dqkv + (row0 + b) * (3 * inner) + h * DH + d;
+      op[inner] = dk * scale;
+      op[2 * inner] = dv;
+    }
+    __syncwarp();
+  }
+}
+
+// ---------------------------------------------------------------------------------------------
 // Backward of the 12 per-AU dots (models/tformer.py:389-401): dx[c*12+i, :] = dl[c,i] w[i,:];  dw[i,:] = sum_c dl[c,i] x[c*12+i,:]
 // ---------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) au_logits_bwd_dx_kernel(const float* __restrict__ dl, int ld_dl, const float* __restrict__ w_last,
@@ -624,9 +762,22 @@ static int launch_attention_bwd(const void* qkv, const void* dout, void* dqkv, i
 
 int attention_bwd(int io_mode, const void* qkv, const void* dout, void* dqkv, int n_seq, int n_tok, int heads, int dim_head, cudaStream_t st,
                   const uint8_t* keep) {
-  AVF_REQUIRE(n_seq > 0 && n_tok > 0 && n_tok <= 64 && heads > 0, AVF_EINVAL, "attention_bwd: n_seq=%d n_tok=%d heads=%d", n_seq, n_tok, heads);
+  AVF_REQUIRE(n_seq > 0 && n_tok > 0 && heads > 0, AVF_EINVAL, "attention_bwd: n_seq=%d n_tok=%d heads=%d", n_seq, n_tok, heads);
   AVF_REQUIRE(dim_head == 32 || dim_head == 64, AVF_EUNSUPPORTED, "attention_bwd: dim_head=%d (supported: 32, 64)", dim_head);
+  AVF_REQUIRE(n_tok <= 64 || (dim_head == 64 && n_tok <= 256), AVF_EUNSUPPORTED,
+              "attention_bwd: n_tok=%d with dim_head=%d (up to 64 tokens; 64-wide heads up to 256)", n_tok, dim_head);
   if (io_mode == AVF_BF16) return attention_bwd_mma_bf16(qkv, dout, dqkv, n_seq, n_tok, heads, dim_head, st, keep);      // tensor cores
+  if (n_tok > 64) {
+    auto kern = keep != nullptr ? attention_bwd_long_f32_kernel<true> : attention_bwd_long_f32_kernel<false>;
+    static PerDeviceOnce once[2];
+    if (once[keep != nullptr].first()) {
+      AVF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, int(attention_bwd_long_smem(256))));
+    }
+    launch_pdl(kern, n_seq * heads, 256, attention_bwd_long_smem(n_tok), st, static_cast<const float*>(qkv), static_cast<const float*>(dout),
+               static_cast<float*>(dqkv), n_tok, heads, rsqrtf(64.f), keep);
+    AVF_LAUNCH_CHECK("attention_bwd_long_f32_kernel");
+    return 0;
+  }
   if (keep != nullptr)
     return dim_head == 32 ? launch_attention_bwd<float, 32, true>(qkv, dout, dqkv, n_seq, n_tok, heads, keep, st)
                           : launch_attention_bwd<float, 64, true>(qkv, dout, dqkv, n_seq, n_tok, heads, keep, st);

@@ -51,7 +51,9 @@ static int check_train_shape(const avf_stack_shape* s) {
   AVF_REQUIRE(s->dim_head == 32 || s->dim_head == 64, AVF_EUNSUPPORTED, "dim_head=%d (supported: 32, 64)", s->dim_head);
   AVF_REQUIRE((s->heads * s->dim_head) % 64 == 0 && s->mlp_dim % 64 == 0, AVF_EUNSUPPORTED, "inner=%d / mlp=%d must be multiples of 64",
               s->heads * s->dim_head, s->mlp_dim);
-  AVF_REQUIRE(s->n_tok <= 64, AVF_EUNSUPPORTED, "n_tok=%d: sequences longer than 64 tokens are not part of this path", s->n_tok);
+  AVF_REQUIRE(s->n_tok <= 64 || s->dim_head == 64, AVF_EUNSUPPORTED,
+              "n_tok=%d: sequences longer than 64 tokens are not part of this path for dim_head=%d", s->n_tok, s->dim_head);
+  AVF_REQUIRE(s->n_tok <= 256, AVF_EUNSUPPORTED, "n_tok=%d: sequences longer than 256 tokens are not part of this path", s->n_tok);
   return 0;
 }
 
