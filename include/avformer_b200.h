@@ -406,6 +406,31 @@ size_t avf_tformer_embed_indexed_bwd_workspace_bytes(int32_t n_clips, int32_t n_
 int avf_tformer_embed_indexed_bwd(int out_mode, const float* dtok, const int32_t* index, int32_t n_clips, int32_t n_frames,
                                   int32_t dim, int32_t n_bank, void* dbank, void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---- attention maps: the softmax probabilities the attention kernels compute (models/heads.py:234, attn = dots.softmax(-1)) ----
+ * probs is a caller-owned DEVICE fp32 buffer.  Element (l, b, h, i, j) of a [depth, n_seq, heads, n_tok, n_tok] map, contiguous, is
+ * p = exp(s_ij - m_i) / l_i for layer l, sequence b, head h, query i and key j, where s is the scaled score after the mask fill (see
+ * "attention masks" above) and m_i, l_i are the kernel's own row maximum and fp32 row sum; in mode AVF_BF16 it is the value before
+ * P is rounded to bf16 for the P V product.  So every row sums to 1 within fp32 rounding, a kept query gets exactly 0.0 on a dropped
+ * key, and a dropped query's row is uniform at 1 / n_tok.  The probabilities are written by the attention launch itself: a map call
+ * issues the launches of the same call with avf_set_fused_enabled(0), never the fused kernel, and its outputs equal that call's bit
+ * for bit.  keep == NULL is the unmasked call.  Workspaces are those of the calls without maps.  Inference only. */
+/* avf_attention_fwd(_masked) + probs [n_seq, heads, n_tok, n_tok] (depth 1). */
+int avf_attention_fwd_probs(int io_mode, const void* qkv, void* out, int32_t n_seq, int32_t n_tok, int32_t heads, int32_t dim_head,
+                            const uint8_t* keep, float* probs, void* stream);
+/* avf_encoder_stack_fwd(_masked) + probs [depth, n_seq, heads, n_tok, n_tok]; pos [n_tok, dim] (optional) is added to x first, as in
+ * avf_token_stack_fwd.  Same workspace as avf_encoder_stack_fwd. */
+int avf_encoder_stack_fwd_probs(int mode, const avf_stack_shape* s, const avf_layer_weights* layers, const uint8_t* keep,
+                                float* x, int32_t ld_x, const float* pos, float* out, int32_t ld_out, float* probs,
+                                void* workspace, size_t workspace_bytes, void* stream);
+/* avf_tformer_fwd(_masked) / avf_tformer_fwd_indexed + probs [depth, n_clips, heads, T+1, T+1].  The last layer's attention runs every
+ * query row so that its map is full; everything after the softmax stays on the cls rows, and cls_out equals the call without maps. */
+int avf_tformer_fwd_probs(int mode, int io_mode, const avf_stack_shape* s, const avf_layer_weights* layers, const uint8_t* keep,
+                          const void* frames, const float* cls_token, const float* pos, float* cls_out, float* probs,
+                          void* workspace, size_t workspace_bytes, void* stream);
+int avf_tformer_fwd_indexed_probs(int mode, int io_mode, const avf_stack_shape* s, const avf_layer_weights* layers,
+                                  const void* bank, int32_t n_bank, const int32_t* index, const float* cls_token, const float* pos,
+                                  float* cls_out, float* probs, void* workspace, size_t workspace_bytes, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

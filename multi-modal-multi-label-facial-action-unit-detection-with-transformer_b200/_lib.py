@@ -142,6 +142,14 @@ SIGNATURES = {
     "avf_tformer_embed_indexed": (ctypes.c_int, [ctypes.c_int, _c_p, _i32, _c_p, _c_p, _c_p, _c_p, _c_p, _i32, _i32, _i32, _c_p]),
     "avf_tformer_embed_indexed_bwd_workspace_bytes": (_sz, [_i32, _i32, _i32]),
     "avf_tformer_embed_indexed_bwd": (ctypes.c_int, [ctypes.c_int, _c_p, _c_p, _i32, _i32, _i32, _i32, _c_p, _c_p, _sz, _c_p]),
+    # ---- attention maps (probs: device fp32 [depth, n_seq, heads, n_tok, n_tok]) ----
+    "avf_attention_fwd_probs": (ctypes.c_int, [ctypes.c_int, _c_p, _c_p, _i32, _i32, _i32, _i32, _c_p, _c_p, _c_p]),
+    "avf_encoder_stack_fwd_probs": (ctypes.c_int, [ctypes.c_int, ctypes.POINTER(StackShape), ctypes.POINTER(LayerWeights), _c_p, _c_p, _i32, _c_p,
+                                                   _c_p, _i32, _c_p, _c_p, _sz, _c_p]),
+    "avf_tformer_fwd_probs": (ctypes.c_int, [ctypes.c_int, ctypes.c_int, ctypes.POINTER(StackShape), ctypes.POINTER(LayerWeights), _c_p, _c_p,
+                                             _c_p, _c_p, _c_p, _c_p, _c_p, _sz, _c_p]),
+    "avf_tformer_fwd_indexed_probs": (ctypes.c_int, [ctypes.c_int, ctypes.c_int, ctypes.POINTER(StackShape), ctypes.POINTER(LayerWeights), _c_p,
+                                                     _i32, _c_p, _c_p, _c_p, _c_p, _c_p, _c_p, _sz, _c_p]),
 }
 
 _lock = threading.Lock()

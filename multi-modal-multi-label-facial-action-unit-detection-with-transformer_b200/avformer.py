@@ -116,6 +116,63 @@ class TwoStreamAuralVisualFormer(nn.Module):
             return torch.zeros(bs, 21, device=clip.device)
         return self.au_head.logits21_(fused, bs)
 
+    MAP_STACKS = ("sformer", "tformer", "audio_au_former", "video_au_former", "fusion_head")
+
+    def attention_maps(self, x, stacks=None):
+        """forward(x) with the attention maps of the encoder stacks: (out21 [B,21], {name: maps}).
+
+        ``stacks`` selects the stacks whose maps are written (None: all of MAP_STACKS; the SFormer's are by far the largest, 8 x 49 x 49
+        fp32 per frame).  Maps are fp32 [depth, n_seq, heads, n_tok, n_tok]: "sformer" [1, B*T, 8, 49, 49], "tformer" [3, B, 8, T+1, T+1]
+        (the last layer full), "audio_au_former" / "video_au_former" [2, B, 8, 12, 12], "fusion_head" [3, B, 8, 12, 12] (absent unless
+        task == "AU", as forward() runs no fusion head then).  The whole call runs with the fused kernel switched off
+        (set_fused_enabled(False), restored on return): a stack with maps runs kernel by kernel, and so do the others, so out21 equals
+        model(x) under set_fused_enabled(False) bit for bit whatever ``stacks`` holds.  Inference only: RuntimeError when autograd would
+        record the call or a stack is in train() with dropout > 0."""
+        names = self.MAP_STACKS if stacks is None else tuple(stacks)
+        unknown = [n for n in names if n not in self.MAP_STACKS]
+        if unknown:
+            raise ValueError(f"attention_maps: unknown stack name(s) {unknown}; the stacks are {list(self.MAP_STACKS)}")
+        audio, clip = x["audio_features"], x["clip"]
+        AF._cuda(clip, "x['clip']")
+        AF._cuda(audio, "x['audio_features']")
+        who = "TwoStreamAuralVisualFormer.attention_maps"
+        if needs_grad(self, clip, audio):
+            raise RuntimeError(f"{who}: attention maps are inference only, and this call would be recorded by autograd; run it under "
+                               f"torch.no_grad() (or freeze the parameters)")
+        for m in self.modules():
+            if isinstance(m, Transformer):
+                m.check_maps_allowed(who)
+        bs = clip.shape[0]
+        vm = self.video_model.video_model
+        maps = {}
+        prev = AF.set_fused_enabled(False)
+        try:
+            fused = torch.empty((bs * 12, 256), dtype=torch.float32, device=clip.device)
+            a_feat = self.audio_model.audio_model(audio).float().contiguous()
+            r = self.audio_model.au_head.tokens_into(a_feat, a_feat.shape[1], bs, out=fused, ld_out=256, maps="audio_au_former" in names)
+            if "audio_au_former" in names:
+                maps["audio_au_former"] = r
+            r = vm.s_former(clip[:, -vm.num_channels:].permute(0, 2, 1, 3, 4), maps="sformer" in names)
+            if "sformer" in names:
+                r, maps["sformer"] = r
+            if "tformer" in names:
+                cls, maps["tformer"] = vm.t_former.attention_maps(r)
+            else:
+                cls = vm.t_former.cls_features(r)
+            r = self.video_model.au_head.tokens_into(cls, cls.shape[1], cls.shape[0], out=fused[:, 128:], ld_out=256,
+                                                     maps="video_au_former" in names)
+            if "video_au_former" in names:
+                maps["video_au_former"] = r
+            if self.task != "AU":
+                return torch.zeros(bs, 21, device=clip.device), maps
+            if "fusion_head" in names:
+                out21, maps["fusion_head"] = self.au_head.logits21_maps_(fused, bs)
+            else:
+                out21 = self.au_head.logits21_(fused, bs)
+            return out21, maps
+        finally:
+            AF.set_fused_enabled(prev)
+
     def _forward_train(self, clip, audio):
         """Same data flow with autograd-visible regions (autograd.py); frozen sub-models (requires_grad=False everywhere,
         inputs without grad) still take the inference kernels inside their modules."""

@@ -116,13 +116,17 @@ static bool fused_rows(int mode, const avf_stack_shape* s, int ld_x, const float
 }
 
 // keep (optional, [n_seq, n_tok] uint8): attention mask of every layer; the fused kernel has none, so a masked stack runs kernel by kernel.
+// probs (optional): layer l's attention probabilities go to probs + l * n_seq*heads*n_tok*n_tok (fp32 [depth, n_seq, heads, n_tok, n_tok]),
+// written by the attention launch itself; the fused kernel keeps them on chip, so such a stack runs kernel by kernel too.
+static size_t probs_per_layer(const avf_stack_shape* s) { return size_t(s->n_seq) * s->heads * s->n_tok * s->n_tok; }
+
 static int encoder_stack(int mode, const avf_stack_shape* s, const avf_layer_weights* L, float* x, int ld_x, float* out, int ld_out,
-                         void* ws, size_t ws_bytes, cudaStream_t st, const uint8_t* keep = nullptr) {
+                         void* ws, size_t ws_bytes, cudaStream_t st, const uint8_t* keep = nullptr, float* probs = nullptr) {
   int e = check_shape(s);
   if (e) return e;
   AVF_REQUIRE(mode == AVF_BF16 || mode == AVF_FP32, AVF_EINVAL, "mode=%d", mode);
   AVF_REQUIRE(L != nullptr && x != nullptr && ws != nullptr, AVF_EINVAL, "null pointer argument");
-  if (keep == nullptr && fused_rows(mode, s, ld_x, out, ld_out))     // whole stack, one persistent kernel
+  if (keep == nullptr && probs == nullptr && fused_rows(mode, s, ld_x, out, ld_out))     // whole stack, one persistent kernel
     return encoder_fused(1, s, L, x, ld_x, out ? out : x, out ? ld_out : ld_x, nullptr, nullptr, nullptr, nullptr, nullptr, st);
   const EncoderWs w = carve_encoder_ws(s, mode, ws);
   AVF_REQUIRE(ws_bytes >= w.total, AVF_EWORKSPACE, "workspace too small: %zu < %zu bytes", ws_bytes, w.total);
@@ -132,7 +136,8 @@ static int encoder_stack(int mode, const avf_stack_shape* s, const avf_layer_wei
     // x + to_out(attn(to_qkv(LN(x))))                                     models/heads.py:175,185,219-239
     if ((e = layernorm(mode, x, ld_x, W.ln1_gamma, W.ln1_beta, w.ln, R, D, st))) return e;
     if ((e = linear(mode, w.ln, D, W.w_qkv, nullptr, nullptr, 0, w.qkv, 3 * I, mode, R, 3 * I, D, 0, st))) return e;
-    if ((e = attention_small(mode, w.qkv, w.attn, s->n_seq, s->n_tok, s->heads, s->dim_head, st, keep))) return e;
+    if ((e = attention_small(mode, w.qkv, w.attn, s->n_seq, s->n_tok, s->heads, s->dim_head, st, keep, probs ? probs + l * probs_per_layer(s) : nullptr)))
+      return e;
     if ((e = linear(mode, w.attn, I, W.w_out, W.b_out, x, ld_x, x, ld_x, AVF_FP32, R, D, I, AVF_EPI_BIAS | AVF_EPI_RESIDUAL, st))) return e;
     // x + W2 gelu(W1 LN(x) + b1) + b2                                     models/heads.py:188-200
     if ((e = layernorm(mode, x, ld_x, W.ln2_gamma, W.ln2_beta, w.ln, R, D, st))) return e;
@@ -157,8 +162,10 @@ static int tformer_check(const avf_stack_shape* s, const avf_layer_weights* laye
 }
 
 // The layers of the TFormer on the embedded tokens x [n_seq*n_tok, dim] fp32 that start the workspace -> cls_out.
+// probs (optional): the maps of every layer (encoder_stack); the last layer's attention then runs every query row (full map) while
+// everything after the softmax stays on the cls rows.
 static int tformer_layers(int mode, const avf_stack_shape* s, const avf_layer_weights* layers, void* workspace, float* cls_out, const uint8_t* keep,
-                          cudaStream_t st) {
+                          cudaStream_t st, float* probs = nullptr) {
   int e = 0;
   const int B = s->n_seq, N = s->n_tok, R = B * N, D = s->dim, I = s->heads * s->dim_head, M = s->mlp_dim;
   uint8_t* p = static_cast<uint8_t*>(workspace);
@@ -173,17 +180,18 @@ static int tformer_layers(int mode, const avf_stack_shape* s, const avf_layer_we
   if (s->depth > 1) {
     avf_stack_shape head = *s;
     head.depth = s->depth - 1;
-    if ((e = encoder_stack(mode, &head, layers, x, D, nullptr, 0, enc_ws, w.total, st, keep))) return e;
+    if ((e = encoder_stack(mode, &head, layers, x, D, nullptr, 0, enc_ws, w.total, st, keep, probs))) return e;
   }
+  float* last_probs = probs ? probs + size_t(s->depth - 1) * probs_per_layer(s) : nullptr;
   // Last layer (models/vformer.py:288-290 returns x[:, 0] only): keys / values need every row, everything after the softmax only
   // the cls row of each clip — out-projection, LayerNorm, MLP run on [n_clips, dim] instead of [n_clips * (T+1), dim].
   const avf_layer_weights& W = layers[s->depth - 1];
   if ((e = layernorm(mode, x, D, W.ln1_gamma, W.ln1_beta, w.ln, R, D, st))) return e;
   if ((e = linear(mode, w.ln, D, W.w_qkv, nullptr, nullptr, 0, w.qkv, 3 * I, mode, R, 3 * I, D, 0, st))) return e;
   if (mode == AVF_BF16) {
-    if ((e = attention_mma_bf16(w.qkv, oc, B, N, s->heads, s->dim_head, st, 1, keep))) return e;
+    if ((e = attention_mma_bf16(w.qkv, oc, B, N, s->heads, s->dim_head, st, 1, keep, last_probs))) return e;
   } else {
-    if ((e = attention_small(mode, w.qkv, w.attn, B, N, s->heads, s->dim_head, st, keep))) return e;
+    if ((e = attention_small(mode, w.qkv, w.attn, B, N, s->heads, s->dim_head, st, keep, last_probs))) return e;
     AVF_CUDA(cudaMemcpy2DAsync(oc, size_t(I) * 4, w.attn, size_t(N) * I * 4, size_t(I) * 4, B, cudaMemcpyDeviceToDevice, st));
   }
   if ((e = rows_gather(x, size_t(N) * D, xc, B, D, st))) return e;
@@ -194,25 +202,26 @@ static int tformer_layers(int mode, const avf_stack_shape* s, const avf_layer_we
 }
 
 static int tformer_fwd(int mode, int io_mode, const avf_stack_shape* s, const avf_layer_weights* layers, const void* frames, const float* cls_token,
-                       const float* pos, float* cls_out, void* workspace, size_t workspace_bytes, const uint8_t* keep, cudaStream_t st) {
+                       const float* pos, float* cls_out, void* workspace, size_t workspace_bytes, const uint8_t* keep, cudaStream_t st,
+                       float* probs = nullptr) {
   int e = tformer_check(s, layers, frames, cls_token, pos, cls_out, workspace, workspace_bytes, avf_tformer_workspace_bytes(s, mode));
   if (e) return e;
   if ((e = tformer_embed(io_mode, frames, cls_token, pos, static_cast<float*>(workspace), s->n_seq, s->n_tok - 1, s->dim, st))) return e;
-  return tformer_layers(mode, s, layers, workspace, cls_out, keep, st);
+  return tformer_layers(mode, s, layers, workspace, cls_out, keep, st, probs);
 }
 
 // Clips described by frame indices into a bank: gather, keep rows and embed in one launch, then the masked layers.  The keep rows
 // follow the workspace of avf_tformer_fwd.
 static int tformer_fwd_indexed(int mode, int io_mode, const avf_stack_shape* s, const avf_layer_weights* layers, const void* bank, int n_bank,
                                const int32_t* index, const float* cls_token, const float* pos, float* cls_out, void* workspace, size_t workspace_bytes,
-                               cudaStream_t st) {
+                               cudaStream_t st, float* probs = nullptr) {
   int e = tformer_check(s, layers, index, cls_token, pos, cls_out, workspace, workspace_bytes, avf_tformer_indexed_workspace_bytes(s, mode));
   if (e) return e;
   AVF_REQUIRE(n_bank >= 0 && (bank != nullptr || n_bank == 0), AVF_EINVAL, "tformer_fwd_indexed: bank of %d frames at %p", n_bank, bank);
   uint8_t* keep = static_cast<uint8_t*>(workspace) + avf_tformer_workspace_bytes(s, mode);
   if ((e = tformer_embed_indexed(io_mode, bank, n_bank, index, cls_token, pos, static_cast<float*>(workspace), keep, s->n_seq, s->n_tok - 1, s->dim, st)))
     return e;
-  return tformer_layers(mode, s, layers, workspace, cls_out, keep, st);
+  return tformer_layers(mode, s, layers, workspace, cls_out, keep, st, probs);
 }
 
 }  // namespace avf
@@ -335,6 +344,25 @@ int avf_attention_fwd_masked(int io_mode, const void* qkv, void* out, int32_t n_
   return attention_small(io_mode, qkv, out, n_seq, n_tok, heads, dim_head, static_cast<cudaStream_t>(stream), keep);
 }
 
+int avf_attention_fwd_probs(int io_mode, const void* qkv, void* out, int32_t n_seq, int32_t n_tok, int32_t heads, int32_t dim_head, const uint8_t* keep,
+                            float* probs, void* stream) {
+  int e = require_device();
+  if (e) return e;
+  AVF_REQUIRE(qkv && out && probs, AVF_EINVAL, "attention_probs: null pointer");
+  return attention_small(io_mode, qkv, out, n_seq, n_tok, heads, dim_head, static_cast<cudaStream_t>(stream), keep, probs);
+}
+
+int avf_encoder_stack_fwd_probs(int mode, const avf_stack_shape* s, const avf_layer_weights* layers, const uint8_t* keep, float* x, int32_t ld_x,
+                                const float* pos, float* out, int32_t ld_out, float* probs, void* workspace, size_t workspace_bytes, void* stream) {
+  int e = require_device();
+  if (e) return e;
+  if ((e = check_shape(s))) return e;
+  AVF_REQUIRE(layers && x && probs && workspace, AVF_EINVAL, "encoder_stack_probs: null pointer");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (pos != nullptr && (e = add_row_periodic(x, ld_x, pos, s->n_seq * s->n_tok, s->dim, s->n_tok, st))) return e;
+  return encoder_stack(mode, s, layers, x, ld_x, out, ld_out, workspace, workspace_bytes, st, keep, probs);
+}
+
 int avf_sformer_tokens_pack(int io_mode, const void* fmap, const float* pos, float* x, int32_t n_frames, int32_t dim, int32_t hw, void* stream) {
   int e = require_device();
   if (e) return e;
@@ -401,6 +429,14 @@ int avf_tformer_fwd_masked(int mode, int io_mode, const avf_stack_shape* s, cons
   return tformer_fwd(mode, io_mode, s, layers, frames, cls_token, pos, cls_out, workspace, workspace_bytes, keep, static_cast<cudaStream_t>(stream));
 }
 
+int avf_tformer_fwd_probs(int mode, int io_mode, const avf_stack_shape* s, const avf_layer_weights* layers, const uint8_t* keep, const void* frames,
+                          const float* cls_token, const float* pos, float* cls_out, float* probs, void* workspace, size_t workspace_bytes, void* stream) {
+  int e = require_device();
+  if (e) return e;
+  AVF_REQUIRE(probs, AVF_EINVAL, "tformer_fwd_probs: null pointer");
+  return tformer_fwd(mode, io_mode, s, layers, frames, cls_token, pos, cls_out, workspace, workspace_bytes, keep, static_cast<cudaStream_t>(stream), probs);
+}
+
 size_t avf_tformer_indexed_workspace_bytes(const avf_stack_shape* s, int mode) {
   if (s == nullptr || s->n_seq <= 0 || s->n_tok <= 0) return 0;
   return avf_tformer_workspace_bytes(s, mode) + align_up(size_t(s->n_seq) * s->n_tok);
@@ -413,6 +449,16 @@ int avf_tformer_fwd_indexed(int mode, int io_mode, const avf_stack_shape* s, con
   if (e) return e;
   return tformer_fwd_indexed(mode, io_mode, s, layers, bank, n_bank, index, cls_token, pos, cls_out, workspace, workspace_bytes,
                              static_cast<cudaStream_t>(stream));
+}
+
+int avf_tformer_fwd_indexed_probs(int mode, int io_mode, const avf_stack_shape* s, const avf_layer_weights* layers, const void* bank, int32_t n_bank,
+                                  const int32_t* index, const float* cls_token, const float* pos, float* cls_out, float* probs, void* workspace,
+                                  size_t workspace_bytes, void* stream) {
+  int e = require_device();
+  if (e) return e;
+  AVF_REQUIRE(probs, AVF_EINVAL, "tformer_fwd_indexed_probs: null pointer");
+  return tformer_fwd_indexed(mode, io_mode, s, layers, bank, n_bank, index, cls_token, pos, cls_out, workspace, workspace_bytes,
+                             static_cast<cudaStream_t>(stream), probs);
 }
 
 int avf_tformer_embed_indexed(int io_mode, const void* bank, int32_t n_bank, const int32_t* index, const float* cls_token, const float* pos, float* x,

@@ -53,10 +53,12 @@ __device__ __forceinline__ float mask_score(float s, bool row_kept, uint64_t km,
 }
 
 // MASKED: keep [n_seq, n_tok] uint8 (1 = keep) masks score (i, j) unless tokens i and j are both kept (mask_score).
-template <int DH, int NP, bool MASKED>    // NP = tokens padded to a multiple of 16 (16 / 32 / 48 / 64)
+// PROBS: also write the softmax probabilities exp2(s - m) / l in fp32 (before P is rounded to bf16 for P V) to probs
+// [n_seq, heads, n_tok, n_tok]; every query row is computed (the map is full) while O is still stored for the first q_rows rows only.
+template <int DH, int NP, bool MASKED, bool PROBS>    // NP = tokens padded to a multiple of 16 (16 / 32 / 48 / 64)
 __global__ void __launch_bounds__(DH == 32 ? 128 : 64) attention_mma_kernel(const __nv_bfloat16* __restrict__ qkv, __nv_bfloat16* __restrict__ out,
                                                             int n_problems, int n_tok, int heads, float scale_log2e, int q_rows,
-                                                            const uint8_t* __restrict__ keep) {
+                                                            const uint8_t* __restrict__ keep, float* __restrict__ probs) {
   pdl_wait();      // programmatic dependent launch: everything above is launch overhead hidden behind the previous kernel
   pdl_trigger();
   // q_rows: only the first q_rows query rows of every sequence are computed and written (compactly: out [n_seq * q_rows, inner]);
@@ -104,7 +106,7 @@ __global__ void __launch_bounds__(DH == 32 ? 128 : 64) attention_mma_kernel(cons
   const int g = lane >> 2, t = lane & 3;
 #pragma unroll 1
   for (int mt = 0; mt < NP / 16; ++mt) {
-    if (mt * 16 >= q_rows) break;
+    if (mt * 16 >= (PROBS ? n_tok : q_rows)) break;
     const int r_lo = mt * 16 + g, r_hi = r_lo + 8;
     // Q fragments (A operand, row-major 16x16 per k-step) from global: lane t of a quad fetches the 16-byte chunks t, t+4, ... of
     // its two rows (the quad reads 64 contiguous bytes per row and instruction instead of 4 x 4 bytes), then the quad transposes
@@ -177,6 +179,18 @@ __global__ void __launch_bounds__(DH == 32 ? 128 : 64) attention_mma_kernel(cons
     l_lo += __shfl_xor_sync(0xffffffffu, l_lo, 2);
     l_hi += __shfl_xor_sync(0xffffffffu, l_hi, 1);
     l_hi += __shfl_xor_sync(0xffffffffu, l_hi, 2);
+    if constexpr (PROBS) {
+      float* p_lo = probs + (size_t(prob) * n_tok + r_lo) * n_tok;
+      float* p_hi = p_lo + size_t(8) * n_tok;
+#pragma unroll
+      for (int nt = 0; nt < NP / 8; ++nt) {
+        const int c = nt * 8 + 2 * t;
+        if (r_lo < n_tok && c < n_tok) p_lo[c] = s[nt][0] / l_lo;
+        if (r_lo < n_tok && c + 1 < n_tok) p_lo[c + 1] = s[nt][1] / l_lo;
+        if (r_hi < n_tok && c < n_tok) p_hi[c] = s[nt][2] / l_hi;
+        if (r_hi < n_tok && c + 1 < n_tok) p_hi[c + 1] = s[nt][3] / l_hi;
+      }
+    }
     // O = P V : the C fragments of two adjacent score tiles are exactly one A fragment
     float o[DH / 8][4];
 #pragma unroll
@@ -214,13 +228,13 @@ __global__ void __launch_bounds__(DH == 32 ? 128 : 64) attention_mma_kernel(cons
   }
 }
 
-template <int DH, int NP, bool MASKED>
-int launch(const void* qkv, void* out, int n_seq, int n_tok, int heads, int q_rows, const uint8_t* keep, cudaStream_t st) {
+template <int DH, int NP, bool MASKED, bool PROBS>
+int launch(const void* qkv, void* out, int n_seq, int n_tok, int heads, int q_rows, const uint8_t* keep, float* probs, cudaStream_t st) {
   const int n_problems = n_seq * heads;
   const float scale_log2e = 1.4426950408889634f / sqrtf(float(DH));
   constexpr int kWarps = DH == 32 ? 4 : 2;
-  launch_pdl(attention_mma_kernel<DH, NP, MASKED>, ceil_div(n_problems, kWarps), kWarps * 32, 0, st, static_cast<const __nv_bfloat16*>(qkv), static_cast<__nv_bfloat16*>(out),
-                                                                      n_problems, n_tok, heads, scale_log2e, q_rows, keep);
+  launch_pdl(attention_mma_kernel<DH, NP, MASKED, PROBS>, ceil_div(n_problems, kWarps), kWarps * 32, 0, st, static_cast<const __nv_bfloat16*>(qkv), static_cast<__nv_bfloat16*>(out),
+                                                                      n_problems, n_tok, heads, scale_log2e, q_rows, keep, probs);
   AVF_LAUNCH_CHECK("attention_mma_kernel");
   return 0;
 }
@@ -585,10 +599,12 @@ __device__ __forceinline__ void long_store(const float (&d)[8][4], __nv_bfloat16
 }
 
 // Forward: two sweeps over the key blocks per 16-row query tile, the first for the exact row max, the second for exp2, l and P V.
-template <bool MASKED>
+// PROBS: l is known only after the second sweep, so a third sweep recomputes the masked scores and writes exp2(s - m) / l in fp32 to
+// probs [n_seq, heads, n_tok, n_tok], each element once; every query row is computed while O is still stored for the first q_rows.
+template <bool MASKED, bool PROBS>
 __global__ void __launch_bounds__(kLongWarps * 32) attention_long_mma_kernel(const __nv_bfloat16* __restrict__ qkv, __nv_bfloat16* __restrict__ out,
                                                                             int n_tok, int heads, float scale_log2e, int q_rows,
-                                                                            const uint8_t* __restrict__ keep) {
+                                                                            const uint8_t* __restrict__ keep, float* __restrict__ probs) {
   pdl_wait();      // programmatic dependent launch: everything above is launch overhead hidden behind the previous kernel
   pdl_trigger();
   extern __shared__ __align__(16) uint8_t smem_long[];
@@ -607,7 +623,7 @@ __global__ void __launch_bounds__(kLongWarps * 32) attention_long_mma_kernel(con
 
   const int g = lane >> 2, t = lane & 3, nkb = NR / 64;
 #pragma unroll 1
-  for (int mt = warp; mt * 16 < q_rows; mt += kLongWarps) {
+  for (int mt = warp; mt * 16 < (PROBS ? n_tok : q_rows); mt += kLongWarps) {
     const int r_lo = mt * 16 + g, r_hi = r_lo + 8;
     uint32_t qf[4][4];
 #pragma unroll
@@ -650,6 +666,24 @@ __global__ void __launch_bounds__(kLongWarps * 32) attention_long_mma_kernel(con
         l_hi += s[nt][2] + s[nt][3];
       }
       long_mma_xm(o, s, Vs + kb * 64, lane);
+    }
+    if constexpr (PROBS) {
+      const float L_lo = quad_sum(l_lo), L_hi = quad_sum(l_hi);
+      float* p_lo = probs + (size_t(blockIdx.x) * n_tok + r_lo) * n_tok;
+      float* p_hi = p_lo + size_t(8) * n_tok;
+#pragma unroll 1
+      for (int kb = 0; kb < nkb; ++kb) {
+        long_mma_abt(s, qf, Ks + kb * 64, g, t);
+        long_mask<MASKED>(s, k_lo, k_hi, MASKED ? km[kb] : 0, n_tok - kb * 64, t);
+#pragma unroll
+        for (int nt = 0; nt < 8; ++nt) {
+          const int c = kb * 64 + nt * 8 + 2 * t;
+          if (r_lo < n_tok && c < n_tok) p_lo[c] = exp2f(fmaf(s[nt][0], scale_log2e, -o_lo)) / L_lo;
+          if (r_lo < n_tok && c + 1 < n_tok) p_lo[c + 1] = exp2f(fmaf(s[nt][1], scale_log2e, -o_lo)) / L_lo;
+          if (r_hi < n_tok && c < n_tok) p_hi[c] = exp2f(fmaf(s[nt][2], scale_log2e, -o_hi)) / L_hi;
+          if (r_hi < n_tok && c + 1 < n_tok) p_hi[c + 1] = exp2f(fmaf(s[nt][3], scale_log2e, -o_hi)) / L_hi;
+        }
+      }
     }
     long_store(o, out + size_t(seq) * q_rows * inner + head * kLongDH, inner, r_lo, q_rows, 1.f / quad_sum(l_lo), 1.f / quad_sum(l_hi), t);
   }
@@ -809,15 +843,15 @@ __global__ void __launch_bounds__(kLongWarps * 32) attention_bwd_long_mma_kernel
 size_t long_fwd_smem(int n_tok) { return size_t(2) * long_rows(n_tok) * kLongPitch * 2 + 4 * sizeof(uint64_t); }
 size_t long_bwd_smem(int n_tok) { return size_t(4) * long_rows(n_tok) * kLongPitch * 2 + size_t(3) * long_rows(n_tok) * 4 + 4 * sizeof(uint64_t); }
 
-template <bool MASKED>
-int launch_long(const void* qkv, void* out, int n_seq, int n_tok, int heads, int q_rows, const uint8_t* keep, cudaStream_t st) {
-  auto kern = attention_long_mma_kernel<MASKED>;
+template <bool MASKED, bool PROBS>
+int launch_long(const void* qkv, void* out, int n_seq, int n_tok, int heads, int q_rows, const uint8_t* keep, float* probs, cudaStream_t st) {
+  auto kern = attention_long_mma_kernel<MASKED, PROBS>;
   static PerDeviceOnce once;
   if (once.first()) {
     AVF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, int(long_fwd_smem(kLongMaxTok))));
   }
   launch_pdl(kern, n_seq * heads, kLongWarps * 32, long_fwd_smem(n_tok), st, static_cast<const __nv_bfloat16*>(qkv), static_cast<__nv_bfloat16*>(out), n_tok,
-             heads, 1.4426950408889634f / sqrtf(float(kLongDH)), q_rows, keep);
+             heads, 1.4426950408889634f / sqrtf(float(kLongDH)), q_rows, keep, probs);
   AVF_LAUNCH_CHECK("attention_long_mma_kernel");
   return 0;
 }
@@ -837,17 +871,27 @@ int launch_bwd_long(const void* qkv, const void* dout, void* dqkv, int n_seq, in
 
 }  // namespace
 
-int attention_mma_bf16(const void* qkv, void* out, int n_seq, int n_tok, int heads, int dim_head, cudaStream_t st, int q_rows, const uint8_t* keep) {
+int attention_mma_bf16(const void* qkv, void* out, int n_seq, int n_tok, int heads, int dim_head, cudaStream_t st, int q_rows, const uint8_t* keep,
+                       float* probs) {
   AVF_REQUIRE(n_tok >= 1 && n_tok <= kLongMaxTok && (n_tok <= 64 || dim_head == kLongDH), AVF_EUNSUPPORTED,
               "attention: n_tok=%d with dim_head=%d (1..64 tokens; 64-wide heads up to 256)", n_tok, dim_head);
   if (q_rows <= 0 || q_rows > n_tok) q_rows = n_tok;
-  if (n_tok > 64)
-    return keep ? launch_long<true>(qkv, out, n_seq, n_tok, heads, q_rows, keep, st) : launch_long<false>(qkv, out, n_seq, n_tok, heads, q_rows, nullptr, st);
+  if (n_tok > 64) {
+    if (probs)
+      return keep ? launch_long<true, true>(qkv, out, n_seq, n_tok, heads, q_rows, keep, probs, st)
+                  : launch_long<false, true>(qkv, out, n_seq, n_tok, heads, q_rows, nullptr, probs, st);
+    return keep ? launch_long<true, false>(qkv, out, n_seq, n_tok, heads, q_rows, keep, nullptr, st)
+                : launch_long<false, false>(qkv, out, n_seq, n_tok, heads, q_rows, nullptr, nullptr, st);
+  }
   const int np = (n_tok + 15) / 16 * 16;
 #define AVF_ATT(D, P)                                                                                   \
-  if (dim_head == D && np == P)                                                                         \
-    return keep ? launch<D, P, true>(qkv, out, n_seq, n_tok, heads, q_rows, keep, st)                   \
-                : launch<D, P, false>(qkv, out, n_seq, n_tok, heads, q_rows, nullptr, st);
+  if (dim_head == D && np == P) {                                                                       \
+    if (probs)                                                                                          \
+      return keep ? launch<D, P, true, true>(qkv, out, n_seq, n_tok, heads, q_rows, keep, probs, st)    \
+                  : launch<D, P, false, true>(qkv, out, n_seq, n_tok, heads, q_rows, nullptr, probs, st); \
+    return keep ? launch<D, P, true, false>(qkv, out, n_seq, n_tok, heads, q_rows, keep, nullptr, st)   \
+                : launch<D, P, false, false>(qkv, out, n_seq, n_tok, heads, q_rows, nullptr, nullptr, st); \
+  }
   AVF_ATT(32, 16) AVF_ATT(32, 32) AVF_ATT(32, 48) AVF_ATT(32, 64)
   AVF_ATT(64, 16) AVF_ATT(64, 32) AVF_ATT(64, 48) AVF_ATT(64, 64)
 #undef AVF_ATT

@@ -41,8 +41,9 @@ int au_confusion(const float* pred, int ld_pred, float thresh, const float* labe
 int linear_f32(const float* a, int lda, const float* w, const float* bias, const float* res, int ld_res, void* c, int ldc,
                int c_mode, int m, int n, int k, int flags, cudaStream_t st);
 // keep (optional): [n_seq, n_tok] uint8, 1 = keep; score (i, j) survives only when tokens i and j are both kept (include/avformer_b200.h).
+// probs (optional): fp32 [n_seq, heads, n_tok, n_tok] receives the softmax probabilities, written inside the same launch.
 int attention_small(int io_mode, const void* qkv, void* out, int n_seq, int n_tok, int heads, int dim_head, cudaStream_t st,
-                    const uint8_t* keep = nullptr);
+                    const uint8_t* keep = nullptr, float* probs = nullptr);
 
 int gemm_f32(int trans_a, int trans_b, const float* a, int lda, const float* w, int ldw, const float* bias, const float* res, int ld_res,
              float* aux, int ld_aux, void* c, int ldc, int c_mode, int m, int n, int k, int flags, cudaStream_t st, DropSpec drop = DropSpec{});
@@ -72,8 +73,9 @@ int adam_step(float* p, const float* g, float* m, float* v, void* shadow, size_t
               int decoupled, float grad_scale, cudaStream_t st);
 
 // avf_attention_mma.cu
+// With probs, every query row's probabilities are written (the map is full) while O is stored for the first q_rows rows only.
 int attention_mma_bf16(const void* qkv, void* out, int n_seq, int n_tok, int heads, int dim_head, cudaStream_t st, int q_rows = 0,
-                       const uint8_t* keep = nullptr);
+                       const uint8_t* keep = nullptr, float* probs = nullptr);
 int attention_bwd_mma_bf16(const void* qkv, const void* dout, void* dqkv, int n_seq, int n_tok, int heads, int dim_head, cudaStream_t st,
                            const uint8_t* keep = nullptr);
 

@@ -167,10 +167,13 @@ __device__ __forceinline__ void store_frag(T* __restrict__ p, const float (&src)
 // MASKED: keep [n_seq, n_tok] uint8 (1 = keep); one warp per staged sequence turns its row into 64 keep bits (behind K|V in shared
 // memory).  A kept query skips the dropped keys; a dropped query attends uniformly to all n_tok keys (every score filled alike), so
 // its running max starts from a real score and never meets -INF - (-INF).
+// PROBS: a second sweep over the keys recomputes each score (same operations, same order) and writes exp2(s - m) / l against the
+// final m and l of the online softmax to probs [n_seq, heads, n_tok, n_tok] in fp32 (exactly 0 on the keys a kept query skips).
 // ---------------------------------------------------------------------------------------------
-template <typename T, int DH, bool MASKED>
+template <typename T, int DH, bool MASKED, bool PROBS>
 __global__ void __launch_bounds__(DH == 32 ? 512 : 256) attention_small_kernel(const T* __restrict__ qkv, T* __restrict__ out, int n_seq, int n_tok,
-                                                              int heads, int spb, int hpb, float scale_log2e, const uint8_t* __restrict__ keep) {
+                                                              int heads, int spb, int hpb, float scale_log2e, const uint8_t* __restrict__ keep,
+                                                              float* __restrict__ probs) {
   pdl_wait();      // programmatic dependent launch: everything above is launch overhead hidden behind the previous kernel
   pdl_trigger();
   extern __shared__ uint8_t smem_attn[];
@@ -244,15 +247,30 @@ __global__ void __launch_bounds__(DH == 32 ? 512 : 256) attention_small_kernel(c
 #pragma unroll
     for (int d = 0; d < DH; ++d) acc[d] *= inv;
     store_frag<T, DH>(out + row * inner + h * DH, acc);
+    if constexpr (PROBS) {
+      float* prow = probs + ((size_t(seq0 + sl) * heads + h) * n_tok + qi) * n_tok;
+      for (int j = 0; j < n_tok; ++j) {
+        if (MASKED && row_kept && !((km >> j) & 1)) { prow[j] = 0.f; continue; }
+        float kf[DH];
+        load_frag<T, DH>(kbase + size_t(j) * 2 * w, kf);
+        float s = 0.f;
+        if (row_kept) {
+#pragma unroll
+          for (int d = 0; d < DH; ++d) s = fmaf(q[d], kf[d], s);
+        }
+        prow[j] = exp2f(s - m) / l;
+      }
+    }
   }
 }
 
 // Masked fp32 attention of 65..256 tokens with 64-wide heads: one CTA per (sequence, head), K|V of the head in shared memory
 // ([n_tok][2][64], the layout of attention_small_kernel with one head per block) and the keep bits as four 64-bit words behind them.
 // Every query row runs the per-thread online softmax of attention_small_kernel in the same order, so an all-kept mask gives the
-// bits of the unmasked call.
+// bits of the unmasked call.  PROBS: the second key sweep of attention_small_kernel writes the probabilities to probs.
+template <bool PROBS>
 __global__ void __launch_bounds__(256) attention_long_f32_kernel(const float* __restrict__ qkv, float* __restrict__ out, int n_tok, int heads,
-                                                                 float scale_log2e, const uint8_t* __restrict__ keep) {
+                                                                 float scale_log2e, const uint8_t* __restrict__ keep, float* __restrict__ probs) {
   pdl_wait();      // programmatic dependent launch: everything above is launch overhead hidden behind the previous kernel
   pdl_trigger();
   constexpr int DH = 64;
@@ -313,6 +331,20 @@ __global__ void __launch_bounds__(256) attention_long_f32_kernel(const float* __
 #pragma unroll
     for (int d = 0; d < DH; ++d) acc[d] *= inv;
     store_frag<float, DH>(out + row * inner + h * DH, acc);
+    if constexpr (PROBS) {
+      float* prow = probs + (size_t(blockIdx.x) * n_tok + qi) * n_tok;
+      for (int j = 0; j < n_tok; ++j) {
+        if (row_kept && !((km[j >> 6] >> (j & 63)) & 1)) { prow[j] = 0.f; continue; }
+        float kf[DH];
+        load_frag<float, DH>(kv + size_t(j) * 2 * DH, kf);
+        float s = 0.f;
+        if (row_kept) {
+#pragma unroll
+          for (int d = 0; d < DH; ++d) s = fmaf(q[d], kf[d], s);
+        }
+        prow[j] = exp2f(s - m) / l;
+      }
+    }
   }
 }
 
@@ -345,8 +377,8 @@ int gemm_f32(int trans_a, int trans_b, const float* a, int lda, const float* w, 
   return 0;
 }
 
-template <typename T, int DH, bool MASKED>
-static int launch_attention(const void* qkv, void* out, int n_seq, int n_tok, int heads, const uint8_t* keep, cudaStream_t st) {
+template <typename T, int DH, bool MASKED, bool PROBS>
+static int launch_attention(const void* qkv, void* out, int n_seq, int n_tok, int heads, const uint8_t* keep, float* probs, cudaStream_t st) {
   const int inner = heads * DH;
   int hpb = heads;                                        // heads staged per block: all of them unless K|V of a sequence exceed 96 KB
   while (hpb > 1 && size_t(n_tok) * 2 * hpb * DH * sizeof(T) > 96 * 1024) hpb = (hpb + 1) / 2;
@@ -358,40 +390,52 @@ static int launch_attention(const void* qkv, void* out, int n_seq, int n_tok, in
   const size_t smem = per_seq * spb + (MASKED ? spb * sizeof(uint64_t) : 0);
   AVF_REQUIRE(smem <= 200 * 1024, AVF_EUNSUPPORTED, "attention: %d tokens x %d inner does not fit shared memory", n_tok, inner);
   int threads = min(kMaxThreads, ceil_div(threads_per_seq * spb, 32) * 32);
-  auto kern = attention_small_kernel<T, DH, MASKED>;
+  auto kern = attention_small_kernel<T, DH, MASKED, PROBS>;
   static PerDeviceOnce once;
   if (once.first()) {
     AVF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
   }
   const float scale_log2e = 1.4426950408889634f / sqrtf(float(DH));
   launch_pdl(kern, dim3(ceil_div(n_seq, spb), ceil_div(heads, hpb)), threads, smem, st, static_cast<const T*>(qkv), static_cast<T*>(out), n_seq, n_tok, heads, spb, hpb,
-                                                                               scale_log2e, keep);
+                                                                               scale_log2e, keep, probs);
   AVF_LAUNCH_CHECK("attention_small_kernel");
   return 0;
 }
 
-int attention_small(int io_mode, const void* qkv, void* out, int n_seq, int n_tok, int heads, int dim_head, cudaStream_t st, const uint8_t* keep) {
+template <bool PROBS>
+static int launch_long_f32(const void* qkv, void* out, int n_seq, int n_tok, int heads, const uint8_t* keep, float* probs, cudaStream_t st) {
+  const size_t smem = size_t(n_tok) * 2 * 64 * sizeof(float) + 4 * sizeof(uint64_t);
+  static PerDeviceOnce once;
+  if (once.first()) {
+    AVF_CUDA(cudaFuncSetAttribute(attention_long_f32_kernel<PROBS>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(256 * 2 * 64 * sizeof(float) + 32)));
+  }
+  launch_pdl(attention_long_f32_kernel<PROBS>, n_seq * heads, 256, smem, st, static_cast<const float*>(qkv), static_cast<float*>(out), n_tok, heads,
+             1.4426950408889634f / sqrtf(64.f), keep, probs);
+  AVF_LAUNCH_CHECK("attention_long_f32_kernel");
+  return 0;
+}
+
+int attention_small(int io_mode, const void* qkv, void* out, int n_seq, int n_tok, int heads, int dim_head, cudaStream_t st, const uint8_t* keep,
+                    float* probs) {
   AVF_REQUIRE(n_seq > 0 && n_tok > 0 && heads > 0, AVF_EINVAL, "attention: n_seq=%d n_tok=%d heads=%d", n_seq, n_tok, heads);
   AVF_REQUIRE(dim_head == 32 || dim_head == 64, AVF_EUNSUPPORTED, "attention: dim_head=%d (supported: 32, 64)", dim_head);
   AVF_REQUIRE(keep == nullptr || n_tok <= 64 || (dim_head == 64 && n_tok <= 256), AVF_EUNSUPPORTED,
               "attention: a keep mask needs n_tok <= 64, or <= 256 with 64-wide heads (n_tok=%d, dim_head=%d)", n_tok, dim_head);
-  if (io_mode == AVF_BF16) return attention_mma_bf16(qkv, out, n_seq, n_tok, heads, dim_head, st, 0, keep);   // tensor cores
-  if (keep != nullptr && n_tok > 64) {
-    const size_t smem = size_t(n_tok) * 2 * 64 * sizeof(float) + 4 * sizeof(uint64_t);
-    static PerDeviceOnce once;
-    if (once.first()) {
-      AVF_CUDA(cudaFuncSetAttribute(attention_long_f32_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(256 * 2 * 64 * sizeof(float) + 32)));
-    }
-    launch_pdl(attention_long_f32_kernel, n_seq * heads, 256, smem, st, static_cast<const float*>(qkv), static_cast<float*>(out), n_tok, heads,
-               1.4426950408889634f / sqrtf(64.f), keep);
-    AVF_LAUNCH_CHECK("attention_long_f32_kernel");
-    return 0;
+  if (io_mode == AVF_BF16) return attention_mma_bf16(qkv, out, n_seq, n_tok, heads, dim_head, st, 0, keep, probs);   // tensor cores
+  if (probs != nullptr) {
+    if (keep != nullptr && n_tok > 64) return launch_long_f32<true>(qkv, out, n_seq, n_tok, heads, keep, probs, st);
+    if (keep != nullptr)
+      return dim_head == 32 ? launch_attention<float, 32, true, true>(qkv, out, n_seq, n_tok, heads, keep, probs, st)
+                            : launch_attention<float, 64, true, true>(qkv, out, n_seq, n_tok, heads, keep, probs, st);
+    return dim_head == 32 ? launch_attention<float, 32, false, true>(qkv, out, n_seq, n_tok, heads, nullptr, probs, st)
+                          : launch_attention<float, 64, false, true>(qkv, out, n_seq, n_tok, heads, nullptr, probs, st);
   }
+  if (keep != nullptr && n_tok > 64) return launch_long_f32<false>(qkv, out, n_seq, n_tok, heads, keep, nullptr, st);
   if (keep != nullptr)
-    return dim_head == 32 ? launch_attention<float, 32, true>(qkv, out, n_seq, n_tok, heads, keep, st)
-                          : launch_attention<float, 64, true>(qkv, out, n_seq, n_tok, heads, keep, st);
-  return dim_head == 32 ? launch_attention<float, 32, false>(qkv, out, n_seq, n_tok, heads, nullptr, st)
-                        : launch_attention<float, 64, false>(qkv, out, n_seq, n_tok, heads, nullptr, st);
+    return dim_head == 32 ? launch_attention<float, 32, true, false>(qkv, out, n_seq, n_tok, heads, keep, nullptr, st)
+                          : launch_attention<float, 64, true, false>(qkv, out, n_seq, n_tok, heads, keep, nullptr, st);
+  return dim_head == 32 ? launch_attention<float, 32, false, false>(qkv, out, n_seq, n_tok, heads, nullptr, nullptr, st)
+                        : launch_attention<float, 64, false, false>(qkv, out, n_seq, n_tok, heads, nullptr, nullptr, st);
 }
 
 }  // namespace avf

@@ -218,3 +218,31 @@ class Transformer(nn.Module):
             return self.forward_train(x.reshape(b * n, d), b, n, keep).view(b, n, d)
         y = x.detach().float().reshape(b * n, d).clone()
         return self.forward_(y, b, n, keep=keep).view(b, n, d)
+
+    # -- attention maps ------------------------------------------------------------------------
+    def check_maps_allowed(self, who: str, *inputs: torch.Tensor) -> None:
+        """Attention maps come from the inference kernels only: refuse a call autograd would record or one that would apply dropout."""
+        if needs_grad(self, *inputs):
+            raise RuntimeError(f"{who}: attention maps are inference only, and this call would be recorded by autograd; run it under "
+                               f"torch.no_grad() (or with parameters and inputs that do not require grad)")
+        if self.training and self.dropout > 0.0:
+            raise RuntimeError(f"{who}: attention maps are inference only, and this stack applies dropout (train() with dropout "
+                               f"{self.dropout}); call eval() first")
+
+    def maps_(self, x2d: torch.Tensor, n_seq: int, n_tok: int, out: Optional[torch.Tensor] = None, ld_out: int = 0,
+              pos: Optional[torch.Tensor] = None, keep: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """forward_ kernel by kernel (never the fused kernel) with the attention maps of every layer written by the attention launches:
+        returns fp32 [depth, n_seq, heads, n_tok, n_tok]; x2d / out receive what forward_ writes with set_fused_enabled(False)."""
+        return AF.encoder_stack_probs_(x2d, self.packed(), self.shape(n_seq, n_tok), keep, pos, out, ld_out)
+
+    def attention_maps(self, x: torch.Tensor, mask=None):
+        """(y, maps): y is ``forward(x, mask)`` as computed with set_fused_enabled(False), bit for bit, and maps fp32 [depth, b, heads, n,
+        n] holds the softmax probabilities of every layer (p = exp(s - m) / l, the kernel's own values; INTEGRATION.md section 1).
+        Inference only: RuntimeError under autograd or in train() with dropout > 0."""
+        AF._cuda(x, "x")
+        self.check_maps_allowed("Transformer.attention_maps", x)
+        b, n, d = x.shape
+        keep = None if mask is None else AF.keep_from_mask(mask, b, n)
+        y = x.detach().float().reshape(b * n, d).clone()
+        maps = self.maps_(y, b, n, keep=keep)
+        return y.view(b, n, d), maps

@@ -250,6 +250,74 @@ def attention_fwd(qkv: torch.Tensor, n_seq: int, n_tok: int, heads: int, dim_hea
 
 
 # ------------------------------------------------------------------------------------------------
+# attention maps: the softmax probabilities written by the attention launches (include/avformer_b200.h, "attention maps")
+# ------------------------------------------------------------------------------------------------
+def _probs(depth: int, n_seq: int, heads: int, n_tok: int, device) -> torch.Tensor:
+    return torch.empty((depth, n_seq, heads, n_tok, n_tok), dtype=torch.float32, device=device)
+
+
+def _keep_or_none(keep: Optional[torch.Tensor], n_seq: int, n_tok: int):
+    return None if keep is None else _keep_ptr(keep, n_seq, n_tok)
+
+
+def attention_fwd_probs(qkv: torch.Tensor, n_seq: int, n_tok: int, heads: int, dim_head: int,
+                        keep: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """attention_fwd and its softmax probabilities from the same launch: (out, probs fp32 [n_seq, heads, n_tok, n_tok])."""
+    qkv = _cuda(qkv, "qkv").contiguous()
+    out = torch.empty((n_seq * n_tok, heads * dim_head), dtype=qkv.dtype, device=qkv.device)
+    probs = _probs(1, n_seq, heads, n_tok, qkv.device)[0]
+    check(_lib.lib().avf_attention_fwd_probs(_io_mode(qkv), _ptr(qkv), _ptr(out), n_seq, n_tok, heads, dim_head, _keep_or_none(keep, n_seq, n_tok),
+                                             _ptr(probs), _stream()), "attention_fwd_probs")
+    return out, probs
+
+
+def encoder_stack_probs_(x: torch.Tensor, packed: PackedStack, shape: StackShape, keep: Optional[torch.Tensor] = None,
+                         pos: Optional[torch.Tensor] = None, out: Optional[torch.Tensor] = None, ld_out: int = 0) -> torch.Tensor:
+    """encoder_stack_fwd_ (+ pos [n_tok, dim] first, if given) kernel by kernel, returning the maps fp32 [depth, n_seq, heads, n_tok,
+    n_tok] of every layer; x (or out) receives what the call without maps writes, bit for bit."""
+    _cuda(x, "x")
+    if x.dtype != torch.float32 or x.stride(-1) != 1:
+        raise TypeError("encoder_stack_probs_: x must be a float32 residual stream with unit column stride")
+    L = _lib.lib()
+    ws = workspace(L.avf_encoder_workspace_bytes(ctypes.byref(shape), packed.mode), x.device)
+    probs = _probs(shape.depth, shape.n_seq, shape.heads, shape.n_tok, x.device)
+    check(L.avf_encoder_stack_fwd_probs(packed.mode, ctypes.byref(shape), packed.array, _keep_or_none(keep, shape.n_seq, shape.n_tok), _ptr(x),
+                                        x.stride(0), _ptr(None if pos is None else _f32c(pos)), _ptr(out), ld_out, _ptr(probs), _ptr(ws), ws.numel(),
+                                        _stream()), "encoder_stack_fwd_probs")
+    return probs
+
+
+def tformer_fwd_probs(frames: torch.Tensor, cls_token: torch.Tensor, pos: torch.Tensor, packed: PackedStack, shape: StackShape,
+                      keep: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """tformer_fwd with the maps of every layer: (cls [n_clips, dim], maps fp32 [depth, n_clips, heads, T+1, T+1]); the last layer's
+    map is full, its cls features equal tformer_fwd's bit for bit."""
+    frames = _cuda(frames, "frames").contiguous()
+    cls = torch.empty((shape.n_seq, shape.dim), dtype=torch.float32, device=frames.device)
+    probs = _probs(shape.depth, shape.n_seq, shape.heads, shape.n_tok, frames.device)
+    L = _lib.lib()
+    ws = workspace(L.avf_tformer_workspace_bytes(ctypes.byref(shape), packed.mode), frames.device)
+    check(L.avf_tformer_fwd_probs(packed.mode, _io_mode(frames), ctypes.byref(shape), packed.array, _keep_or_none(keep, shape.n_seq, shape.n_tok),
+                                  _ptr(frames), _ptr(_f32c(cls_token)), _ptr(_f32c(pos)), _ptr(cls), _ptr(probs), _ptr(ws), ws.numel(), _stream()),
+          "tformer_fwd_probs")
+    return cls, probs
+
+
+def tformer_fwd_indexed_probs(bank: torch.Tensor, index: torch.Tensor, cls_token: torch.Tensor, pos: torch.Tensor, packed: PackedStack,
+                              shape: StackShape) -> Tuple[torch.Tensor, torch.Tensor]:
+    """tformer_fwd_indexed with the maps of every layer, as tformer_fwd_probs."""
+    bank = _cuda(bank, "bank").contiguous()
+    index = _index_i32(index, shape.n_seq, shape.n_tok - 1, "tformer_fwd_indexed_probs")
+    cls = torch.empty((shape.n_seq, shape.dim), dtype=torch.float32, device=bank.device)
+    probs = _probs(shape.depth, shape.n_seq, shape.heads, shape.n_tok, bank.device)
+    L = _lib.lib()
+    ws = workspace(L.avf_tformer_indexed_workspace_bytes(ctypes.byref(shape), packed.mode), bank.device)
+    check(L.avf_tformer_fwd_indexed_probs(packed.mode, _io_mode(bank), ctypes.byref(shape), packed.array, _ptr(bank), bank.shape[0], _ptr(index),
+                                          _ptr(_f32c(cls_token)), _ptr(_f32c(pos)), _ptr(cls), _ptr(probs), _ptr(ws), ws.numel(), _stream()),
+          "tformer_fwd_indexed_probs")
+    return cls, probs
+
+
+# ------------------------------------------------------------------------------------------------
 # a6 / a7 / a8 / a9 / a11 / a12
 # ------------------------------------------------------------------------------------------------
 def sformer_fwd(fmap: torch.Tensor, pos: torch.Tensor, packed: PackedStack, heads: int, dim_head: int, mlp_dim: int,

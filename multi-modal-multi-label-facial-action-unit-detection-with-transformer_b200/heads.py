@@ -68,12 +68,15 @@ class AU_former(nn.Module):
             self._last = _PackedLast([getattr(self, f"AU_linear_last{i}") for i in range(1, 13)])
         return self._last
 
-    def tokens_into(self, emb: torch.Tensor, ld_emb: int, n_clips: int, out: Optional[torch.Tensor] = None, ld_out: int = 0):
+    def tokens_into(self, emb: torch.Tensor, ld_emb: int, n_clips: int, out: Optional[torch.Tensor] = None, ld_out: int = 0,
+                    maps: bool = False):
         """BN -> 12 projections -> + pos -> 2 encoder layers.  ``emb`` may be a strided view (row stride
         ld_emb): the cls rows of a TFormer token matrix are consumed in place.  The last layer's result goes
         to ``out`` (row stride ld_out) when given — that is how the audio and video halves of the
         [B,12,256] fusion input get written side by side without a cat (models/avformer.py:100).  With
-        BatchNorm in eval() the positional add is part of the encoder-stack launch."""
+        BatchNorm in eval() the positional add is part of the encoder-stack launch.  ``maps``: run the stack kernel by kernel
+        (Transformer.maps_) and return its attention maps [2, n_clips, 8, 12, 12] instead of the tokens, which still go to out / x."""
+        stack = self.corr_transformer.maps_ if maps else self.corr_transformer.forward_
         f = self._packed_front()
         bn = self.AU_BN1
         if bn.training:
@@ -82,9 +85,9 @@ class AU_former(nn.Module):
             x, _ = AF.au_former_front_train(view, n_clips, bn.weight, bn.bias, bn.running_mean, bn.running_var, True,
                                             0.1 if bn.momentum is None else bn.momentum, f.w, f.b, self.pos_embedding[0], f.mode)
             bn.num_batches_tracked += 1
-            return self.corr_transformer.forward_(x, n_clips, 12, out, ld_out)
+            return stack(x, n_clips, 12, out, ld_out)
         x = AF.au_former_front(emb, ld_emb, n_clips, (bn.weight, bn.bias, bn.running_mean, bn.running_var), f.w, f.b, None, f.mode)
-        return self.corr_transformer.forward_(x, n_clips, 12, out, ld_out, pos=self.pos_embedding[0])
+        return stack(x, n_clips, 12, out, ld_out, pos=self.pos_embedding[0])
 
     def front_params(self):
         return [p for i in range(1, 13) for p in (getattr(self, f"AU_linear_p{i}").weight, getattr(self, f"AU_linear_p{i}").bias)]
@@ -133,6 +136,12 @@ class former_AU_head(nn.Module):
             return AF.au_logits(tokens2d, self._packed_last().w, n_clips, want_decisions)
         return AF.token_stack_fwd_(tokens2d, t.packed(), t.shape(n_clips, 12), self.pos_embedding[0], w_last=self._packed_last().w,
                                    want_decisions=want_decisions)
+
+    def logits21_maps_(self, tokens2d: torch.Tensor, n_clips: int):
+        """logits21_ kernel by kernel with the attention maps of the three layers: ([B,21], maps [3, n_clips, 8, 12, 12]); the logits
+        equal logits21_'s with set_fused_enabled(False) bit for bit (the same positional add, layers and logits launches)."""
+        maps = self.corr_transformer.maps_(tokens2d, n_clips, 12, pos=self.pos_embedding[0])
+        return AF.au_logits(tokens2d, self._packed_last().w, n_clips), maps
 
     def last_params(self):
         return [getattr(self, f"AU_linear_last{i}").weight for i in range(1, 13)]

@@ -99,11 +99,25 @@ class ResFormer(nn.Module):
             return SFormerFn.apply(fmap, self.pos_embedding, st, *st.param_list())
         return AF.sformer_fwd(fmap, self.pos_embedding[0, :n_tok], st.packed(), st.heads, st.dim_head, st.mlp_dim, out=out)
 
-    def forward(self, x):
+    def sformer_maps(self, fmap):
+        """sformer() kernel by kernel with the attention maps of the spatial transformer: (fmap_out, maps [depth, F, heads, H*W, H*W]);
+        fmap_out equals sformer()'s with set_fused_enabled(False) bit for bit (the same pack, layers and unpack launches)."""
+        st = self.spatial_transformer
+        n_tok = fmap.shape[2] * fmap.shape[3]
+        if n_tok > self.pos_embedding.shape[1]:
+            raise ValueError(f"stage-3 map has {n_tok} positions but pos_embedding holds {self.pos_embedding.shape[1]}")
+        st.check_maps_allowed("ResFormer.sformer_maps", fmap, self.pos_embedding)
+        x = AF.sformer_tokens_pack(fmap, self.pos_embedding[0, :n_tok])
+        maps = st.maps_(x, fmap.shape[0], n_tok)
+        return AF.sformer_tokens_unpack(x, fmap.shape, fmap.dtype), maps
+
+    def forward(self, x, maps: bool = False):
+        """x [b,t,c,h,w] -> [b*t, 512]; ``maps``: also return the SFormer's attention maps (sformer_maps)."""
         b, t, c, h, w = x.shape
         fmap = self.stem_to_stage3(x.contiguous().view(-1, c, h, w))
-        fmap = self.sformer(fmap)
-        return torch.flatten(self.avgpool(self.layer4(fmap)), 1)
+        fmap, smaps = self.sformer_maps(fmap) if maps else (self.sformer(fmap), None)
+        feat = torch.flatten(self.avgpool(self.layer4(fmap)), 1)
+        return (feat, smaps) if maps else feat
 
 
 class SFormerBlock(nn.Module):
@@ -231,6 +245,28 @@ class TFormer(nn.Module):
                 raise ValueError(f"TFormer.{who}: index entries must lie in [-1, {bank_shape[0]}) (-1 = missing frame), got "
                                  f"[{lo}, {hi}]")
         return index.to(device=device, dtype=torch.int32).contiguous()
+
+    def attention_maps(self, x, mask=None):
+        """(cls, maps): cls equals ``cls_features(x, mask)`` bit for bit and maps fp32 [depth, n_clips, heads, T+1, T+1] holds the
+        softmax probabilities of every layer; the last layer's attention runs every query row, so its map is full (which frames and
+        which frames' tokens each token attended to).  Inference only: RuntimeError under autograd or in train() with dropout > 0."""
+        n_clips = self._n_clips(x)
+        st = self.spatial_transformer
+        st.check_maps_allowed("TFormer.attention_maps", x, self.cls_token, self.pos_embedding)
+        keep = None if mask is None else AF.keep_from_mask(mask, n_clips, self.num_patches + 1)
+        return AF.tformer_fwd_probs(x.detach(), self.cls_token.view(-1), self.pos_embedding[0], st.packed(), st.shape(n_clips, self.num_patches + 1),
+                                    keep)
+
+    def attention_maps_indexed(self, bank, index):
+        """attention_maps on clips described by frame indices, bit for bit ``attention_maps(bank[index.clamp(min=0)].reshape(-1, dim),
+        mask=index >= 0)`` without the gathered copy.  ``bank`` / ``index`` as in cls_features_indexed, with the same checks and errors.
+        Whole videos: ``eng.frame_features`` for the bank, then this call with the clips' index table."""
+        AF._cuda(bank, "bank")
+        st = self.spatial_transformer
+        st.check_maps_allowed("TFormer.attention_maps_indexed", bank, self.cls_token, self.pos_embedding)
+        index = self.bank_index(bank.shape, bank.device, index, "attention_maps_indexed")
+        return AF.tformer_fwd_indexed_probs(bank.detach(), index, self.cls_token.view(-1), self.pos_embedding[0], st.packed(),
+                                            st.shape(index.shape[0], self.num_patches + 1))
 
     def forward(self, x, mask=None):
         """x [n_clips*T, dim] frame features -> cls features [n_clips, dim].  ``mask`` (optional): bool [n_clips, T], True = a real
