@@ -431,6 +431,28 @@ int avf_tformer_fwd_indexed_probs(int mode, int io_mode, const avf_stack_shape* 
                                   const void* bank, int32_t n_bank, const int32_t* index, const float* cls_token, const float* pos,
                                   float* cls_out, float* probs, void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---- attention relevance: gradient-weighted attention maps from the attention backward (models/heads.py:234, attn) -------------
+ * gmap(s) is a caller-owned DEVICE fp32 buffer [depth, n_seq, heads, n_tok, n_tok], contiguous.  Element (l, b, h, i, j) is
+ * G = P_ij * dP_ij for layer l, sequence b, head h, query i and key j: P is the backward kernel's own recomputed softmax (the same
+ * quantity as the attention maps above, fp32) and dP = dout V^T the gradient wrt that probability before the softmax backward
+ * (mode AVF_BF16: the MMA of bf16 dout and V with fp32 accumulation); the product is formed in fp32.  So a kept query gets exactly
+ * 0.0 on a dropped key and a dropped query's row is (1 / n_tok) * dP.  The maps are written by the attention backward launch itself,
+ * in the pass that already holds P and dP; dqkv / dx and every gradient equal those of the call without maps bit for bit.
+ * keep == NULL is the unmasked call.  Workspaces are those of the calls without maps. */
+/* avf_attention_bwd(_masked) + gmap [n_seq, heads, n_tok, n_tok] (depth 1); models/heads.py:234 (attn) and its gradient. */
+int avf_attention_bwd_gradmaps(int io_mode, const void* qkv, const void* dout, void* dqkv, int32_t n_seq, int32_t n_tok,
+                               int32_t heads, int32_t dim_head, const uint8_t* keep, float* gmap, void* stream);
+/* avf_encoder_stack_bwd(_masked) + gmaps (models/heads.py:234, attn, of every layer): layer l's map goes to gmaps + l * n_seq*heads*n_tok*n_tok.  A NULL field of grads (or
+ * grads == NULL) launches no weight-gradient kernel for it, so with grads == NULL the call computes activation gradients only. */
+int avf_encoder_stack_bwd_gradmaps(int mode, const avf_stack_shape* s, const avf_layer_weights* layers, const uint8_t* keep,
+                                   const void* tape, size_t tape_bytes, float* dx, int32_t ld_dx,
+                                   const avf_layer_grads* grads, int accumulate, void* workspace, size_t workspace_bytes,
+                                   float dropout_p, uint64_t dropout_seed, const uint32_t* dropout_salt, float* gmaps, void* stream);
+/* Rollout of the gradient maps of models/heads.py:234 (attn) (Chefer, Gur, Wolf, ICCV 2021, self-attention rule), per sequence b, fp32:  A_l = mean over h of max(G[l, b, h], 0),
+ * R_0 = I, R_l = R_{l-1} + A_l R_{l-1}, R[b] = R_depth (no row normalisation) -> R [n_seq, n_tok, n_tok] DEVICE fp32.
+ * n_tok <= 256.  Deterministic: every sum runs in a fixed order, no atomics.  One launch. */
+int avf_attention_rollout(const float* gmaps, int32_t depth, int32_t n_seq, int32_t heads, int32_t n_tok, float* R, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

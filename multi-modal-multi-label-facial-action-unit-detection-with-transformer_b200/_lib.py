@@ -150,6 +150,12 @@ SIGNATURES = {
                                              _c_p, _c_p, _c_p, _c_p, _c_p, _sz, _c_p]),
     "avf_tformer_fwd_indexed_probs": (ctypes.c_int, [ctypes.c_int, ctypes.c_int, ctypes.POINTER(StackShape), ctypes.POINTER(LayerWeights), _c_p,
                                                      _i32, _c_p, _c_p, _c_p, _c_p, _c_p, _c_p, _sz, _c_p]),
+    # ---- attention relevance (gmaps: device fp32 [depth, n_seq, heads, n_tok, n_tok]; R: [n_seq, n_tok, n_tok]) ----
+    "avf_attention_bwd_gradmaps": (ctypes.c_int, [ctypes.c_int, _c_p, _c_p, _c_p, _i32, _i32, _i32, _i32, _c_p, _c_p, _c_p]),
+    "avf_encoder_stack_bwd_gradmaps": (ctypes.c_int, [ctypes.c_int, ctypes.POINTER(StackShape), ctypes.POINTER(LayerWeights), _c_p, _c_p, _sz, _c_p,
+                                                      _i32, ctypes.POINTER(LayerGrads), ctypes.c_int, _c_p, _sz, ctypes.c_float, ctypes.c_uint64,
+                                                      _c_p, _c_p, _c_p]),
+    "avf_attention_rollout": (ctypes.c_int, [_c_p, _i32, _i32, _i32, _i32, _c_p, _c_p]),
 }
 
 _lock = threading.Lock()

@@ -3,6 +3,7 @@
 and test_aff2.py:58-117 can use them unchanged.  Every transformer region runs in libavformer_b200.so."""
 from __future__ import annotations
 
+import numbers
 from collections import OrderedDict
 
 import torch
@@ -172,6 +173,90 @@ class TwoStreamAuralVisualFormer(nn.Module):
             return out21, maps
         finally:
             AF.set_fused_enabled(prev)
+
+    def attention_relevance(self, x, au, stacks=None):
+        """Per-AU attention relevance (gradient-weighted attention with rollout, INTEGRATION.md section 1): (out21 [B,21], {name: (gmaps, R)}).
+
+        ``au`` is the target: an int j (the logit of AU j), a float [12] weight vector or a float [B, 12] per-clip weight matrix; the
+        backward is seeded with d out21[:, :12] = weights and d out21[:, 12:] = 0.  gmaps fp32 [depth, n_seq, heads, n_tok, n_tok] are
+        the gradient maps G = P o dP of every layer, written by the attention backward kernels, and R fp32 [n_seq, n_tok, n_tok] their
+        rollout R = prod_l (I + mean_h max(G_l, 0)).  Names, shapes and ``stacks`` as in attention_maps (the TFormer's last layer is
+        full).  The forward is the tape-keeping one of every region, so out21 equals _forward_train's when every region is recorded
+        there, bit for bit; the backward runs only as far as the deepest selected stack (the SFormer's passes through stage 4 and
+        the pool with torch autograd; the conv stem, stages 1-3 and the audio ResNet run no backward).  No parameter gradient is
+        created or changed and no autograd graph outlives the call, whatever the requires_grad flags and the grad mode.  Needs eval()
+        (RuntimeError otherwise) and task == "AU"; ValueError for an unknown stack or a malformed ``au``."""
+        names = self.MAP_STACKS if stacks is None else tuple(stacks)
+        unknown = [n for n in names if n not in self.MAP_STACKS]
+        if unknown:
+            raise ValueError(f"attention_relevance: unknown stack name(s) {unknown}; the stacks are {list(self.MAP_STACKS)}")
+        audio, clip = x["audio_features"], x["clip"]
+        AF._cuda(clip, "x['clip']")
+        AF._cuda(audio, "x['audio_features']")
+        who = "TwoStreamAuralVisualFormer.attention_relevance"
+        in_train = [n or type(self).__name__ for n, m in self.named_modules() if m.training]
+        if in_train:
+            raise RuntimeError(f"{who}: attention relevance needs eval(); {in_train[0]} is in train(), where dropout and BatchNorm batch "
+                               f"statistics would couple the clips of a batch and BatchNorm would update its running statistics; call "
+                               f"model.eval() first")
+        if self.task != "AU":
+            raise RuntimeError(f"{who}: relevance explains the AU logits, which only task 'AU' computes (task is {self.task!r})")
+        bs = clip.shape[0]
+        weights = self._relevance_weights(au, bs, clip.device)
+        vm = self.video_model.video_model
+        rf, tf = vm.s_former, vm.t_former
+        st = rf.spatial_transformer
+        a_head, v_head = self.audio_model.au_head, self.video_model.au_head
+        want_sf = "sformer" in names
+        want_tf = want_sf or "tformer" in names
+        want_v = want_tf or "video_au_former" in names
+        gm = {}
+        with torch.no_grad():
+            # forward: the tape-keeping kernels of every region (the data flow of _forward_train)
+            tok_a, a_ctx = a_head.relevance_fwd_(self.audio_model.audio_model(audio), bs)
+            fmap = rf.stem_to_stage3(clip[:, -vm.num_channels:].permute(0, 2, 1, 3, 4).contiguous().flatten(0, 1))
+            F_, C, H, W = fmap.shape
+            s_tok = AF.sformer_tokens_pack(fmap, rf.pos_embedding.detach().reshape(-1, C)[: H * W])
+            s_y, s_tape = st.relevance_fwd_(s_tok, F_, H * W)
+            s_out = AF.sformer_tokens_unpack(s_y, fmap.shape, fmap.dtype)
+            with torch.enable_grad():              # stage 4 and the pool: torch autograd, differentiated wrt the SFormer's output only
+                s_out.requires_grad_(want_sf)
+                feat = torch.flatten(rf.avgpool(rf.layer4(s_out)), 1)
+            t_y, t_tape, _ = tf.relevance_fwd_(feat)
+            T1 = tf.num_patches + 1
+            tok_v, v_ctx = v_head.relevance_fwd_(t_y.view(bs, T1, tf.dim)[:, 0], bs)
+            out21, f_ctx = self.au_head.relevance_fwd_(torch.cat([tok_a, tok_v], dim=1), bs)
+            # backward from the weighted logits, as deep as the selected stacks need
+            if names:
+                gm["fusion_head"], dfused = self.au_head.relevance_bwd_(f_ctx, weights, maps="fusion_head" in names)
+                if "audio_au_former" in names:
+                    gm["audio_au_former"], _ = a_head.relevance_bwd_(a_ctx, dfused[:, :a_head.token_dim].contiguous())
+                if want_v:
+                    gm["video_au_former"], demb = v_head.relevance_bwd_(v_ctx, dfused[:, a_head.token_dim:].contiguous(),
+                                                                        maps="video_au_former" in names, want_emb=want_tf)
+                if want_tf:
+                    dtok, gm["tformer"] = tf.relevance_bwd_(t_tape, bs, demb, maps="tformer" in names)
+                if want_sf:
+                    dfeat = dtok.view(bs, T1, tf.dim)[:, 1:].reshape(feat.shape)
+                    (dfmap,) = torch.autograd.grad(feat, s_out, dfeat)
+                    gm["sformer"] = st.relevance_bwd_(AF.sformer_tokens_pack(dfmap, None), s_tape, F_, H * W)
+            return out21, {n: (gm[n], AF.attention_rollout(gm[n])) for n in self.MAP_STACKS if n in names}
+
+    @staticmethod
+    def _relevance_weights(au, bs, device) -> torch.Tensor:
+        """The seed d out21[:, :12] of attention_relevance as fp32 [bs, 12] on ``device``."""
+        if isinstance(au, numbers.Integral) and not isinstance(au, bool):
+            if not 0 <= int(au) < 12:
+                raise ValueError(f"attention_relevance: au={au} is not an AU index (0..11)")
+            w = torch.zeros((bs, 12), dtype=torch.float32, device=device)
+            w[:, int(au)] = 1.0
+            return w
+        t = au if torch.is_tensor(au) else None
+        if t is None or not t.dtype.is_floating_point or tuple(t.shape) not in ((12,), (bs, 12)):
+            desc = f"{t.dtype} {tuple(t.shape)}" if t is not None else type(au).__name__
+            raise ValueError(f"attention_relevance: au must be an int in 0..11, a float [12] weight vector or a float [{bs}, 12] weight "
+                             f"matrix, got {desc}")
+        return t.detach().to(device=device, dtype=torch.float32).expand(bs, 12).contiguous()
 
     def _forward_train(self, clip, audio):
         """Same data flow with autograd-visible regions (autograd.py); frozen sub-models (requires_grad=False everywhere,

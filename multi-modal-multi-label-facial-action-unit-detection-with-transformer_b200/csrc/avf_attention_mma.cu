@@ -257,12 +257,14 @@ struct BwdCfg {
 
 // MASKED: the scores are masked as in the forward (mask_score); dS is 0 wherever a score was filled, and the uniform P of a dropped
 // query still carries its dO into dV.
-template <int DH, int NP, bool MASKED>
+// GMAP: pass 1 also writes the gradient map G = P o dP (fp32 P and fp32-accumulated dP, multiplied once in fp32) to gmap
+// [n_seq, heads, n_tok, n_tok]; pass 1 visits every (query, key), and the stores are its only addition.
+template <int DH, int NP, bool MASKED, bool GMAP>
 __global__ void __launch_bounds__(BwdCfg<DH, NP>::WARPS * 32) attention_bwd_mma_kernel(const __nv_bfloat16* __restrict__ qkv,
                                                                                        const __nv_bfloat16* __restrict__ dout,
                                                                                        __nv_bfloat16* __restrict__ dqkv, int n_problems,
                                                                                        int n_tok, int heads, float scale,
-                                                                                       const uint8_t* __restrict__ keep) {
+                                                                                       const uint8_t* __restrict__ keep, float* __restrict__ gmap) {
   pdl_wait();      // programmatic dependent launch: everything above is launch overhead hidden behind the previous kernel
   pdl_trigger();
   using Cfg = BwdCfg<DH, NP>;
@@ -416,6 +418,18 @@ __global__ void __launch_bounds__(BwdCfg<DH, NP>::WARPS * 32) attention_bwd_mma_
     d_lo += __shfl_xor_sync(0xffffffffu, d_lo, 2);
     d_hi += __shfl_xor_sync(0xffffffffu, d_hi, 1);
     d_hi += __shfl_xor_sync(0xffffffffu, d_hi, 2);
+    if constexpr (GMAP) {                      // s = P, dp = dP here; __fmul_rn keeps the product out of the FMAs of delta and dS
+      float* g_lo = gmap + (size_t(prob) * n_tok + r_lo) * n_tok;
+      float* g_hi = g_lo + size_t(8) * n_tok;
+#pragma unroll
+      for (int nt = 0; nt < NP / 8; ++nt) {
+        const int c = nt * 8 + 2 * t;
+        if (r_lo < n_tok && c < n_tok) g_lo[c] = __fmul_rn(s[nt][0], dp[nt][0]);
+        if (r_lo < n_tok && c + 1 < n_tok) g_lo[c + 1] = __fmul_rn(s[nt][1], dp[nt][1]);
+        if (r_lo + 8 < n_tok && c < n_tok) g_hi[c] = __fmul_rn(s[nt][2], dp[nt][2]);
+        if (r_lo + 8 < n_tok && c + 1 < n_tok) g_hi[c + 1] = __fmul_rn(s[nt][3], dp[nt][3]);
+      }
+    }
     if (t == 0) {
       st_m[r_lo] = o_lo; st_il[r_lo] = i_lo; st_d[r_lo] = d_lo;
       st_m[r_lo + 8] = o_hi; st_il[r_lo + 8] = i_hi; st_d[r_lo + 8] = d_hi;
@@ -480,12 +494,12 @@ __global__ void __launch_bounds__(BwdCfg<DH, NP>::WARPS * 32) attention_bwd_mma_
   }
 }
 
-template <int DH, int NP, bool MASKED>
-int launch_bwd(const void* qkv, const void* dout, void* dqkv, int n_seq, int n_tok, int heads, const uint8_t* keep, cudaStream_t st) {
+template <int DH, int NP, bool MASKED, bool GMAP>
+int launch_bwd(const void* qkv, const void* dout, void* dqkv, int n_seq, int n_tok, int heads, const uint8_t* keep, float* gmap, cudaStream_t st) {
   const int n_problems = n_seq * heads;
   constexpr int kWarps = BwdCfg<DH, NP>::WARPS;
-  launch_pdl(attention_bwd_mma_kernel<DH, NP, MASKED>, ceil_div(n_problems, kWarps), kWarps * 32, 0, st, static_cast<const __nv_bfloat16*>(qkv), static_cast<const __nv_bfloat16*>(dout), static_cast<__nv_bfloat16*>(dqkv), n_problems, n_tok, heads,
-      1.0f / sqrtf(float(DH)), keep);
+  launch_pdl(attention_bwd_mma_kernel<DH, NP, MASKED, GMAP>, ceil_div(n_problems, kWarps), kWarps * 32, 0, st, static_cast<const __nv_bfloat16*>(qkv), static_cast<const __nv_bfloat16*>(dout), static_cast<__nv_bfloat16*>(dqkv), n_problems, n_tok, heads,
+      1.0f / sqrtf(float(DH)), keep, gmap);
   AVF_LAUNCH_CHECK("attention_bwd_mma_kernel");
   return 0;
 }
@@ -692,11 +706,14 @@ __global__ void __launch_bounds__(kLongWarps * 32) attention_long_mma_kernel(con
 // Backward, the two passes of attention_bwd_mma_kernel with Q, K, V, dO of the (sequence, head) in shared memory:
 //   pass 1 (rows = queries): sweep 1 the row max, sweep 2 l and sum_j e_j dP_j (delta = that / l), sweep 3 dS and dQ = dS K;
 //   pass 2 (rows = keys): one sweep over 64-query blocks, P^T and dS^T from the saved statistics, dV = P^T dO, dK = dS^T Q.
-template <bool MASKED>
+// GMAP: sweep 3 of pass 1, which visits every (query, key) with P and dP in registers, also writes G = P o dP in fp32 to gmap
+// [n_seq, heads, n_tok, n_tok].
+template <bool MASKED, bool GMAP>
 __global__ void __launch_bounds__(kLongWarps * 32) attention_bwd_long_mma_kernel(const __nv_bfloat16* __restrict__ qkv,
                                                                                 const __nv_bfloat16* __restrict__ dout,
                                                                                 __nv_bfloat16* __restrict__ dqkv, int n_tok, int heads,
-                                                                                float scale, const uint8_t* __restrict__ keep) {
+                                                                                float scale, const uint8_t* __restrict__ keep,
+                                                                                float* __restrict__ gmap) {
   pdl_wait();      // programmatic dependent launch: everything above is launch overhead hidden behind the previous kernel
   pdl_trigger();
   extern __shared__ __align__(16) uint8_t smem_long[];
@@ -774,6 +791,21 @@ __global__ void __launch_bounds__(kLongWarps * 32) attention_bwd_long_mma_kernel
       long_mma_abt(s, qf, Ks + kb * 64, g, t);
       long_mask<MASKED>(s, k_lo, k_hi, MASKED ? km[kb] : 0, n_tok - kb * 64, t);
       long_mma_abt(dp, of, Vs + kb * 64, g, t);
+      if constexpr (GMAP) {                    // the P of the dS below (the same expression), times dP
+        float* g_lo = gmap + (size_t(blockIdx.x) * n_tok + r_lo) * n_tok + kb * 64;
+        float* g_hi = g_lo + size_t(8) * n_tok;
+        const int cols = n_tok - kb * 64;
+#pragma unroll
+        for (int nt = 0; nt < 8; ++nt) {
+          const int c = nt * 8 + 2 * t;
+          const float p0 = exp2f(fmaf(s[nt][0], scale_log2e, -o_lo)) * i_lo, p1 = exp2f(fmaf(s[nt][1], scale_log2e, -o_lo)) * i_lo;
+          const float p2 = exp2f(fmaf(s[nt][2], scale_log2e, -o_hi)) * i_hi, p3 = exp2f(fmaf(s[nt][3], scale_log2e, -o_hi)) * i_hi;
+          if (r_lo < n_tok && c < cols) g_lo[c] = __fmul_rn(p0, dp[nt][0]);
+          if (r_lo < n_tok && c + 1 < cols) g_lo[c + 1] = __fmul_rn(p1, dp[nt][1]);
+          if (r_hi < n_tok && c < cols) g_hi[c] = __fmul_rn(p2, dp[nt][2]);
+          if (r_hi < n_tok && c + 1 < cols) g_hi[c + 1] = __fmul_rn(p3, dp[nt][3]);
+        }
+      }
 #pragma unroll
       for (int nt = 0; nt < 8; ++nt) {        // dS (the 1/sqrt(dh) is applied once when dQ is stored)
         s[nt][0] = exp2f(fmaf(s[nt][0], scale_log2e, -o_lo)) * i_lo * (dp[nt][0] - d_lo);
@@ -856,15 +888,15 @@ int launch_long(const void* qkv, void* out, int n_seq, int n_tok, int heads, int
   return 0;
 }
 
-template <bool MASKED>
-int launch_bwd_long(const void* qkv, const void* dout, void* dqkv, int n_seq, int n_tok, int heads, const uint8_t* keep, cudaStream_t st) {
-  auto kern = attention_bwd_long_mma_kernel<MASKED>;
+template <bool MASKED, bool GMAP>
+int launch_bwd_long(const void* qkv, const void* dout, void* dqkv, int n_seq, int n_tok, int heads, const uint8_t* keep, float* gmap, cudaStream_t st) {
+  auto kern = attention_bwd_long_mma_kernel<MASKED, GMAP>;
   static PerDeviceOnce once;
   if (once.first()) {
     AVF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, int(long_bwd_smem(kLongMaxTok))));
   }
   launch_pdl(kern, n_seq * heads, kLongWarps * 32, long_bwd_smem(n_tok), st, static_cast<const __nv_bfloat16*>(qkv), static_cast<const __nv_bfloat16*>(dout),
-             static_cast<__nv_bfloat16*>(dqkv), n_tok, heads, 1.0f / sqrtf(float(kLongDH)), keep);
+             static_cast<__nv_bfloat16*>(dqkv), n_tok, heads, 1.0f / sqrtf(float(kLongDH)), keep, gmap);
   AVF_LAUNCH_CHECK("attention_bwd_long_mma_kernel");
   return 0;
 }
@@ -903,17 +935,25 @@ int attention_mma_bf16(const void* qkv, void* out, int n_seq, int n_tok, int hea
 
 namespace avf {
 int attention_bwd_mma_bf16(const void* qkv, const void* dout, void* dqkv, int n_seq, int n_tok, int heads, int dim_head, cudaStream_t st,
-                           const uint8_t* keep) {
+                           const uint8_t* keep, float* gmap) {
   AVF_REQUIRE(n_tok >= 1 && n_tok <= kLongMaxTok && (n_tok <= 64 || dim_head == kLongDH), AVF_EUNSUPPORTED,
               "attention_bwd: n_tok=%d with dim_head=%d (1..64 tokens; 64-wide heads up to 256)", n_tok, dim_head);
-  if (n_tok > 64)
-    return keep ? launch_bwd_long<true>(qkv, dout, dqkv, n_seq, n_tok, heads, keep, st)
-                : launch_bwd_long<false>(qkv, dout, dqkv, n_seq, n_tok, heads, nullptr, st);
+  if (n_tok > 64) {
+    if (gmap)
+      return keep ? launch_bwd_long<true, true>(qkv, dout, dqkv, n_seq, n_tok, heads, keep, gmap, st)
+                  : launch_bwd_long<false, true>(qkv, dout, dqkv, n_seq, n_tok, heads, nullptr, gmap, st);
+    return keep ? launch_bwd_long<true, false>(qkv, dout, dqkv, n_seq, n_tok, heads, keep, nullptr, st)
+                : launch_bwd_long<false, false>(qkv, dout, dqkv, n_seq, n_tok, heads, nullptr, nullptr, st);
+  }
   const int np = (n_tok + 15) / 16 * 16;
-#define AVF_ATT(D, P)                                                                                   \
-  if (dim_head == D && np == P)                                                                         \
-    return keep ? launch_bwd<D, P, true>(qkv, dout, dqkv, n_seq, n_tok, heads, keep, st)                \
-                : launch_bwd<D, P, false>(qkv, dout, dqkv, n_seq, n_tok, heads, nullptr, st);
+#define AVF_ATT(D, P)                                                                                      \
+  if (dim_head == D && np == P) {                                                                          \
+    if (gmap)                                                                                              \
+      return keep ? launch_bwd<D, P, true, true>(qkv, dout, dqkv, n_seq, n_tok, heads, keep, gmap, st)     \
+                  : launch_bwd<D, P, false, true>(qkv, dout, dqkv, n_seq, n_tok, heads, nullptr, gmap, st); \
+    return keep ? launch_bwd<D, P, true, false>(qkv, dout, dqkv, n_seq, n_tok, heads, keep, nullptr, st)   \
+                : launch_bwd<D, P, false, false>(qkv, dout, dqkv, n_seq, n_tok, heads, nullptr, nullptr, st); \
+  }
   AVF_ATT(32, 16) AVF_ATT(32, 32) AVF_ATT(32, 48) AVF_ATT(32, 64)
   AVF_ATT(64, 16) AVF_ATT(64, 32) AVF_ATT(64, 48) AVF_ATT(64, 64)
 #undef AVF_ATT

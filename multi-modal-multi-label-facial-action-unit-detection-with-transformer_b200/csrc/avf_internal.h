@@ -61,8 +61,11 @@ int layernorm_bwd(const float* x, int ld_x, const float* gamma, const float* dyn
 // y = x * mask(drop) as bf16 / fp32 (dense [rows, dim]); without dropout a plain cast / copy
 int masked_copy(const float* x, void* y, int y_mode, int rows, int dim, DropSpec drop, cudaStream_t st);
 int dropout_mask(float* out, int rows, int cols, DropSpec drop, cudaStream_t st);
+// gmap (optional): fp32 [n_seq, heads, n_tok, n_tok] receives G = P o dP from the same launch; dqkv is the same as without it.
 int attention_bwd(int io_mode, const void* qkv, const void* dout, void* dqkv, int n_seq, int n_tok, int heads, int dim_head, cudaStream_t st,
-                  const uint8_t* keep = nullptr);
+                  const uint8_t* keep = nullptr, float* gmap = nullptr);
+// R [n_seq, n_tok, n_tok] = the rollout of the gradient maps gmaps [depth, n_seq, heads, n_tok, n_tok] (avf_attention_rollout)
+int attention_rollout(const float* gmaps, int depth, int n_seq, int heads, int n_tok, float* R, cudaStream_t st);
 int au_logits_bwd(const float* dl, int ld_dl, const float* x, int ld_x, const float* w_last, float* dx, int ld_dx, float* dw, int n_clips,
                   int dim, cudaStream_t st);
 int bn_train_fwd(int out_mode, const float* x, int ld_x, const float* g, const float* b, float* run_mean, float* run_var, float momentum,
@@ -77,7 +80,7 @@ int adam_step(float* p, const float* g, float* m, float* v, void* shadow, size_t
 int attention_mma_bf16(const void* qkv, void* out, int n_seq, int n_tok, int heads, int dim_head, cudaStream_t st, int q_rows = 0,
                        const uint8_t* keep = nullptr, float* probs = nullptr);
 int attention_bwd_mma_bf16(const void* qkv, const void* dout, void* dqkv, int n_seq, int n_tok, int heads, int dim_head, cudaStream_t st,
-                           const uint8_t* keep = nullptr);
+                           const uint8_t* keep = nullptr, float* gmap = nullptr);
 
 // avf_layer_fused.cu: whole encoder stack in one persistent tcgen05 kernel (dim 256 or 128, 8 heads x 32)
 bool encoder_fused_supported(const avf_stack_shape* s);

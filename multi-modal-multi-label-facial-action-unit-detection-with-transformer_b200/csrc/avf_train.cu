@@ -269,10 +269,12 @@ __global__ void __launch_bounds__(256) dropout_mask_kernel(float* __restrict__ o
 // Sequences are 12 / 17 / 49 tokens: everything of one head lives in shared memory as fp32.
 // MASKED: keep [n_seq, n_tok] uint8 (1 = keep), turned into 64 keep bits by two ballots of every warp.  Scores of a kept query on
 // dropped keys are -INF (P = 0); a dropped query's scores are all equal (uniform P); dS = 0 on every filled score.
+// GMAP: the row pass, which holds P and dP of every (query, key), also writes G = P o dP in fp32 to gmap [n_seq, heads, n_tok, n_tok].
 // ---------------------------------------------------------------------------------------------
-template <typename T, int DH, bool MASKED>
+template <typename T, int DH, bool MASKED, bool GMAP>
 __global__ void __launch_bounds__(128) attention_bwd_kernel(const T* __restrict__ qkv, const T* __restrict__ dout, T* __restrict__ dqkv,
-                                                            int n_tok, int heads, float scale, const uint8_t* __restrict__ keep) {
+                                                            int n_tok, int heads, float scale, const uint8_t* __restrict__ keep,
+                                                            float* __restrict__ gmap) {
   pdl_wait();      // programmatic dependent launch: everything above is launch overhead hidden behind the previous kernel
   pdl_trigger();
   extern __shared__ float sm[];
@@ -335,6 +337,7 @@ __global__ void __launch_bounds__(128) attention_bwd_kernel(const T* __restrict_
       const float p = sp[a * NP + b] * inv;
       sp[a * NP + b] = p;
       delta += p * sds[a * NP + b];
+      if constexpr (GMAP) gmap[(size_t(blockIdx.x) * N + a) * N + b] = __fmul_rn(p, sds[a * NP + b]);     // sds holds dP here
     }
     delta = warp_sum(delta);
     const bool filled_row = MASKED && !((km >> a) & 1);
@@ -362,17 +365,17 @@ __global__ void __launch_bounds__(128) attention_bwd_kernel(const T* __restrict_
 //   pass 1, K | V staged, rows = queries: scores and dP, softmax statistics (max, 1/sum, delta) to shared memory, dQ = scale dS K;
 //   pass 2, Q | dO restaged, rows = keys: P and dS again from the statistics, dV = P^T dO, dK = scale dS^T Q.
 // The row's own operand pair sits in a per-warp slot (broadcast reads) and its scores in a per-warp line.  Masks as in
-// attention_bwd_kernel, with the keep bits in four 64-bit words.
+// attention_bwd_kernel, with the keep bits in four 64-bit words.  GMAP: pass 1 also writes G = P o dP (attention_bwd_kernel).
 // ---------------------------------------------------------------------------------------------
 constexpr int kLongF32Pitch = 64 + 1;
 __host__ __device__ constexpr size_t attention_bwd_long_smem(int n_tok) {
   return (size_t(2) * n_tok * kLongF32Pitch + 8 * (2 * 64 + 2 * 256) + 3 * 256) * sizeof(float) + 4 * sizeof(uint64_t);
 }
 
-template <bool MASKED>
+template <bool MASKED, bool GMAP>
 __global__ void __launch_bounds__(256) attention_bwd_long_f32_kernel(const float* __restrict__ qkv, const float* __restrict__ dout,
                                                                      float* __restrict__ dqkv, int n_tok, int heads, float scale,
-                                                                     const uint8_t* __restrict__ keep) {
+                                                                     const uint8_t* __restrict__ keep, float* __restrict__ gmap) {
   pdl_wait();      // programmatic dependent launch: everything above is launch overhead hidden behind the previous kernel
   pdl_trigger();
   constexpr int DH = 64, P = kLongF32Pitch;
@@ -441,6 +444,7 @@ __global__ void __launch_bounds__(256) attention_bwd_long_f32_kernel(const float
     for (int b = lane; b < N; b += 32) {
       const float p = exp2f(l0[b] - mx) * il;
       delta += p * l1[b];
+      if constexpr (GMAP) gmap[(size_t(blockIdx.x) * N + a) * N + b] = __fmul_rn(p, l1[b]);     // l1 holds dP here
       l0[b] = p;
     }
     delta = warp_sum(delta);
@@ -491,6 +495,64 @@ __global__ void __launch_bounds__(256) attention_bwd_long_f32_kernel(const float
       op[2 * inner] = dv;
     }
     __syncwarp();
+  }
+}
+
+// ---------------------------------------------------------------------------------------------
+// Rollout of gradient maps (Chefer, Gur, Wolf, ICCV 2021, self-attention rule), per sequence b, in fp32:
+//   A_l = mean_h max(G[l, b, h], 0);  R_0 = I;  R_l = R_{l-1} + A_l R_{l-1};  R[b] = R_depth      (gmaps [depth, n_seq, heads, N, N])
+// The columns of R evolve independently (R_l[:, J] = R_{l-1}[:, J] + A_l R_{l-1}[:, J]), so a CTA owns `cols` columns of one sequence
+// (all of them up to 64 tokens: the 12-token heads, the 17-token TFormer, the 49-token SFormer; 64-column blocks beyond) with the
+// current and the next column block in shared memory, and stages kRollRows rows of A_l at a time, the head mean and the clamp of each
+// element computed once per CTA.  Every sum runs in a fixed order (no atomics), so the result is deterministic.
+// ---------------------------------------------------------------------------------------------
+constexpr int kRollRows = 16;
+static int rollout_cols(int n_tok) { return n_tok <= 64 ? n_tok : 64; }
+static size_t rollout_smem(int n_tok) { return (size_t(2) * n_tok * rollout_cols(n_tok) + size_t(kRollRows) * n_tok) * sizeof(float); }
+
+__global__ void __launch_bounds__(256) attention_rollout_kernel(const float* __restrict__ gmaps, int depth, int n_seq, int heads, int n_tok,
+                                                                int cols, float* __restrict__ R) {
+  pdl_wait();      // programmatic dependent launch: everything above is launch overhead hidden behind the previous kernel
+  pdl_trigger();
+  extern __shared__ float sm_roll[];
+  const int N = n_tok, n_blk = (N + cols - 1) / cols;
+  const int b = blockIdx.x / n_blk, c0 = (blockIdx.x - b * n_blk) * cols, cb = min(cols, N - c0);
+  float* cur = sm_roll;                   // [N][cols]  R_{l-1}[:, c0 : c0 + cb]
+  float* nxt = cur + N * cols;            // [N][cols]  R_l
+  float* arow = nxt + N * cols;           // [kRollRows][N]  rows of A_l
+  for (int e = threadIdx.x; e < N * cols; e += blockDim.x) {
+    const int k = e / cols, j = e - k * cols;
+    cur[e] = k == c0 + j ? 1.f : 0.f;
+  }
+  const size_t nn = size_t(N) * N;
+  const float inv_h = 1.f / float(heads);
+  for (int l = 0; l < depth; ++l) {
+    const float* g = gmaps + (size_t(l) * n_seq + b) * heads * nn;
+    for (int i0 = 0; i0 < N; i0 += kRollRows) {
+      const int rows = min(kRollRows, N - i0);
+      __syncthreads();                    // cur written, arow free
+      for (int e = threadIdx.x; e < rows * N; e += blockDim.x) {
+        const size_t off = size_t(i0) * N + e;
+        float a = 0.f;
+        for (int h = 0; h < heads; ++h) a += fmaxf(g[h * nn + off], 0.f);
+        arow[e] = a * inv_h;
+      }
+      __syncthreads();
+      for (int e = threadIdx.x; e < rows * cb; e += blockDim.x) {
+        const int i = e / cb, j = e - i * cb;
+        float acc = 0.f;
+        for (int k = 0; k < N; ++k) acc = fmaf(arow[i * N + k], cur[k * cols + j], acc);
+        nxt[(i0 + i) * cols + j] = cur[(i0 + i) * cols + j] + acc;
+      }
+    }
+    float* t = cur;
+    cur = nxt;
+    nxt = t;
+  }
+  __syncthreads();
+  for (int e = threadIdx.x; e < N * cb; e += blockDim.x) {
+    const int i = e / cb, j = e - i * cb;
+    R[(size_t(b) * N + i) * N + c0 + j] = cur[i * cols + j];
   }
 }
 
@@ -745,44 +807,71 @@ int dropout_mask(float* out, int rows, int cols, DropSpec drop, cudaStream_t st)
   return 0;
 }
 
-template <typename T, int DH, bool MASKED>
-static int launch_attention_bwd(const void* qkv, const void* dout, void* dqkv, int n_seq, int n_tok, int heads, const uint8_t* keep, cudaStream_t st) {
+template <typename T, int DH, bool MASKED, bool GMAP>
+static int launch_attention_bwd(const void* qkv, const void* dout, void* dqkv, int n_seq, int n_tok, int heads, const uint8_t* keep, float* gmap,
+                                cudaStream_t st) {
   const size_t smem = (size_t(4) * n_tok * (DH + 1) + size_t(2) * n_tok * (n_tok + 1)) * sizeof(float);
   AVF_REQUIRE(smem <= 200 * 1024, AVF_EUNSUPPORTED, "attention_bwd: %d tokens x %d do not fit shared memory", n_tok, DH);
-  auto kern = attention_bwd_kernel<T, DH, MASKED>;
+  auto kern = attention_bwd_kernel<T, DH, MASKED, GMAP>;
   static PerDeviceOnce once;
   if (once.first()) {
     AVF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
   }
   launch_pdl(kern, n_seq * heads, 128, smem, st, static_cast<const T*>(qkv), static_cast<const T*>(dout), static_cast<T*>(dqkv), n_tok, heads,
-                                         rsqrtf(float(DH)), keep);
+                                         rsqrtf(float(DH)), keep, gmap);
   AVF_LAUNCH_CHECK("attention_bwd_kernel");
   return 0;
 }
 
+template <bool GMAP>
+static int launch_attention_bwd_long(const void* qkv, const void* dout, void* dqkv, int n_seq, int n_tok, int heads, const uint8_t* keep, float* gmap,
+                                     cudaStream_t st) {
+  auto kern = keep != nullptr ? attention_bwd_long_f32_kernel<true, GMAP> : attention_bwd_long_f32_kernel<false, GMAP>;
+  static PerDeviceOnce once[2];
+  if (once[keep != nullptr].first()) {
+    AVF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, int(attention_bwd_long_smem(256))));
+  }
+  launch_pdl(kern, n_seq * heads, 256, attention_bwd_long_smem(n_tok), st, static_cast<const float*>(qkv), static_cast<const float*>(dout),
+             static_cast<float*>(dqkv), n_tok, heads, rsqrtf(64.f), keep, gmap);
+  AVF_LAUNCH_CHECK("attention_bwd_long_f32_kernel");
+  return 0;
+}
+
+template <bool GMAP>
+static int attention_bwd_f32(const void* qkv, const void* dout, void* dqkv, int n_seq, int n_tok, int heads, int dim_head, const uint8_t* keep,
+                             float* gmap, cudaStream_t st) {
+  if (n_tok > 64) return launch_attention_bwd_long<GMAP>(qkv, dout, dqkv, n_seq, n_tok, heads, keep, gmap, st);
+  if (keep != nullptr)
+    return dim_head == 32 ? launch_attention_bwd<float, 32, true, GMAP>(qkv, dout, dqkv, n_seq, n_tok, heads, keep, gmap, st)
+                          : launch_attention_bwd<float, 64, true, GMAP>(qkv, dout, dqkv, n_seq, n_tok, heads, keep, gmap, st);
+  return dim_head == 32 ? launch_attention_bwd<float, 32, false, GMAP>(qkv, dout, dqkv, n_seq, n_tok, heads, nullptr, gmap, st)
+                        : launch_attention_bwd<float, 64, false, GMAP>(qkv, dout, dqkv, n_seq, n_tok, heads, nullptr, gmap, st);
+}
+
 int attention_bwd(int io_mode, const void* qkv, const void* dout, void* dqkv, int n_seq, int n_tok, int heads, int dim_head, cudaStream_t st,
-                  const uint8_t* keep) {
+                  const uint8_t* keep, float* gmap) {
   AVF_REQUIRE(n_seq > 0 && n_tok > 0 && heads > 0, AVF_EINVAL, "attention_bwd: n_seq=%d n_tok=%d heads=%d", n_seq, n_tok, heads);
   AVF_REQUIRE(dim_head == 32 || dim_head == 64, AVF_EUNSUPPORTED, "attention_bwd: dim_head=%d (supported: 32, 64)", dim_head);
   AVF_REQUIRE(n_tok <= 64 || (dim_head == 64 && n_tok <= 256), AVF_EUNSUPPORTED,
               "attention_bwd: n_tok=%d with dim_head=%d (up to 64 tokens; 64-wide heads up to 256)", n_tok, dim_head);
-  if (io_mode == AVF_BF16) return attention_bwd_mma_bf16(qkv, dout, dqkv, n_seq, n_tok, heads, dim_head, st, keep);      // tensor cores
-  if (n_tok > 64) {
-    auto kern = keep != nullptr ? attention_bwd_long_f32_kernel<true> : attention_bwd_long_f32_kernel<false>;
-    static PerDeviceOnce once[2];
-    if (once[keep != nullptr].first()) {
-      AVF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, int(attention_bwd_long_smem(256))));
-    }
-    launch_pdl(kern, n_seq * heads, 256, attention_bwd_long_smem(n_tok), st, static_cast<const float*>(qkv), static_cast<const float*>(dout),
-               static_cast<float*>(dqkv), n_tok, heads, rsqrtf(64.f), keep);
-    AVF_LAUNCH_CHECK("attention_bwd_long_f32_kernel");
-    return 0;
+  if (io_mode == AVF_BF16) return attention_bwd_mma_bf16(qkv, dout, dqkv, n_seq, n_tok, heads, dim_head, st, keep, gmap);      // tensor cores
+  return gmap ? attention_bwd_f32<true>(qkv, dout, dqkv, n_seq, n_tok, heads, dim_head, keep, gmap, st)
+              : attention_bwd_f32<false>(qkv, dout, dqkv, n_seq, n_tok, heads, dim_head, keep, nullptr, st);
+}
+
+int attention_rollout(const float* gmaps, int depth, int n_seq, int heads, int n_tok, float* R, cudaStream_t st) {
+  AVF_REQUIRE(gmaps && R, AVF_EINVAL, "attention_rollout: null pointer");
+  AVF_REQUIRE(depth > 0 && n_seq > 0 && heads > 0 && n_tok > 0, AVF_EINVAL, "attention_rollout: depth=%d n_seq=%d heads=%d n_tok=%d", depth, n_seq,
+              heads, n_tok);
+  AVF_REQUIRE(n_tok <= 256, AVF_EUNSUPPORTED, "attention_rollout: n_tok=%d (up to 256 tokens)", n_tok);
+  static PerDeviceOnce once;
+  if (once.first()) {
+    AVF_CUDA(cudaFuncSetAttribute(attention_rollout_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(rollout_smem(256))));
   }
-  if (keep != nullptr)
-    return dim_head == 32 ? launch_attention_bwd<float, 32, true>(qkv, dout, dqkv, n_seq, n_tok, heads, keep, st)
-                          : launch_attention_bwd<float, 64, true>(qkv, dout, dqkv, n_seq, n_tok, heads, keep, st);
-  return dim_head == 32 ? launch_attention_bwd<float, 32, false>(qkv, dout, dqkv, n_seq, n_tok, heads, nullptr, st)
-                        : launch_attention_bwd<float, 64, false>(qkv, dout, dqkv, n_seq, n_tok, heads, nullptr, st);
+  const int cols = rollout_cols(n_tok);
+  launch_pdl(attention_rollout_kernel, n_seq * ceil_div(n_tok, cols), 256, rollout_smem(n_tok), st, gmaps, depth, n_seq, heads, n_tok, cols, R);
+  AVF_LAUNCH_CHECK("attention_rollout_kernel");
+  return 0;
 }
 
 int au_logits_bwd(const float* dl, int ld_dl, const float* x, int ld_x, const float* w_last, float* dx, int ld_dx, float* dw, int n_clips,

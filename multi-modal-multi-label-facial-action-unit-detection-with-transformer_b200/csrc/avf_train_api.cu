@@ -161,9 +161,11 @@ static BwdWs carve_bwd_ws(const avf_stack_shape* s, int mode, void* base) {
   return w;
 }
 
+// gmaps (optional): layer l's gradient map G = P o dP goes to gmaps + l * n_seq*heads*n_tok*n_tok (fp32 [depth, n_seq, heads, n_tok, n_tok]),
+// written by that layer's attention backward launch.
 static int encoder_bwd(int mode, const avf_stack_shape* s, const avf_layer_weights* L, const void* tape, size_t tape_bytes, float* dx, int ld_dx,
                        const avf_layer_grads* G, int accumulate, void* ws, size_t ws_bytes, float p_drop, uint64_t seed, const uint32_t* salt,
-                       cudaStream_t st, const uint8_t* keep = nullptr) {
+                       cudaStream_t st, const uint8_t* keep = nullptr, float* gmaps = nullptr) {
   int e = check_train_shape(s);
   if (e) return e;
   AVF_REQUIRE(p_drop >= 0.f && p_drop < 1.f, AVF_EINVAL, "dropout p=%f", p_drop);
@@ -206,7 +208,8 @@ static int encoder_bwd(int mode, const avf_stack_shape* s, const avf_layer_weigh
     // ---- attention sub-layer:  x_mid = x_in + Wo attn(Wqkv LN1(x_in)) + bo -----------------------------------
     if (g.w_out && (e = gemm(mode, 1, 1, dyb, ld_dyb, t.o, I, nullptr, nullptr, 0, nullptr, 0, g.w_out, I, AVF_FP32, D, I, R, wg, w.red, w.red_bytes, st))) return e;
     if ((e = gemm(mode, 0, 1, dyb, ld_dyb, W.w_out, I, nullptr, nullptr, 0, nullptr, 0, w.dob, I, mode, R, I, D, 0, nullptr, 0, st))) return e;
-    if ((e = attention_bwd(mode, t.qkv, w.dob, w.big, s->n_seq, s->n_tok, s->heads, s->dim_head, st, keep))) return e;
+    float* gmap = gmaps ? gmaps + size_t(l) * s->n_seq * s->heads * s->n_tok * s->n_tok : nullptr;
+    if ((e = attention_bwd(mode, t.qkv, w.dob, w.big, s->n_seq, s->n_tok, s->heads, s->dim_head, st, keep, gmap))) return e;
     if (g.w_qkv && (e = gemm(mode, 1, 1, w.big, 3 * I, t.xn1, D, nullptr, nullptr, 0, nullptr, 0, g.w_qkv, D, AVF_FP32, 3 * I, D, R, wg, w.red, w.red_bytes, st))) return e;
     if ((e = gemm(mode, 0, 1, w.big, 3 * I, W.w_qkv, D, nullptr, nullptr, 0, nullptr, 0, w.dxn, D, AVF_FP32, R, D, 3 * I, 0, nullptr, 0, st))) return e;
     if ((e = layernorm_bwd(t.x_in, D, W.ln1_gamma, w.dxn, dx, ld_dx, dxb_out, mode, g.ln1_gamma, g.ln1_beta, g.b_out, beta, R, D, w.red, w.red_bytes, st,
@@ -346,6 +349,31 @@ int avf_attention_bwd_masked(int io_mode, const void* qkv, const void* dout, voi
   if (e) return e;
   AVF_REQUIRE(qkv && dout && dqkv, AVF_EINVAL, "attention_bwd: null pointer");
   return attention_bwd(io_mode, qkv, dout, dqkv, n_seq, n_tok, heads, dim_head, static_cast<cudaStream_t>(stream), keep);
+}
+
+int avf_attention_bwd_gradmaps(int io_mode, const void* qkv, const void* dout, void* dqkv, int32_t n_seq, int32_t n_tok, int32_t heads,
+                               int32_t dim_head, const uint8_t* keep, float* gmap, void* stream) {
+  int e = require_device_train();
+  if (e) return e;
+  AVF_REQUIRE(qkv && dout && dqkv && gmap, AVF_EINVAL, "attention_bwd_gradmaps: null pointer");
+  return attention_bwd(io_mode, qkv, dout, dqkv, n_seq, n_tok, heads, dim_head, static_cast<cudaStream_t>(stream), keep, gmap);
+}
+
+int avf_encoder_stack_bwd_gradmaps(int mode, const avf_stack_shape* s, const avf_layer_weights* layers, const uint8_t* keep, const void* tape,
+                                   size_t tape_bytes, float* dx, int32_t ld_dx, const avf_layer_grads* grads, int accumulate, void* workspace,
+                                   size_t workspace_bytes, float dropout_p, uint64_t dropout_seed, const uint32_t* dropout_salt, float* gmaps,
+                                   void* stream) {
+  int e = require_device_train();
+  if (e) return e;
+  AVF_REQUIRE(gmaps, AVF_EINVAL, "encoder_stack_bwd_gradmaps: null pointer");
+  return encoder_bwd(mode, s, layers, tape, tape_bytes, dx, ld_dx, grads, accumulate, workspace, workspace_bytes, dropout_p, dropout_seed, dropout_salt,
+                     static_cast<cudaStream_t>(stream), keep, gmaps);
+}
+
+int avf_attention_rollout(const float* gmaps, int32_t depth, int32_t n_seq, int32_t heads, int32_t n_tok, float* R, void* stream) {
+  int e = require_device_train();
+  if (e) return e;
+  return attention_rollout(gmaps, depth, n_seq, heads, n_tok, R, static_cast<cudaStream_t>(stream));
 }
 
 /* ---- AU_former front end with tape ------------------------------------------------------------------------- */

@@ -246,3 +246,43 @@ class Transformer(nn.Module):
         y = x.detach().float().reshape(b * n, d).clone()
         maps = self.maps_(y, b, n, keep=keep)
         return y.view(b, n, d), maps
+
+    # -- attention relevance -------------------------------------------------------------------
+    def check_relevance_allowed(self, who: str) -> None:
+        """Relevance differentiates the eval() computation: refuse a stack in train() (dropout, and batch statistics in the model)."""
+        if self.training:
+            raise RuntimeError(f"{who}: attention relevance needs eval(); in train() dropout and BatchNorm batch statistics would couple "
+                               f"the clips of a batch and BatchNorm would update its running statistics; call eval() first")
+
+    def relevance_fwd_(self, x2d: torch.Tensor, n_seq: int, n_tok: int, keep: Optional[torch.Tensor] = None):
+        """The tape-keeping forward without dropout of an fp32 token matrix [n_seq*n_tok, dim] (left untouched): (y, tape), y bit-equal
+        to forward_train's."""
+        return AF.encoder_stack_fwd_train(x2d, self.packed(), self.shape(n_seq, n_tok), keep=keep)
+
+    def relevance_bwd_(self, d2d: torch.Tensor, tape: torch.Tensor, n_seq: int, n_tok: int, keep: Optional[torch.Tensor] = None,
+                       maps: bool = True) -> Optional[torch.Tensor]:
+        """Backward of relevance_fwd_ for the activations only, in place on d2d (dL/dy in, dL/dx out; no parameter gradient).  Returns
+        the gradient maps fp32 [depth, n_seq, heads, n_tok, n_tok] (maps=True) or None."""
+        shape = self.shape(n_seq, n_tok)
+        if maps:
+            return AF.encoder_stack_bwd_gradmaps_(d2d, self.packed(), shape, tape, keep)
+        AF.encoder_stack_bwd_(d2d, self.packed(), shape, tape, [False] * (len(AF.LayerWeights._fields_) * self.depth), keep=keep)
+        return None
+
+    def attention_relevance(self, x: torch.Tensor, dy: torch.Tensor, mask=None):
+        """(y, gmaps, R) for the target whose gradient wrt the output is ``dy`` [b, n, dim]: y is the tape-keeping forward's output
+        (forward_train's, bit for bit), gmaps fp32 [depth, b, heads, n, n] the gradient maps G = P o dP of every layer from the
+        attention backward kernels, and R fp32 [b, n, n] their rollout R = prod_l (I + mean_h max(G_l, 0)) (INTEGRATION.md section 1).
+        No parameter gradient is computed or changed.  RuntimeError in train()."""
+        AF._cuda(x, "x")
+        AF._cuda(dy, "dy")
+        self.check_relevance_allowed("Transformer.attention_relevance")
+        b, n, d = x.shape
+        if tuple(dy.shape) != (b, n, d):
+            raise ValueError(f"Transformer.attention_relevance: dy must have the shape of x {(b, n, d)}, got {tuple(dy.shape)}")
+        keep = None if mask is None else AF.keep_from_mask(mask, b, n)
+        with torch.no_grad():
+            y, tape = self.relevance_fwd_(x.detach().float().reshape(b * n, d).contiguous(), b, n, keep)
+            dx = dy.detach().reshape(b * n, d).to(torch.float32, copy=True, memory_format=torch.contiguous_format)
+            gmaps = self.relevance_bwd_(dx, tape, b, n, keep)
+            return y.view(b, n, d), gmaps, AF.attention_rollout(gmaps)

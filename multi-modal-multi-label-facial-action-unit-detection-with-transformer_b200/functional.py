@@ -636,6 +636,52 @@ def encoder_stack_bwd_(dx: torch.Tensor, packed: PackedStack, shape: StackShape,
     return dx, grads
 
 
+# ------------------------------------------------------------------------------------------------
+# attention relevance: gradient maps G = P o dP written by the attention backward, and their rollout
+# (include/avformer_b200.h, "attention relevance")
+# ------------------------------------------------------------------------------------------------
+def attention_bwd_gradmaps(qkv: torch.Tensor, dout: torch.Tensor, n_seq: int, n_tok: int, heads: int, dim_head: int,
+                           keep: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """attention_bwd and the gradient map of the same launch: (dqkv, gmap fp32 [n_seq, heads, n_tok, n_tok]); dqkv equals
+    attention_bwd's bit for bit."""
+    qkv, dout = _cuda(qkv, "qkv").contiguous(), _cuda(dout, "dout").contiguous()
+    dqkv = torch.empty_like(qkv)
+    gmap = _probs(1, n_seq, heads, n_tok, qkv.device)[0]
+    check(_lib.lib().avf_attention_bwd_gradmaps(_io_mode(qkv), _ptr(qkv), _ptr(dout), _ptr(dqkv), n_seq, n_tok, heads, dim_head,
+                                                _keep_or_none(keep, n_seq, n_tok), _ptr(gmap), _stream()), "attention_bwd_gradmaps")
+    return dqkv, gmap
+
+
+def encoder_stack_bwd_gradmaps_(dx: torch.Tensor, packed: PackedStack, shape: StackShape, tape: torch.Tensor,
+                                keep: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """encoder_stack_bwd_ of activations only (no parameter gradient is computed, no wgrad kernel launched), in place on dx [rows,
+    dim] fp32 dense (dL/dy on entry, dL/dx on return, bit-equal to encoder_stack_bwd_), returning the gradient maps fp32 [depth,
+    n_seq, heads, n_tok, n_tok] of every layer.  No dropout: the tape must come from a forward without it."""
+    _cuda(dx, "dx")
+    if dx.dtype != torch.float32 or not dx.is_contiguous():
+        raise TypeError("encoder_stack_bwd_gradmaps_: dx must be a contiguous float32 gradient stream")
+    L = _lib.lib()
+    ws = workspace(L.avf_encoder_bwd_workspace_bytes(ctypes.byref(shape), packed.mode), dx.device)
+    gmaps = _probs(shape.depth, shape.n_seq, shape.heads, shape.n_tok, dx.device)
+    check(L.avf_encoder_stack_bwd_gradmaps(packed.mode, ctypes.byref(shape), packed.array, _keep_or_none(keep, shape.n_seq, shape.n_tok), _ptr(tape),
+                                           tape.numel(), _ptr(dx), dx.stride(0), None, 0, _ptr(ws), ws.numel(), 0.0, 0, None, _ptr(gmaps), _stream()),
+          "encoder_stack_bwd_gradmaps")
+    return gmaps
+
+
+def attention_rollout(gmaps: torch.Tensor) -> torch.Tensor:
+    """Rollout of gradient maps fp32 [depth, n_seq, heads, n_tok, n_tok] -> R fp32 [n_seq, n_tok, n_tok]: R = prod over layers of
+    (I + mean_h max(G_l, 0)), the last layer leftmost (avf_attention_rollout)."""
+    _cuda(gmaps, "gmaps")
+    if gmaps.dtype != torch.float32 or gmaps.dim() != 5 or gmaps.shape[-1] != gmaps.shape[-2] or not gmaps.is_contiguous():
+        raise ValueError(f"attention_rollout: gmaps must be a contiguous float32 tensor [depth, n_seq, heads, n_tok, n_tok], got {gmaps.dtype} "
+                         f"{tuple(gmaps.shape)}")
+    depth, n_seq, heads, n_tok, _ = gmaps.shape
+    R = torch.empty((n_seq, n_tok, n_tok), dtype=torch.float32, device=gmaps.device)
+    check(_lib.lib().avf_attention_rollout(_ptr(gmaps), depth, n_seq, heads, n_tok, _ptr(R), _stream()), "attention_rollout")
+    return R
+
+
 def sformer_tokens_pack(fmap: torch.Tensor, pos: Optional[torch.Tensor]) -> torch.Tensor:
     """[F,C,H,W] -> fp32 tokens [F*H*W, C] (+ pos [H*W, C]); pos=None is the plain transpose."""
     fmap = _cuda(fmap, "fmap").contiguous()

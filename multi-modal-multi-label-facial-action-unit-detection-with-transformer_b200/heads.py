@@ -98,6 +98,31 @@ class AU_former(nn.Module):
         x = AUFrontFn.apply(emb, self.AU_BN1.weight, self.AU_BN1.bias, self.pos_embedding, self, n_clips, *self.front_params())
         return self.corr_transformer.forward_train(x, n_clips, 12)
 
+    def relevance_fwd_(self, emb: torch.Tensor, n_clips: int):
+        """tokens_train's forward (running statistics: eval()) without recording: (tokens [n_clips*12, emb_dim], ctx for relevance_bwd_);
+        the tokens equal tokens_train's bit for bit."""
+        f = self._packed_front()
+        bn = self.AU_BN1
+        emb_d = emb.detach()
+        if emb_d.dtype != torch.float32 or emb_d.stride(-1) != 1:
+            emb_d = emb_d.float().contiguous()
+        x, ftape = AF.au_former_front_train(emb_d, n_clips, bn.weight.detach(), bn.bias.detach(), bn.running_mean, bn.running_var, False,
+                                            0.1 if bn.momentum is None else bn.momentum, f.w, f.b, self.pos_embedding.detach()[0], f.mode)
+        y, tape = self.corr_transformer.relevance_fwd_(x, n_clips, 12)
+        return y, (emb_d, f, ftape, tape, n_clips)
+
+    def relevance_bwd_(self, ctx, dy: torch.Tensor, maps: bool = True, want_emb: bool = False):
+        """Backward of relevance_fwd_ from dy [n_clips*12, emb_dim] fp32 dense (used as scratch), activations only: (gradient maps
+        [2, n_clips, 8, 12, 12] or None, dL/demb [n_clips, in_dim] or None)."""
+        emb_d, f, ftape, tape, n_clips = ctx
+        gmaps = self.corr_transformer.relevance_bwd_(dy, tape, n_clips, 12, maps=maps)
+        demb = None
+        if want_emb:
+            bn = self.AU_BN1
+            demb = AF.au_former_front_bwd(emb_d, n_clips, bn.weight.detach(), bn.running_mean, bn.running_var, False, f.w, ftape, dy, f.mode,
+                                          want_emb=True, want_bn=False, want_w=False)[0]
+        return gmaps, demb
+
     def forward(self, emb):
         AF._cuda(emb, "emb")
         bs = emb.shape[0]
@@ -152,6 +177,21 @@ class former_AU_head(nn.Module):
         x = AddPosFn.apply(tokens2d, self.pos_embedding, 12)
         x = self.corr_transformer.forward_train(x, n_clips, 12)
         return AULogitsFn.apply(x, self, n_clips, *self.last_params())
+
+    def relevance_fwd_(self, tokens2d: torch.Tensor, n_clips: int):
+        """logits21_train's forward without recording: ([B,21] equal to logits21_train's bit for bit, ctx for relevance_bwd_)."""
+        x = AF.add_row_periodic_(tokens2d.detach().float().contiguous().clone(), self.pos_embedding.detach().reshape(12, -1), 12)
+        y, tape = self.corr_transformer.relevance_fwd_(x, n_clips, 12)
+        last = self._packed_last()
+        return AF.au_logits(y, last.w, n_clips), (y, tape, last, n_clips)
+
+    def relevance_bwd_(self, ctx, weights: torch.Tensor, maps: bool = True):
+        """Backward of relevance_fwd_ seeded with d out21[:, :12] = weights [n_clips, 12] fp32 (d out21[:, 12:] = 0), activations only:
+        (gradient maps [3, n_clips, 8, 12, 12] or None, dL/dtokens [n_clips*12, emb_dim])."""
+        y, tape, last, n_clips = ctx
+        dx, _ = AF.au_logits_bwd(weights, y, last.w, n_clips, want_dx=True, want_dw=False)
+        gmaps = self.corr_transformer.relevance_bwd_(dx, tape, n_clips, 12, maps=maps)
+        return gmaps, dx
 
     def forward(self, input):
         AF._cuda(input, "input")

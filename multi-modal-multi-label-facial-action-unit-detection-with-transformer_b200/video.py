@@ -268,6 +268,41 @@ class TFormer(nn.Module):
         return AF.tformer_fwd_indexed_probs(bank.detach(), index, self.cls_token.view(-1), self.pos_embedding[0], st.packed(),
                                             st.shape(index.shape[0], self.num_patches + 1))
 
+    def relevance_fwd_(self, x, keep=None):
+        """The tape-keeping forward of forward() with autograd, without recording: (tokens [n_clips*(T+1), dim], tape, n_clips) for
+        relevance_bwd_; the cls rows c*(T+1) of the tokens are forward()'s output bit for bit."""
+        n_clips = self._n_clips(x)
+        tok = AF.tformer_embed(x.detach(), self.cls_token.detach().reshape(-1), self.pos_embedding.detach()[0], self.num_patches)
+        y, tape = self.spatial_transformer.relevance_fwd_(tok, n_clips, self.num_patches + 1, keep)
+        return y, tape, n_clips
+
+    def relevance_bwd_(self, tape, n_clips, d_cls, keep=None, maps=True):
+        """Backward of relevance_fwd_ seeded with d_cls [n_clips, dim] on the cls rows: (dtok [n_clips*(T+1), dim] = the gradient wrt
+        the embedded tokens, gradient maps [depth, n_clips, heads, T+1, T+1] or None)."""
+        T1 = self.num_patches + 1
+        dtok = torch.zeros((n_clips * T1, self.dim), dtype=torch.float32, device=d_cls.device)
+        dtok.view(n_clips, T1, self.dim)[:, 0] = d_cls
+        gmaps = self.spatial_transformer.relevance_bwd_(dtok, tape, n_clips, T1, keep, maps)
+        return dtok, gmaps
+
+    def attention_relevance(self, frame_feat, d_cls, mask=None):
+        """(cls, gmaps, R) for the target whose gradient wrt the cls features is ``d_cls`` [n_clips, dim]: cls equals forward()'s with
+        autograd bit for bit (the tape-keeping kernels), gmaps fp32 [depth, n_clips, heads, T+1, T+1] are the gradient maps
+        G = P o dP of every layer (the last one full: the tape path runs every row) and R fp32 [n_clips, T+1, T+1] their rollout;
+        R[:, 0, 1:] is the relevance of each frame for the cls token.  ``mask``: frames kept, as in forward().  No parameter gradient
+        is computed or changed.  RuntimeError in train()."""
+        n_clips = self._n_clips(frame_feat)
+        AF._cuda(d_cls, "d_cls")
+        self.spatial_transformer.check_relevance_allowed("TFormer.attention_relevance")
+        if tuple(d_cls.shape) != (n_clips, self.dim):
+            raise ValueError(f"TFormer.attention_relevance: d_cls must be [{n_clips}, {self.dim}], got {tuple(d_cls.shape)}")
+        keep = None if mask is None else AF.keep_from_mask(mask, n_clips, self.num_patches + 1)
+        with torch.no_grad():
+            y, tape, _ = self.relevance_fwd_(frame_feat, keep)
+            _, gmaps = self.relevance_bwd_(tape, n_clips, d_cls.detach().float(), keep)
+            cls = y.view(n_clips, self.num_patches + 1, self.dim)[:, 0].contiguous()
+            return cls, gmaps, AF.attention_rollout(gmaps)
+
     def forward(self, x, mask=None):
         """x [n_clips*T, dim] frame features -> cls features [n_clips, dim].  ``mask`` (optional): bool [n_clips, T], True = a real
         frame; clips with fewer real frames can share a batch with full ones (the padding frames' values do not matter)."""
